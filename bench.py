@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the pixel-reconstruction path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c2|c3_444|c3_gray|c4|c5]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (dequant + IDCT + upsample + YCbCr->RGB, reference src/worker.rs:32)
 over one batch of synthetic images.  Default workload = BASELINE.json configs[1]: a batch of 256 synthetic
@@ -97,6 +98,24 @@ def cpu_threads() -> int:
 IMAGENET_MEAN = (123.675, 116.28, 103.53, 0.0)
 IMAGENET_INV_STD = (1 / 58.395, 1 / 57.12, 1 / 57.375, 1.0)
 REF_FIXTURE = os.path.join(ROOT, "tests", "golden", "ref", "test-baseline.jpg")
+DUMP_BYTES = 64_000_000    # --dump-outputs writes at most this much
+DUMP_SEED = 2024
+
+
+def dump_outputs(out_dir: str, n_images: int, out_bytes: int, pixels) -> None:
+    """--dump-outputs: the pixel buffers the timed path wrote in its last step, as DIR/pixels.npy (float32, one row per
+    image of the batch).  When the whole batch does not fit in DUMP_BYTES, a row holds the bytes at k sorted positions
+    drawn from a generator seeded with (DUMP_SEED, image index): the same positions for the same arguments, so that the
+    files of two builds compare element for element.  pixels(b) returns image b's output bytes (uint8)."""
+    k = min(out_bytes, (DUMP_BYTES - 4096) // 4 // n_images)
+    rows = np.empty((n_images, k), np.float32)
+    for b in range(n_images):
+        px = pixels(b)
+        if k < out_bytes:
+            px = px[np.sort(np.random.default_rng([DUMP_SEED, b]).integers(0, out_bytes, k))]
+        rows[b] = px
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pixels.npy"), rows)
 
 
 def make_pool(cfg: str, n_distinct: int, rank: int):
@@ -277,9 +296,13 @@ def run_reference(args):
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
-    for _ in range(args.steps):
+    for _ in range(args.steps - bool(args.dump_outputs)):
         step()
+    if args.dump_outputs:     # the last timed step keeps its outputs (only here: holding them slows the host allocator)
+        last = [oracle.reconstruct(im, threads=threads) for im in imgs]
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, len(last), last[0].size, last.__getitem__)
     value = mp_step * args.steps / dt
     sample = f"{n_sample} of the workload's images per step ({n_sample}x {w}x{h}), coefficient planes in RAM -> pixels in RAM"
     line = {
@@ -388,6 +411,8 @@ def run_ours(args):
     ms_max = pl.max(ms)
     total_mp = pl.sum(mp_step * args.steps * reps)
     value = total_mp / (ms_max / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batch, out_bytes, lambda b: dev_out[b].download(stream=stream.ptr))
 
     # ---- sustained: the same launch back to back for >= args.sustain_seconds (the 20-step region above is a burst of ~70 ms;
     # this shows what the kernel holds once power / clocks have settled), clocks sampled during it
@@ -756,7 +781,12 @@ def main():
                     help="images of the whole-decode leg: one per host thread is in its (ragged) last round, so few images under-report")
     ap.add_argument("--no-consumer", action="store_true", help="skip the device-side consumer leg (planes -> normalised planar f16)")
     ap.add_argument("--no-check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the pixels of the last step to DIR/pixels.npy "
+                    "(float32, one row per image; a seeded sample of each image when the batch exceeds 64 MB; rank 0 only).  "
+                    "--impl reference times and dumps a smaller sample of images, so its file has another shape than the GPU path's")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     import __graft_entry__
     if not os.path.exists(__graft_entry__.LIB):

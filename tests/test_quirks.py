@@ -7,19 +7,18 @@ has one test-only switch per quirk (zj_host_set_quirks); its coefficient planes 
 
     quirks as written -> the deviation listed below;   the ONE named quirk off -> within +-5 of libjpeg everywhere.
 
-Files: tests/golden/ref/ = copies of /root/reference/{test-images,tests/inputs} (reference-held vectors)."""
+Files: tests/golden/ref/ = copies of the reference's {test-images,tests/inputs} (reference-held vectors, tests/ref_files.py)."""
 import io
-import os
 
 import numpy as np
 import pytest
 from PIL import Image
 
+import ref_files
 from sane_ref import sane_pixels
 from zune_jpeg_b200 import _ffi
 from zune_jpeg_b200.decoder import ColorSpace, DecodeErrors, Decoder, ZuneJpegOptions
 
-REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref")
 Q9, Q10, Q11, ALL = _ffi.QUIRK_Q9, _ffi.QUIRK_Q10, _ffi.QUIRK_Q11, _ffi.QUIRK_ALL
 
 
@@ -55,7 +54,7 @@ CASES = [
 
 @pytest.mark.parametrize("name,quirk,as_written", CASES)
 def test_fixture_deviation_is_the_cited_quirk(name, quirk, as_written):
-    data = open(os.path.join(REF, name), "rb").read()
+    data = ref_files.read(name)
     mx, share = _deviation(data, ALL)
     if quirk is None:
         assert mx <= 5, (name, mx)

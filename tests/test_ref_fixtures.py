@@ -1,23 +1,19 @@
 """The reference's own JPEG files through the PRODUCT path on the GPU (BASELINE configs[0] and the inputs of the
-reference's integration tests, /root/reference/tests/{large,medium,random}_images.rs, which only eyeball their outputs).
+reference's integration tests, tests/{large,medium,random}_images.rs, which only eyeball their outputs).
 
-Every file under tests/golden/ref/ (copies of reference fixtures) -- and, when /root/reference is mounted, every other file
-of its test-images/, tests/inputs/ and benches/images/ -- is decoded by Decoder.decode_buffer, decode_batch and
-decode_batch(gpu_entropy=True) and must equal, byte for byte, the oracle fed with the planes of the SEQUENTIAL host stage."""
+Every file under tests/golden/ref/ (verbatim copies of files of the reference's test-images/ and tests/inputs/, see
+tests/ref_files.py) is decoded by Decoder.decode_buffer, decode_batch and decode_batch(gpu_entropy=True) and must
+equal, byte for byte, the oracle fed with the planes of the SEQUENTIAL host stage."""
 import glob
+import hashlib
 import os
 
 import numpy as np
 import pytest
 
 import oracle
+import ref_files
 from zune_jpeg_b200.decoder import ColorSpace, DecodeErrors, Decoder, ZuneJpegOptions, decode_batch
-
-HERE = os.path.dirname(os.path.abspath(__file__))
-LOCAL = sorted(glob.glob(os.path.join(HERE, "golden", "ref", "*.jp*g")))
-MOUNTED = [p for d in ("test-images", "tests/inputs", "benches/images") for p in sorted(glob.glob(os.path.join("/root/reference", d, "*.jp*g")))
-           if os.path.basename(p) not in {os.path.basename(q) for q in LOCAL}]
-FILES = LOCAL + MOUNTED
 
 
 def _want(data: bytes, out_cs: ColorSpace):
@@ -33,19 +29,20 @@ def _want(data: bytes, out_cs: ColorSpace):
 
 
 def test_fixture_copies_are_the_reference_files():
-    """tests/golden/ref/ holds reference files verbatim (checked whenever the reference tree is mounted)."""
-    assert len(LOCAL) >= 7
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("reference tree not mounted")
-    for p in LOCAL:
-        hits = [q for d in ("test-images", "tests/inputs") for q in glob.glob(os.path.join("/root/reference", d, os.path.basename(p)))]
-        assert hits and open(hits[0], "rb").read() == open(p, "rb").read(), p
+    """tests/golden/ref/ holds the files of its manifest and nothing else, and each, as ref_files.read() returns it, has
+    the recorded length and SHA-256."""
+    stored = sorted(os.path.basename(p) for p in glob.glob(os.path.join(ref_files.DIR, "*.jp*g")))
+    assert len(stored) >= 7 and stored == ref_files.NAMES
+    for name in ref_files.NAMES:
+        data = ref_files.read(name)
+        assert len(data) == ref_files.MANIFEST[name]["bytes"], name
+        assert hashlib.sha256(data).hexdigest() == ref_files.MANIFEST[name]["sha256"], name
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("path", FILES, ids=[os.path.basename(p) for p in FILES])
-def test_reference_file_through_the_product(path):
-    data = open(path, "rb").read()
+@pytest.mark.parametrize("name", ref_files.NAMES)
+def test_reference_file_through_the_product(name):
+    data = ref_files.read(name)
     for out_cs in (ColorSpace.RGB, ColorSpace.RGBA, ColorSpace.GRAYSCALE, ColorSpace.YCbCr):
         want = _want(data, out_cs)
         opts = ZuneJpegOptions().set_out_colorspace(out_cs)
@@ -58,19 +55,19 @@ def test_reference_file_through_the_product(path):
         d = Decoder.new_with_options(opts)      # default 4 threads: restart-interval-parallel host stage when DRI is present
         got = np.frombuffer(d.decode_buffer(data), np.uint8)
         assert got.size == d.width() * d.height() * d.get_output_colorspace().num_components()
-        assert np.array_equal(got, want), (os.path.basename(path), out_cs, "decode_buffer")
+        assert np.array_equal(got, want), (name, out_cs, "decode_buffer")
         if out_cs in (ColorSpace.RGB, ColorSpace.GRAYSCALE):
             a, b = decode_batch([data, data], opts, threads=2)
-            assert a == want.tobytes() and b == a, (os.path.basename(path), out_cs, "decode_batch")
+            assert a == want.tobytes() and b == a, (name, out_cs, "decode_batch")
             stats = {}
             g = decode_batch([data], opts, threads=2, gpu_entropy=True, stats=stats)[0]
-            assert g == want.tobytes(), (os.path.basename(path), out_cs, "decode_batch gpu_entropy", stats)
+            assert g == want.tobytes(), (name, out_cs, "decode_batch gpu_entropy", stats)
 
 
 @pytest.mark.gpu
 def test_single_qt_restart_fixture_takes_the_gpu_entropy_route():
     """single_qt.jpeg (DRI = 1005 MCUs: not row-aligned, 4:2:2) is the reference's one real restart-marker file."""
-    data = open(os.path.join(HERE, "golden", "ref", "single_qt.jpeg"), "rb").read()
+    data = ref_files.read("single_qt.jpeg")
     stats = {}
     got = decode_batch([data], threads=2, gpu_entropy=True, stats=stats)[0]
     assert got == _want(data, ColorSpace.RGB).tobytes()
