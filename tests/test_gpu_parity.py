@@ -245,7 +245,7 @@ def test_sparse_and_dense_blocks_mix():
 def test_warp_uniform_sparsity_classes_at_the_limits(mode):
     """Every short form of the rolled IDCT taken by WHOLE warps (the class is the same in every block of a plane), with
     coefficients over the full i16 range and quantisers up to 255: the regrouped butterflies (idct8 / idct8_lo4 / idct8_lo6 --
-    multiply-adds re-associated in Z/2^32, `ZF_IDCT_MAD`) and the 4- / 6- / 8-input column passes must wrap exactly like the
+    multiply-adds re-associated in Z/2^32) and the 4- / 6- / 8-input column passes must wrap exactly like the
     oracle's literal form.  Classes = (rows kept, columns kept)."""
     from zune_jpeg_b200 import gpu
     rng = np.random.default_rng(4242)
@@ -479,18 +479,6 @@ def test_gpu_entropy_decode_device_outputs():
         assert b.download(len(w_)).tobytes() == w_
     res = decode_batch(ins, threads=4, device_out=[(b.ptr, 1000) for b in bufs])
     assert all(isinstance(r, DecodeErrors) for r in res)
-
-
-def test_gpu_entropy_decode_in_chunks():
-    """ZJ_GPU_ENTROPY_CHUNKS=4 (files, entropy kernels and reconstruction chunk by chunk on auxiliary streams; the setting is read
-    once per process, hence the child process): same pixels, same statuses."""
-    import os
-    import subprocess
-    import sys
-    if os.environ.get("ZJ_GPU_ENTROPY_CHUNKS") != "4":
-        env = dict(os.environ, ZJ_GPU_ENTROPY_CHUNKS="4")
-        r = subprocess.run([sys.executable, "-m", "pytest", "-x", "-q", "-m", "gpu", __file__, "-k", "test_gpu_entropy_decode"], env=env, capture_output=True, text=True)
-        assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
 
 
 def test_gpu_entropy_decode_fuzz():

@@ -1,4 +1,4 @@
-"""The regrouped 1-D butterflies of the CUDA kernels (zj_kernels.cu: idct8 / idct8_lo4 / idct8_lo6 with ZF_IDCT_MAD) restated in
+"""The regrouped 1-D butterflies of the CUDA kernels (zj_kernels.cu: idct8 / idct8_lo4 / idct8_lo6) restated in
 numpy and compared with the reference's literal operation order (src/idct/scalar.rs:79-166 == src/idct/avx2.rs:251-331) over
 Z/2^32: the regrouping (bias folded into one shift-add, odd outputs as chains of two multiply-adds, constants summed up front in
 the short forms) must be exact for EVERY 32-bit input, wrap-around included.  CPU only -- the GPU suite proves the same on the

@@ -1,7 +1,6 @@
 #!/usr/bin/env python
 """tools/gpu_entropy_devout_probe.py [n] -- zj_decode_batch_gpu_device on n 4K 4:2:0 JPEGs with one restart interval per MCU row:
-pinned JPEG bytes in, pixels left in device memory; ZJ_GPU_ENTROPY_CHUNKS=1..4 sets the number of upload/kernel chunks,
-ZJ_GPU_ENTROPY_TRACE=1 prints phase times (adds synchronisation)."""
+pinned JPEG bytes in, pixels left in device memory; ZJ_GPU_ENTROPY_TRACE=1 prints phase times (adds synchronisation)."""
 import os
 import sys
 import time
@@ -35,4 +34,4 @@ for rep in range(6):
     times.append(time.perf_counter() - t0)
 assert dev[0].download().tobytes() == ref
 best = min(times[1:])
-print(f"chunks={os.environ.get('ZJ_GPU_ENTROPY_CHUNKS', '4')}: {n} x {w}x{h}: best {1e3 * best:.1f} ms = {n * w * h / 1e6 / best:.0f} MP/s (all: {' '.join('%.1f' % (1e3 * t) for t in times)}), on GPU: {stats}")
+print(f"{n} x {w}x{h}: best {1e3 * best:.1f} ms = {n * w * h / 1e6 / best:.0f} MP/s (all: {' '.join('%.1f' % (1e3 * t) for t in times)}), on GPU: {stats}")

@@ -616,13 +616,11 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
 
 // Staging state of zj_gpu_reconstruct_submit, leased per host thread (see there); the idle ones are what
 // zj_release_device_caches frees.
-constexpr int ZJ_NS_MAX = 4;
+constexpr int ZJ_NS = 3;   // staging streams per device: the sub-batches of a call take turns on them
 struct StreamCache {
-    cudaStream_t s[64][ZJ_NS_MAX] = {};
-    uint8_t *buf[64][ZJ_NS_MAX] = {};
-    size_t cap[64][ZJ_NS_MAX] = {};
-    cudaEvent_t ev[64][ZJ_NS_MAX][3] = {};   // per staging buffer: planes uploaded / kernels done / pixels downloaded
-    bool ev_rec[64][ZJ_NS_MAX] = {};
+    cudaStream_t s[64][ZJ_NS] = {};
+    uint8_t *buf[64][ZJ_NS] = {};
+    size_t cap[64][ZJ_NS] = {};
 };
 struct CachePool {
     std::mutex mu;
@@ -630,7 +628,7 @@ struct CachePool {
 };
 static CachePool g_stream_pool;
 
-// frees the streams, events and device staging buffers of every cache no thread holds (hidden symbol; the exported entry
+// frees the streams and device staging buffers of every cache no thread holds (hidden symbol; the exported entry
 // point is zj_release_device_caches in zj_host_decoder.cpp)
 extern "C" void zj_capi_release_stream_caches(void)
 {
@@ -644,12 +642,11 @@ extern "C" void zj_capi_release_stream_caches(void)
     for (StreamCache *c : drop) {
         for (int dev = 0; dev < 64; dev++) {
             bool any = false;
-            for (int k = 0; k < ZJ_NS_MAX; k++) any = any || c->s[dev][k] || c->buf[dev][k];
+            for (int k = 0; k < ZJ_NS; k++) any = any || c->s[dev][k] || c->buf[dev][k];
             if (!any || cudaSetDevice(dev) != cudaSuccess) continue;
-            for (int k = 0; k < ZJ_NS_MAX; k++) {
+            for (int k = 0; k < ZJ_NS; k++) {
                 if (c->s[dev][k]) cudaStreamSynchronize(c->s[dev][k]);
                 if (c->buf[dev][k]) cudaFree(c->buf[dev][k]);
-                for (int e = 0; e < 3; e++) if (c->ev[dev][k][e]) cudaEventDestroy(c->ev[dev][k][e]);
                 if (c->s[dev][k]) cudaStreamDestroy(c->s[dev][k]);
             }
         }
@@ -666,9 +663,9 @@ extern "C" void zj_capi_release_stream_caches(void)
 struct zj_pending {
     int device = 0;
     int ns = 0;
-    cudaStream_t st[4] = {};
+    cudaStream_t st[ZJ_NS] = {};
     cudaStream_t user = nullptr;
-    cudaEvent_t done[4] = {};
+    cudaEvent_t done[ZJ_NS] = {};
     std::vector<zj_batch *> batches;
 };
 
@@ -709,13 +706,7 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
     const double t_in = trace ? now_ms() : 0;
     auto lap = [&](const char *what) { if (trace) fprintf(stderr, "[zj submit] %-22s +%.3f ms\n", what, now_ms() - t_in); };
     cudaStream_t user = (cudaStream_t)stream;
-    constexpr int NS_MAX = 4;
-    const char *env_ns = getenv("ZJ_E2E_STREAMS"), *env_mb = getenv("ZJ_E2E_BUDGET_MB");
-    // ZJ_E2E_PIPE=1: one stream per direction (uploads / kernels / downloads) over a ring of four staging buffers chained by
-    // events, instead of whole sub-batches alternating over the streams
-    const bool pipe = getenv("ZJ_E2E_PIPE") != nullptr && atoi(getenv("ZJ_E2E_PIPE")) != 0;
-    const int NS = pipe ? 3 : std::max(1, std::min(NS_MAX, env_ns ? atoi(env_ns) : 3));
-    cudaStream_t st[NS_MAX];
+    cudaStream_t st[ZJ_NS];
     // the staging streams are created once per host thread and device and reused: creating / destroying streams takes
     // driver-wide locks, which hurts when many threads call in (zj_decode_batch)
     // ... and so is the device staging buffer of every stream (grown on demand, reused in stream order): memory that the
@@ -739,7 +730,7 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
     if (!lease.c) return ZJ_ERR_OOM;
     StreamCache &cache = *lease.c;
     if (device >= 64) return ZJ_ERR_NO_DEVICE;
-    for (int k = 0; k < NS; k++) {
+    for (int k = 0; k < ZJ_NS; k++) {
         if (!cache.s[device][k]) CU(cudaStreamCreateWithFlags(&cache.s[device][k], cudaStreamNonBlocking));
         st[k] = cache.s[device][k];
     }
@@ -747,21 +738,18 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
     cudaEvent_t ev_in;
     CU(cudaEventCreateWithFlags(&ev_in, cudaEventDisableTiming));
     CU(cudaEventRecord(ev_in, user));
-    for (int k = 0; k < NS; k++) CU(cudaStreamWaitEvent(st[k], ev_in, 0));
+    for (int k = 0; k < ZJ_NS; k++) CU(cudaStreamWaitEvent(st[k], ev_in, 0));
     cudaEventDestroy(ev_in);   // (released once the recorded work has completed)
     lap("streams + entry event");
 
     zj_pending *pd = new (std::nothrow) zj_pending;
     if (!pd) return ZJ_ERR_OOM;
     pd->device = device;
-    pd->ns = NS;
+    pd->ns = ZJ_NS;
     pd->user = user;
-    for (int k = 0; k < NS; k++) pd->st[k] = st[k];
+    for (int k = 0; k < ZJ_NS; k++) pd->st[k] = st[k];
 
-#define CUB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = cuda_fail(e_, #call); break; } }   // (inside the loop: fall through to the common clean-up)
-    const size_t budget = (size_t)(env_mb ? std::max(16, atoi(env_mb)) : 256) << 20;  // device staging per sub-batch
-    static const bool prime = getenv("ZJ_E2E_NO_PRIME") == nullptr;
-    const size_t first_budget = prime ? budget / 8 : budget;
+    const size_t budget = (size_t)256 << 20;  // device staging per sub-batch
     size_t i = 0;
     int which = 0;
     rc = ZJ_OK;
@@ -772,25 +760,17 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
             for (uint32_t z = 0; z < plans[j].ncomp_used; z++) coef += (size_t)plans[j].n_strips * plans[j].chunk[z] * 2;
             need += coef + coef / 8 + 4096;      // (planes uploaded as one span may carry the gaps between them)
             // (the first sub-batch is a small one: kernels and downloads start after 1/8 of the usual upload)
-            if (j > i && bytes + need > (i == 0 ? first_budget : budget)) break;
+            if (j > i && bytes + need > (i == 0 ? budget / 8 : budget)) break;
             bytes += need + 4 * 256;
             j++;
         }
-        cudaStream_t s = st[pipe ? 0 : which];
-        which = (which + 1) % (pipe ? NS_MAX : NS);
-        const int slot = (which + (pipe ? NS_MAX : NS) - 1) % (pipe ? NS_MAX : NS);          // index of stream s / of the staging buffer
-        cudaStream_t s_up = pipe ? st[0] : s, s_k = pipe ? st[1] : s, s_dn = pipe ? st[2] : s;
+        const int slot = which;                   // stream s and its staging buffer
+        cudaStream_t s = st[slot];
+        which = (which + 1) % ZJ_NS;
         cudaError_t e = cudaSuccess;
-        if (pipe) {
-            for (int q = 0; q < 3; q++)
-                if (!cache.ev[device][slot][q]) CUB(cudaEventCreateWithFlags(&cache.ev[device][slot][q], cudaEventDisableTiming));
-            if (rc != ZJ_OK) break;
-            // the buffer is free once the pixels of its last sub-batch have been downloaded
-            if (cache.ev_rec[device][slot]) CUB(cudaStreamWaitEvent(s_up, cache.ev[device][slot][2], 0));
-        }
         if (cache.cap[device][slot] < bytes) {
             if (cache.buf[device][slot]) {
-                if (pipe) { for (int q = 0; q < 3; q++) cudaStreamSynchronize(st[q]); } else cudaStreamSynchronize(s);
+                cudaStreamSynchronize(s);
                 cudaFree(cache.buf[device][slot]); cache.buf[device][slot] = nullptr; cache.cap[device][slot] = 0;
             }
             e = cudaMalloc((void **)&cache.buf[device][slot], bytes + bytes / 8);
@@ -834,44 +814,40 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
             dlens[k - i] = plans[k].out_size;
         }
         zj_batch *b = nullptr;
-        rc = batch_create_impl(device, dimgs.data(), dimgs.size(), douts.data(), dlens.data(), &b, true, s_k);
+        rc = batch_create_impl(device, dimgs.data(), dimgs.size(), douts.data(), dlens.data(), &b, true, s);
         if (rc != ZJ_OK) break;
         for (size_t k = i; k < j && rc == ZJ_OK; k++) {
             if (span[k - i]) {
-                e = cudaMemcpyAsync((void *)dimgs[k - i].comp[0].coeff, imgs[k].comp[0].coeff, span[k - i], cudaMemcpyHostToDevice, s_up);
+                e = cudaMemcpyAsync((void *)dimgs[k - i].comp[0].coeff, imgs[k].comp[0].coeff, span[k - i], cudaMemcpyHostToDevice, s);
                 if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(H2D)");
                 continue;
             }
             for (uint32_t z = 0; z < plans[k].ncomp_used; z++) {
                 const size_t nb = (size_t)plans[k].n_strips * plans[k].chunk[z] * 2;
-                e = cudaMemcpyAsync((void *)dimgs[k - i].comp[z].coeff, imgs[k].comp[z].coeff, nb, cudaMemcpyHostToDevice, s_up);
+                e = cudaMemcpyAsync((void *)dimgs[k - i].comp[z].coeff, imgs[k].comp[z].coeff, nb, cudaMemcpyHostToDevice, s);
                 if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemcpyAsync(H2D)"); break; }
             }
         }
         if (rc != ZJ_OK) { zj_batch_destroy(b); break; }
         lap("descriptors + uploads");
         pd->batches.push_back(b);
-        if (pipe) { CUB(cudaEventRecord(cache.ev[device][slot][0], s_up)); CUB(cudaStreamWaitEvent(s_k, cache.ev[device][slot][0], 0)); }
-        rc = zj_batch_run(b, s_k);
+        rc = zj_batch_run(b, s);
         if (rc != ZJ_OK) break;
-        if (pipe) { CUB(cudaEventRecord(cache.ev[device][slot][1], s_k)); CUB(cudaStreamWaitEvent(s_dn, cache.ev[device][slot][1], 0)); }
         for (size_t k = i; k < j; k++) {
-            e = cudaMemcpyAsync(out[k], douts[k - i], plans[k].out_size, cudaMemcpyDeviceToHost, s_dn);
+            e = cudaMemcpyAsync(out[k], douts[k - i], plans[k].out_size, cudaMemcpyDeviceToHost, s);
             if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemcpyAsync(D2H)"); break; }
         }
-        if (pipe && rc == ZJ_OK) { CUB(cudaEventRecord(cache.ev[device][slot][2], s_dn)); cache.ev_rec[device][slot] = true; }
         lap("kernels + downloads");
         i = j;
     }
     if (rc == ZJ_OK) {
-        for (int k = 0; k < NS; k++) {
+        for (int k = 0; k < ZJ_NS; k++) {
             if (cudaEventCreateWithFlags(&pd->done[k], cudaEventDisableTiming | cudaEventBlockingSync) != cudaSuccess) { pd->done[k] = nullptr; cudaGetLastError(); continue; }
             if (cudaEventRecord(pd->done[k], st[k]) != cudaSuccess) { cudaEventDestroy(pd->done[k]); pd->done[k] = nullptr; cudaGetLastError(); }
         }
         *pending = pd;
         return ZJ_OK;
     }
-#undef CUB
     const int rc_submit = rc;
     zj_gpu_reconstruct_finish(pd);   // waits for what was queued, releases the descriptors
     return rc_submit;

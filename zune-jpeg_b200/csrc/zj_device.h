@@ -20,37 +20,22 @@ enum OutKind : int {
 // (including the chroma halo blocks):                 blocks / MCU column        + halo
 //   (per 128 threads) NONE: 3 blocks -> TM 40 -> 120  H: 8 -> TM 15 -> 120 + 8
 //   V:    4 blocks  -> TM 32 -> 128                   HV: 12 -> TM 10 -> 120 + 8 (+4 in tile 0)
-#ifndef ZJ_CFG_THREADS
-#define ZJ_CFG_THREADS 256
-#endif
-#ifndef ZJ_CFG_MINBLOCKS
-#define ZJ_CFG_MINBLOCKS 3
-#endif
-constexpr int ZJ_THREADS = ZJ_CFG_THREADS;
-constexpr int ZJ_MINBLOCKS = ZJ_CFG_MINBLOCKS;  // CTAs per SM the register allocation is capped for
+constexpr int ZJ_THREADS = 256;
+constexpr int ZJ_MINBLOCKS = 3;  // CTAs per SM the register allocation is capped for
 constexpr int ZJ_SLOW_CAP = 192;  // edge units per tile queued for the generic path
 // tile widths scale with the CTA size (128 threads: 40 / 15 / 32 / 10)
 constexpr int TM_NONE = 40 * ZJ_THREADS / 128, TM_H = 15 * ZJ_THREADS / 128, TM_V = 32 * ZJ_THREADS / 128, TM_HV = 10 * ZJ_THREADS / 128, TM_GRAY = 128;
 
 // The fast kernel (X86 variant): 256 threads = 128 producers (IDCT, two 8x8 blocks per thread and strip) + 128
 // consumers (up-sampling / colour / stores, two 16-sample units per thread and strip).
-#ifndef ZF_CFG_MINBLOCKS
-#define ZF_CFG_MINBLOCKS 3
-#endif
-#ifndef ZF_CFG_SPC
-#define ZF_CFG_SPC 40
-#endif
 constexpr int ZF_THREADS = 256, ZF_PRODUCERS = 128, ZF_CONSUMERS = 128;
-constexpr int ZF_MINBLOCKS = ZF_CFG_MINBLOCKS;
-constexpr int ZF_DEFAULT_SPC = ZF_CFG_SPC;      // target strips per CTA (see strips_per_cta)
+constexpr int ZF_MINBLOCKS = 3;
+constexpr int ZF_DEFAULT_SPC = 40;      // target strips per CTA (see strips_per_cta)
 // unit columns (16 luma samples) per tile: 2 * ZF_CONSUMERS / row groups per strip
 constexpr int ZF_XU_GRAY = 32;                  // luma-only fast kernel: 512-sample tiles
 // (4:2:2: 15 instead of 16 -- the strip-tile's block list, 2 x 30 luma + 2 x 2 x 15 chroma + 8 halo blocks, is then exactly
 // 128 = one IDCT pass of the four producer warps; with 16 it is 136 and the producers' critical path a second pass)
-#ifndef ZF_CFG_XU_H
-#define ZF_CFG_XU_H 15
-#endif
-constexpr int ZF_XU_NONE = 2 * ZF_CONSUMERS / 8, ZF_XU_H = ZF_CFG_XU_H, ZF_XU_V = 2 * ZF_CONSUMERS / 8, ZF_XU_HV = 2 * ZF_CONSUMERS / 16;
+constexpr int ZF_XU_NONE = 2 * ZF_CONSUMERS / 8, ZF_XU_H = 15, ZF_XU_V = 2 * ZF_CONSUMERS / 8, ZF_XU_HV = 2 * ZF_CONSUMERS / 16;
 
 struct DevImage {
     const int16_t *coeff[3];  // device pointers, whole-image planes

@@ -264,12 +264,10 @@ static int launch_lanes(const EntImage *d_images, uint32_t n_images, uint32_t ma
 int launch_entropy(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, void *stream)
 {
     if (n_images == 0 || max_seg == 0) return 0;
-    static const int forced = [] { const char *e = getenv("ZJ_ENTROPY_LANES"); return e ? atoi(e) : 0; }();
     const uint64_t intervals = (uint64_t)n_images * max_seg;          // (an upper bound: images of one launch may differ)
-    const int lanes = forced ? forced : (intervals < 12000 ? 8 : (intervals < 24000 ? 16 : 32));
     cudaStream_t s = (cudaStream_t)stream;
-    if (lanes <= 8) return launch_lanes<8>(d_images, n_images, max_seg, s);
-    if (lanes <= 16) return launch_lanes<16>(d_images, n_images, max_seg, s);
+    if (intervals < 12000) return launch_lanes<8>(d_images, n_images, max_seg, s);
+    if (intervals < 24000) return launch_lanes<16>(d_images, n_images, max_seg, s);
     return launch_lanes<32>(d_images, n_images, max_seg, s);
 }
 

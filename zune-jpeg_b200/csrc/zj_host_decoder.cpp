@@ -1797,8 +1797,7 @@ ZJ_API int zj_decode_batch_multi(const zj_options *o, const int *devices, size_t
 // them; a buffer larger than ZJ_RETAIN_MB (default 16384: never, in practice) is freed when the call that grew it ends.
 struct GpuSlot {
     cudaStream_t s = nullptr; uint8_t *mem = nullptr; size_t cap = 0;
-    std::vector<zj_batch *> batches;          // one reconstruction launch plan per chunk (below)
-    std::vector<size_t> chunk_t;              // chunk c = images [chunk_t[c], chunk_t[c + 1]) of `take`
+    std::vector<zj_batch *> batches;          // reconstruction launch plans whose kernels may still be running
     std::vector<size_t> take, idx;            // images of the sub-batch in stage 1 / images whose pixels are on their way
     std::vector<zj::EntImage> eimg;
     std::vector<uint8_t *> pix;
@@ -1806,24 +1805,8 @@ struct GpuSlot {
     uint8_t *meta_host = nullptr, *st_host = nullptr;   // pinned: descriptors + tables + interval starts up, statuses down
     size_t meta_cap = 0, st_cap = 0;
     bool staged = false;
-    // ZJ_GPU_ENTROPY_CHUNKS > 1: the files of a sub-batch go up in chunks on auxiliary streams, each followed by the entropy
-    // kernel of its images and the download of their statuses, and stage 2 reconstructs a chunk as soon as its statuses are in
-    static constexpr int NAUX = 4;
-    cudaStream_t aux[NAUX] = {};
-    cudaEvent_t ev_meta = nullptr, ev_chunk[NAUX] = {};
-    bool aux_ready()
+    void release()      // stream, device staging memory and the pinned descriptor / status blocks
     {
-        for (int k = 0; k < NAUX; k++) {
-            if (!aux[k] && cudaStreamCreateWithFlags(&aux[k], cudaStreamNonBlocking) != cudaSuccess) { cudaGetLastError(); return false; }
-            if (!ev_chunk[k] && cudaEventCreateWithFlags(&ev_chunk[k], cudaEventDisableTiming | cudaEventBlockingSync) != cudaSuccess) { cudaGetLastError(); return false; }
-        }
-        if (!ev_meta && cudaEventCreateWithFlags(&ev_meta, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); return false; }
-        return true;
-    }
-    void release()      // streams, device staging memory and the pinned descriptor / status blocks
-    {
-        for (int k = 0; k < NAUX; k++) { if (aux[k]) cudaStreamDestroy(aux[k]); if (ev_chunk[k]) cudaEventDestroy(ev_chunk[k]); }
-        if (ev_meta) cudaEventDestroy(ev_meta);
         if (mem) cudaFree(mem);
         if (s) cudaStreamDestroy(s);
         if (meta_host) cudaFreeHost(meta_host);
@@ -2005,8 +1988,7 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
     std::vector<uint8_t *> malloced(n, nullptr);
     auto drain = [&](GpuSlot &sl) {   // wait for the slot's downloads, publish its images
         if (sl.idx.empty() && sl.batches.empty()) return;
-        bool ok = cudaStreamSynchronize(sl.s) == cudaSuccess;
-        for (int k = 0; k < GpuSlot::NAUX; k++) if (sl.aux[k]) ok = (cudaStreamSynchronize(sl.aux[k]) == cudaSuccess) && ok;
+        const bool ok = cudaStreamSynchronize(sl.s) == cudaSuccess;
         if (!ok) cudaGetLastError();
         for (zj_batch *b : sl.batches) zj_batch_destroy(b);
         sl.batches.clear();
@@ -2095,28 +2077,11 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
         }
         if (ok) memcpy(sl.meta_host, sl.eimg.data(), take.size() * sizeof(zj::EntImage));
         ok = ok && off <= sl.cap && cudaMemcpyAsync(d_meta, sl.meta_host, meta_bytes, cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
-        // files + entropy kernels, chunk by chunk on the auxiliary streams (behind the cleared planes and the descriptors)
-        static const size_t n_chunks_env = [] { const char *e = getenv("ZJ_GPU_ENTROPY_CHUNKS"); long v = e ? atol(e) : 1; return (size_t)std::max(1L, std::min(v, (long)GpuSlot::NAUX)); }();   // (measured on 256 4K images: 1 chunk 27.6 ms every time, 4 chunks 26.5 ms at best with outliers of 50-230 ms)
-        const size_t n_chunks = (take.size() >= 2 * n_chunks_env && sl.aux_ready()) ? n_chunks_env : 1;
-        ok = ok && (n_chunks == 1 || cudaEventRecord(sl.ev_meta, sl.s) == cudaSuccess);
-        sl.chunk_t.assign(n_chunks + 1, 0);
-        for (size_t c = 0; c <= n_chunks; c++) sl.chunk_t[c] = take.size() * c / n_chunks;
-        for (size_t c = 0; c < n_chunks && ok; c++) {
-            const size_t t0 = sl.chunk_t[c], t1 = sl.chunk_t[c + 1];
-            cudaStream_t cs = n_chunks == 1 ? sl.s : sl.aux[c];
-            if (n_chunks > 1) ok = ok && cudaStreamWaitEvent(cs, sl.ev_meta, 0) == cudaSuccess;
-            uint32_t chunk_seg = 0;
-            for (size_t t = t0; t < t1 && ok; t++) {
-                ok = cudaMemcpyAsync(const_cast<uint8_t *>(sl.eimg[t].data), bufs[take[t]], lens[take[t]], cudaMemcpyHostToDevice, cs) == cudaSuccess;
-                chunk_seg = std::max(chunk_seg, sl.eimg[t].n_seg);
-            }
-            ok = ok && zj::launch_entropy(reinterpret_cast<const zj::EntImage *>(d_meta) + t0, (uint32_t)(t1 - t0), chunk_seg, cs) == 0;
-            // the chunk's statuses come back behind its kernel: stage 2 reconstructs a chunk as soon as they are in, while the
-            // other chunks are still being entropy-decoded
-            const size_t s0 = sl.st_off[t0], s1 = t1 < take.size() ? sl.st_off[t1] : st_total;
-            ok = ok && (s1 == s0 || cudaMemcpyAsync(sl.st_host + s0, d_status + s0, s1 - s0, cudaMemcpyDeviceToHost, cs) == cudaSuccess);
-            if (n_chunks > 1) ok = ok && cudaEventRecord(sl.ev_chunk[c], cs) == cudaSuccess;
-        }
+        // files + entropy kernel (behind the cleared planes and the descriptors), then the statuses come back
+        for (size_t t = 0; t < take.size() && ok; t++)
+            ok = cudaMemcpyAsync(const_cast<uint8_t *>(sl.eimg[t].data), bufs[take[t]], lens[take[t]], cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
+        ok = ok && zj::launch_entropy(reinterpret_cast<const zj::EntImage *>(d_meta), (uint32_t)take.size(), max_seg, sl.s) == 0;
+        ok = ok && (st_total == 0 || cudaMemcpyAsync(sl.st_host, d_status, st_total, cudaMemcpyDeviceToHost, sl.s) == cudaSuccess);
         lap("files + entropy kernels", sl.s);
         if (!ok) cudaGetLastError();
         sl.staged = ok;   // (not staged: nothing is published, these images go through the host path)
@@ -2126,40 +2091,34 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
     auto stage2 = [&](GpuSlot &sl) {
         if (!sl.staged) return;
         sl.staged = false;
-        const size_t n_chunks = sl.chunk_t.size() - 1;
-        for (size_t c = 0; c < n_chunks; c++) {
-            cudaStream_t cs = n_chunks == 1 ? sl.s : sl.aux[c];
-            // (a blocking-sync event: the thread sleeps until this chunk's statuses are on the host)
-            const cudaError_t e = n_chunks == 1 ? cudaStreamSynchronize(cs) : cudaEventSynchronize(sl.ev_chunk[c]);
-            if (e != cudaSuccess) { cudaGetLastError(); continue; }
-            std::vector<zj_image> dimgs;
-            std::vector<uint8_t *> douts;
-            std::vector<size_t> dlens, who;
-            for (size_t t = sl.chunk_t[c]; t < sl.chunk_t[c + 1]; t++) {
-                const size_t i = sl.take[t];
-                Item &it = items[i];
-                bool all = true;
-                for (size_t k = 0; k < it.pp.n_seg; k++) all = all && sl.st_host[sl.st_off[t] + k] == 0;
-                if (!all) continue;
-                zj_image di = it.img;
-                for (uint32_t z = 0; z < di.n_comp; z++) di.comp[z].coeff = sl.eimg[t].plane[z];
-                dimgs.push_back(di); douts.push_back(sl.pix[t]); dlens.push_back(it.need); who.push_back(i);
+        if (cudaStreamSynchronize(sl.s) != cudaSuccess) { cudaGetLastError(); return; }
+        std::vector<zj_image> dimgs;
+        std::vector<uint8_t *> douts;
+        std::vector<size_t> dlens, who;
+        for (size_t t = 0; t < sl.take.size(); t++) {
+            const size_t i = sl.take[t];
+            Item &it = items[i];
+            bool all = true;
+            for (size_t k = 0; k < it.pp.n_seg; k++) all = all && sl.st_host[sl.st_off[t] + k] == 0;
+            if (!all) continue;
+            zj_image di = it.img;
+            for (uint32_t z = 0; z < di.n_comp; z++) di.comp[z].coeff = sl.eimg[t].plane[z];
+            dimgs.push_back(di); douts.push_back(sl.pix[t]); dlens.push_back(it.need); who.push_back(i);
+        }
+        if (dimgs.empty()) return;
+        zj_batch *b = nullptr;
+        int rc = zj_batch_create(opt.device, dimgs.data(), dimgs.size(), douts.data(), dlens.data(), &b);
+        if (rc == ZJ_OK) { sl.batches.push_back(b); rc = zj_batch_run(b, sl.s); }
+        for (size_t t = 0; t < who.size() && rc == ZJ_OK; t++) {
+            const size_t i = who[t];
+            if (!dev_out) {
+                uint8_t *dst = out[i];
+                if (!dst) { dst = (uint8_t *)malloc(items[i].need); malloced[i] = dst; }
+                if (!dst) continue;
+                if (cudaMemcpyAsync(dst, douts[t], dlens[t], cudaMemcpyDeviceToHost, sl.s) != cudaSuccess) { cudaGetLastError(); continue; }
             }
-            if (dimgs.empty()) continue;
-            zj_batch *b = nullptr;
-            int rc = zj_batch_create(opt.device, dimgs.data(), dimgs.size(), douts.data(), dlens.data(), &b);
-            if (rc == ZJ_OK) { sl.batches.push_back(b); rc = zj_batch_run(b, cs); }
-            for (size_t t = 0; t < who.size() && rc == ZJ_OK; t++) {
-                const size_t i = who[t];
-                if (!dev_out) {
-                    uint8_t *dst = out[i];
-                    if (!dst) { dst = (uint8_t *)malloc(items[i].need); malloced[i] = dst; }
-                    if (!dst) continue;
-                    if (cudaMemcpyAsync(dst, douts[t], dlens[t], cudaMemcpyDeviceToHost, cs) != cudaSuccess) { cudaGetLastError(); continue; }
-                }
-                on_gpu[i] = 1;
-                sl.idx.push_back(i);
-            }
+            on_gpu[i] = 1;
+            sl.idx.push_back(i);
         }
         lap("status + reconstruct (+ d2h)", trace ? sl.s : nullptr);
     };

@@ -18,55 +18,8 @@
 
 #include "zj_device.h"
 
-// tuning switches of the fast kernel (tools/build_variant.sh)
-#ifndef ZF_HINTS
-#define ZF_HINTS 1
-#endif
-#ifndef ZF_T2PAIR
-#define ZF_T2PAIR 1
-#endif
-#ifndef ZF_LO6
-#define ZF_LO6 1        // 1: a 6-input column pass for jobs whose rows 6-7 are zero in every block of the warp
-#endif
-#if ZF_HINTS
 #define ZF_LIKELY(x) __builtin_expect(!!(x), 1)
 #define ZF_UNLIKELY(x) __builtin_expect(!!(x), 0)
-#else
-#define ZF_LIKELY(x) (x)
-#define ZF_UNLIKELY(x) (x)
-#endif
-#ifndef ZF_WARP_ROTATE
-#define ZF_WARP_ROTATE 1
-#endif
-#ifndef ZF_EXPERIMENT_SKIPC
-#define ZF_EXPERIMENT_SKIPC 0   // timing experiment only (wrong chroma): skip the pass-1 IDCT
-#endif
-#ifndef ZF_EXPERIMENT_PAD
-#define ZF_EXPERIMENT_PAD 0     // timing experiment only: extra dynamic shared memory per CTA (limits CTAs per SM)
-#endif
-#ifndef ZF_EMIT_LOOP
-#define ZF_EMIT_LOOP 0
-#endif
-#ifndef ZF_EARLY_NEXT
-#define ZF_EARLY_NEXT 1      // producers without a pass-1 job prefetch their next strip from pass 0 (see the producer loop)
-#endif
-#ifndef ZF_ROTATE_HV
-#define ZF_ROTATE_HV 0       // 4:2:0: the pass-1 producer jobs (Cb, Cr, halo) rotate over the four producer warps with the strip (measured: 589 against 608 GP/s with the static assignment, 626 against 643 once both forms copied early -- kept for the record, off)
-#endif
-#ifndef ZF_DEFER_EMPTY
-#define ZF_DEFER_EMPTY 1     // (rotated form) wait for the plane buffer between the row pass and the column pass (measured: no difference)
-#endif
-
-// The per-sample generic path (slow_pixel) used to be kept out of line.  With that call inside a consumer warp,
-// compute-sanitizer's synccheck reported divergent threads at the next named barrier (results and racecheck were clean);
-// inlined -- only its leaf ChromaView::at stays a call -- memcheck, racecheck and synccheck are all clean and the headline
-// config is no slower (tools/sanitize_cases.py).
-#ifndef ZJ_NOINLINE
-#define ZJ_NOINLINE __forceinline__
-#endif
-#ifndef ZJ_NOINLINE_AT
-#define ZJ_NOINLINE_AT __noinline__   // ChromaView::at, the leaf every generic sample fetch goes through, stays a call (code size)
-#endif
 
 namespace zj {
 
@@ -75,19 +28,15 @@ typedef uint32_t u32;
 // ------------------------------------------------------------------------------------------------ IDCT
 // 1-D 8-point kernel: reference src/idct/scalar.rs:79-166 == src/idct/avx2.rs:251-331.  All arithmetic is
 // in Z/2^32 (u32), the final shift is arithmetic.
-// ZF_IDCT_MAD: the butterfly written as the 43 operations it needs (27 multiply-adds / adds of the even and odd parts + 16 for
-// the final sums and shifts) with the multiply-adds pinned as `mad.lo` -- the plain expression form below compiled to 50 (the
+// The butterfly is written as the 43 operations it needs (27 multiply-adds / adds of the even and odd parts + 16 for the final
+// sums and shifts) with the multiply-adds pinned as `mad.lo` -- the reference's plain expression form compiled to 50 (the
 // rounding bias as four separate adds, the products of p3 / p4 formed once and added twice).  Regrouping is exact: all of it is
-// arithmetic in Z/2^32.
-#ifndef ZF_IDCT_MAD
-#define ZF_IDCT_MAD 1
-#endif
+// arithmetic in Z/2^32 (tests/test_idct_regroup.py checks it against the reference's literal order).
 template <int K> __device__ __forceinline__ u32 madk(u32 a, u32 c) { u32 d; asm("mad.lo.s32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "n"(K), "r"(c)); return d; }
 
 template <int SH>
 __device__ __forceinline__ void idct8(u32 &s0, u32 &s1, u32 &s2, u32 &s3, u32 &s4, u32 &s5, u32 &s6, u32 &s7, const u32 bias)
 {
-#if ZF_IDCT_MAD
     const u32 p1 = (s2 + s6) * 2217u;
     const u32 t2 = madk<-7567>(s6, p1), t3 = madk<3135>(s2, p1);
     const u32 v = (s0 << 12) + bias;
@@ -100,23 +49,6 @@ __device__ __forceinline__ void idct8(u32 &s0, u32 &s1, u32 &s2, u32 &s3, u32 &s
     const u32 c = madk<12586>(s3, madk<-8034>(p3, r2));
     const u32 b = madk<8410>(s5, madk<-1597>(p4, r2));
     const u32 d = madk<6149>(s1, madk<-1597>(p4, r1));
-#else
-    u32 p1 = (s2 + s6) * 2217u;
-    u32 t2 = p1 + s6 * (u32)(-7567);
-    u32 t3 = p1 + s2 * 3135u;
-    u32 t0 = (s0 + s4) << 12;
-    u32 t1 = (s0 - s4) << 12;
-    u32 x0 = t0 + t3 + bias, x3 = t0 - t3 + bias, x1 = t1 + t2 + bias, x2 = t1 - t2 + bias;
-    u32 a = s7, b = s5, c = s3, d = s1;
-    u32 p3 = a + c, p4 = b + d, q1 = a + d, q2 = b + c;
-    u32 p5 = (p3 + p4) * 4816u;
-    a *= 1223u; b *= 8410u; c *= 12586u; d *= 6149u;
-    q1 = p5 + q1 * (u32)(-3685);
-    q2 = p5 + q2 * (u32)(-10497);
-    p3 *= (u32)(-8034);
-    p4 *= (u32)(-1597);
-    d += q1 + p4; c += q2 + p3; b += q2 + p4; a += q1 + p3;
-#endif
     s0 = (u32)((int)(x0 + d) >> SH);
     s1 = (u32)((int)(x1 + c) >> SH);
     s2 = (u32)((int)(x2 + b) >> SH);
@@ -133,7 +65,6 @@ __device__ __forceinline__ void idct8(u32 &s0, u32 &s1, u32 &s2, u32 &s3, u32 &s
 template <int SH>
 __device__ __forceinline__ void idct8_lo4(u32 &s0, u32 &s1, u32 &s2, u32 &s3, u32 &s4, u32 &s5, u32 &s6, u32 &s7, const u32 bias)
 {
-#if ZF_IDCT_MAD
     // 29 operations: every intermediate is a two-term combination of (s0, s2) or (s1, s3) with the constants summed up front
     const u32 t0 = (s0 << 12) + bias;
     const u32 x0 = madk<2217 + 3135>(s2, t0), x3 = madk<-(2217 + 3135)>(s2, t0), x1 = madk<2217>(s2, t0), x2 = madk<-2217>(s2, t0);
@@ -142,19 +73,6 @@ __device__ __forceinline__ void idct8_lo4(u32 &s0, u32 &s1, u32 &s2, u32 &s3, u3
     const u32 cc = madk<12586 - 10497 + 4816 - 8034>(s3, d48);          // c * 12586 + q2 + p3
     const u32 bb = madk<4816 - 10497>(s3, s1 * (u32)(4816 - 1597));     // q2 + p4
     const u32 aa = madk<4816 - 3685>(s1, s3 * (u32)(4816 - 8034));      // q1 + p3
-#else
-    const u32 t2 = s2 * 2217u;                 // p1 + s6 * -7567 with s6 = 0
-    const u32 t3 = s2 * (2217u + 3135u);       // p1 + s2 * 3135
-    const u32 t0 = (s0 << 12) + bias;          // t0 == t1 when s4 = 0
-    const u32 x0 = t0 + t3, x3 = t0 - t3, x1 = t0 + t2, x2 = t0 - t2;
-    const u32 c = s3, d = s1;                  // a = s7 = 0, b = s5 = 0
-    const u32 p5 = (c + d) * 4816u;
-    const u32 q1 = p5 + d * (u32)(-3685);      // p1 = a + d = d
-    const u32 q2 = p5 + c * (u32)(-10497);     // p2 = b + c = c
-    const u32 p3 = c * (u32)(-8034);           // p3 = a + c = c
-    const u32 p4 = d * (u32)(-1597);           // p4 = b + d = d
-    const u32 dd = d * 6149u + q1 + p4, cc = c * 12586u + q2 + p3, bb = q2 + p4, aa = q1 + p3;
-#endif
     s0 = (u32)((int)(x0 + dd) >> SH);
     s1 = (u32)((int)(x1 + cc) >> SH);
     s2 = (u32)((int)(x2 + bb) >> SH);
@@ -404,42 +322,11 @@ __device__ __forceinline__ void col_pass(const bool active, const bool dconly, c
     }
 }
 
-// ---- halo blocks: ONE sample column instead of the whole block.  The consumers' packed path reads exactly one column of a
-// chroma halo block -- the last one of the left neighbour, the first one of the right neighbour (and of the "stale neighbour"
-// block of tile 0) -- so for a job that holds nothing but halo blocks the row pass only produces that column:
-//   out[r][0] = (E + O + 512) >> 10,  out[r][7] = (E - O + 512) >> 10   with, from the butterfly of idct8 (all in Z/2^32, so the
-//   regrouping is exact):  E = 4096 (s0 + s4) + 5352 s2 + 2217 s6,   O = 5683 s1 + 4816 s3 + 3219 s5 + 1131 s7
-// and leaves it in the scratch where the ORDINARY column pass of column group 0 finds it (position 0 for a first column, position 3
-// for a last column, whose four output bytes then land on block columns 4-7); the other three columns of that group are computed
-// from stale scratch and land in halo samples nobody reads.  About 400 instead of 940 warp-instructions for the halo job of a
-// strip-tile (12 blocks in 32 lanes: it was a seventh of the producers' instructions in 4:2:0) for 60 lines of new hot code --
-// a separate single-column column pass was measured too: 345 SASS lines more, and the 4:2:0 kernel LOST 5.5 % (instruction cache).
-// Only taken when no unit of the tile goes through the per-sample path and the raw row tail (Q4g) stays inside the tile.
-#ifndef ZF_HALO_COL
-#define ZF_HALO_COL 0      // (measured twice: 590 against 598 and 594 against 608 GP/s -- the extra hot code costs more than the instructions it saves; off)
-#endif
-#ifndef ZF_UNROLL_HV
-#define ZF_UNROLL_HV 1
-#endif
-#ifndef ZF_UNROLL_V
-#define ZF_UNROLL_V 1
-#endif
-#ifndef ZF_UNROLL_H
-#define ZF_UNROLL_H 4
-#endif
-#ifndef ZF_UNROLL_NONE
-#define ZF_UNROLL_NONE 4
-#endif
-#ifndef ZF_UNROLL_GRAY
-#define ZF_UNROLL_GRAY 4
-#endif
 // UNROLL: 1 = the row-pair loop stays rolled (4:2:0 / 4:4:0: the consumers' hot code leaves no room in the 32 KB instruction
 // cache for more); 4 = unrolled (everything that depends on the row pair becomes static: +7 % on 4:2:2, +10 % luma-only)
-// halo: 0 = an ordinary job; warp-uniform non-zero = a job of halo blocks reduced to one column each (1: this lane's block
-// needs its first column, 2: its last column)
-template <int UNROLL, bool HALO, bool LO6, typename AfterRows>
+template <int UNROLL, bool LO6, typename AfterRows>
 __device__ __forceinline__ void idct_rolled(const bool active, const u32 sl, const u32 sc, const u32 *__restrict__ qtw, uint8_t *__restrict__ dst, const int dst_stride,
-                                            const int halo, AfterRows after_rows)
+                                            AfterRows after_rows)
 {
     constexpr u32 CH = 16u * ZF_PRODUCERS;
     // Row pairs are visited from the bottom (rows 6-7) to the top (rows 0-1): the first word of the LAST visited pair is then
@@ -447,28 +334,6 @@ __device__ __forceinline__ void idct_rolled(const bool active, const u32 sl, con
     // everything except that word's low half (all 63 AC coefficients); nz collects, one bit per pair, which pairs were
     // transformed (warp-uniform: bit 3 = rows 6-7 ... bit 0 = rows 0-1).
     u32 acc = 0, carry = 0, nz = 0;
-    // (the vote makes the condition warp-uniform FOR THE COMPILER: `halo` derives from the thread index, and a branch it takes
-    // for divergent wraps the ordinary loop below in convergence barriers and takes its counters out of the uniform registers --
-    // measured: 6 % of the whole kernel)
-    const bool halo_job = HALO && __any_sync(0xffffffffu, halo != 0);
-    if (halo_job) {
-        const u32 sg = halo == 2 ? 0xffffffffu : 1u;
-        const u32 k1 = 5683u * sg, k3 = 4816u * sg, k5 = 3219u * sg, k7 = 1131u * sg;
-        const u32 o = sc + (halo == 2 ? 12u : 0u);
-#pragma unroll 1
-        for (int r = 7; r >= 0; r--) {            // bottom-up, as below: `carry` is left with the word that holds the DC coefficient
-            u32 w0, w1, w2, w3;
-            lds128(sl ^ (u32)(r << 4), w0, w1, w2, w3);
-            acc |= carry | w1 | w2 | w3;
-            carry = w0;
-            const uint4 q = *reinterpret_cast<const uint4 *>(qtw + 4 * r);
-            const u32 s0 = dp2a_lo(w0, q.x), s1 = dp2a_hi(w0, q.x), s2 = dp2a_lo(w1, q.y), s3 = dp2a_hi(w1, q.y);
-            const u32 s4 = dp2a_lo(w2, q.z), s5 = dp2a_hi(w2, q.z), s6 = dp2a_lo(w3, q.w), s7 = dp2a_hi(w3, q.w);
-            const u32 v = 512u + ((s0 + s4) << 12) + s2 * 5352u + s6 * 2217u + s1 * k1 + s3 * k3 + s5 * k5 + s7 * k7;
-            asm volatile("st.shared.b32 [%0], %1;" ::"r"(o + (u32)(2 * r) * CH), "r"((u32)((int)v >> 10)) : "memory");
-        }
-        nz = 0xfu;                                 // every row was produced: the 8-input column pass
-    } else
 #pragma unroll UNROLL
     for (int i = 96; i >= 0; i -= 32) {        // i = 32 * row pair: byte offset in the slot and in the table, 1/256 of the scratch offset
         u32 a0, a1, a2, a3, b0, b1, b2, b3;
@@ -530,15 +395,12 @@ __device__ __forceinline__ void idct_rolled(const bool active, const u32 sl, con
 #pragma unroll 1
         for (int g = 0; g < 2; g++) col_pass<4>(active, dconly, dcword, sc + (u32)g * CH, dst + 4 * g, dst_stride);
     } else {
-        // (a halo job: column group 0 only, and a last column's four bytes go to block columns 4-7)
-        const int g1 = halo_job ? 1 : 2;
-        uint8_t *const d0 = (HALO && halo == 2) ? dst + 4 : dst;
         if (LO6 && !rows67) {                 // rows 6-7 are zero in every block of the warp (five luma jobs in six of a quality-90 photo)
 #pragma unroll 1
-            for (int g = 0; g < g1; g++) col_pass<6>(active, dconly, dcword, sc + (u32)g * CH, d0 + 4 * g, dst_stride);
+            for (int g = 0; g < 2; g++) col_pass<6>(active, dconly, dcword, sc + (u32)g * CH, dst + 4 * g, dst_stride);
         } else {
 #pragma unroll 1
-            for (int g = 0; g < g1; g++) col_pass<8>(active, dconly, dcword, sc + (u32)g * CH, d0 + 4 * g, dst_stride);
+            for (int g = 0; g < 2; g++) col_pass<8>(active, dconly, dcword, sc + (u32)g * CH, dst + 4 * g, dst_stride);
         }
     }
 }
@@ -562,7 +424,7 @@ struct ChromaView {
     int lhb, rhb, spb;  // block columns held in the left / right / special halo slots (-1 = none)
     int cs;          // smem row stride (samples)
     unsigned long long magic_w;  // ceil(2^40 / W)
-    __device__ ZJ_NOINLINE_AT int at(int row, int col) const
+    __device__ __noinline__ int at(int row, int col) const   // the leaf every generic sample fetch goes through stays a call (code size)
     {
         int lc;
         if (col >= c0 && col < c1) lc = 8 + (col - c0);
@@ -709,9 +571,12 @@ __device__ __forceinline__ void ycc_to_rgb(int y, int cb, int cr, u32 &r, u32 &g
 }
 
 
-// ------------------------------------------------------------------------- generic (edge) path, out of line
-// Every quirk of the reference, any variant, one sample at a time.  (ZJ_NOINLINE: see the top of the file; the hot loop of
-// the kernel stays small enough for the instruction cache; only edge units of a tile come here.
+// ------------------------------------------------------------------------- generic (edge) path
+// Every quirk of the reference, any variant, one sample at a time; only edge units of a tile come here.
+// slow_pixel used to be kept out of line.  With that call inside a consumer warp, compute-sanitizer's synccheck reported
+// divergent threads at the next named barrier (results and racecheck were clean); inlined -- only its leaf ChromaView::at
+// stays a call, which keeps the hot loop of the kernel small enough for the instruction cache -- memcheck, racecheck and
+// synccheck are all clean and the headline config is no slower (tools/sanitize_cases.py).
 template <typename ST>
 struct SlowCtx {
     ChromaView<ST> cv[2];
@@ -723,7 +588,7 @@ struct SlowCtx {
 };
 
 template <int MODE, int VARIANT, typename ST>
-__device__ ZJ_NOINLINE void slow_pixel(const SlowCtx<ST> &c, int yl, int x)  // x = tile-local luma column
+__device__ __forceinline__ void slow_pixel(const SlowCtx<ST> &c, int yl, int x)  // x = tile-local luma column
 {
     const u32 y = c.y_base + yl;
     if (y >= c.height) return;                 // rows past the image are truncated (mcu.rs:375)
@@ -752,7 +617,7 @@ __device__ ZJ_NOINLINE void slow_pixel(const SlowCtx<ST> &c, int yl, int x)  // 
 // width < 16: the first 16 samples (zero-padded past Wp) are converted into a 16*nc-byte temp and its first
 // width*nc bytes are copied out (worker.rs:176-198).  A single tile covers the row.
 template <int MODE, int VARIANT, typename ST>
-__device__ ZJ_NOINLINE void slow_small_width(const SlowCtx<ST> &c, int rows, int tid)
+__device__ __forceinline__ void slow_small_width(const SlowCtx<ST> &c, int rows, int tid)
 {
     const u32 rowbytes = c.width * c.nc;
     for (int u = tid; u < rows * 16; u += ZJ_THREADS) {
@@ -823,42 +688,20 @@ __device__ __forceinline__ void convert_pair(u32 y, u32 cb, u32 cr, u32 &r, u32 
     b = (minu2(maxu2(cb * 113u + (y32 << 1), 0x38803880u), 0x787F787Fu) - 0x38803880u) >> 6;
 }
 
-// The same with the results left in bytes 1 and 3 (ZF_CONV_HI): the final `>> 5` / `>> 6` (a shift: ALU pipe, the busier one in
-// the consumers) becomes `* 8` / `* 4` on lanes that are already clamped to 13 / 14 bits (a multiply: FMA pipe), and the byte
+// The same with the results left in bytes 1 and 3: the final `>> 5` / `>> 6` (a shift: ALU pipe, the busier one in the
+// consumers) becomes `* 8` / `* 4` on lanes that are already clamped to 13 / 14 bits (a multiply: FMA pipe), and the byte
 // interleave picks bytes 1 and 3 instead of 0 and 2.  The blue channel is clamped from above as unsigned lanes first
 // (64y + 113cb reaches 48751), then shifted down by 14464 and clamped at zero as signed lanes: one instruction fewer.
-#ifndef ZF_CONV_HI
-#define ZF_CONV_HI 2
-#endif
-#ifndef ZF_KR
-#define ZF_KR 2         // 1: the red channel's bias rides on a second lane constant (one 32-bit add fewer per lane pair, one register more); 2: red and green also share the biased luma term
-#endif
+// Every channel is biased so that ONE lane constant (k = -16384, kept in a register by the caller) brings it back: the biases
+// ride on immediates of 32-bit adds (all lanes stay inside [0, 65535], so the lanes never carry into each other).  Red and
+// green share y32g = 32y + 20767 (one LEA; 20767 = 16384 + 4352 + 31); red's lane constant takes the difference back
+// (kr = -5760 - 20767, the lane-wise add wraps mod 2^16 and the true result lies in [-5760, 15315]).
 __device__ __forceinline__ void convert_pair_hi(u32 y, u32 cb, u32 cr, u32 &r, u32 &g, u32 &b, const u32 k, const u32 kr)
 {
-    const u32 y32 = y << 5;
-#if ZF_CONV_HI == 2
-    // every channel is biased so that ONE lane constant (-16384, kept in a register by the caller) brings it back: the biases
-    // ride on immediates of 32-bit adds (all lanes stay inside [0, 65535], so the lanes never carry into each other)
-#if ZF_KR == 2
-    // red and green share y32g = 32y + 20767 (one LEA); red's lane constant takes the difference back (kr = -5760 - 20767, the
-    // lane-wise add wraps mod 2^16 and the true result lies in [-5760, 15315])
     const u32 y32g = y * 32u + 0x511F511Fu;
     r = minrelu2(vadd2(cr * 45u + y32g, kr), 0x1FFF1FFFu) * 8u;
     g = minrelu2(vadd2(y32g - cb * 11u - cr * 23u, k), 0x1FFF1FFFu) * 8u;
-    b = minrelu2(vadd2(minu2(cb * 113u + y * 64u + 0x07800780u, 0x7FFF7FFFu), k), 0x3FFF3FFFu) * 4u;
-    return;
-#elif ZF_KR
-    r = minrelu2(vadd2(cr * 45u + y32, kr), 0x1FFF1FFFu) * 8u;                                     // kr = -5760 on both lanes: 45cr + 32y never leaves [0, 21075]
-#else
-    r = minrelu2(vadd2(cr * 45u + y32 + 0x29802980u, k), 0x1FFF1FFFu) * 8u;                        // +10624 = 16384 - 5760
-#endif
-    g = minrelu2(vadd2(y32 + 0x511F511Fu - cb * 11u - cr * 23u, k), 0x1FFF1FFFu) * 8u;             // +20767 = 16384 + 4352 + 31
     b = minrelu2(vadd2(minu2(cb * 113u + y * 64u + 0x07800780u, 0x7FFF7FFFu), k), 0x3FFF3FFFu) * 4u;   // +1920 = 16384 - 14464
-#else
-    r = minrelu2(vadd2(cr * 45u + y32, 0xE980E980u), 0x1FFF1FFFu) * 8u;
-    g = minrelu2(vadd2(y32 + 0x331F331Fu - cb * 11u - cr * 23u, 0xDE00DE00u), 0x1FFF1FFFu) * 8u;
-    b = minrelu2(vadd2(minu2(cb * 113u + y * 64u, 0x787F787Fu), 0xC780C780u), 0x3FFF3FFFu) * 4u;   // min(., 30847) - 14464, relu
-#endif
 }
 
 // 8 pixels -> 24 interleaved bytes.  c0/c1/c2 hold channel pairs with the values in bytes 0 and 2.
@@ -1243,11 +1086,12 @@ template <int MODE> struct FastTraits {
     static constexpr int YB = TWY / 8, CB = TWC / 8;  // blocks per block row of the tile
     static constexpr int CS = TWC + 24;               // chroma smem row: left halo | tile | right halo | special
     static constexpr int NSLOT = MODE == MODE_H ? 2 : (MODE == MODE_HV ? 3 : 0);  // halo block columns per chroma plane
-    // row-pair loop of the IDCT: unrolled where the instruction cache has room for it (measured per mode)
     // a 6-input column pass for jobs whose rows 6-7 are zero in every block of the warp: pays where the row-pair loop is rolled or
     // the strip is short (4:2:0 +1.1 %, 4:2:2 +0.6 %); with the unrolled loops of 4:4:4 / luma-only its code costs more than it saves
-    static constexpr bool LO6 = ZF_LO6 && (MODE == MODE_HV || MODE == MODE_H);
-    static constexpr int IDCT_UNROLL = MODE == MODE_HV ? ZF_UNROLL_HV : (MODE == MODE_V ? ZF_UNROLL_V : (MODE == MODE_H ? ZF_UNROLL_H : ZF_UNROLL_NONE));
+    static constexpr bool LO6 = MODE == MODE_HV || MODE == MODE_H;
+    // row-pair loop of the IDCT: unrolled where the instruction cache has room for it (measured per mode); 4:2:0 / 4:4:0 stay
+    // rolled, their consumers' hot code leaves no room in the 32 KB instruction cache for more (see idct_rolled)
+    static constexpr int IDCT_UNROLL = (MODE == MODE_HV || MODE == MODE_V) ? 1 : 4;
     static constexpr int NY = YBR * YB, NC = CBR * CB, PER = NC + NSLOT * CBR;
     static constexpr int YBYTES = ROWS * TWY, CBYTES = CROWS * CS, BUF = YBYTES + 2 * CBYTES;  // one buffer of sample planes
     static_assert(NY + 2 * PER <= 2 * ZF_PRODUCERS, "two 8x8 blocks per producer thread");
@@ -1260,33 +1104,19 @@ template <int MODE> struct FastTraits {
 // n = T(a, b), f = T(b, a) on both lanes, sharing a + b + 2:  3a + b + 2 = (a + b + 2) + 2a
 __device__ __forceinline__ void T2pair(u32 a, u32 b, u32 &n, u32 &f)
 {
-#if ZF_T2PAIR
     const u32 s = a + b + 0x00020002u;
     n = ((s + 2u * a) >> 2) & 0x00ff00ffu;
     f = ((s + 2u * b) >> 2) & 0x00ff00ffu;
-#else
-    n = ((a * 3u + b + 0x00020002u) >> 2) & 0x00ff00ffu;
-    f = ((b * 3u + a + 0x00020002u) >> 2) & 0x00ff00ffu;
-#endif
 }
-// ZF_VSCALE (4:2:0 packed path): the vertical blend hands 4 * T(a, b) (1) or 4 * T(a, b) + 2 (2) to the horizontal filter instead
-// of T(a, b): the `>> 2` of the blend becomes part of the filter's own shift --
-//   (3 * 4N + 4L + 8) >> 4  ==  (3N + L + 2) >> 2  ==  (3 * (4N + 2) + (4L + 2)) >> 4      (exact: everything is a multiple of 4)
-// which takes two shifts out of every T2pair (1) and the filter's separate add out of every output pair as well (2).
-// Lanes stay below 3 * 1538 + 1538 + 8 = 6160.
-#ifndef ZF_VSCALE
-#define ZF_VSCALE 1
-#endif
-__device__ __forceinline__ void T2pair_s(u32 a, u32 b, u32 &n, u32 &f, const u32 mask)
+// 4:2:0 packed path: the vertical blend hands 4 * T(a, b) to the horizontal filter instead of T(a, b), and the `>> 2` of the
+// blend becomes part of the filter's own shift --
+//   (3 * 4N + 4L + 8) >> 4  ==  (3N + L + 2) >> 2      (exact: everything is a multiple of 4)
+// which takes two shifts out of every T2pair.  Lanes stay below 3 * 1536 + 1536 + 8 = 6152.
+__device__ __forceinline__ void T2pair_s(u32 a, u32 b, u32 &n, u32 &f)
 {
     const u32 s = a + b + 0x00020002u;
-#if ZF_VSCALE == 2
-    n = ((s + 2u * a) & mask) | 0x00020002u;
-    f = ((s + 2u * b) & mask) | 0x00020002u;
-#else
     n = (s + 2u * a) & 0xFFFCFFFCu;
     f = (s + 2u * b) & 0xFFFCFFFCu;
-#endif
 }
 __device__ __forceinline__ u32 evens(u32 w) { return prmt(w, 0u, 0x4240u); }  // bytes 0,2 -> 16-bit lanes
 __device__ __forceinline__ u32 odds(u32 w) { return prmt(w, 0u, 0x4341u); }   // bytes 1,3 -> 16-bit lanes
@@ -1318,7 +1148,7 @@ __device__ __forceinline__ void hfilter16(u32 h, const u32 r[4], u32 E[4], u32 O
     }
 }
 
-// the same filter on inputs scaled as ZF_VSCALE says (r[k], h = 4 * sample (+ 2)); results are the unscaled ones of hfilter16
+// the same filter on inputs scaled by 4 (r[k], h = 4 * sample, see T2pair_s); results are the unscaled ones of hfilter16
 __device__ __forceinline__ void hfilter16_s(u32 h, const u32 r[4], u32 E[4], u32 O[4])
 {
     u32 L[5];
@@ -1329,14 +1159,9 @@ __device__ __forceinline__ void hfilter16_s(u32 h, const u32 r[4], u32 E[4], u32
     L[4] = prmt(r[3], h, 0x7632u);
 #pragma unroll
     for (int k = 0; k < 4; k++) {
-#if ZF_VSCALE == 2
-        E[k] = ((r[k] * 3u + L[k]) >> 4) & 0x01ff01ffu;
-        O[k] = ((r[k] * 3u + L[k + 1]) >> 4) & 0x01ff01ffu;
-#else
         const u32 p3 = r[k] * 3u + 0x00080008u;
         E[k] = ((p3 + L[k]) >> 4) & 0x01ff01ffu;
         O[k] = ((p3 + L[k + 1]) >> 4) & 0x01ff01ffu;
-#endif
     }
 }
 
@@ -1356,13 +1181,8 @@ __device__ __forceinline__ void emit16(uint8_t *dst, const u32 yw[4], const u32 
         if (ycc) {  // `as u8` interleave (color_convert/scalar.rs:152-161)
             c0E = yE; c1E = cbE[k]; c2E = crE[k]; c0O = yO; c1O = cbO[k]; c2O = crO[k];
         } else {
-#if ZF_CONV_HI
             convert_pair_hi(yE, cbE[k], crE[k], c0E, c1E, c2E, kk, kr);
             convert_pair_hi(yO, cbO[k], crO[k], c0O, c1O, c2O, kk, kr);
-#else
-            convert_pair(yE, cbE[k], crE[k], c0E, c1E, c2E);
-            convert_pair(yO, cbO[k], crO[k], c0O, c1O, c2O);
-#endif
         }
         const u32 rgE = prmt(c0E, c1E, sel);   // [R0 G0 R2 G2]
         const u32 brO = prmt(c2E, c0O, sel);   // [B0 R1 B2 R3]
@@ -1390,13 +1210,8 @@ __device__ __forceinline__ void load16(const uint8_t *p, const bool a16, u32 w[4
     else { const uint2 v0 = *reinterpret_cast<const uint2 *>(p), v1 = *reinterpret_cast<const uint2 *>(p + 8); w[0] = v0.x; w[1] = v0.y; w[2] = v1.x; w[3] = v1.y; }
 }
 
-#ifndef ZF_NBUF
-#define ZF_NBUF 2
-#endif
-#ifndef ZF_ROLEMAP
-#define ZF_ROLEMAP 0    // 0: warps 0-3 produce, 4-7 consume (both roles on every SM sub-partition); 1: sub-partitions 0,1 produce, 2,3 consume
-#endif
-enum { BAR_FULL = 1, BAR_EMPTY = 1 + ZF_NBUF, BAR_QUEUE = 1 + 2 * ZF_NBUF };  // + buffer index
+constexpr int ZF_NB = 2;   // plane buffers in flight
+enum { BAR_FULL = 1, BAR_EMPTY = 3, BAR_QUEUE = 5 };  // + buffer index (BAR_QUEUE + 1: the producers' own barrier)
 
 template <int MODE>
 __global__ void __launch_bounds__(ZF_THREADS, ZF_MINBLOCKS)
@@ -1407,8 +1222,7 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
     constexpr int ROWS = FT::ROWS, TWY = FT::TWY, CS = FT::CS, NRG = FT::NRG, XU = FT::XU, RPU = FT::RPU;
     constexpr bool HALO = FT::NSLOT > 0;
 
-    constexpr int NB = (MODE == MODE_V || MODE == MODE_NONE) ? 2 : ZF_NBUF;   // plane buffers in flight
-    extern __shared__ __align__(128) uint8_t sDynAll[];  // [staging slots ZF_PRODUCERS * 128 B | row-pass scratch ZF_PRODUCERS * 256 B | NB plane buffers of [Y | Cb | Cr]]
+    extern __shared__ __align__(128) uint8_t sDynAll[];  // [staging slots ZF_PRODUCERS * 128 B | row-pass scratch ZF_PRODUCERS * 256 B | ZF_NB plane buffers of [Y | Cb | Cr]]
     ST *const sPlanes = sDynAll + 3 * ZF_PRODUCERS * 128 + 128;   // (+ one all-zero slot)
     __shared__ __align__(16) u32 sQ[3][32];
     __shared__ int sSlowN;
@@ -1455,19 +1269,8 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
     if (tid == 0) sSlowN = 0;
     __syncthreads();
 
-#if ZF_ROLEMAP == 1
-    const int warp = tid >> 5;
-    const bool producer = (warp & 2) == 0;
-    const int rtid = ((warp >> 2) * 64) + ((warp & 1) * 32) + (tid & 31);   // thread index inside the role
-#elif ZF_ROLEMAP == 2
-    // producers in the UPPER warps of the CTA: the warp scheduler favours higher warp slots, and the producers are the
-    // critical path of the pipeline
-    const bool producer = tid >= ZF_CONSUMERS;
-    const int rtid = producer ? tid - ZF_CONSUMERS : tid;
-#else
     const bool producer = tid < ZF_PRODUCERS;
     const int rtid = producer ? tid : tid - ZF_PRODUCERS;
-#endif
     if (producer) {
         // ================================================================= producers: dequantise + IDCT
         // Blocks rtid and rtid + ZF_PRODUCERS of the tile's list [Y | Cb tile | Cr tile | Cb halo | Cr halo]: every warp
@@ -1479,7 +1282,7 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
         // Which of the four producer jobs a hardware warp takes is rotated with the CTA index: the jobs are not equally heavy
         // (in 4:2:0 two warps carry a luma AND a chroma pass), warp w always runs on SM sub-partition w mod 4, and the three
         // resident CTAs of an SM would otherwise pile their heavy warps onto the same two sub-partitions.
-        const int lane = tid & 31, wq = ((rtid >> 5) + ZF_WARP_ROTATE * (int)(blockIdx.x + blockIdx.y + blockIdx.z)) & 3;
+        const int lane = tid & 31, wq = ((rtid >> 5) + (int)(blockIdx.x + blockIdx.y + blockIdx.z)) & 3;
         const int ybpr = Wp >> 3;
         // block index -> plane, block row, global block column (-1: none), smem column
         auto decode = [&](int b, int &comp, int &br, int &gcol, int &lcol) {
@@ -1502,7 +1305,8 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
         const u32 stepY = (u32)(FT::YBR * ybpr * 64), stepC = (u32)(FT::CBR * mcu_x * 64);   // i16 per strip
         // One staging job = the 32 consecutive list entries [B0, B0 + 32) of a warp: where this lane's block of the job goes (pk),
         // how the warp copies the job's runs (g0 / g1 lane pointers at the CTA's first strip, jm).
-        //   pk: bits 0-15 byte offset in the plane buffer, 16 active, 17 chroma, 18-19 table, 20 left halo block
+        //   pk: bits 0-15 byte offset in the plane buffer, 16 active, 17 chroma, 18-19 table, 20 left halo block (nothing reads it;
+        //       the compiler schedules the setup differently without it, so it goes with the next change that re-measures the kernel)
         //   jm: bits 0-7 chunk k of the cooperative copy is inside the run, bit 8 the lane copies its own (lone) block
         auto setup_job = [&](const int B0, u32 &pkj, const int16_t *&g0, const int16_t *&g1, u32 &jmj) {
             int comp, br, gcol, lcol;
@@ -1510,7 +1314,7 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
             const bool active = gcol >= 0;
             pkj = (comp == 0 ? (u32)(br * 8 * TWY + lcol) : (u32)(FT::YBYTES + (comp - 1) * FT::CBYTES + br * 8 * CS + lcol)) |
                   (active ? 0x10000u : 0u) | (comp ? 0x20000u : 0u) | ((u32)comp << 18) |
-                  ((comp != 0 && lcol == 0) ? 0x100000u : 0u);   // bit 20: left halo block (its LAST column is the one the consumers read)
+                  ((comp != 0 && lcol == 0) ? 0x100000u : 0u);   // bit 20: see pk above
             const int lsub = lane >> 3, lch = lane & 7;
             g0 = g1 = im.coeff[0];
             int mode = 0, lim0 = 0, lim1 = 0;   // mode: 0 none, 1 one run of 32, 2 two runs of 16, 3 lone blocks
@@ -1553,104 +1357,23 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
         // (these four are a few integer operations each from the lane index; made opaque so that they are kept instead of
         // being recomputed in every pass)
         asm volatile("" : "+r"(const_cast<u32 &>(d_even)), "+r"(const_cast<u32 &>(d_odd)), "+r"(const_cast<u32 &>(slx)), "+r"(const_cast<u32 &>(scr)));
-        auto issue = [&](const int ps, const int16_t *g0, const int16_t *g1, const u32 m) {
-            const u32 off = 0u;
+        auto issue = [&](const int16_t *g0, const int16_t *g1, const u32 m) {
             if (ZF_LIKELY(m == 0xffu)) {   // a full job: no per-chunk predicates
 #pragma unroll
                 for (int k = 0; k < 8; k++)
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(((k & 1) ? d_odd : d_even) + off + k * 512u), "l"((k < 4 ? g0 : g1) + k * 256) : "memory");
+                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(((k & 1) ? d_odd : d_even) + k * 512u), "l"((k < 4 ? g0 : g1) + k * 256) : "memory");
             } else if (m & 0x100u) {
 #pragma unroll
                 for (int r = 0; r < 8; r++)
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((slx + off) ^ (u32)(r << 4)), "l"(g0 + r * 8) : "memory");
+                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(slx ^ (u32)(r << 4)), "l"(g0 + r * 8) : "memory");
             } else {
 #pragma unroll
                 for (int k = 0; k < 8; k++)
                     if (m & (1u << k))
-                        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(((k & 1) ? d_odd : d_even) + off + k * 512u), "l"((k < 4 ? g0 : g1) + k * 256) : "memory");
+                        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(((k & 1) ? d_odd : d_even) + k * 512u), "l"((k < 4 ? g0 : g1) + k * 256) : "memory");
             }
             asm volatile("cp.async.commit_group;" ::: "memory");
         };
-#if ZF_ROTATE_HV
-        if constexpr (MODE == MODE_HV) {
-            // 4:2:0 / the seven jobs of a strip-tile (4 luma, Cb, Cr, halo) over four warps: every warp transforms its own luma
-            // job in pass 0; the three pass-1 jobs ROTATE with the strip so that no warp is the heavy one all the time (statically
-            // assigned, two warps carried a chroma pass in every strip and set the pace of the whole CTA while the fourth idled
-            // at the `empty` barrier).  pair = which chroma plane a warp alternates on, half = on which strip parity:
-            //   strip parity == half: the warp's chroma job;  else, every other time ((it >> 1) & 1 == pair): the halo job.
-            //   it:      0        1        2        3
-            //   warp 0   Cb       halo     Cb       -          (pair 0, half 0)
-            //   warp 1   Cr       -        Cr       halo       (pair 1, half 0)
-            //   warp 2   halo     Cb       -        Cb         (pair 0, half 1)
-            //   warp 3   -        Cr       halo     Cr         (pair 1, half 1)
-            // Per four strips every warp does 4 luma + 2 chroma + 1 halo job.  The wait for the consumers to release the plane
-            // buffer sits between the row pass (which only writes the warp's scratch) and the column pass of pass 0.
-            // (through votes: wq derives from the thread index, and a branch on anything the compiler cannot prove warp-uniform
-            // wraps the transform loops in convergence barriers and takes their counters out of the uniform registers)
-            const int pair = __any_sync(0xffffffffu, (wq & 1) != 0) ? 1 : 0, half = __any_sync(0xffffffffu, (wq & 2) != 0) ? 1 : 0;
-            u32 pkL, pkC, pkH, jmL, jmC, jmH;
-            const int16_t *aL, *bL, *aC, *bC, *aH, *bH;
-            setup_job(wq * 32, pkL, aL, bL, jmL);
-            setup_job(FT::NY + pair * FT::NC, pkC, aC, bC, jmC);
-            setup_job(FT::NY + 2 * FT::NC, pkH, aH, bH, jmH);
-            aC += (u32)half * stepC; bC += (u32)half * stepC;                  // first strip of the warp's chroma job
-            aH += (u32)((1 - half) + 2 * pair) * stepC;                       // ... and of its halo job
-            const bool workL = __any_sync(0xffffffffu, (pkL & 0x10000u) != 0), workC = __any_sync(0xffffffffu, (pkC & 0x10000u) != 0),
-                       workH = __any_sync(0xffffffffu, (pkH & 0x10000u) != 0);
-            // the halo job may be reduced to the one column per block the consumers' packed path reads (idct_rolled): not when a unit
-            // of the tile goes through the per-sample path (it reads halo samples anywhere), nor when the raw row tail (Q4g) starts
-            // left of the tile (decided in front of the first pass 1, see below)
-            constexpr bool HALO_JOBS = ZF_HALO_COL && !FT::DENSE && ((FT::NY + 2 * FT::NC) % 32) == 0;
-            const bool tail_in_halo = cb0 + ncb == mcu_x && W - 36 - cb0 * 8 < 0;
-            bool halo_ok = HALO_JOBS;
-            issue(0, aL, bL, jmL);
-            aL += stepY; bL += stepY;
-            int buf = 0;
-            for (int it = 0; it < n_it; it++) {
-                ST *planes = sPlanes + buf * FT::BUF;
-                const bool hasC = (it & 1) == half, hasH = !hasC && ((it >> 1) & 1) == pair;
-                // a strip without a pass-1 job: the next strip's luma job is copied from pass 0 and pass 1 is skipped (ZF_EARLY_NEXT)
-                const bool early = ZF_EARLY_NEXT && !HALO_JOBS && !(hasC || hasH);
-#pragma unroll 1
-                for (int ps = 0; ps < 2; ps++) {
-                    if (ps == 1 && early) break;
-                    const u32 pkk = ps ? (hasC ? pkC : pkH) : pkL;
-                    const bool work = ps ? (hasC ? workC : (hasH && workH)) : workL;
-                    const bool active = (pkk & 0x10000u) != 0;
-                    asm volatile("cp.async.wait_group 0;" ::: "memory");
-                    __syncwarp();
-#if !ZF_DEFER_EMPTY
-                    if (ps == 0 && it >= NB) bar_sync(BAR_EMPTY + buf);
-#endif
-                    // the copy issued from this pass: the warp's pass-1 job of this strip (if it has one), or its luma job of the next strip
-                    auto refill = [&]() {
-#if ZF_DEFER_EMPTY
-                        if (ps == 0 && it >= NB) bar_sync(BAR_EMPTY + buf);   // the consumers are done with this buffer
-#endif
-                        const bool nxt = ps || early;
-                        const int16_t *g0 = nxt ? aL : (hasC ? aC : aH), *g1 = nxt ? bL : (hasC ? bC : aH);
-                        const u32 m = nxt ? (it + 1 < n_it ? jmL : 0u) : (hasC ? jmC : (hasH ? jmH : 0u));
-                        issue(ps, g0, g1, m);
-                        if (nxt) { aL += stepY; bL += stepY; }
-                        else if (hasC) { aC += 2u * stepC; bC += 2u * stepC; }
-                        else if (hasH) aH += 4u * stepC;
-                    };
-                    if (HALO_JOBS && ps && it == 0) {
-                        // the consumers have counted their per-sample units long before the producers' first pass 1 (they arrived at
-                        // this barrier when their queue was complete): nobody waits here, it only orders the read of the count
-                        asm volatile("bar.sync %0, %1;" ::"r"((int)BAR_QUEUE + 2), "n"(ZF_THREADS) : "memory");
-                        halo_ok = halo_ok && sSlowN == 0 && !tail_in_halo;
-                    }
-                    const int halo = (HALO_JOBS && ps && hasH && halo_ok) ? ((pkk & 0x100000u) ? 2 : 1) : 0;
-                    if (work) idct_rolled<FT::IDCT_UNROLL, HALO_JOBS, FT::LO6>(active, active ? slx : zslot, scr, sQ[(pkk >> 18) & 3u], planes + (pkk & 0xffffu), (pkk & 0x20000u) ? CS : TWY, halo, refill);
-                    else refill();
-                }
-                bar_arrive(BAR_FULL + buf);
-                buf = buf + 1 == NB ? 0 : buf + 1;
-            }
-            return;
-        }
-#endif
         // this thread's own two blocks / this warp's staging jobs
         u32 pk[2], jm[2];
         const int16_t *q0[2], *q1[2];    // lane pointers into run 0 / run 1 (lone blocks: the lane's own block)
@@ -1671,15 +1394,7 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
         // one staging slot per thread: the copy of the next pass is issued as soon as the row pass has drained the slot
         // and lands while the column pass runs
         const bool work0 = __any_sync(0xffffffffu, (pk0 & 0x10000u) != 0), work1 = __any_sync(0xffffffffu, (pk1 & 0x10000u) != 0);   // any block in the warp
-        // the pass-1 job of this warp holds nothing but halo blocks (4:2:0: entries 192-203 of the list) ...
-        constexpr bool HALO_JOBS = ZF_HALO_COL && MODE == MODE_HV && !FT::DENSE && ((FT::NY + 2 * FT::NC) % 32) == 0;
-        const int jw1 = (wq + ((MODE == MODE_NONE || MODE == MODE_H) ? 2 : 0)) & 3;
-        bool halo1 = HALO_JOBS && (ZF_PRODUCERS + jw1 * 32 >= FT::NY + 2 * FT::NC);
-        // ... and may be reduced to the one column per block the consumers' packed path reads: not when a unit of the tile goes
-        // through the per-sample path (it reads halo samples anywhere), nor when the raw row tail (Q4g) starts left of the tile
-        // (decided in front of the first pass 1, see below)
-        const bool tail_in_halo = cb0 + ncb == mcu_x && W - 36 - cb0 * 8 < 0;
-        issue(0, qa0, qb0, jm0);
+        issue(qa0, qb0, jm0);
         qa0 += st0; qb0 += st0;
         int buf = 0;
         for (int it = 0; it < n_it; it++) {
@@ -1690,34 +1405,24 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
                 // strip's job as soon as the row pass of pass 0 has drained the slot, and skips pass 1: issued from pass 1 the copy
                 // had no lead at all -- the warp waited for it at the top of the next strip (10 % of all stall samples of the
                 // 1080p 4:2:2 config sat on that wait).
-                if (ZF_EARLY_NEXT && !HALO_JOBS && ps == 1 && !work1) break;
+                if (ps == 1 && !work1) break;
                 const u32 pkk = ps ? pk1 : pk0;
                 const bool active = (pkk & 0x10000u) != 0;
                 asm volatile("cp.async.wait_group 0;" ::: "memory");
                 __syncwarp();
-                if (ps == 0 && it >= NB) bar_sync(BAR_EMPTY + buf);   // the consumers are done with this buffer
+                if (ps == 0 && it >= ZF_NB) bar_sync(BAR_EMPTY + buf);   // the consumers are done with this buffer
                 // the copy issued from this pass: the warp's pass-1 job of this strip, or its pass-0 job of the next strip
                 // (one call site: the copy code exists once in the loop)
                 auto refill = [&]() {
-                    const bool nxt = ps || (ZF_EARLY_NEXT && !HALO_JOBS && !work1);           // the next strip's pass-0 job
-                    issue(ps, nxt ? qa0 : qa1, nxt ? qb0 : qb1, nxt ? (it + 1 < n_it ? jm0 : 0u) : jm1);
+                    const bool nxt = ps || !work1;           // the next strip's pass-0 job
+                    issue(nxt ? qa0 : qa1, nxt ? qb0 : qb1, nxt ? (it + 1 < n_it ? jm0 : 0u) : jm1);
                     if (nxt) { qa0 += st0; qb0 += st0; } else { qa1 += st1; qb1 += st1; }
                 };
-                if (HALO_JOBS && ps && it == 0) {
-                    // the consumers have counted their per-sample units long before the producers' first pass 1 (they arrived at
-                    // this barrier when their queue was complete): nobody waits here, it only orders the read of the count
-                    asm volatile("bar.sync %0, %1;" ::"r"((int)BAR_QUEUE + 2), "n"(ZF_THREADS) : "memory");
-                    halo1 = halo1 && sSlowN == 0 && !tail_in_halo;
-#ifdef ZF_HALO_FORCE_OFF
-                    halo1 = halo1 && spc < 0;      // (experiment: the code is there but never taken)
-#endif
-                }
-                const int halo = (HALO_JOBS && ps && halo1) ? ((pkk & 0x100000u) ? 2 : 1) : 0;
-                if (ps ? (work1 && !ZF_EXPERIMENT_SKIPC) : work0) idct_rolled<FT::IDCT_UNROLL, HALO_JOBS, FT::LO6>(active, active ? slx : zslot, scr, sQ[(pkk >> 18) & 3u], planes + (pkk & 0xffffu), (pkk & 0x20000u) ? CS : TWY, halo, refill);
+                if (ps ? work1 : work0) idct_rolled<FT::IDCT_UNROLL, FT::LO6>(active, active ? slx : zslot, scr, sQ[(pkk >> 18) & 3u], planes + (pkk & 0xffffu), (pkk & 0x20000u) ? CS : TWY, refill);
                 else refill();
             }
             bar_arrive(BAR_FULL + buf);
-            buf = buf + 1 == NB ? 0 : buf + 1;
+            buf = buf + 1 == ZF_NB ? 0 : buf + 1;
         }
         return;
     }
@@ -1726,15 +1431,10 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
     const int tc = rtid;
     const int xu = tc % XU, rgA = tc / XU;                // this thread's units: (xu, rgA) and (xu, rgA + NRG/2)
     const bool ycc = im.out_kind == OUT_YCC;
-    u32 esel = (ZF_CONV_HI && !ycc) ? 0x7351u : 0x6240u, ekk = 0xC000C000u ^ ((u32)spc >> 30);   // (spc < 2^30: a constant ptxas cannot see)
+    u32 esel = !ycc ? 0x7351u : 0x6240u, ekk = 0xC000C000u ^ ((u32)spc >> 30);   // (spc < 2^30: a constant ptxas cannot see)
     asm volatile("" : "+r"(esel), "+r"(ekk));   // (opaque: kept in registers instead of being rematerialised in front of every use)
-    u32 ekr = (ZF_KR == 2 ? 0x98619861u : 0xE980E980u) ^ ((u32)spc >> 30), emask = 0xFFFCFFFCu ^ ((u32)spc >> 30);
-#if ZF_KR
+    u32 ekr = 0x98619861u ^ ((u32)spc >> 30);
     asm volatile("" : "+r"(ekr));
-#endif
-#if ZF_VSCALE == 2
-    asm volatile("" : "+r"(emask));
-#endif
     int xs = X0 + 16 * xu;                                // first sample of the unit in the padded row
     // Where the unit's 48 bytes go (worker.rs:201-246, SURVEY A.5): samples < n_norm ("normal" 16-sample chunks) sit at
     // byte 3*s, except bytes the tail chunk overwrites; the tail chunk (samples Wp-16..Wp-1) sits at T; the rest is never written
@@ -1787,7 +1487,6 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
         }
     bar_sync_consumers(BAR_QUEUE);   // the queue is complete (consumer warps only)
     const int nslow = sSlowN;
-    if (ZF_HALO_COL && MODE == MODE_HV && !FT::DENSE && ((FT::NY + 2 * FT::NC) % 32) == 0) bar_arrive(BAR_QUEUE + 2);   // ... and the producers may read its length
 
     // bytes of a row nobody writes: [P, stride) minus the tail chunk [T, T+48) (Q5: 16 zero bytes; Q6: the w "alpha"
     // bytes) = [z0, stride); every tile zeroes its share, with the widest stores the alignment allows
@@ -1859,15 +1558,9 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
                     const u32 Ah = aL | (aR << 16), Bh = bL | (bR << 16);
                     u32 N[4], F[4];
                     u32 Nh, Fh;
-#if ZF_VSCALE
 #pragma unroll
-                    for (int k = 0; k < 4; k++) T2pair_s(A[k], B[k], N[k], F[k], emask);
-                    T2pair_s(Ah, Bh, Nh, Fh, emask);
-#else
-#pragma unroll
-                    for (int k = 0; k < 4; k++) T2pair(A[k], B[k], N[k], F[k]);
-                    T2pair(Ah, Bh, Nh, Fh);
-#endif
+                    for (int k = 0; k < 4; k++) T2pair_s(A[k], B[k], N[k], F[k]);
+                    T2pair_s(Ah, Bh, Nh, Fh);
                     // AVX2 form: lane 0 of a vector takes 3*(in+in'+2)>>2 of its OWN first element as "previous" value,
                     // lane 15 the same expression of the next vector's first element as "next" value (Q4e)
                     u32 pv = (3u * ((sel0 ? (a.x & 0xffu) + (b.x & 0xffu) : aR + bR) + 2u)) >> 2;
@@ -1886,19 +1579,12 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
                             pv = (3u * (y0 + y1 + 2u)) >> 2;
                         }
                     }
-#if ZF_VSCALE
-                    pv = pv * 4u + (ZF_VSCALE == 2 ? 2u : 0u);            // (<= 4 * 384 + 2: one lane)
-#endif
+                    pv = pv * 4u;                                          // (<= 4 * 384: one lane)
                     const u32 keep = sel0 ? 0xffff0000u : 0x0000ffffu, ins = sel0 ? pv : pv << 16;
                     Nh = (Nh & keep) | ins;
                     Fh = (Fh & keep) | ins;
-#if ZF_VSCALE
                     hfilter16_s(Nh, N, E0[c], O0[c]);
                     hfilter16_s(Fh, F, E1[c], O1[c]);
-#else
-                    hfilter16(Nh, N, E0[c], O0[c]);
-                    hfilter16(Fh, F, E1[c], O1[c]);
-#endif
                     if (firstvec && cc0 == 0) E1[c][0] = prmt(E1[c][0], O1[c][0], 0x3254u);   // far rows: out[0] = out[1] (avx2.rs:330)
                 } else {
                     // last 32 outputs of the double-row: out[O+2k] = T(in[c], in[c-1]), out[O+2k+1] = T(in[c], in[c+1]),
@@ -1918,25 +1604,6 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
                     }
                 }
             }
-#if ZF_EMIT_LOOP
-            // one copy of the colour / pack / store code (it is a third of the hot instructions): the second row's chroma
-            // is moved into the first row's registers between the two trips
-#pragma unroll 1
-            for (int row = 0; row < RPU; row++) {
-                const int yl = row ? yl1 : yl0;
-                if (y_base + yl < im.height) {
-                    u32 yw[4];
-                    load16(planes + yl * TWY + xl, FT::H == 2 || y16, yw);
-                    emit16(out + (size_t)(y_base + yl) * stride + dst_off, yw, E0[0], O0[0], E0[1], O0[1], ycc, nw, vec, esel, ekk, ekr);
-                }
-                if (RPU == 2) {
-#pragma unroll
-                    for (int c = 0; c < 2; c++)
-#pragma unroll
-                        for (int k = 0; k < 4; k++) { E0[c][k] = E1[c][k]; O0[c][k] = O1[c][k]; }
-                }
-            }
-#else
             if (y_base + yl0 < im.height) {
                 u32 yw[4];
                 load16(planes + yl0 * TWY + xl, FT::H == 2 || y16, yw);
@@ -1947,7 +1614,6 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
                 load16(planes + yl1 * TWY + xl, FT::H == 2 || y16, yw);
                 emit16(out + (size_t)(y_base + yl1) * stride + dst_off, yw, E1[0], O1[0], E1[1], O1[1], ycc, nw, vec, esel, ekk, ekr);
             }
-#endif
         }
         if (ZF_UNLIKELY(nslow > 0)) {
             SlowCtx<ST> sc;
@@ -1982,8 +1648,8 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
             }
             __syncwarp();
         }
-        if (it + NB < n_it) bar_arrive(BAR_EMPTY + buf);          // the producers may refill this buffer
-        buf = buf + 1 == NB ? 0 : buf + 1;
+        if (it + ZF_NB < n_it) bar_arrive(BAR_EMPTY + buf);          // the producers may refill this buffer
+        buf = buf + 1 == ZF_NB ? 0 : buf + 1;
         if (ZF_UNLIKELY(zcnt > 0)) {
             // thread -> (row zr0 + i * zrpp, store zk0 + j * ZF_CONSUMERS): no divisions inside the strip loop
             for (int yl = zr0; yl < ROWS; yl += zrpp) {
@@ -2139,7 +1805,7 @@ gray_fast_kernel(const DevImage *__restrict__ images, const int spc)
             auto refill = [&]() {
                 if (it + 1 < n_it) { issue(q0, row_exists(it + 1)); q0 += step; }
             };
-            if (work && row_exists(it)) idct_rolled<ZF_UNROLL_GRAY, false, false>(active, active ? slx : zslot, scr, sQ, planes + dsto, ZG_TW, 0, refill);
+            if (work && row_exists(it)) idct_rolled<4, false>(active, active ? slx : zslot, scr, sQ, planes + dsto, ZG_TW, refill);
             else refill();
             bar_arrive(BAR_FULL + (it & 1));
         }
@@ -2209,8 +1875,7 @@ static cudaError_t launch_fast(const DevImage *d_images, const LaunchGroup &g, c
     const int spc = strips_per_cta(g);
     dim3 grid(g.max_tiles, (g.max_strips + spc - 1) / spc + 1, g.count);
     typedef FastTraits<MODE> FT;
-    constexpr int NB = (MODE == MODE_V || MODE == MODE_NONE) ? 2 : ZF_NBUF;
-    constexpr size_t smem = 3 * ZF_PRODUCERS * 128 + 128 + (size_t)NB * FT::BUF + ZF_EXPERIMENT_PAD;
+    constexpr size_t smem = 3 * ZF_PRODUCERS * 128 + 128 + (size_t)ZF_NB * FT::BUF;
     static bool configured[64] = {false};
     int dev = 0;
     cudaGetDevice(&dev);
