@@ -199,6 +199,42 @@ ZJ_API int zj_gpu_convert_device(int device, void *stream, const uint8_t *src_de
 ZJ_API int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs, size_t n, const zj_output_desc *d,
                                         void *const *out_dev, const size_t *out_len);
 
+/* ---------------------------------------------------- cropped, resized batch tensors (DESIGN.md section 4.5.1) */
+/* What a model reads: one N x OC x OH x OW (CHW) or N x OH x OW x OC (HWC) tensor, slot i at i * zj_resize_slot_size bytes,
+ * each slot a crop of image i resized to out_w x out_h, in the type / layout / channels / normalisation of a zj_output_desc
+ * (scale_log2 must be 0).  torchvision's resized_crop: crop first, then resize; neighbours are clamped to the crop and pixels
+ * outside it never contribute.  p[r][c][ch] = the u8 the reference writes at crop row r, column c; every fp32 operation is
+ * one IEEE round-to-nearest operation, in the order written, no FMA:
+ *   ZJ_FILTER_AREA      adaptive average pooling: output row i covers crop rows [i*h/OH, ceil((i+1)*h/OH)), columns alike;
+ *                       s = exact integer sum of the window's bytes, n = its pixel count.  u8: (s + n/2) / n (integer);
+ *                       float: v = float(s) / float(n).  At exactly half size this is the scale_log2 = 1 consumer.
+ *   ZJ_FILTER_BILINEAR  torch interpolate(mode="bilinear", align_corners=False, antialias=False): sx = float(w) / float(OW),
+ *                       fx = max((float(j) + 0.5f) * sx - 0.5f, 0), c0 = min(int(fx), w - 1), c1 = min(c0 + 1, w - 1),
+ *                       ax = fx - float(c0), bx = 1 - ax; rows alike (sy, r0, r1, ay, by).  top = bx*p[r0][c0] + ax*p[r0][c1],
+ *                       bot = bx*p[r1][c0] + ax*p[r1][c1], v = by*top + ay*bot.  u8: v rounded to nearest even, clamped to [0, 255].
+ *   float outputs       (v - mean[c]) * inv_std[c]; f16 = that value rounded to nearest even.
+ * OC = nc, or 3 when channels = 3 and nc = 4; every image of a call must have the same OC. */
+typedef struct zj_roi { uint32_t x, y, w, h; } zj_roi;                      /* w, h >= 1, x + w <= width, y + h <= height */
+typedef struct zj_resize { uint32_t out_w, out_h, filter, reserved; } zj_resize;   /* out_w, out_h 1..65535; reserved = 0 */
+enum { ZJ_FILTER_AREA = 0, ZJ_FILTER_BILINEAR = 1 };
+/* bytes of one slot for images of nc bytes per pixel (0 on a bad descriptor) */
+ZJ_API size_t zj_resize_slot_size(const zj_output_desc *d, const zj_resize *r, uint32_t nc);
+/* The smallest strip range (zj_image_strip_range) whose rows cover [row_begin, row_end), as a virtual image *sub; *sub_row0 =
+ * the row of row_begin inside it.  The range that reaches the last strip also owns the rows below it, which the reference never
+ * writes.  A range too short to be planned as an image of its own (the output-capacity rule of mcu.rs:198-209 refuses a last
+ * strip of a few rows on its own) starts at earlier strips; an image the strip rule cannot cut (ZJ_ERR_UNSUPPORTED there) is
+ * returned whole, *sub_row0 = row_begin. */
+ZJ_API int zj_image_rows(const zj_image *img, uint32_t row_begin, uint32_t row_end, zj_image *sub, uint32_t *sub_row0);
+/* The resize alone over width*height*nc interleaved u8 in device memory (width, height <= 65535; any alignment: no byte
+ * outside those width*height*nc is read): crop `roi` (NULL = the whole image) into the dst_dev slot.  Asynchronous on `stream`. */
+ZJ_API int zj_gpu_resize_device(int device, void *stream, const uint8_t *src_dev, uint32_t width, uint32_t height, uint32_t nc,
+                                const zj_roi *roi, const zj_output_desc *d, const zj_resize *r, void *dst_dev, size_t dst_len);
+/* Device coefficient planes in, one batch tensor out (out_len >= n slots).  Only the strips that hold rois[i]'s rows
+ * (zj_image_rows) are reconstructed, into a stream-ordered u8 scratch buffer, in sub-batches of at most ZJ_CONSUMER_CHUNK_MB
+ * megabytes as zj_gpu_reconstruct_device_ex does; rois = NULL: whole images.  Returns after `stream` has drained. */
+ZJ_API int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *imgs, size_t n, const zj_roi *rois,
+                                             const zj_output_desc *d, const zj_resize *r, void *out_dev, size_t out_len);
+
 /* Memory helpers so a non-CUDA host language can stage buffers without linking the CUDA runtime. */
 ZJ_API int zj_gpu_pinned_alloc(size_t bytes, void **p);
 ZJ_API int zj_gpu_pinned_free(void *p);
@@ -341,6 +377,13 @@ ZJ_API int zj_decode_batch_gpu_device(const zj_options *o, const uint8_t *const 
 ZJ_API int zj_decode_batch_gpu_device_ex(const zj_options *o, const uint8_t *const *bufs, const size_t *lens, size_t n,
                                          const zj_output_desc *d, void *const *out_dev, size_t *out_len, int *status,
                                          size_t *n_gpu_entropy);
+/* ... and cropped and resized into one batch tensor (zj_gpu_reconstruct_device_resized above; out_len >= n slots, the slot size
+ * from the OC that o->out_colorspace gives).  Whole images are decoded; statuses and zj_batch_error* are those of
+ * zj_decode_batch, and a decoded image whose roi does not fit it (known only after its headers) or whose OC differs gets
+ * ZJ_ERR_INVALID_ARG.  The slot of a failed image is left untouched.  rois = NULL: whole images. */
+ZJ_API int zj_decode_batch_gpu_device_resized(const zj_options *o, const uint8_t *const *bufs, const size_t *lens, size_t n,
+                                              const zj_roi *rois, const zj_output_desc *d, const zj_resize *r, void *out_dev,
+                                              size_t out_len, int *status, size_t *n_gpu_entropy);
 /* TEST-ONLY switches for three bugs of the reference's host stage that this library reproduces by default so that its
  * coefficient planes are the reference's (DESIGN.md section 2).  A cleared bit makes the cited lines behave like libjpeg:
  *   Q9  src/huffman.rs:249-252   fast-AC entry `(k << 10) + ...` is an i16: |k| >= 32 loses its top bits

@@ -5,15 +5,16 @@ from ._ffi import (  # noqa: F401
     VARIANT_SCALAR, VARIANT_X86, ZjComponent, ZjImage, ZjImageInfo, ZjOptions,
 )
 
-__all__ = ["Decoder", "ZuneJpegOptions", "JpegDecoder", "DecoderOptions", "ColorSpace", "DecodeErrors", "ImageInfo", "reconstruct", "decode_batch"]
+__all__ = ["Decoder", "ZuneJpegOptions", "JpegDecoder", "DecoderOptions", "ColorSpace", "DecodeErrors", "ImageInfo", "reconstruct", "decode_batch",
+           "decode_batch_resized", "Resize"]
 
 
 def __getattr__(name):  # lazy: importing the package must not require the built library
     if name in ("Decoder", "ZuneJpegOptions", "ColorSpace", "DecodeErrors", "ImageInfo", "UnsupportedSchemes", "decode_batch",
-                "JpegDecoder", "DecoderOptions"):
+                "decode_batch_resized", "JpegDecoder", "DecoderOptions"):
         from . import decoder as _d
         return getattr(_d, name)
-    if name in ("reconstruct", "Batch", "DeviceBuffer", "PinnedBuffer", "make_image"):
+    if name in ("reconstruct", "Batch", "DeviceBuffer", "PinnedBuffer", "make_image", "Resize"):
         from . import gpu as _g
         return getattr(_g, name)
     raise AttributeError(name)

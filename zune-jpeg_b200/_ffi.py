@@ -60,6 +60,17 @@ class ZjOutputDesc(C.Structure):
     ]
 
 
+FILTER_AREA, FILTER_BILINEAR = 0, 1
+
+
+class ZjRoi(C.Structure):
+    _fields_ = [("x", C.c_uint32), ("y", C.c_uint32), ("w", C.c_uint32), ("h", C.c_uint32)]
+
+
+class ZjResize(C.Structure):
+    _fields_ = [("out_w", C.c_uint32), ("out_h", C.c_uint32), ("filter", C.c_uint32), ("reserved", C.c_uint32)]
+
+
 class ZjOptions(C.Structure):
     _fields_ = [
         ("use_unsafe", C.c_uint32),
@@ -115,6 +126,15 @@ SYMBOLS = {
     "zj_gpu_reconstruct_device_ex": (C.c_int, [C.c_int, _P, C.POINTER(ZjImage), C.c_size_t, C.POINTER(ZjOutputDesc), _PP, C.POINTER(C.c_size_t)]),
     "zj_decode_batch_gpu_device_ex": (C.c_int, [C.POINTER(ZjOptions), C.POINTER(_P), C.POINTER(C.c_size_t), C.c_size_t, C.POINTER(ZjOutputDesc),
                                                 C.POINTER(_P), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_size_t)]),
+    "zj_resize_slot_size": (C.c_size_t, [C.POINTER(ZjOutputDesc), C.POINTER(ZjResize), C.c_uint32]),
+    "zj_image_rows": (C.c_int, [C.POINTER(ZjImage), C.c_uint32, C.c_uint32, C.POINTER(ZjImage), C.POINTER(C.c_uint32)]),
+    "zj_gpu_resize_device": (C.c_int, [C.c_int, _P, _P, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(ZjRoi), C.POINTER(ZjOutputDesc),
+                                       C.POINTER(ZjResize), _P, C.c_size_t]),
+    "zj_gpu_reconstruct_device_resized": (C.c_int, [C.c_int, _P, C.POINTER(ZjImage), C.c_size_t, C.POINTER(ZjRoi), C.POINTER(ZjOutputDesc),
+                                                    C.POINTER(ZjResize), _P, C.c_size_t]),
+    "zj_decode_batch_gpu_device_resized": (C.c_int, [C.POINTER(ZjOptions), C.POINTER(_P), C.POINTER(C.c_size_t), C.c_size_t, C.POINTER(ZjRoi),
+                                                     C.POINTER(ZjOutputDesc), C.POINTER(ZjResize), _P, C.c_size_t, C.POINTER(C.c_int),
+                                                     C.POINTER(C.c_size_t)]),
     "zj_gpu_pinned_alloc": (C.c_int, [C.c_size_t, _PP]),
     "zj_gpu_pinned_free": (C.c_int, [_P]),
     "zj_gpu_device_alloc": (C.c_int, [C.c_int, C.c_size_t, _PP]),

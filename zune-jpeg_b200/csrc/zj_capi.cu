@@ -10,6 +10,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <functional>
 #include <mutex>
 #include <new>
 #include <thread>
@@ -21,6 +22,7 @@
 namespace zj {
 cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream);
 cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
+cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
 }
 
 using namespace zj;
@@ -536,6 +538,46 @@ static size_t consumer_chunk_bytes()
     return v;
 }
 
+// Sub-batches of consecutive images whose u8 intermediates fit consumer_chunk_bytes() together (at least one image each)
+struct ConsumerChunk { size_t first, count, bytes; };
+// places image i's intermediate of `bytes` bytes in the last sub-batch or a new one; returns its offset in the scratch buffer
+static size_t chunk_place(std::vector<ConsumerChunk> &chunks, size_t i, size_t bytes)
+{
+    const size_t padded = (bytes + 255) & ~(size_t)255;
+    if (chunks.empty() || chunks.back().bytes + padded > consumer_chunk_bytes()) chunks.push_back({i, 0, 0});
+    const size_t off = chunks.back().bytes;
+    chunks.back().bytes += padded;
+    chunks.back().count++;
+    return off;
+}
+
+// Reconstructs the sub-batches one after the other into `scratch` (image i at u8_off[i], u8_size[i] bytes) on `s`, and after
+// each calls second_pass(chunk), which launches the kernels that read it.  Then waits for `s` and releases the plans.  Nothing
+// runs unless rc (the status so far) is ZJ_OK.
+static int reconstruct_chunks(int device, cudaStream_t s, const zj_image *imgs, const std::vector<ConsumerChunk> &chunks, uint8_t *scratch,
+                              const std::vector<size_t> &u8_off, const std::vector<size_t> &u8_size, int rc,
+                              const std::function<int(const ConsumerChunk &)> &second_pass)
+{
+    std::vector<zj_batch *> batches;
+    for (size_t c = 0; c < chunks.size() && rc == ZJ_OK; c++) {
+        const ConsumerChunk &ch = chunks[c];
+        std::vector<uint8_t *> outs(ch.count);
+        std::vector<size_t> lens(ch.count);
+        for (size_t k = 0; k < ch.count; k++) { outs[k] = scratch + u8_off[ch.first + k]; lens[k] = u8_size[ch.first + k]; }
+        zj_batch *b = nullptr;
+        rc = batch_create_impl(device, imgs + ch.first, ch.count, outs.data(), lens.data(), &b, true, s);
+        if (rc) break;
+        batches.push_back(b);
+        rc = zj_batch_run(b, s);
+        if (rc == ZJ_OK) rc = second_pass(ch);
+    }
+    // the descriptor arrays and the scratch must outlive the kernels
+    cudaError_t e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess && rc == ZJ_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
+    for (zj_batch *b : batches) zj_batch_destroy(b);
+    return rc;
+}
+
 int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs, size_t n, const zj_output_desc *d,
                                  void *const *out_dev, const size_t *out_len)
 {
@@ -549,8 +591,7 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
     // geometry, sizes, sub-batches of consecutive images
     std::vector<ConvImage> conv(n);
     std::vector<size_t> u8_size(n), u8_off(n);
-    struct Chunk { size_t first, count, bytes; };
-    std::vector<Chunk> chunks;
+    std::vector<ConsumerChunk> chunks;
     size_t scratch_bytes = 0;
     for (size_t i = 0; i < n; i++) {
         u8_size[i] = zj_output_size(&imgs[i]);
@@ -562,11 +603,7 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
         if (!out_dev[i]) return ZJ_ERR_INVALID_ARG;
         if (out_len[i] < (size_t)ci.ow * ci.oh * ci.oc * dtype_size(d->dtype)) return ZJ_ERR_SHORT_OUTPUT;
         ci.dst = out_dev[i];
-        const size_t padded = (u8_size[i] + 255) & ~(size_t)255;
-        if (chunks.empty() || chunks.back().bytes + padded > consumer_chunk_bytes()) chunks.push_back({i, 0, 0});
-        u8_off[i] = chunks.back().bytes;
-        chunks.back().bytes += padded;
-        chunks.back().count++;
+        u8_off[i] = chunk_place(chunks, i, u8_size[i]);
         scratch_bytes = std::max(scratch_bytes, chunks.back().bytes);
     }
     if (n == 0) return ZJ_OK;
@@ -577,20 +614,10 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
     if (e != cudaSuccess) { cudaFreeAsync(scratch, s); return cuda_fail(e, "cudaMallocAsync(consumer descriptors)"); }
     for (size_t i = 0; i < n; i++) conv[i].src = scratch + u8_off[i];
     e = cudaMemcpyAsync(d_conv, conv.data(), n * sizeof(ConvImage), cudaMemcpyHostToDevice, s);
-    std::vector<zj_batch *> batches;
     if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(consumer descriptors)");
-    for (size_t c = 0; c < chunks.size() && rc == ZJ_OK; c++) {
-        const Chunk &ch = chunks[c];
-        std::vector<uint8_t *> outs(ch.count);
-        std::vector<size_t> lens(ch.count);
-        for (size_t k = 0; k < ch.count; k++) { outs[k] = scratch + u8_off[ch.first + k]; lens[k] = u8_size[ch.first + k]; }
-        zj_batch *b = nullptr;
-        rc = batch_create_impl(device, imgs + ch.first, ch.count, outs.data(), lens.data(), &b, true, s);
-        if (rc) break;
-        batches.push_back(b);
-        rc = zj_batch_run(b, s);
+    rc = reconstruct_chunks(device, s, imgs, chunks, scratch, u8_off, u8_size, rc, [&](const ConsumerChunk &ch) {
         // one consumer launch per run of images with the same number of source bytes per pixel
-        for (size_t k = 0; k < ch.count && rc == ZJ_OK;) {
+        for (size_t k = 0; k < ch.count;) {
             size_t k1 = k;
             uint32_t mw = 0, mh = 0;
             while (k1 < ch.count && conv[ch.first + k1].nc == conv[ch.first + k].nc) {
@@ -598,19 +625,193 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
                 k1++;
             }
             if (mw && mh) {
-                e = launch_convert(d_conv + ch.first + k, (uint32_t)(k1 - k), conv[ch.first + k].nc, mw, mh, *d, s);
+                cudaError_t le = launch_convert(d_conv + ch.first + k, (uint32_t)(k1 - k), conv[ch.first + k].nc, mw, mh, *d, s);
                 g_launches.fetch_add(1);
-                if (e != cudaSuccess) rc = cuda_fail(e, "consumer launch");
+                if (le != cudaSuccess) return cuda_fail(le, "consumer launch");
             }
             k = k1;
         }
-    }
-    // the descriptor arrays and the scratch must outlive the kernels
-    e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess && rc == ZJ_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-    for (zj_batch *b : batches) zj_batch_destroy(b);
+        return (int)ZJ_OK;
+    });
     cudaFreeAsync(d_conv, s);
     cudaFreeAsync(scratch, s);
+    return rc;
+}
+
+// ------------------------------------------------------------------------------------- cropped, resized batch tensors
+static int resize_check(const zj_output_desc *d, const zj_resize *r)
+{
+    int rc = desc_check(d);
+    if (rc) return rc;
+    // (sizes up to 65535, as for images: the kernels' window products fit 32 bits)
+    if (d->scale_log2 != 0 || !r || r->out_w == 0 || r->out_h == 0 || r->out_w > 65535 || r->out_h > 65535 || r->filter > ZJ_FILTER_BILINEAR ||
+        r->reserved != 0)
+        return ZJ_ERR_INVALID_ARG;
+    return ZJ_OK;
+}
+
+static uint32_t resize_oc(const zj_output_desc *d, uint32_t nc) { return (d->channels == 3 && nc == 4) ? 3u : nc; }
+
+size_t zj_resize_slot_size(const zj_output_desc *d, const zj_resize *r, uint32_t nc)
+{
+    if (resize_check(d, r) != ZJ_OK || (nc != 1 && nc != 3 && nc != 4)) return 0;
+    return (size_t)r->out_w * r->out_h * resize_oc(d, nc) * dtype_size(d->dtype);
+}
+
+// *out = the crop of a width x height image that `roi` names (NULL = the whole image)
+static int roi_resolve(const zj_roi *roi, uint32_t width, uint32_t height, zj_roi *out)
+{
+    if (!roi) { *out = {0, 0, width, height}; return ZJ_OK; }
+    if (roi->w == 0 || roi->h == 0 || (uint64_t)roi->x + roi->w > width || (uint64_t)roi->y + roi->h > height) return ZJ_ERR_INVALID_ARG;
+    *out = *roi;
+    return ZJ_OK;
+}
+
+// src: the width x height (rows of it) u8 image the crop lies in, from its row `row0` on
+static ResizeImage resize_image(const uint8_t *src, uint32_t width, uint32_t height, uint32_t nc, uint32_t row0, const zj_roi &roi, void *dst,
+                                const zj_resize &r)
+{
+    ResizeImage ri{};
+    ri.pitch = width * nc;
+    ri.lo = src;
+    ri.hi = src + (size_t)height * ri.pitch;
+    ri.src = src + (size_t)row0 * ri.pitch + (size_t)roi.x * nc;
+    ri.dst = dst;
+    ri.w = roi.w; ri.h = roi.h;
+    ri.sx = (float)roi.w / (float)r.out_w;   // IEEE single-precision division, as the kernel's other operations
+    ri.sy = (float)roi.h / (float)r.out_h;
+    return ri;
+}
+
+// one resize launch per run of at most 65535 images with the same nc (d_ri / ri: the same descriptors on the device / host)
+static int launch_resize_runs(const ResizeImage *d_ri, const uint32_t *nc, size_t n, const zj_output_desc &d, const zj_resize &r, cudaStream_t s)
+{
+    for (size_t k = 0; k < n;) {
+        size_t k1 = k;
+        while (k1 < n && nc[k1] == nc[k] && k1 - k < 65535) k1++;
+        const cudaError_t e = launch_resize(d_ri + k, (uint32_t)(k1 - k), nc[k], d, r, s);
+        g_launches.fetch_add(1);
+        if (e != cudaSuccess) return cuda_fail(e, "resize launch");
+        k = k1;
+    }
+    return ZJ_OK;
+}
+
+int zj_image_rows(const zj_image *img, uint32_t row_begin, uint32_t row_end, zj_image *sub, uint32_t *sub_row0)
+{
+    Plan pl;
+    int rc = plan_image(img, &pl);
+    if (rc) return rc;
+    if (!sub || !sub_row0 || row_begin >= row_end || row_end > img->height) return ZJ_ERR_INVALID_ARG;
+    // strips [s0, s1): the strips the rows fall in; rows at or below the last strip belong to the range that ends with it
+    const uint32_t ns = pl.n_strips;
+    const uint32_t s0 = ns ? std::min(row_begin / pl.rows, ns - 1) : 0;
+    const uint32_t s1 = ns ? std::min((row_end + pl.rows - 1) / pl.rows, ns) : 0;
+    // A virtual image is planned like any image, so the output-capacity rule (mcu.rs:198-209) applies to it on its own: a short
+    // range at the bottom (one row of a last strip) can be refused where the whole image is not.  Such a range starts at earlier
+    // strips instead; an image that cannot be cut at all (ZJ_ERR_UNSUPPORTED) is returned whole.
+    for (uint32_t b = s0;; b--) {
+        rc = zj_image_strip_range(img, b, s1, sub, nullptr, nullptr, nullptr);
+        if (rc == ZJ_OK) { *sub_row0 = row_begin - b * pl.rows; return ZJ_OK; }
+        if (rc == ZJ_ERR_UNSUPPORTED || (rc == ZJ_ERR_REF_PANIC && b == 0)) break;
+        if (rc != ZJ_ERR_REF_PANIC) return rc;
+    }
+    *sub = *img;
+    *sub_row0 = row_begin;
+    return ZJ_OK;
+}
+
+int zj_gpu_resize_device(int device, void *stream, const uint8_t *src_dev, uint32_t width, uint32_t height, uint32_t nc, const zj_roi *roi,
+                         const zj_output_desc *d, const zj_resize *r, void *dst_dev, size_t dst_len)
+{
+    const size_t slot = zj_resize_slot_size(d, r, nc);
+    if (slot == 0 || width == 0 || height == 0 || width > 65535 || height > 65535 || !src_dev || !dst_dev) return ZJ_ERR_INVALID_ARG;
+    zj_roi crop;
+    int rc = roi_resolve(roi, width, height, &crop);
+    if (rc) return rc;
+    if (dst_len < slot) return ZJ_ERR_SHORT_OUTPUT;
+    rc = set_device(device);
+    if (rc) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const ResizeImage ri = resize_image(src_dev, width, height, nc, crop.y, crop, dst_dev, *r);
+    ResizeImage *d_ri = nullptr;
+    CU(pool_alloc((void **)&d_ri, sizeof(ri), device, s));
+    cudaError_t e = cudaMemcpyAsync(d_ri, &ri, sizeof(ri), cudaMemcpyHostToDevice, s);   // (pageable source: staged before the call returns)
+    rc = e == cudaSuccess ? launch_resize_runs(d_ri, &nc, 1, *d, *r, s) : cuda_fail(e, "cudaMemcpyAsync(resize descriptor)");
+    cudaFreeAsync(d_ri, s);
+    return rc;
+}
+
+int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *imgs, size_t n, const zj_roi *rois, const zj_output_desc *d,
+                                      const zj_resize *r, void *out_dev, size_t out_len)
+{
+    int rc = resize_check(d, r);
+    if (rc) return rc;
+    if ((!imgs || !out_dev) && n) return ZJ_ERR_INVALID_ARG;
+    // per image: the crop, the strips that hold its rows, where their u8 pixels go in the scratch buffer
+    std::vector<zj_image> subs(n);
+    std::vector<zj_roi> crops(n);
+    std::vector<uint32_t> row0(n), nc(n);
+    std::vector<size_t> u8_size(n), u8_off(n);
+    std::vector<ConsumerChunk> chunks;
+    size_t scratch_bytes = 0;
+    for (size_t i = 0; i < n; i++) {
+        if (zj_output_size(&imgs[i]) == 0) { rc = zj_validate_image(&imgs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
+        nc[i] = (uint32_t)num_components(imgs[i].out_cs);
+        if (resize_oc(d, nc[i]) != resize_oc(d, nc[0])) return ZJ_ERR_INVALID_ARG;   // one tensor: one channel count
+        rc = roi_resolve(rois ? &rois[i] : nullptr, imgs[i].width, imgs[i].height, &crops[i]);
+        if (rc) return rc;
+        rc = zj_image_rows(&imgs[i], crops[i].y, crops[i].y + crops[i].h, &subs[i], &row0[i]);
+        if (rc) return rc;
+        u8_size[i] = zj_output_size(&subs[i]);
+        if (u8_size[i] == 0) { rc = zj_validate_image(&subs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
+        u8_off[i] = chunk_place(chunks, i, u8_size[i]);
+        scratch_bytes = std::max(scratch_bytes, chunks.back().bytes);
+    }
+    const size_t slot = n ? zj_resize_slot_size(d, r, nc[0]) : 0;
+    if (n && out_len / slot < n) return ZJ_ERR_SHORT_OUTPUT;
+    rc = set_device(device);
+    if (rc) return rc;
+    if (n == 0) return ZJ_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    uint8_t *scratch = nullptr;
+    ResizeImage *d_ri = nullptr;
+    CU(pool_alloc((void **)&scratch, scratch_bytes, device, s));
+    cudaError_t e = pool_alloc((void **)&d_ri, n * sizeof(ResizeImage), device, s);
+    if (e != cudaSuccess) { cudaFreeAsync(scratch, s); return cuda_fail(e, "cudaMallocAsync(resize descriptors)"); }
+    std::vector<ResizeImage> ri(n);
+    for (size_t i = 0; i < n; i++)
+        ri[i] = resize_image(scratch + u8_off[i], imgs[i].width, subs[i].height, nc[i], row0[i], crops[i], static_cast<uint8_t *>(out_dev) + i * slot, *r);
+    e = cudaMemcpyAsync(d_ri, ri.data(), n * sizeof(ResizeImage), cudaMemcpyHostToDevice, s);
+    if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(resize descriptors)");
+    rc = reconstruct_chunks(device, s, subs.data(), chunks, scratch, u8_off, u8_size, rc, [&](const ConsumerChunk &ch) {
+        return launch_resize_runs(d_ri + ch.first, nc.data() + ch.first, ch.count, *d, *r, s);
+    });
+    cudaFreeAsync(d_ri, s);
+    cudaFreeAsync(scratch, s);
+    return rc;
+}
+
+// Hidden helper for zj_decode_batch_gpu_device_resized (zj_host_decoder.cpp): the resize over decoded u8 images already in
+// device memory, image i into slot dst_slot[i] of out_dev; the arguments were checked by the caller.
+extern "C" int zj_capi_resize_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
+                                   const zj_roi *crops,
+                                   const size_t *dst_slot, size_t n, const zj_output_desc *d, const zj_resize *r, void *out_dev)
+{
+    int rc = resize_check(d, r);
+    if (rc) return rc;
+    rc = set_device(device);
+    if (rc) return rc;
+    if (n == 0) return ZJ_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t slot = zj_resize_slot_size(d, r, nc[0]);
+    std::vector<ResizeImage> ri(n);
+    for (size_t i = 0; i < n; i++) ri[i] = resize_image(src[i], w[i], h[i], nc[i], crops[i].y, crops[i], static_cast<uint8_t *>(out_dev) + dst_slot[i] * slot, *r);
+    ResizeImage *d_ri = nullptr;
+    CU(pool_alloc((void **)&d_ri, n * sizeof(ResizeImage), device, s));
+    cudaError_t e = cudaMemcpyAsync(d_ri, ri.data(), n * sizeof(ResizeImage), cudaMemcpyHostToDevice, s);   // (pageable: staged before the call returns)
+    rc = e == cudaSuccess ? launch_resize_runs(d_ri, nc, n, *d, *r, s) : cuda_fail(e, "cudaMemcpyAsync(resize descriptors)");
+    cudaFreeAsync(d_ri, s);
     return rc;
 }
 

@@ -190,4 +190,279 @@ cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t n
     }
 }
 
+// ------------------------------------------------------------------------------------------------------ resize
+// A crop of each image's u8 pixels resized to one out_w x out_h slot of a batch tensor (zj_gpu_resize_device and the
+// *_resized entry points; the specification is the header's, DESIGN.md section 4.5.1).  Every value is a function of the u8
+// bytes of the crop alone: neighbours are clamped to the crop and pixels outside it never contribute.
+//   ZJ_FILTER_AREA      output row i covers crop rows [floor(i*h/OH), ceil((i+1)*h/OH)), columns alike; s = exact sum of the
+//                       window's bytes, n = its pixel count; u8 = (s + n/2) / n, float = float(s) / float(n)
+//   ZJ_FILTER_BILINEAR  torch interpolate(bilinear, align_corners=False, antialias=False) in the stated fp32 order;
+//                       u8 = round-to-nearest-even of the value, clamped to [0, 255]
+// then (v - mean[c]) * inv_std[c] for floats, every fp32 operation a single IEEE round-to-nearest one (no FMA).
+
+struct ResizeParams {
+    float mean[4], inv_std[4];
+    uint32_t ow, oh;
+};
+
+constexpr int RZ_ROWS = 8;   // output rows per CTA: one warp each (256 threads)
+
+template <typename T> __device__ __forceinline__ u32 to_bits(T v);
+template <> __device__ __forceinline__ u32 to_bits<uint8_t>(uint8_t v) { return v; }
+template <> __device__ __forceinline__ u32 to_bits<__half>(__half v) { return __half_as_ushort(v); }
+template <> __device__ __forceinline__ u32 to_bits<float>(float v) { return __float_as_uint(v); }
+template <typename T> __device__ __forceinline__ T from_bits(u32 b);
+template <> __device__ __forceinline__ uint8_t from_bits<uint8_t>(u32 b) { return (uint8_t)b; }
+template <> __device__ __forceinline__ __half from_bits<__half>(u32 b) { return __ushort_as_half((unsigned short)b); }
+template <> __device__ __forceinline__ float from_bits<float>(u32 b) { return __uint_as_float(b); }
+
+// 8 consecutive output pixels (n valid) of output row y, all OC channels, into the slot: per plane (CHW) or as 8 * OC
+// interleaved elements (HWC); 16-byte stores where the address allows them (store8)
+template <typename T, bool CHW, int OC>
+__device__ __forceinline__ void store_px8(T *dst, const ResizeParams &prm, u32 y, u32 x0, int n, const T (&v)[8][OC])
+{
+    if (CHW) {
+        const size_t plane = (size_t)prm.ow * prm.oh;
+#pragma unroll
+        for (int c = 0; c < OC; c++) {
+            T u[8];
+#pragma unroll
+            for (int e = 0; e < 8; e++) u[e] = v[e][c];
+            T *q = dst + (size_t)c * plane + (size_t)y * prm.ow + x0;
+            store8<T>(q, u, n, (reinterpret_cast<uintptr_t>(q) & 15) == 0);
+        }
+    } else {
+        T *q = dst + ((size_t)y * prm.ow + x0) * OC;
+        const bool vec = (reinterpret_cast<uintptr_t>(q) & 15) == 0 && n == 8;
+#pragma unroll
+        for (int g = 0; g < OC; g++) {
+            T u[8];
+#pragma unroll
+            for (int e = 0; e < 8; e++) u[e] = v[(8 * g + e) / OC][(8 * g + e) % OC];
+            const int left = n * OC - 8 * g;
+            if (left <= 0) break;
+            store8<T>(q + 8 * g, u, left < 8 ? left : 8, vec);
+        }
+    }
+}
+
+template <typename T> __device__ __forceinline__ T normalise(float v, float mean, float inv_std)
+{
+    return cvt<T>(__fmul_rn(__fsub_rn(v, mean), inv_std));
+}
+
+// dp4a mask of the bytes of channel c in a word whose byte 0 belongs to channel ph
+template <int NC> __device__ __forceinline__ u32 chan_mask(int ph, int c)
+{
+    if (NC == 1) return 0x01010101u;
+    int k = c - ph;
+    if (k < 0) k += NC;
+    if (NC == 4) return 1u << (8 * k);
+    return k == 0 ? 0x01000001u : 1u << (8 * k);   // NC == 3: bytes k and k + 3
+}
+
+// (s + n/2) / n for s <= 255 * n, without a 64-bit division: a float estimate (off by less than 0.001) corrected by one step
+__device__ __forceinline__ u32 div_round(uint64_t s, u32 n)
+{
+    const uint64_t t = s + n / 2;
+    u32 q = (u32)__fdividef(__ull2float_rn(t), __uint2float_rn(n));
+    if ((uint64_t)q * n > t) q--;
+    else if ((uint64_t)(q + 1) * n <= t) q++;
+    return q;
+}
+
+// Sums the bytes [b, e) of one window row per channel into acc: the aligned words from a = b & ~3 on, one dp4a per word and
+// channel against m[c] (the channel's bytes of the word) and keep (the bytes inside [b, e)).  INSIDE: every word lies in the source
+// image; otherwise a word that does not is assembled from the window's bytes by byte loads, so no load leaves the image.
+template <int NC, int OC, bool INSIDE>
+__device__ __forceinline__ void area_span(uintptr_t a, const uintptr_t b, const uintptr_t e, u32 (&m)[OC], u32 (&acc)[OC])
+{
+    for (; a < e; a += 4) {
+        u32 keep = 0xffffffffu;
+        if (a < b) keep = 0xffffffffu << (8 * (u32)(b - a));
+        if (a + 4 > e) keep &= 0xffffffffu >> (8 * (u32)(a + 4 - e));
+        u32 wd;
+        if (INSIDE || (a >= b && a + 4 <= e)) wd = __ldg(reinterpret_cast<const u32 *>(a));
+        else {
+            wd = 0;
+#pragma unroll
+            for (int k = 0; k < 4; k++)
+                if (a + k >= b && a + k < e) wd |= (u32)__ldg(reinterpret_cast<const uint8_t *>(a + k)) << (8 * k);
+        }
+#pragma unroll
+        for (int c = 0; c < OC; c++) acc[c] = __dp4a(wd, m[c] & keep, acc[c]);
+        if (NC == 3) {   // the next word starts one channel later
+            u32 t[OC];
+#pragma unroll
+            for (int c = 0; c < OC; c++) t[c] = m[c];
+#pragma unroll
+            for (int c = 0; c < OC; c++) m[c] = t[(c + 2) % 3];
+        }
+    }
+}
+
+// ZJ_FILTER_AREA.  A warp owns 32 consecutive output columns of one output row, a lane one column: in every source row of the
+// window the warp reads one contiguous span, each lane its own window's bytes as the aligned 32-bit words that hold them, summed
+// per channel by one dp4a against a byte mask (bytes outside the window or of another channel weigh 0).  No load reaches outside
+// the source image: the one or two words that would are read byte by byte.  Groups of 8 lanes then hand their values to one
+// lane, which stores 8 pixels.
+template <typename T, bool CHW, int NC, int OC>
+__global__ void __launch_bounds__(256) resize_area_kernel(const ResizeImage *__restrict__ images, const ResizeParams prm)
+{
+    const ResizeImage im = images[blockIdx.z];
+    const u32 lane = threadIdx.x & 31;
+    const u32 i = blockIdx.y * RZ_ROWS + (threadIdx.x >> 5);
+    if (i >= prm.oh) return;   // (warp-uniform: the shuffles below see every lane of a warp that gets there)
+    const u32 j = blockIdx.x * 32u + lane;
+    const bool live = j < prm.ow;
+    // (crop and output sizes are at most 65535: the products fit 32 bits)
+    const u32 r0 = i * im.h / prm.oh, r1 = ((i + 1) * im.h + prm.oh - 1) / prm.oh;
+    const u32 c0 = live ? j * im.w / prm.ow : 0u;
+    const u32 c1 = live ? ((j + 1) * im.w + prm.ow - 1) / prm.ow : 0u;
+    uint64_t sum[OC];
+#pragma unroll
+    for (int c = 0; c < OC; c++) sum[c] = 0;
+    const uintptr_t lo = reinterpret_cast<uintptr_t>(im.lo), hi = reinterpret_cast<uintptr_t>(im.hi);
+    const uint8_t *row = im.src + (size_t)r0 * im.pitch;
+    for (u32 r = r0; r < r1; r++, row += im.pitch) {
+        const uintptr_t b = reinterpret_cast<uintptr_t>(row) + (size_t)c0 * NC, e = reinterpret_cast<uintptr_t>(row) + (size_t)c1 * NC;
+        uintptr_t a = b & ~(uintptr_t)3;
+        // channel of the first word's byte 0 (the crop starts on a pixel)
+        const int ph = (int)(((long long)c0 * NC - (long long)(b - a)) % NC + NC) % NC;
+        u32 m[OC];
+#pragma unroll
+        for (int c = 0; c < OC; c++) m[c] = chan_mask<NC>(ph, c);
+        u32 acc[OC];
+#pragma unroll
+        for (int c = 0; c < OC; c++) acc[c] = 0;
+        // every aligned word of the span lies inside the source image (all rows but the image's first and last, at most)
+        if (a >= lo && ((e + 3) & ~(uintptr_t)3) <= hi) area_span<NC, OC, true>(a, b, e, m, acc);
+        else area_span<NC, OC, false>(a, b, e, m, acc);
+#pragma unroll
+        for (int c = 0; c < OC; c++) sum[c] += acc[c];
+    }
+    const u32 n = (r1 - r0) * (c1 - c0);
+    u32 bits[OC];
+#pragma unroll
+    for (int c = 0; c < OC; c++) {
+        if (!live) bits[c] = 0;
+        else if (sizeof(T) == 1) bits[c] = div_round(sum[c], n);
+        else bits[c] = to_bits<T>(normalise<T>(__fdiv_rn(__ull2float_rn(sum[c]), __uint2float_rn(n)), prm.mean[c], prm.inv_std[c]));
+    }
+    T v[8][OC];
+    if (sizeof(T) == 1) {   // u8: the OC channels of a pixel travel in one word
+        u32 packed = 0;
+#pragma unroll
+        for (int c = 0; c < OC; c++) packed |= bits[c] << (8 * c);
+#pragma unroll
+        for (int k = 0; k < 8; k++) {
+            const u32 p = __shfl_sync(0xffffffffu, packed, (lane & ~7u) + k);
+#pragma unroll
+            for (int c = 0; c < OC; c++) v[k][c] = from_bits<T>((p >> (8 * c)) & 0xffu);
+        }
+    } else {
+#pragma unroll
+        for (int k = 0; k < 8; k++)
+#pragma unroll
+            for (int c = 0; c < OC; c++) v[k][c] = from_bits<T>(__shfl_sync(0xffffffffu, bits[c], (lane & ~7u) + k));
+    }
+    const u32 x0 = j;   // for the storing lanes (lane % 8 == 0)
+    if ((lane & 7) == 0 && x0 < prm.ow)
+        store_px8<T, CHW, OC>(reinterpret_cast<T *>(im.dst), prm, i, x0, (int)min(8u, prm.ow - x0), v);
+}
+
+// source index, weights of output index j (crop size n_in, scale s = float(n_in) / float(n_out)) -- the exact fp32 sequence
+// of the specification
+__device__ __forceinline__ void bilinear_coord(u32 j, u32 n_in, float s, int &i0, float &a, float &b)
+{
+    float f = __fsub_rn(__fmul_rn(__fadd_rn(__uint2float_rn(j), 0.5f), s), 0.5f);
+    if (f < 0.0f) f = 0.0f;
+    i0 = min((int)f, (int)n_in - 1);
+    a = __fsub_rn(f, (float)i0);
+    b = __fsub_rn(1.0f, a);
+}
+
+// ZJ_FILTER_BILINEAR.  A CTA covers 256 output columns x 8 output rows of one image; their coordinate tables are built once in
+// shared memory.  A thread produces 8 consecutive output pixels of a row: four byte loads per pixel and channel.
+template <typename T, bool CHW, int NC, int OC>
+__global__ void __launch_bounds__(256) resize_bilinear_kernel(const ResizeImage *__restrict__ images, const ResizeParams prm)
+{
+    __shared__ int s_c0[256];
+    __shared__ float s_ax[256], s_bx[256];
+    __shared__ int s_r0[RZ_ROWS];
+    __shared__ float s_ay[RZ_ROWS], s_by[RZ_ROWS];
+    const ResizeImage im = images[blockIdx.z];
+    const u32 jt = blockIdx.x * 256u, it = blockIdx.y * RZ_ROWS;
+    const u32 t = threadIdx.x;
+    if (jt + t < prm.ow) bilinear_coord(jt + t, im.w, im.sx, s_c0[t], s_ax[t], s_bx[t]);
+    if (t < RZ_ROWS && it + t < prm.oh) bilinear_coord(it + t, im.h, im.sy, s_r0[t], s_ay[t], s_by[t]);
+    __syncthreads();
+    const u32 ly = t >> 5, xl = 8u * (t & 31);
+    const u32 y = it + ly, x0 = jt + xl;
+    if (y >= prm.oh || x0 >= prm.ow) return;
+    const int n = (int)min(8u, prm.ow - x0);
+    const int r0 = s_r0[ly], r1 = min(r0 + 1, (int)im.h - 1);
+    const float ay = s_ay[ly], by = s_by[ly];
+    const uint8_t *p0 = im.src + (size_t)r0 * im.pitch, *p1 = im.src + (size_t)r1 * im.pitch;
+    T v[8][OC];
+#pragma unroll
+    for (int e = 0; e < 8; e++) {
+        const int k = xl + min(e, n - 1);   // (columns past the row's end repeat the last one; they are not stored)
+        const int c0 = s_c0[k], c1 = min(c0 + 1, (int)im.w - 1);
+        const float ax = s_ax[k], bx = s_bx[k];
+#pragma unroll
+        for (int c = 0; c < OC; c++) {
+            const float p00 = __ldg(p0 + c0 * NC + c), p01 = __ldg(p0 + c1 * NC + c);
+            const float p10 = __ldg(p1 + c0 * NC + c), p11 = __ldg(p1 + c1 * NC + c);
+            const float top = __fadd_rn(__fmul_rn(bx, p00), __fmul_rn(ax, p01));
+            const float bot = __fadd_rn(__fmul_rn(bx, p10), __fmul_rn(ax, p11));
+            const float val = __fadd_rn(__fmul_rn(by, top), __fmul_rn(ay, bot));
+            if (sizeof(T) == 1) v[e][c] = (T)min(max(__float2int_rn(val), 0), 255);
+            else v[e][c] = normalise<T>(val, prm.mean[c], prm.inv_std[c]);
+        }
+    }
+    store_px8<T, CHW, OC>(reinterpret_cast<T *>(im.dst), prm, y, x0, n, v);
+}
+
+template <typename T, bool CHW, int NC, int OC>
+static void launch_resize_k(const ResizeImage *d_images, uint32_t count, bool area, const ResizeParams &prm, cudaStream_t s)
+{
+    const uint32_t gy = (prm.oh + RZ_ROWS - 1) / RZ_ROWS;
+    if (area) resize_area_kernel<T, CHW, NC, OC><<<dim3((prm.ow + 31) / 32, gy, count), 256, 0, s>>>(d_images, prm);
+    else resize_bilinear_kernel<T, CHW, NC, OC><<<dim3((prm.ow + 255) / 256, gy, count), 256, 0, s>>>(d_images, prm);
+}
+
+template <typename T, bool CHW>
+static void launch_resize_nc(const ResizeImage *d_images, uint32_t count, uint32_t nc, uint32_t oc, bool area, const ResizeParams &prm, cudaStream_t s)
+{
+    if (nc == 1) launch_resize_k<T, CHW, 1, 1>(d_images, count, area, prm, s);
+    else if (nc == 3) launch_resize_k<T, CHW, 3, 3>(d_images, count, area, prm, s);
+    else if (oc == 3) launch_resize_k<T, CHW, 4, 3>(d_images, count, area, prm, s);
+    else launch_resize_k<T, CHW, 4, 4>(d_images, count, area, prm, s);
+}
+
+template <typename T>
+static void launch_resize_t(const ResizeImage *d_images, uint32_t count, uint32_t nc, uint32_t oc, bool chw, bool area, const ResizeParams &prm, cudaStream_t s)
+{
+    if (chw) launch_resize_nc<T, true>(d_images, count, nc, oc, area, prm, s);
+    else launch_resize_nc<T, false>(d_images, count, nc, oc, area, prm, s);
+}
+
+// images [0, count) of d_images (count <= 65535) share nc; the descriptors were checked by the caller
+cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s)
+{
+    ResizeParams prm;
+    for (int c = 0; c < 4; c++) { prm.mean[c] = d.mean[c]; prm.inv_std[c] = d.inv_std[c]; }
+    prm.ow = r.out_w;
+    prm.oh = r.out_h;
+    const bool chw = d.layout == ZJ_LAYOUT_CHW, area = r.filter == ZJ_FILTER_AREA;
+    const uint32_t oc = (d.channels == 3 && nc == 4) ? 3u : nc;
+    switch (d.dtype) {
+    case ZJ_DTYPE_U8: launch_resize_t<uint8_t>(d_images, count, nc, oc, chw, area, prm, s); break;
+    case ZJ_DTYPE_F16: launch_resize_t<__half>(d_images, count, nc, oc, chw, area, prm, s); break;
+    default: launch_resize_t<float>(d_images, count, nc, oc, chw, area, prm, s); break;
+    }
+    return cudaGetLastError();
+}
+
 }  // namespace zj

@@ -78,4 +78,15 @@ struct ConvImage {
     uint32_t ow, oh, oc;          // output geometry (oc = channels written)
 };
 
+// One image of a resize launch (zj_consumer.cu): a crop of interleaved u8 pixels in, one slot of the batch tensor out.  The
+// output size, layout, type and channels are the launch's.
+struct ResizeImage {
+    const uint8_t *src;           // byte 0 of the crop's pixel (0, 0)
+    const uint8_t *lo, *hi;       // the source image's bytes: no load reaches outside [lo, hi)
+    void *dst;                    // the image's slot
+    uint32_t pitch;               // bytes per source row (width * nc)
+    uint32_t w, h;                // crop size in pixels
+    float sx, sy;                 // bilinear scales float(w) / float(out_w), float(h) / float(out_h) (one IEEE division each)
+};
+
 }  // namespace zj

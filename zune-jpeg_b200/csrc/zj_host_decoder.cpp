@@ -1828,6 +1828,9 @@ extern "C" void zj_capi_release_stream_caches(void);   // zj_capi.cu (hidden)
 extern "C" void zj_capi_trim_pools(void);
 extern "C" int zj_capi_pool_alloc(void **p, size_t bytes, int device, void *stream);
 extern "C" void zj_capi_pool_free(void *p, void *stream);
+extern "C" int zj_capi_resize_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
+                                   const zj_roi *crops,
+                                   const size_t *dst_slot, size_t n, const zj_output_desc *d, const zj_resize *r, void *out_dev);
 extern "C" int zj_capi_convert_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
                                     void *const *dst, size_t n, const zj_output_desc *d);
 
@@ -2242,6 +2245,77 @@ ZJ_API int zj_decode_batch_gpu_device_ex(const zj_options *o, const uint8_t *con
             csrc.push_back(mid[i]); cdst.push_back(out_dev[i]); cw.push_back(g.w); ch.push_back(g.h); cnc.push_back(g.nc);
         }
         int crc = zj_capi_convert_many(opt.device, nullptr, csrc.data(), cw.data(), ch.data(), cnc.data(), cdst.data(), csrc.size(), d);
+        if (crc == ZJ_OK && cudaStreamSynchronize(nullptr) != cudaSuccess) { cudaGetLastError(); crc = ZJ_ERR_CUDA; }
+        if (crc != ZJ_OK) failed = crc;
+    }
+    zj_capi_pool_free(scratch, nullptr);
+    return failed;
+}
+
+// The batch-tensor call: whole images decoded into a stream-ordered u8 scratch buffer (as zj_decode_batch_gpu_device_ex does),
+// then each decoded image's crop resized into its slot (zj_consumer.cu).
+ZJ_API int zj_decode_batch_gpu_device_resized(const zj_options *o, const uint8_t *const *bufs, const size_t *lens, size_t n,
+                                              const zj_roi *rois, const zj_output_desc *d, const zj_resize *r, void *out_dev,
+                                              size_t out_len, int *status, size_t *n_gpu_entropy)
+{
+    if ((!bufs || !lens || !out_dev || !status) && n) return ZJ_ERR_INVALID_ARG;
+    zj_options opt;
+    if (o) opt = *o; else zj_options_default(&opt);
+    // every slot has the channel count the options' colourspace gives
+    const uint32_t cs_opt = opt.out_colorspace;
+    if (cs_opt > ZJ_CS_RGBX) return ZJ_ERR_INVALID_ARG;
+    const uint32_t nc_opt = cs_opt == ZJ_CS_GRAYSCALE ? 1u : ((cs_opt == ZJ_CS_RGB || cs_opt == ZJ_CS_YCBCR) ? 3u : 4u);
+    const size_t slot = zj_resize_slot_size(d, r, nc_opt);
+    if (slot == 0) return ZJ_ERR_INVALID_ARG;
+    if (n && out_len / slot < n) return ZJ_ERR_SHORT_OUTPUT;
+    const uint32_t oc_opt = (d->channels == 3 && nc_opt == 4) ? 3u : nc_opt;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= opt.device) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
+    if (cudaSetDevice(opt.device) != cudaSuccess) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
+    // geometry of every image from its headers: the u8 intermediate is sized before decoding
+    struct Geo { uint32_t w = 0, h = 0, nc = 0; size_t u8 = 0, off = 0; bool ok = false; };
+    std::vector<Geo> geo(n);
+    size_t total = 0;
+    for (size_t i = 0; i < n; i++) {
+        zj_decoder *dd = zj_decoder_new(&opt);
+        zj_image_info info;
+        if (dd && zj_decoder_read_headers(dd, bufs[i], lens[i]) == ZJ_OK && zj_decoder_info(dd, &info) == ZJ_OK && info.valid) {
+            Geo &g = geo[i];
+            g.w = info.width; g.h = info.height;
+            const uint32_t cs = zj_decoder_out_colorspace(dd);
+            g.nc = cs == ZJ_CS_GRAYSCALE ? 1u : ((cs == ZJ_CS_RGB || cs == ZJ_CS_YCBCR) ? 3u : 4u);
+            g.u8 = (size_t)g.w * g.h * g.nc;
+            g.off = total;
+            total += (g.u8 + 255) & ~(size_t)255;
+            g.ok = true;
+        }
+        if (dd) zj_decoder_free(dd);
+    }
+    uint8_t *scratch = nullptr;
+    if (total) { const int arc = zj_capi_pool_alloc((void **)&scratch, total, opt.device, nullptr); if (arc != ZJ_OK) return arc; }
+    std::vector<uint8_t *> mid(n);
+    std::vector<size_t> mid_len(n);
+    // (images whose headers do not parse get a dummy one-byte slot: the decode call reports their error)
+    for (size_t i = 0; i < n; i++) { mid[i] = geo[i].ok ? scratch + geo[i].off : scratch; mid_len[i] = geo[i].ok ? geo[i].u8 : 0; }
+    int rc = zj_decode_batch_gpu_device(&opt, bufs, lens, n, mid.data(), mid_len.data(), status, n_gpu_entropy);
+    int failed = rc;
+    if (rc >= 0) {
+        // every decoded image whose crop fits it and whose channel count is the slots' through the resize
+        std::vector<const uint8_t *> src;
+        std::vector<uint32_t> w, h, nc;
+        std::vector<zj_roi> crops;
+        std::vector<size_t> slots;
+        for (size_t i = 0; i < n; i++) {
+            if (status[i] != ZJ_OK) continue;
+            const Geo &g = geo[i];
+            zj_roi c = {0, 0, g.w, g.h};
+            if (rois) c = rois[i];
+            const bool fits = c.w && c.h && (uint64_t)c.x + c.w <= g.w && (uint64_t)c.y + c.h <= g.h;
+            const uint32_t oc = (d->channels == 3 && g.nc == 4) ? 3u : g.nc;
+            if (!fits || oc != oc_opt) { status[i] = ZJ_ERR_INVALID_ARG; failed++; continue; }
+            src.push_back(mid[i]); w.push_back(g.w); h.push_back(g.h); nc.push_back(g.nc); crops.push_back(c); slots.push_back(i);
+        }
+        int crc = zj_capi_resize_many(opt.device, nullptr, src.data(), w.data(), h.data(), nc.data(), crops.data(), slots.data(), src.size(), d, r, out_dev);
         if (crc == ZJ_OK && cudaStreamSynchronize(nullptr) != cudaSuccess) { cudaGetLastError(); crc = ZJ_ERR_CUDA; }
         if (crc != ZJ_OK) failed = crc;
     }

@@ -363,3 +363,52 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
             finally:
                 lib.zj_buffer_free(outs[i])
     return res
+
+
+def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpegOptions | None = None, threads: int = 0):
+    """zj_decode_batch_gpu_device_resized: JPEG byte strings in, one batch tensor in device memory out -- every image decoded
+    whole, its crop resized to `resize` (a gpu.Resize) in the layout / type / normalisation of `desc` (a gpu.OutputDesc, scale
+    must be full size; default HWC u8).  rois: None, or one (x, y, w, h) or None (= the whole image) per image.
+
+    Returns (gpu.DeviceArray of shape (N, C, OH, OW) or (N, OH, OW, C), [None | DecodeErrors per image]).  The errors are the
+    ones decode_batch reports for the same inputs; a crop that does not fit its image, or an image whose channel count is not
+    the one the options' colourspace gives, fails with status ZJ_ERR_INVALID_ARG.  The slot of a failed image is not written."""
+    from . import gpu
+    lib = _ffi.load()
+    options = options if options is not None else ZuneJpegOptions()
+    desc = desc if desc is not None else gpu.OutputDesc()
+    raw = options._raw()
+    raw.num_threads = int(threads)
+    n = len(buffers)
+    keep = [b if isinstance(b, np.ndarray) else bytes(b) for b in buffers]
+    bufs = (C.c_void_p * n)(*[b.ctypes.data if isinstance(b, np.ndarray) else C.cast(C.c_char_p(b), C.c_void_p).value for b in keep])
+    lens = (C.c_size_t * n)(*[b.nbytes if isinstance(b, np.ndarray) else len(b) for b in keep])
+    sizes = [(0, 0)] * n
+    if rois is not None and any(r is None for r in rois) and not all(r is None for r in rois):
+        # whole-image entries next to crops: the sizes come from the headers (a file whose headers fail reports that error)
+        for i, r in enumerate(rois):
+            if r is None:
+                d = Decoder(options)
+                try:
+                    d.read_headers(keep[i])
+                    sizes[i] = (d.width(), d.height())
+                except DecodeErrors:
+                    sizes[i] = (1, 1)
+    nc = ColorSpace(options.get_out_colorspace()).num_components()
+    slot = resize.slot_size(desc, nc)
+    out = gpu.DeviceBuffer(max(slot * n, 1), options.get_device())
+    status = (C.c_int * n)()
+    n_gpu = C.c_size_t(0)
+    rc = lib.zj_decode_batch_gpu_device_resized(C.byref(raw), bufs, lens, n, gpu._roi_array(rois, sizes), C.byref(desc.c), C.byref(resize.c),
+                                                out.ptr, slot * n, status, C.byref(n_gpu))
+    if rc < 0:
+        raise DecodeErrors(13, lib.zj_gpu_strerror(rc).decode(), rc)
+    errs = []
+    for i in range(n):
+        if status[i] == 0:
+            errs.append(None)
+            continue
+        kind = lib.zj_batch_error_kind(i)
+        text = lib.zj_batch_error(i).decode(errors="replace") if kind else lib.zj_gpu_strerror(status[i]).decode()
+        errs.append(DecodeErrors(kind or (13 if status[i] != _ffi.ERR_DECODE else 1), text, status[i]))
+    return gpu.DeviceArray(out, (n, *resize.slot_shape(desc, nc)), desc.c.dtype), errs

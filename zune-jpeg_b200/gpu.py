@@ -323,3 +323,121 @@ def convert_device(src: DeviceBuffer, width: int, height: int, nc: int, desc: Ou
     _check(lib.zj_gpu_convert_device(device, stream, src.ptr, width, height, nc, C.byref(desc.c), b.ptr, sz), "zj_gpu_convert_device")
     synchronize(device, stream)
     return DeviceArray(b, (oc, oh, ow) if desc.chw else (oh, ow, oc), desc.c.dtype)
+
+
+# ------------------------------------------------------------------ cropped, resized batch tensors (DESIGN.md section 4.5.1)
+_FILTERS = {"area": _ffi.FILTER_AREA, "bilinear": _ffi.FILTER_BILINEAR}
+
+
+def _nc_of(img: ZjImage) -> int:
+    return {0: 3, 1: 1, 2: 3}.get(int(img.out_cs), 4)
+
+
+def _roi_array(rois, sizes):
+    """zj_roi[n] for a list of (x, y, w, h) or None (= the whole image, sizes[i] = (width, height)) entries; None -> NULL"""
+    if rois is None or all(r is None for r in rois):
+        return None
+    arr = (_ffi.ZjRoi * len(rois))()
+    for i, r in enumerate(rois):
+        arr[i].x, arr[i].y, arr[i].w, arr[i].h = r if r is not None else (0, 0, *sizes[i])
+    return arr
+
+
+class Resize:
+    """zj_resize: each image's crop resized to size = (OH, OW) with filter "area" (adaptive average pooling: the anti-aliased
+    choice for down-scales) or "bilinear" (torch interpolate, align_corners=False, antialias=False).  Every value is the
+    function of the crop's u8 bytes that expected() states."""
+
+    def __init__(self, size, filter: str = "area"):
+        oh, ow = size
+        r = _ffi.ZjResize()
+        r.out_w, r.out_h, r.filter = int(ow), int(oh), _FILTERS[filter]
+        self.c = r
+
+    @property
+    def size(self):
+        return (self.c.out_h, self.c.out_w)
+
+    def slot_shape(self, desc: OutputDesc, nc: int):
+        oc = 3 if (desc.c.channels == 3 and nc == 4) else nc
+        return (oc, self.c.out_h, self.c.out_w) if desc.chw else (self.c.out_h, self.c.out_w, oc)
+
+    def slot_size(self, desc: OutputDesc, nc: int) -> int:
+        return int(_ffi.load().zj_resize_slot_size(C.byref(desc.c), C.byref(self.c), nc))
+
+    def expected(self, u8: np.ndarray, width: int, height: int, nc: int, desc: OutputDesc | None = None, roi=None) -> np.ndarray:
+        """The specification, applied to the reference's bytes with numpy (tests: `u8` comes from the oracle).  Every float32
+        operation is one numpy float32 operation, in the order the header states."""
+        desc = desc if desc is not None else OutputDesc()
+        f32 = np.float32
+        x, y, w, h = roi if roi is not None else (0, 0, width, height)
+        oc = 3 if (desc.c.channels == 3 and nc == 4) else nc
+        p = np.asarray(u8, np.uint8).reshape(height, width, nc)[y:y + h, x:x + w, :oc]
+        OH, OW = self.c.out_h, self.c.out_w
+        u8_out = desc.c.dtype == _ffi.DTYPE_U8
+        if self.c.filter == _ffi.FILTER_AREA:
+            def windows(n_out, n_in):
+                i = np.arange(n_out, dtype=np.int64)
+                return (i * n_in) // n_out, ((i + 1) * n_in + n_out - 1) // n_out
+            r0, r1 = windows(OH, h)
+            c0, c1 = windows(OW, w)
+            sat = np.zeros((h + 1, w + 1, oc), np.uint64)           # summed-area table: exact window sums
+            sat[1:, 1:] = p.astype(np.uint64).cumsum(axis=0).cumsum(axis=1)
+            s = sat[r1][:, c1] - sat[r0][:, c1] - sat[r1][:, c0] + sat[r0][:, c0]
+            n = ((r1 - r0)[:, None] * (c1 - c0)[None, :]).astype(np.uint64)[:, :, None]
+            v = ((s + n // np.uint64(2)) // n).astype(np.uint8) if u8_out else s.astype(f32) / n.astype(f32)
+        else:
+            def coords(n_out, n_in):
+                sc = f32(n_in) / f32(n_out)
+                f = (np.arange(n_out, dtype=f32) + f32(0.5)) * sc - f32(0.5)
+                f = np.maximum(f, f32(0))
+                i0 = np.minimum(f.astype(np.int64), n_in - 1)
+                i1 = np.minimum(i0 + 1, n_in - 1)
+                a = f - i0.astype(f32)
+                return i0, i1, a, f32(1) - a
+            r0, r1, ay, by = coords(OH, h)
+            c0, c1, ax, bx = coords(OW, w)
+            q = p.astype(f32)
+            ax, bx, ay, by = ax[None, :, None], bx[None, :, None], ay[:, None, None], by[:, None, None]
+            top = bx * q[r0][:, c0] + ax * q[r0][:, c1]
+            bot = bx * q[r1][:, c0] + ax * q[r1][:, c1]
+            v = by * top + ay * bot
+            if u8_out:
+                v = np.clip(np.rint(v), 0, 255).astype(np.uint8)    # (rint: round half to even)
+        if not u8_out:
+            mean = np.array(list(desc.c.mean)[:oc], f32)
+            inv = np.array(list(desc.c.inv_std)[:oc], f32)
+            v = (v - mean) * inv
+        v = v.astype(desc.np_dtype)
+        return np.ascontiguousarray(v.transpose(2, 0, 1)) if desc.chw else np.ascontiguousarray(v)
+
+
+def resize_device(src: DeviceBuffer, width: int, height: int, nc: int, resize: Resize, desc: OutputDesc | None = None, roi=None,
+                  device: int = 0, stream=None) -> DeviceArray:
+    """zj_gpu_resize_device: the resize alone over interleaved u8 pixels already in device memory; roi = (x, y, w, h) or None."""
+    lib = _ffi.load()
+    desc = desc if desc is not None else OutputDesc()
+    sz = resize.slot_size(desc, nc)
+    b = DeviceBuffer(max(sz, 1), device)
+    r = _roi_array([roi], [(width, height)])
+    _check(lib.zj_gpu_resize_device(device, stream, src.ptr, width, height, nc, r, C.byref(desc.c), C.byref(resize.c), b.ptr, sz),
+           "zj_gpu_resize_device")
+    synchronize(device, stream)
+    return DeviceArray(b, resize.slot_shape(desc, nc), desc.c.dtype)
+
+
+def reconstruct_device_resized(images, resize: Resize, desc: OutputDesc | None = None, rois=None, device: int = 0, stream=None) -> DeviceArray:
+    """zj_gpu_reconstruct_device_resized: `images` carry DEVICE coefficient planes; returns one (N, C, OH, OW) or (N, OH, OW, C)
+    DeviceArray.  rois: None, or one (x, y, w, h) or None (= the whole image) per image; only the strips that hold a crop's rows
+    are reconstructed."""
+    lib = _ffi.load()
+    desc = desc if desc is not None else OutputDesc()
+    n = len(images)
+    nc = _nc_of(images[0]) if n else 3
+    slot = resize.slot_size(desc, nc)
+    b = DeviceBuffer(max(slot * n, 1), device)
+    arr = _img_array(images)
+    r = _roi_array(rois, [(im.width, im.height) for im in images])
+    _check(lib.zj_gpu_reconstruct_device_resized(device, stream, arr, n, r, C.byref(desc.c), C.byref(resize.c), b.ptr, slot * n),
+           "zj_gpu_reconstruct_device_resized")
+    return DeviceArray(b, (n, *resize.slot_shape(desc, nc)), desc.c.dtype)
