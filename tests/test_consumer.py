@@ -110,6 +110,36 @@ def test_consumer_sub_batches():
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("entry", ["zj_gpu_reconstruct_device_ex", "zj_gpu_reconstruct_device_resized"])
+def test_more_than_65535_images_of_one_format(entry):
+    """65537 small images of one pixel format fit one sub-batch, but a launch takes at most 65535 (the image index is gridDim.z):
+    the reconstruction and the second pass each run in two launches."""
+    from zune_jpeg_b200 import _ffi, gpu
+    lib = _ffi.load()
+    n = 65537
+    imgs, wants, keep = _device_images(gpu, np.random.default_rng(17), [(17, 33, "444", 0)])
+    arr = (_ffi.ZjImage * n).from_buffer_copy(bytes(imgs[0]) * n)      # every descriptor names the same device planes
+    desc = gpu.OutputDesc("CHW", "f16", False, 0, MEAN, INV)
+    if entry == "zj_gpu_reconstruct_device_ex":
+        exp = desc.expected(wants[0], 17, 33, 3)
+        out = gpu.DeviceBuffer(exp.nbytes * n)
+        ptrs = (C.c_void_p * n)(*range(out.ptr, out.ptr + exp.nbytes * n, exp.nbytes))
+        lens = (C.c_size_t * n)(*[exp.nbytes] * n)
+        call = lambda: lib.zj_gpu_reconstruct_device_ex(0, None, arr, n, C.byref(desc.c), ptrs, lens)
+    else:
+        rz = gpu.Resize((8, 16), "area")
+        exp = rz.expected(wants[0], 17, 33, 3, desc)
+        out = gpu.DeviceBuffer(exp.nbytes * n)
+        call = lambda: lib.zj_gpu_reconstruct_device_resized(0, None, arr, n, None, C.byref(desc.c), C.byref(rz.c), out.ptr, exp.nbytes * n)
+    before = gpu.launch_count()
+    assert call() == 0
+    assert gpu.launch_count() - before == 4      # (65535 + 2 images) x (reconstruction + second pass)
+    got = out.download().reshape(n, exp.nbytes)
+    bad = np.nonzero((got != np.frombuffer(exp.tobytes(), np.uint8)).any(axis=1))[0]
+    assert bad.size == 0, f"{bad.size} slots differ, first {bad[:8]}"
+
+
+@pytest.mark.gpu
 def test_cuda_array_interface_and_dlpack():
     """The hand-off: torch reads the consumer's output in place through __cuda_array_interface__ / DLPack."""
     import torch

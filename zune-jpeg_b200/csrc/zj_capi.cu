@@ -10,20 +10,14 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
-#include <functional>
 #include <mutex>
 #include <new>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/zune_jpeg_b200.h"
 #include "zj_device.h"
-
-namespace zj {
-cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream);
-cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
-cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
-}
 
 using namespace zj;
 
@@ -38,7 +32,7 @@ static int cuda_fail(cudaError_t e, const char *what)
 }
 #define CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(e_, #call); } while (0)
 
-static int num_components(uint32_t cs)  // ColorSpace::num_components, reference src/misc.rs:108-118
+int zj::num_components(uint32_t cs)  // ColorSpace::num_components, reference src/misc.rs:108-118
 {
     switch (cs) {
     case ZJ_CS_RGB: case ZJ_CS_YCBCR: return 3;
@@ -257,7 +251,7 @@ static cudaError_t pool_alloc(void **p, size_t bytes, int device, cudaStream_t s
     return pool ? cudaMallocFromPoolAsync(p, bytes, pool, s) : cudaMallocAsync(p, bytes, s);
 }
 // gives the pool's cached memory back to the driver (zj_release_device_caches)
-extern "C" void zj_capi_trim_pools(void)
+void zj::trim_pools()
 {
     std::lock_guard<std::mutex> lock(g_pool_mu);
     for (int d = 0; d < 64; d++) if (g_pool[d]) cudaMemPoolTrimTo(g_pool[d], 0);
@@ -415,7 +409,10 @@ int zj_gpu_reconstruct_device(int device, void *stream, const zj_image *imgs, si
     return rc;
 }
 
+}  // extern "C"
+
 // ------------------------------------------------------------------------------------- device-side consumers
+// (The header gives the zj_* functions below their C linkage; the templates this part shares cannot have it.)
 void zj_output_desc_default(zj_output_desc *d)
 {
     if (!d) return;
@@ -436,6 +433,9 @@ int zj_output_desc_is_default(const zj_output_desc *d)
 
 static size_t dtype_size(uint32_t dt) { return dt == ZJ_DTYPE_U8 ? 1 : (dt == ZJ_DTYPE_F16 ? 2 : 4); }
 
+// channels written per pixel of nc source bytes (channels = 3 drops the fourth byte)
+static uint32_t out_channels(const zj_output_desc *d, uint32_t nc) { return (d->channels == 3 && nc == 4) ? 3u : nc; }
+
 static int conv_shape(uint32_t width, uint32_t height, uint32_t nc, const zj_output_desc *d, uint32_t *ow, uint32_t *oh, uint32_t *oc)
 {
     int rc = desc_check(d);
@@ -443,8 +443,14 @@ static int conv_shape(uint32_t width, uint32_t height, uint32_t nc, const zj_out
     if (nc != 1 && nc != 3 && nc != 4) return ZJ_ERR_INVALID_ARG;
     *ow = width >> d->scale_log2;
     *oh = height >> d->scale_log2;
-    *oc = (d->channels == 3 && nc == 4) ? 3u : nc;
+    *oc = out_channels(d, nc);
     return ZJ_OK;
+}
+
+size_t zj::convert_size(uint32_t width, uint32_t height, uint32_t nc, const zj_output_desc *d)
+{
+    uint32_t ow, oh, oc;
+    return conv_shape(width, height, nc, d, &ow, &oh, &oc) == ZJ_OK ? (size_t)ow * oh * oc * dtype_size(d->dtype) : 0;
 }
 
 int zj_consumer_output_shape(const zj_image *img, const zj_output_desc *d, uint32_t *out_w, uint32_t *out_h, uint32_t *out_c)
@@ -455,9 +461,52 @@ int zj_consumer_output_shape(const zj_image *img, const zj_output_desc *d, uint3
 
 size_t zj_consumer_output_size(const zj_image *img, const zj_output_desc *d)
 {
-    uint32_t ow, oh, oc;
-    if (!img || zj_output_size(img) == 0 || zj_consumer_output_shape(img, d, &ow, &oh, &oc) != ZJ_OK) return 0;
-    return (size_t)ow * oh * oc * dtype_size(d->dtype);
+    if (!img || zj_output_size(img) == 0) return 0;
+    return convert_size(img->width, img->height, (uint32_t)num_components(img->out_cs), d);
+}
+
+// One launch of the second pass (the consumer for ConvImage, the resize for ResizeImage) per run of consecutive images with the
+// same bytes per pixel, at most 65535 images each: the image index is gridDim.z.  dev / host: the same descriptors in device /
+// host memory, nc[i]: image i's bytes per pixel, r: the resize's parameters.
+template <class Img>
+static int launch_runs(const Img *dev, const Img *host, const uint32_t *nc, size_t n, const zj_output_desc &d, const zj_resize *r, cudaStream_t s)
+{
+    constexpr bool convert = std::is_same<Img, ConvImage>::value;
+    for (size_t k = 0, k1 = 0; k < n; k = k1) {
+        uint32_t mw = 0, mh = 0;   // the consumer's grid covers the run's largest output
+        for (k1 = k; k1 < n && nc[k1] == nc[k] && k1 - k < 65535; k1++)
+            if constexpr (convert) { mw = std::max(mw, host[k1].ow); mh = std::max(mh, host[k1].oh); }
+        cudaError_t e;
+        if constexpr (convert) {
+            if (!mw || !mh) continue;   // nothing to write (half size of images one pixel wide or high)
+            e = launch_convert(dev + k, (uint32_t)(k1 - k), nc[k], mw, mh, d, s);
+        } else {
+            e = launch_resize(dev + k, (uint32_t)(k1 - k), nc[k], d, *r, s);
+        }
+        g_launches.fetch_add(1);
+        if (e != cudaSuccess) return cuda_fail(e, convert ? "consumer launch" : "resize launch");
+    }
+    return ZJ_OK;
+}
+
+// Copies the descriptors host[0, n) into a stream-ordered pool allocation, calls use(that copy) and frees it, all in the order of s
+template <class Img, class Use>
+static int with_device_copy(const Img *host, size_t n, int device, cudaStream_t s, Use use)
+{
+    Img *dev = nullptr;
+    CU(pool_alloc((void **)&dev, n * sizeof(Img), device, s));
+    // (pageable source: the async copy returns once the data sits in the driver's staging buffer)
+    const cudaError_t e = cudaMemcpyAsync(dev, host, n * sizeof(Img), cudaMemcpyHostToDevice, s);
+    const int rc = e == cudaSuccess ? use(static_cast<const Img *>(dev)) : cuda_fail(e, "cudaMemcpyAsync(descriptors)");
+    cudaFreeAsync(dev, s);
+    return rc;
+}
+
+// The second pass over n images whose u8 pixels are already in device memory
+template <class Img>
+static int run_pass(int device, cudaStream_t s, const Img *host, const uint32_t *nc, size_t n, const zj_output_desc &d, const zj_resize *r)
+{
+    return with_device_copy(host, n, device, s, [&](const Img *dev) { return launch_runs(dev, host, nc, n, d, r, s); });
 }
 
 int zj_gpu_convert_device(int device, void *stream, const uint8_t *src_dev, uint32_t width, uint32_t height, uint32_t nc,
@@ -467,60 +516,12 @@ int zj_gpu_convert_device(int device, void *stream, const uint8_t *src_dev, uint
     int rc = conv_shape(width, height, nc, d, &ci.ow, &ci.oh, &ci.oc);
     if (rc) return rc;
     if (!src_dev || !dst_dev) return ZJ_ERR_INVALID_ARG;
-    if (dst_len < (size_t)ci.ow * ci.oh * ci.oc * dtype_size(d->dtype)) return ZJ_ERR_SHORT_OUTPUT;
+    if (dst_len < convert_size(width, height, nc, d)) return ZJ_ERR_SHORT_OUTPUT;
     rc = set_device(device);
     if (rc) return rc;
     if (ci.ow == 0 || ci.oh == 0) return ZJ_OK;
     ci.src = src_dev; ci.dst = dst_dev; ci.width = width; ci.height = height; ci.nc = nc;
-    cudaStream_t s = (cudaStream_t)stream;
-    ConvImage *d_ci = nullptr;
-    CU(pool_alloc((void **)&d_ci, sizeof(ci), device, s));
-    cudaError_t e = cudaMemcpyAsync(d_ci, &ci, sizeof(ci), cudaMemcpyHostToDevice, s);   // (pageable source: staged before the call returns)
-    if (e == cudaSuccess) { e = launch_convert(d_ci, 1, nc, ci.ow, ci.oh, *d, s); g_launches.fetch_add(1); }
-    cudaFreeAsync(d_ci, s);
-    if (e != cudaSuccess) return cuda_fail(e, "zj_gpu_convert_device");
-    return ZJ_OK;
-}
-
-// Hidden helpers for zj_decode_batch_gpu_device_ex (zj_host_decoder.cpp): scratch from this library's stream-ordered pool, and
-// the consumer over many images in as few launches as their pixel formats allow.
-extern "C" int zj_capi_pool_alloc(void **p, size_t bytes, int device, void *stream)
-{
-    int rc = set_device(device);
-    if (rc) return rc;
-    CU(pool_alloc(p, bytes, device, (cudaStream_t)stream));
-    return ZJ_OK;
-}
-extern "C" void zj_capi_pool_free(void *p, void *stream) { if (p) cudaFreeAsync(p, (cudaStream_t)stream); }
-extern "C" int zj_capi_convert_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
-                                    void *const *dst, size_t n, const zj_output_desc *d)
-{
-    int rc = desc_check(d);
-    if (rc) return rc;
-    rc = set_device(device);
-    if (rc) return rc;
-    if (n == 0) return ZJ_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    std::vector<ConvImage> conv(n);
-    for (size_t i = 0; i < n; i++) {
-        ConvImage &ci = conv[i];
-        ci.src = src[i]; ci.dst = dst[i]; ci.width = w[i]; ci.height = h[i]; ci.nc = nc[i];
-        rc = conv_shape(w[i], h[i], nc[i], d, &ci.ow, &ci.oh, &ci.oc);
-        if (rc) return rc;
-    }
-    ConvImage *d_conv = nullptr;
-    CU(pool_alloc((void **)&d_conv, n * sizeof(ConvImage), device, s));
-    cudaError_t e = cudaMemcpyAsync(d_conv, conv.data(), n * sizeof(ConvImage), cudaMemcpyHostToDevice, s);   // (pageable: staged before the call returns)
-    for (size_t k = 0; k < n && e == cudaSuccess;) {
-        size_t k1 = k;
-        uint32_t mw = 0, mh = 0;
-        while (k1 < n && conv[k1].nc == conv[k].nc && k1 - k < 65535) { mw = std::max(mw, conv[k1].ow); mh = std::max(mh, conv[k1].oh); k1++; }
-        if (mw && mh) { e = launch_convert(d_conv + k, (uint32_t)(k1 - k), conv[k].nc, mw, mh, *d, s); g_launches.fetch_add(1); }
-        k = k1;
-    }
-    cudaFreeAsync(d_conv, s);
-    if (e != cudaSuccess) return cuda_fail(e, "consumer launch");
-    return ZJ_OK;
+    return run_pass(device, (cudaStream_t)stream, &ci, &nc, 1, *d, nullptr);
 }
 
 // Sub-batch budget of the u8 intermediate (scratch memory of the call).  Measured on 128 4K images (profiles/README.md):
@@ -551,30 +552,47 @@ static size_t chunk_place(std::vector<ConsumerChunk> &chunks, size_t i, size_t b
     return off;
 }
 
-// Reconstructs the sub-batches one after the other into `scratch` (image i at u8_off[i], u8_size[i] bytes) on `s`, and after
-// each calls second_pass(chunk), which launches the kernels that read it.  Then waits for `s` and releases the plans.  Nothing
-// runs unless rc (the status so far) is ZJ_OK.
-static int reconstruct_chunks(int device, cudaStream_t s, const zj_image *imgs, const std::vector<ConsumerChunk> &chunks, uint8_t *scratch,
-                              const std::vector<size_t> &u8_off, const std::vector<size_t> &u8_size, int rc,
-                              const std::function<int(const ConsumerChunk &)> &second_pass)
+// The planes route of the second pass: subs[i] is reconstructed into u8_size[i] bytes of a stream-ordered scratch buffer, in
+// sub-batches that take turns in it, and each sub-batch is followed by the pass over its images.  build(i, image i's u8
+// pixels) gives image i's descriptor; the descriptors are uploaded once.  Returns after `s` has drained.
+template <class Build>
+static int reconstruct_then(int device, cudaStream_t s, const zj_image *subs, const std::vector<size_t> &u8_size, const uint32_t *nc,
+                            const zj_output_desc &d, const zj_resize *r, Build build)
 {
-    std::vector<zj_batch *> batches;
-    for (size_t c = 0; c < chunks.size() && rc == ZJ_OK; c++) {
-        const ConsumerChunk &ch = chunks[c];
-        std::vector<uint8_t *> outs(ch.count);
-        std::vector<size_t> lens(ch.count);
-        for (size_t k = 0; k < ch.count; k++) { outs[k] = scratch + u8_off[ch.first + k]; lens[k] = u8_size[ch.first + k]; }
-        zj_batch *b = nullptr;
-        rc = batch_create_impl(device, imgs + ch.first, ch.count, outs.data(), lens.data(), &b, true, s);
-        if (rc) break;
-        batches.push_back(b);
-        rc = zj_batch_run(b, s);
-        if (rc == ZJ_OK) rc = second_pass(ch);
+    using Img = decltype(build(0, nullptr));
+    const size_t n = u8_size.size();
+    std::vector<ConsumerChunk> chunks;
+    std::vector<size_t> u8_off(n);
+    size_t scratch_bytes = 0;
+    for (size_t i = 0; i < n; i++) {
+        u8_off[i] = chunk_place(chunks, i, u8_size[i]);
+        scratch_bytes = std::max(scratch_bytes, chunks.back().bytes);
     }
-    // the descriptor arrays and the scratch must outlive the kernels
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess && rc == ZJ_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
-    for (zj_batch *b : batches) zj_batch_destroy(b);
+    uint8_t *scratch = nullptr;
+    CU(pool_alloc((void **)&scratch, scratch_bytes, device, s));
+    std::vector<Img> host(n);
+    for (size_t i = 0; i < n; i++) host[i] = build(i, scratch + u8_off[i]);
+    const int rc = with_device_copy(host.data(), n, device, s, [&](const Img *dev) {
+        int rc = ZJ_OK;
+        std::vector<zj_batch *> batches;
+        for (size_t c = 0; c < chunks.size() && rc == ZJ_OK; c++) {
+            const ConsumerChunk &ch = chunks[c];
+            std::vector<uint8_t *> outs(ch.count);
+            for (size_t k = 0; k < ch.count; k++) outs[k] = scratch + u8_off[ch.first + k];
+            zj_batch *b = nullptr;
+            rc = batch_create_impl(device, subs + ch.first, ch.count, outs.data(), u8_size.data() + ch.first, &b, true, s);
+            if (rc) break;
+            batches.push_back(b);
+            rc = zj_batch_run(b, s);
+            if (rc == ZJ_OK) rc = launch_runs(dev + ch.first, host.data() + ch.first, nc + ch.first, ch.count, d, r, s);
+        }
+        // the descriptor arrays and the scratch must outlive the kernels
+        cudaError_t e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess && rc == ZJ_OK) rc = cuda_fail(e, "cudaStreamSynchronize");
+        for (zj_batch *b : batches) zj_batch_destroy(b);
+        return rc;
+    });
+    cudaFreeAsync(scratch, s);
     return rc;
 }
 
@@ -587,55 +605,25 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
     if ((!imgs || !out_dev || !out_len) && n) return ZJ_ERR_INVALID_ARG;
     rc = set_device(device);
     if (rc) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
-    // geometry, sizes, sub-batches of consecutive images
     std::vector<ConvImage> conv(n);
-    std::vector<size_t> u8_size(n), u8_off(n);
-    std::vector<ConsumerChunk> chunks;
-    size_t scratch_bytes = 0;
+    std::vector<uint32_t> nc(n);
+    std::vector<size_t> u8_size(n);
     for (size_t i = 0; i < n; i++) {
         u8_size[i] = zj_output_size(&imgs[i]);
         if (u8_size[i] == 0) { rc = zj_validate_image(&imgs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
         ConvImage &ci = conv[i];
-        ci.width = imgs[i].width; ci.height = imgs[i].height; ci.nc = (uint32_t)num_components(imgs[i].out_cs);
+        ci.width = imgs[i].width; ci.height = imgs[i].height; ci.nc = nc[i] = (uint32_t)num_components(imgs[i].out_cs);
         rc = conv_shape(ci.width, ci.height, ci.nc, d, &ci.ow, &ci.oh, &ci.oc);
         if (rc) return rc;
         if (!out_dev[i]) return ZJ_ERR_INVALID_ARG;
-        if (out_len[i] < (size_t)ci.ow * ci.oh * ci.oc * dtype_size(d->dtype)) return ZJ_ERR_SHORT_OUTPUT;
+        if (out_len[i] < convert_size(ci.width, ci.height, ci.nc, d)) return ZJ_ERR_SHORT_OUTPUT;
         ci.dst = out_dev[i];
-        u8_off[i] = chunk_place(chunks, i, u8_size[i]);
-        scratch_bytes = std::max(scratch_bytes, chunks.back().bytes);
     }
     if (n == 0) return ZJ_OK;
-    uint8_t *scratch = nullptr;
-    ConvImage *d_conv = nullptr;
-    CU(pool_alloc((void **)&scratch, scratch_bytes, device, s));
-    cudaError_t e = pool_alloc((void **)&d_conv, n * sizeof(ConvImage), device, s);
-    if (e != cudaSuccess) { cudaFreeAsync(scratch, s); return cuda_fail(e, "cudaMallocAsync(consumer descriptors)"); }
-    for (size_t i = 0; i < n; i++) conv[i].src = scratch + u8_off[i];
-    e = cudaMemcpyAsync(d_conv, conv.data(), n * sizeof(ConvImage), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(consumer descriptors)");
-    rc = reconstruct_chunks(device, s, imgs, chunks, scratch, u8_off, u8_size, rc, [&](const ConsumerChunk &ch) {
-        // one consumer launch per run of images with the same number of source bytes per pixel
-        for (size_t k = 0; k < ch.count;) {
-            size_t k1 = k;
-            uint32_t mw = 0, mh = 0;
-            while (k1 < ch.count && conv[ch.first + k1].nc == conv[ch.first + k].nc) {
-                mw = std::max(mw, conv[ch.first + k1].ow); mh = std::max(mh, conv[ch.first + k1].oh);
-                k1++;
-            }
-            if (mw && mh) {
-                cudaError_t le = launch_convert(d_conv + ch.first + k, (uint32_t)(k1 - k), conv[ch.first + k].nc, mw, mh, *d, s);
-                g_launches.fetch_add(1);
-                if (le != cudaSuccess) return cuda_fail(le, "consumer launch");
-            }
-            k = k1;
-        }
-        return (int)ZJ_OK;
+    return reconstruct_then(device, (cudaStream_t)stream, imgs, u8_size, nc.data(), *d, nullptr, [&](size_t i, const uint8_t *u8) {
+        conv[i].src = u8;
+        return conv[i];
     });
-    cudaFreeAsync(d_conv, s);
-    cudaFreeAsync(scratch, s);
-    return rc;
 }
 
 // ------------------------------------------------------------------------------------- cropped, resized batch tensors
@@ -650,12 +638,10 @@ static int resize_check(const zj_output_desc *d, const zj_resize *r)
     return ZJ_OK;
 }
 
-static uint32_t resize_oc(const zj_output_desc *d, uint32_t nc) { return (d->channels == 3 && nc == 4) ? 3u : nc; }
-
 size_t zj_resize_slot_size(const zj_output_desc *d, const zj_resize *r, uint32_t nc)
 {
     if (resize_check(d, r) != ZJ_OK || (nc != 1 && nc != 3 && nc != 4)) return 0;
-    return (size_t)r->out_w * r->out_h * resize_oc(d, nc) * dtype_size(d->dtype);
+    return (size_t)r->out_w * r->out_h * out_channels(d, nc) * dtype_size(d->dtype);
 }
 
 // *out = the crop of a width x height image that `roi` names (NULL = the whole image)
@@ -665,6 +651,12 @@ static int roi_resolve(const zj_roi *roi, uint32_t width, uint32_t height, zj_ro
     if (roi->w == 0 || roi->h == 0 || (uint64_t)roi->x + roi->w > width || (uint64_t)roi->y + roi->h > height) return ZJ_ERR_INVALID_ARG;
     *out = *roi;
     return ZJ_OK;
+}
+
+int zj::resize_admit(const zj_output_desc *d, uint32_t slot_nc, const zj_roi *roi, uint32_t width, uint32_t height, uint32_t nc, zj_roi *crop)
+{
+    if (out_channels(d, nc) != out_channels(d, slot_nc)) return ZJ_ERR_INVALID_ARG;   // one tensor: one channel count
+    return roi_resolve(roi, width, height, crop);
 }
 
 // src: the width x height (rows of it) u8 image the crop lies in, from its row `row0` on
@@ -681,20 +673,6 @@ static ResizeImage resize_image(const uint8_t *src, uint32_t width, uint32_t hei
     ri.sx = (float)roi.w / (float)r.out_w;   // IEEE single-precision division, as the kernel's other operations
     ri.sy = (float)roi.h / (float)r.out_h;
     return ri;
-}
-
-// one resize launch per run of at most 65535 images with the same nc (d_ri / ri: the same descriptors on the device / host)
-static int launch_resize_runs(const ResizeImage *d_ri, const uint32_t *nc, size_t n, const zj_output_desc &d, const zj_resize &r, cudaStream_t s)
-{
-    for (size_t k = 0; k < n;) {
-        size_t k1 = k;
-        while (k1 < n && nc[k1] == nc[k] && k1 - k < 65535) k1++;
-        const cudaError_t e = launch_resize(d_ri + k, (uint32_t)(k1 - k), nc[k], d, r, s);
-        g_launches.fetch_add(1);
-        if (e != cudaSuccess) return cuda_fail(e, "resize launch");
-        k = k1;
-    }
-    return ZJ_OK;
 }
 
 int zj_image_rows(const zj_image *img, uint32_t row_begin, uint32_t row_end, zj_image *sub, uint32_t *sub_row0)
@@ -732,14 +710,8 @@ int zj_gpu_resize_device(int device, void *stream, const uint8_t *src_dev, uint3
     if (dst_len < slot) return ZJ_ERR_SHORT_OUTPUT;
     rc = set_device(device);
     if (rc) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
     const ResizeImage ri = resize_image(src_dev, width, height, nc, crop.y, crop, dst_dev, *r);
-    ResizeImage *d_ri = nullptr;
-    CU(pool_alloc((void **)&d_ri, sizeof(ri), device, s));
-    cudaError_t e = cudaMemcpyAsync(d_ri, &ri, sizeof(ri), cudaMemcpyHostToDevice, s);   // (pageable source: staged before the call returns)
-    rc = e == cudaSuccess ? launch_resize_runs(d_ri, &nc, 1, *d, *r, s) : cuda_fail(e, "cudaMemcpyAsync(resize descriptor)");
-    cudaFreeAsync(d_ri, s);
-    return rc;
+    return run_pass(device, (cudaStream_t)stream, &ri, &nc, 1, *d, r);
 }
 
 int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *imgs, size_t n, const zj_roi *rois, const zj_output_desc *d,
@@ -748,71 +720,74 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     int rc = resize_check(d, r);
     if (rc) return rc;
     if ((!imgs || !out_dev) && n) return ZJ_ERR_INVALID_ARG;
-    // per image: the crop, the strips that hold its rows, where their u8 pixels go in the scratch buffer
+    // per image: the crop, the strips that hold its rows and the size of their u8 pixels
     std::vector<zj_image> subs(n);
     std::vector<zj_roi> crops(n);
     std::vector<uint32_t> row0(n), nc(n);
-    std::vector<size_t> u8_size(n), u8_off(n);
-    std::vector<ConsumerChunk> chunks;
-    size_t scratch_bytes = 0;
+    std::vector<size_t> u8_size(n);
     for (size_t i = 0; i < n; i++) {
         if (zj_output_size(&imgs[i]) == 0) { rc = zj_validate_image(&imgs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
         nc[i] = (uint32_t)num_components(imgs[i].out_cs);
-        if (resize_oc(d, nc[i]) != resize_oc(d, nc[0])) return ZJ_ERR_INVALID_ARG;   // one tensor: one channel count
-        rc = roi_resolve(rois ? &rois[i] : nullptr, imgs[i].width, imgs[i].height, &crops[i]);
+        rc = resize_admit(d, nc[0], rois ? &rois[i] : nullptr, imgs[i].width, imgs[i].height, nc[i], &crops[i]);
         if (rc) return rc;
         rc = zj_image_rows(&imgs[i], crops[i].y, crops[i].y + crops[i].h, &subs[i], &row0[i]);
         if (rc) return rc;
         u8_size[i] = zj_output_size(&subs[i]);
         if (u8_size[i] == 0) { rc = zj_validate_image(&subs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
-        u8_off[i] = chunk_place(chunks, i, u8_size[i]);
-        scratch_bytes = std::max(scratch_bytes, chunks.back().bytes);
     }
     const size_t slot = n ? zj_resize_slot_size(d, r, nc[0]) : 0;
     if (n && out_len / slot < n) return ZJ_ERR_SHORT_OUTPUT;
     rc = set_device(device);
     if (rc) return rc;
     if (n == 0) return ZJ_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    uint8_t *scratch = nullptr;
-    ResizeImage *d_ri = nullptr;
-    CU(pool_alloc((void **)&scratch, scratch_bytes, device, s));
-    cudaError_t e = pool_alloc((void **)&d_ri, n * sizeof(ResizeImage), device, s);
-    if (e != cudaSuccess) { cudaFreeAsync(scratch, s); return cuda_fail(e, "cudaMallocAsync(resize descriptors)"); }
-    std::vector<ResizeImage> ri(n);
-    for (size_t i = 0; i < n; i++)
-        ri[i] = resize_image(scratch + u8_off[i], imgs[i].width, subs[i].height, nc[i], row0[i], crops[i], static_cast<uint8_t *>(out_dev) + i * slot, *r);
-    e = cudaMemcpyAsync(d_ri, ri.data(), n * sizeof(ResizeImage), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(resize descriptors)");
-    rc = reconstruct_chunks(device, s, subs.data(), chunks, scratch, u8_off, u8_size, rc, [&](const ConsumerChunk &ch) {
-        return launch_resize_runs(d_ri + ch.first, nc.data() + ch.first, ch.count, *d, *r, s);
+    return reconstruct_then(device, (cudaStream_t)stream, subs.data(), u8_size, nc.data(), *d, r, [&](size_t i, const uint8_t *u8) {
+        return resize_image(u8, imgs[i].width, subs[i].height, nc[i], row0[i], crops[i], static_cast<uint8_t *>(out_dev) + i * slot, *r);
     });
-    cudaFreeAsync(d_ri, s);
-    cudaFreeAsync(scratch, s);
-    return rc;
 }
 
-// Hidden helper for zj_decode_batch_gpu_device_resized (zj_host_decoder.cpp): the resize over decoded u8 images already in
-// device memory, image i into slot dst_slot[i] of out_dev; the arguments were checked by the caller.
-extern "C" int zj_capi_resize_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
-                                   const zj_roi *crops,
-                                   const size_t *dst_slot, size_t n, const zj_output_desc *d, const zj_resize *r, void *out_dev)
+// ------------------------------------------------------------------------------------- the JPEG-bytes route's second pass
+int zj::scratch_alloc(void **p, size_t bytes, int device, void *stream)
+{
+    int rc = set_device(device);
+    if (rc) return rc;
+    CU(pool_alloc(p, bytes, device, (cudaStream_t)stream));
+    return ZJ_OK;
+}
+void zj::scratch_free(void *p, void *stream) { if (p) cudaFreeAsync(p, (cudaStream_t)stream); }
+
+int zj::convert_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d)
+{
+    int rc = desc_check(d);
+    if (rc) return rc;
+    rc = set_device(device);
+    if (rc) return rc;
+    if (n == 0) return ZJ_OK;
+    std::vector<ConvImage> conv(n);
+    std::vector<uint32_t> nc(n);
+    for (size_t i = 0; i < n; i++) {
+        ConvImage &ci = conv[i];
+        ci.src = imgs[i].src; ci.dst = imgs[i].dst; ci.width = imgs[i].width; ci.height = imgs[i].height; ci.nc = nc[i] = imgs[i].nc;
+        rc = conv_shape(ci.width, ci.height, ci.nc, d, &ci.ow, &ci.oh, &ci.oc);
+        if (rc) return rc;
+    }
+    return run_pass(device, (cudaStream_t)stream, conv.data(), nc.data(), n, *d, nullptr);
+}
+
+// (the crops and channel counts were admitted by the caller: resize_admit)
+int zj::resize_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d, const zj_resize *r)
 {
     int rc = resize_check(d, r);
     if (rc) return rc;
     rc = set_device(device);
     if (rc) return rc;
     if (n == 0) return ZJ_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t slot = zj_resize_slot_size(d, r, nc[0]);
     std::vector<ResizeImage> ri(n);
-    for (size_t i = 0; i < n; i++) ri[i] = resize_image(src[i], w[i], h[i], nc[i], crops[i].y, crops[i], static_cast<uint8_t *>(out_dev) + dst_slot[i] * slot, *r);
-    ResizeImage *d_ri = nullptr;
-    CU(pool_alloc((void **)&d_ri, n * sizeof(ResizeImage), device, s));
-    cudaError_t e = cudaMemcpyAsync(d_ri, ri.data(), n * sizeof(ResizeImage), cudaMemcpyHostToDevice, s);   // (pageable: staged before the call returns)
-    rc = e == cudaSuccess ? launch_resize_runs(d_ri, nc, n, *d, *r, s) : cuda_fail(e, "cudaMemcpyAsync(resize descriptors)");
-    cudaFreeAsync(d_ri, s);
-    return rc;
+    std::vector<uint32_t> nc(n);
+    for (size_t i = 0; i < n; i++) {
+        nc[i] = imgs[i].nc;
+        ri[i] = resize_image(imgs[i].src, imgs[i].width, imgs[i].height, nc[i], imgs[i].crop.y, imgs[i].crop, imgs[i].dst, *r);
+    }
+    return run_pass(device, (cudaStream_t)stream, ri.data(), nc.data(), n, *d, r);
 }
 
 // Staging state of zj_gpu_reconstruct_submit, leased per host thread (see there); the idle ones are what
@@ -829,9 +804,9 @@ struct CachePool {
 };
 static CachePool g_stream_pool;
 
-// frees the streams and device staging buffers of every cache no thread holds (hidden symbol; the exported entry
-// point is zj_release_device_caches in zj_host_decoder.cpp)
-extern "C" void zj_capi_release_stream_caches(void)
+// frees the streams and device staging buffers of every cache no thread holds (the exported entry point is
+// zj_release_device_caches in zj_host_decoder.cpp)
+void zj::release_stream_caches()
 {
     std::vector<StreamCache *> drop;
     {
@@ -856,6 +831,8 @@ extern "C" void zj_capi_release_stream_caches(void)
     if (prev >= 0) cudaSetDevice(prev);
     cudaGetLastError();
 }
+
+extern "C" {
 
 // Host entry point: stage planes H2D, run, copy pixels D2H.  Images are processed in sub-batches on internal streams so
 // that the copies of one sub-batch overlap the kernels of the other.  Split in two halves: zj_gpu_reconstruct_submit queues

@@ -1,10 +1,15 @@
-// zj_device.h -- descriptors shared by the host-side planner (zj_capi.cu) and the kernels (zj_kernels.cu).
+// zj_device.h -- descriptors shared by the host-side planner (zj_capi.cu) and the kernels (zj_kernels.cu), and the
+// declarations of the library's functions that one source file calls in another.
 //
 // Vocabulary follows the reference: an image is cut into MCU-row *strips* (the unit of
 // worker::post_process, reference src/worker.rs:32; geometry src/mcu.rs:139-226, src/mcu_prog.rs:132-203);
 // a strip is cut into *tiles* of TM MCU columns, one CTA per tile.
 #pragma once
+#include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
+
+#include "../../include/zune_jpeg_b200.h"
 
 namespace zj {
 
@@ -88,5 +93,35 @@ struct ResizeImage {
     uint32_t w, h;                // crop size in pixels
     float sx, sy;                 // bilinear scales float(w) / float(out_w), float(h) / float(out_h) (one IEEE division each)
 };
+
+// Kernel launches: zj_kernels.cu (reconstruction), zj_consumer.cu (consumer, resize)
+cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream);
+cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
+cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
+
+// ---- zj_capi.cu for zj_host_decoder.cpp (hidden symbols, not part of the C ABI)
+int num_components(uint32_t cs);   // output bytes per pixel of colourspace cs (ColorSpace::num_components); 0 = not a colourspace
+// bytes the consumer writes for a width x height image of nc bytes per pixel; 0 = a bad descriptor or nc
+size_t convert_size(uint32_t width, uint32_t height, uint32_t nc, const zj_output_desc *d);
+// *crop = the crop `roi` of a width x height image of nc bytes per pixel (NULL = the whole image), into a batch tensor of
+// slot_nc-byte source pixels; ZJ_ERR_INVALID_ARG when it does not fit the image or the image's channel count is not the slots'
+int resize_admit(const zj_output_desc *d, uint32_t slot_nc, const zj_roi *roi, uint32_t width, uint32_t height, uint32_t nc, zj_roi *crop);
+// device memory from this library's stream-ordered pool of `device`, allocated / freed in the order of `stream`
+int scratch_alloc(void **p, size_t bytes, int device, void *stream);
+void scratch_free(void *p, void *stream);
+
+// One decoded image in device memory: the input of the second pass of the JPEG-bytes route
+struct U8Image {
+    const uint8_t *src;           // u8, interleaved, width * height * nc
+    uint32_t width, height, nc;
+    zj_roi crop;                  // resize_many: the crop
+    void *dst;                    // convert_many: the image's output; resize_many: its slot
+};
+// the consumer / the resize over n decoded images, one launch per run of equal pixel formats; asynchronous on `stream`
+int convert_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d);
+int resize_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d, const zj_resize *r);
+
+void release_stream_caches();   // the idle staging streams and buffers of zj_gpu_reconstruct_submit
+void trim_pools();              // the stream-ordered pools' cached memory back to the driver
 
 }  // namespace zj

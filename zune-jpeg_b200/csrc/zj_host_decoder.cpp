@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "../../include/zune_jpeg_b200.h"
+#include "zj_device.h"
 #include "zj_entropy.h"
 
 // Worker threads pull their work from a shared counter, so a pool that could not be grown (std::system_error: thread limit)
@@ -1587,9 +1588,7 @@ ZJ_API int zj_decoder_decode_buffer(zj_decoder *d, const uint8_t *buf, size_t le
     // the size comes from the headers (mcu.rs:375-379: width * height * out components); they are parsed again by the decode
     int rc = zj_decoder_read_headers(d, buf, len);
     if (rc) return rc;
-    const uint32_t cs = d->options.out_colorspace;
-    const size_t nc = cs == ZJ_CS_GRAYSCALE ? 1 : ((cs == ZJ_CS_RGB || cs == ZJ_CS_YCBCR) ? 3 : 4);
-    const size_t cap = (size_t)d->info.width * d->info.height * nc;
+    const size_t cap = (size_t)d->info.width * d->info.height * zj::num_components(d->options.out_colorspace);
     uint8_t *o = (uint8_t *)malloc(cap ? cap : 1);
     if (!o) return ZJ_ERR_OOM;
     size_t n = 0;
@@ -1824,16 +1823,6 @@ static size_t slot_retain_bytes()
     static const size_t v = [] { const char *e = getenv("ZJ_RETAIN_MB"); long mb = e ? atol(e) : 16384; return (size_t)(mb < 0 ? 0 : mb) << 20; }();
     return v;
 }
-extern "C" void zj_capi_release_stream_caches(void);   // zj_capi.cu (hidden)
-extern "C" void zj_capi_trim_pools(void);
-extern "C" int zj_capi_pool_alloc(void **p, size_t bytes, int device, void *stream);
-extern "C" void zj_capi_pool_free(void *p, void *stream);
-extern "C" int zj_capi_resize_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
-                                   const zj_roi *crops,
-                                   const size_t *dst_slot, size_t n, const zj_output_desc *d, const zj_resize *r, void *out_dev);
-extern "C" int zj_capi_convert_many(int device, void *stream, const uint8_t *const *src, const uint32_t *w, const uint32_t *h, const uint32_t *nc,
-                                    void *const *dst, size_t n, const zj_output_desc *d);
-
 ZJ_API void zj_release_device_caches(void)
 {
     {
@@ -1843,8 +1832,8 @@ ZJ_API void zj_release_device_caches(void)
         g_slot_cache.device = -1;
         cudaGetLastError();
     }
-    zj_capi_release_stream_caches();
-    zj_capi_trim_pools();
+    zj::release_stream_caches();
+    zj::trim_pools();
 }
 
 // Batch front door with the entropy stage on the GPU as well (zj_entropy.cu) for the JPEGs that allow it: baseline scans
@@ -2187,6 +2176,49 @@ ZJ_API int zj_decode_batch_gpu_device(const zj_options *o, const uint8_t *const 
     return decode_batch_gpu_impl(o, bufs, lens, n, const_cast<uint8_t **>(out_dev), out_len, status, n_gpu_entropy, true);
 }
 
+// The first pass of the device-output calls with a second pass: every image decoded into a stream-ordered u8 scratch buffer
+// (zj_decode_batch_gpu_device), then second_pass(img, failed) over img[i] = image i's geometry and pixels.  second_pass checks
+// each decoded image, counts the images it turns down in `failed`, queues its launches and returns their status.  Returns
+// zj_decode_batch's result with those images added, or a negative zj_status; the pixels are in place on return.
+static int decode_then(const zj_options &opt, const uint8_t *const *bufs, const size_t *lens, size_t n, int *status, size_t *n_gpu_entropy,
+                       const std::function<int(std::vector<zj::U8Image> &, int &)> &second_pass)
+{
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= opt.device) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
+    if (cudaSetDevice(opt.device) != cudaSuccess) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
+    // geometry of every image from its headers: the u8 intermediate is sized before decoding
+    std::vector<zj::U8Image> img(n);
+    std::vector<size_t> off(n), len(n);
+    std::vector<bool> parsed(n);
+    size_t total = 0;
+    for (size_t i = 0; i < n; i++) {
+        zj_decoder *dd = zj_decoder_new(&opt);
+        zj_image_info info;
+        if (dd && zj_decoder_read_headers(dd, bufs[i], lens[i]) == ZJ_OK && zj_decoder_info(dd, &info) == ZJ_OK && info.valid) {
+            img[i].width = info.width; img[i].height = info.height;
+            img[i].nc = (uint32_t)zj::num_components(zj_decoder_out_colorspace(dd));
+            len[i] = (size_t)img[i].width * img[i].height * img[i].nc;
+            off[i] = total;
+            total += (len[i] + 255) & ~(size_t)255;
+            parsed[i] = true;
+        }
+        if (dd) zj_decoder_free(dd);
+    }
+    uint8_t *scratch = nullptr;
+    if (total) { const int arc = zj::scratch_alloc((void **)&scratch, total, opt.device, nullptr); if (arc != ZJ_OK) return arc; }
+    std::vector<uint8_t *> mid(n);
+    // (images whose headers do not parse get a dummy one-byte slot: the decode call reports their error)
+    for (size_t i = 0; i < n; i++) { mid[i] = parsed[i] ? scratch + off[i] : scratch; img[i].src = mid[i]; }
+    int failed = zj_decode_batch_gpu_device(&opt, bufs, lens, n, mid.data(), len.data(), status, n_gpu_entropy);
+    if (failed >= 0) {
+        int crc = second_pass(img, failed);
+        if (crc == ZJ_OK && cudaStreamSynchronize(nullptr) != cudaSuccess) { cudaGetLastError(); crc = ZJ_ERR_CUDA; }
+        if (crc != ZJ_OK) failed = crc;
+    }
+    zj::scratch_free(scratch, nullptr);
+    return failed;
+}
+
 // The device-output call with a consumer descriptor: the pixels are reconstructed into a stream-ordered u8 scratch buffer and
 // converted from there (zj_consumer.cu); with the default descriptor this IS zj_decode_batch_gpu_device.
 ZJ_API int zj_decode_batch_gpu_device_ex(const zj_options *o, const uint8_t *const *bufs, const size_t *lens, size_t n,
@@ -2199,57 +2231,20 @@ ZJ_API int zj_decode_batch_gpu_device_ex(const zj_options *o, const uint8_t *con
     if ((!bufs || !lens || !out_dev || !out_len || !status) && n) return ZJ_ERR_INVALID_ARG;
     zj_options opt;
     if (o) opt = *o; else zj_options_default(&opt);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= opt.device) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
-    if (cudaSetDevice(opt.device) != cudaSuccess) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
-    // geometry of every image from its headers: the u8 intermediate and the caller's buffers are sized before decoding
-    struct Geo { uint32_t w = 0, h = 0, nc = 0; size_t u8 = 0, off = 0; bool ok = false; };
-    std::vector<Geo> geo(n);
-    size_t total = 0;
-    for (size_t i = 0; i < n; i++) {
-        zj_decoder *dd = zj_decoder_new(&opt);
-        zj_image_info info;
-        if (dd && zj_decoder_read_headers(dd, bufs[i], lens[i]) == ZJ_OK && zj_decoder_info(dd, &info) == ZJ_OK && info.valid) {
-            Geo &g = geo[i];
-            g.w = info.width; g.h = info.height;
-            const uint32_t cs = zj_decoder_out_colorspace(dd);
-            g.nc = cs == ZJ_CS_GRAYSCALE ? 1u : ((cs == ZJ_CS_RGB || cs == ZJ_CS_YCBCR) ? 3u : 4u);
-            g.u8 = (size_t)g.w * g.h * g.nc;
-            g.off = total;
-            total += (g.u8 + 255) & ~(size_t)255;
-            g.ok = true;
-        }
-        if (dd) zj_decoder_free(dd);
-    }
-    uint8_t *scratch = nullptr;
-    if (total) { const int arc = zj_capi_pool_alloc((void **)&scratch, total, opt.device, nullptr); if (arc != ZJ_OK) return arc; }
-    std::vector<uint8_t *> mid(n);
-    std::vector<size_t> mid_len(n);
-    // (images whose headers do not parse get a dummy one-byte slot: the decode call reports their error)
-    for (size_t i = 0; i < n; i++) { mid[i] = geo[i].ok ? scratch + geo[i].off : scratch; mid_len[i] = geo[i].ok ? geo[i].u8 : 0; }
-    int rc = zj_decode_batch_gpu_device(&opt, bufs, lens, n, mid.data(), mid_len.data(), status, n_gpu_entropy);
-    int failed = rc;
-    if (rc >= 0) {
+    return decode_then(opt, bufs, lens, n, status, n_gpu_entropy, [&](std::vector<zj::U8Image> &img, int &failed) {
         // every decoded image through the consumer: one launch per run of equal pixel formats
-        std::vector<const uint8_t *> csrc;
-        std::vector<void *> cdst;
-        std::vector<uint32_t> cw, ch, cnc;
-        const size_t es = d->dtype == ZJ_DTYPE_U8 ? 1 : (d->dtype == ZJ_DTYPE_F16 ? 2 : 4);
+        std::vector<zj::U8Image> conv;
         for (size_t i = 0; i < n; i++) {
             if (status[i] != ZJ_OK) { out_len[i] = 0; continue; }
-            const Geo &g = geo[i];
-            const size_t need = (size_t)(g.w >> d->scale_log2) * (g.h >> d->scale_log2) * ((d->channels == 3 && g.nc == 4) ? 3 : g.nc) * es;
+            const size_t need = zj::convert_size(img[i].width, img[i].height, img[i].nc, d);
             if (!out_dev[i]) { status[i] = ZJ_ERR_INVALID_ARG; failed++; out_len[i] = 0; continue; }
             if (out_len[i] < need) { status[i] = ZJ_ERR_SHORT_OUTPUT; failed++; out_len[i] = 0; continue; }
             out_len[i] = need;
-            csrc.push_back(mid[i]); cdst.push_back(out_dev[i]); cw.push_back(g.w); ch.push_back(g.h); cnc.push_back(g.nc);
+            img[i].dst = out_dev[i];
+            conv.push_back(img[i]);
         }
-        int crc = zj_capi_convert_many(opt.device, nullptr, csrc.data(), cw.data(), ch.data(), cnc.data(), cdst.data(), csrc.size(), d);
-        if (crc == ZJ_OK && cudaStreamSynchronize(nullptr) != cudaSuccess) { cudaGetLastError(); crc = ZJ_ERR_CUDA; }
-        if (crc != ZJ_OK) failed = crc;
-    }
-    zj_capi_pool_free(scratch, nullptr);
-    return failed;
+        return zj::convert_many(opt.device, nullptr, conv.data(), conv.size(), d);
+    });
 }
 
 // The batch-tensor call: whole images decoded into a stream-ordered u8 scratch buffer (as zj_decode_batch_gpu_device_ex does),
@@ -2262,65 +2257,23 @@ ZJ_API int zj_decode_batch_gpu_device_resized(const zj_options *o, const uint8_t
     zj_options opt;
     if (o) opt = *o; else zj_options_default(&opt);
     // every slot has the channel count the options' colourspace gives
-    const uint32_t cs_opt = opt.out_colorspace;
-    if (cs_opt > ZJ_CS_RGBX) return ZJ_ERR_INVALID_ARG;
-    const uint32_t nc_opt = cs_opt == ZJ_CS_GRAYSCALE ? 1u : ((cs_opt == ZJ_CS_RGB || cs_opt == ZJ_CS_YCBCR) ? 3u : 4u);
+    const uint32_t nc_opt = (uint32_t)zj::num_components(opt.out_colorspace);
     const size_t slot = zj_resize_slot_size(d, r, nc_opt);
     if (slot == 0) return ZJ_ERR_INVALID_ARG;
     if (n && out_len / slot < n) return ZJ_ERR_SHORT_OUTPUT;
-    const uint32_t oc_opt = (d->channels == 3 && nc_opt == 4) ? 3u : nc_opt;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= opt.device) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
-    if (cudaSetDevice(opt.device) != cudaSuccess) { cudaGetLastError(); return ZJ_ERR_NO_DEVICE; }
-    // geometry of every image from its headers: the u8 intermediate is sized before decoding
-    struct Geo { uint32_t w = 0, h = 0, nc = 0; size_t u8 = 0, off = 0; bool ok = false; };
-    std::vector<Geo> geo(n);
-    size_t total = 0;
-    for (size_t i = 0; i < n; i++) {
-        zj_decoder *dd = zj_decoder_new(&opt);
-        zj_image_info info;
-        if (dd && zj_decoder_read_headers(dd, bufs[i], lens[i]) == ZJ_OK && zj_decoder_info(dd, &info) == ZJ_OK && info.valid) {
-            Geo &g = geo[i];
-            g.w = info.width; g.h = info.height;
-            const uint32_t cs = zj_decoder_out_colorspace(dd);
-            g.nc = cs == ZJ_CS_GRAYSCALE ? 1u : ((cs == ZJ_CS_RGB || cs == ZJ_CS_YCBCR) ? 3u : 4u);
-            g.u8 = (size_t)g.w * g.h * g.nc;
-            g.off = total;
-            total += (g.u8 + 255) & ~(size_t)255;
-            g.ok = true;
-        }
-        if (dd) zj_decoder_free(dd);
-    }
-    uint8_t *scratch = nullptr;
-    if (total) { const int arc = zj_capi_pool_alloc((void **)&scratch, total, opt.device, nullptr); if (arc != ZJ_OK) return arc; }
-    std::vector<uint8_t *> mid(n);
-    std::vector<size_t> mid_len(n);
-    // (images whose headers do not parse get a dummy one-byte slot: the decode call reports their error)
-    for (size_t i = 0; i < n; i++) { mid[i] = geo[i].ok ? scratch + geo[i].off : scratch; mid_len[i] = geo[i].ok ? geo[i].u8 : 0; }
-    int rc = zj_decode_batch_gpu_device(&opt, bufs, lens, n, mid.data(), mid_len.data(), status, n_gpu_entropy);
-    int failed = rc;
-    if (rc >= 0) {
+    return decode_then(opt, bufs, lens, n, status, n_gpu_entropy, [&](std::vector<zj::U8Image> &img, int &failed) {
         // every decoded image whose crop fits it and whose channel count is the slots' through the resize
-        std::vector<const uint8_t *> src;
-        std::vector<uint32_t> w, h, nc;
-        std::vector<zj_roi> crops;
-        std::vector<size_t> slots;
+        std::vector<zj::U8Image> admitted;
         for (size_t i = 0; i < n; i++) {
             if (status[i] != ZJ_OK) continue;
-            const Geo &g = geo[i];
-            zj_roi c = {0, 0, g.w, g.h};
-            if (rois) c = rois[i];
-            const bool fits = c.w && c.h && (uint64_t)c.x + c.w <= g.w && (uint64_t)c.y + c.h <= g.h;
-            const uint32_t oc = (d->channels == 3 && g.nc == 4) ? 3u : g.nc;
-            if (!fits || oc != oc_opt) { status[i] = ZJ_ERR_INVALID_ARG; failed++; continue; }
-            src.push_back(mid[i]); w.push_back(g.w); h.push_back(g.h); nc.push_back(g.nc); crops.push_back(c); slots.push_back(i);
+            if (zj::resize_admit(d, nc_opt, rois ? &rois[i] : nullptr, img[i].width, img[i].height, img[i].nc, &img[i].crop) != ZJ_OK) {
+                status[i] = ZJ_ERR_INVALID_ARG; failed++; continue;
+            }
+            img[i].dst = static_cast<uint8_t *>(out_dev) + i * slot;
+            admitted.push_back(img[i]);
         }
-        int crc = zj_capi_resize_many(opt.device, nullptr, src.data(), w.data(), h.data(), nc.data(), crops.data(), slots.data(), src.size(), d, r, out_dev);
-        if (crc == ZJ_OK && cudaStreamSynchronize(nullptr) != cudaSuccess) { cudaGetLastError(); crc = ZJ_ERR_CUDA; }
-        if (crc != ZJ_OK) failed = crc;
-    }
-    zj_capi_pool_free(scratch, nullptr);
-    return failed;
+        return zj::resize_many(opt.device, nullptr, admitted.data(), admitted.size(), d, r);
+    });
 }
 
 ZJ_API void zj_host_set_quirks(uint32_t mask) { g_quirks.store(mask & ZJ_QUIRK_ALL); }

@@ -296,6 +296,24 @@ JpegDecoder = Decoder
 DecoderOptions = ZuneJpegOptions
 
 
+def _input_arrays(buffers):
+    """(keep, bufs, lens): the inputs as bytes or uint8 arrays (the caller keeps them alive during the call) and the pointer and
+    length arrays the batch calls take"""
+    n = len(buffers)
+    keep = [b if isinstance(b, np.ndarray) else bytes(b) for b in buffers]
+    bufs = (C.c_void_p * n)(*[b.ctypes.data if isinstance(b, np.ndarray) else C.cast(C.c_char_p(b), C.c_void_p).value for b in keep])
+    lens = (C.c_size_t * n)(*[b.nbytes if isinstance(b, np.ndarray) else len(b) for b in keep])
+    return keep, bufs, lens
+
+
+def _image_error(lib, i: int, status: int, batch_errors: bool = True) -> DecodeErrors:
+    """image i's failure in a batch call: the variant and text Decoder.decode_buffer raises for the same input
+    (zj_batch_error_kind / zj_batch_error, which the call records when `batch_errors`)"""
+    kind = lib.zj_batch_error_kind(i) if batch_errors else 0
+    text = lib.zj_batch_error(i).decode(errors="replace") if kind else lib.zj_gpu_strerror(status).decode()
+    return DecodeErrors(kind or (13 if status != _ffi.ERR_DECODE else 1), text, status)
+
+
 def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int = 0, out=None, gpu_entropy: bool = False, stats: dict | None = None,
                  device_out=None, desc=None, devices=None):
     """zj_decode_batch: JPEG byte strings in, pixel bytes out, `threads` host threads (0 = one per hardware thread)
@@ -311,15 +329,12 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
     image, a `DecodeErrors` instance for a failed one.  `out`: optional list of writable buffers (e.g. PinnedBuffer.array
     slices), one per image, large enough for width*height*components.  Inputs may be `bytes` or uint8 numpy arrays (e.g. views
     of pinned memory, which upload at the full PCIe rate)."""
-    import numpy as np
     lib = _ffi.load()
     options = options if options is not None else ZuneJpegOptions()
     raw = options._raw()
     raw.num_threads = int(threads)
     n = len(buffers)
-    keep = [b if isinstance(b, np.ndarray) else bytes(b) for b in buffers]
-    bufs = (C.c_void_p * n)(*[b.ctypes.data if isinstance(b, np.ndarray) else C.cast(C.c_char_p(b), C.c_void_p).value for b in keep])
-    lens = (C.c_size_t * n)(*[b.nbytes if isinstance(b, np.ndarray) else len(b) for b in keep])
+    keep, bufs, lens = _input_arrays(buffers)
     outs = (C.c_void_p * n)()
     out_len = (C.c_size_t * n)()
     status = (C.c_int * n)()
@@ -351,10 +366,7 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
     res = []
     for i in range(n):
         if status[i] != 0:
-            # the variant and text Decoder.decode_buffer raises for the same input (zj_batch_error_kind / zj_batch_error)
-            kind = lib.zj_batch_error_kind(i) if devices is None else 0
-            text = lib.zj_batch_error(i).decode(errors="replace") if kind else lib.zj_gpu_strerror(status[i]).decode()
-            res.append(DecodeErrors(kind or (13 if status[i] != _ffi.ERR_DECODE else 1), text, status[i]))
+            res.append(_image_error(lib, i, status[i], batch_errors=devices is None))
         elif out is not None or device_out is not None:
             res.append(int(out_len[i]))
         else:
@@ -380,9 +392,7 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
     raw = options._raw()
     raw.num_threads = int(threads)
     n = len(buffers)
-    keep = [b if isinstance(b, np.ndarray) else bytes(b) for b in buffers]
-    bufs = (C.c_void_p * n)(*[b.ctypes.data if isinstance(b, np.ndarray) else C.cast(C.c_char_p(b), C.c_void_p).value for b in keep])
-    lens = (C.c_size_t * n)(*[b.nbytes if isinstance(b, np.ndarray) else len(b) for b in keep])
+    keep, bufs, lens = _input_arrays(buffers)
     sizes = [(0, 0)] * n
     if rois is not None and any(r is None for r in rois) and not all(r is None for r in rois):
         # whole-image entries next to crops: the sizes come from the headers (a file whose headers fail reports that error)
@@ -403,12 +413,5 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
                                                 out.ptr, slot * n, status, C.byref(n_gpu))
     if rc < 0:
         raise DecodeErrors(13, lib.zj_gpu_strerror(rc).decode(), rc)
-    errs = []
-    for i in range(n):
-        if status[i] == 0:
-            errs.append(None)
-            continue
-        kind = lib.zj_batch_error_kind(i)
-        text = lib.zj_batch_error(i).decode(errors="replace") if kind else lib.zj_gpu_strerror(status[i]).decode()
-        errs.append(DecodeErrors(kind or (13 if status[i] != _ffi.ERR_DECODE else 1), text, status[i]))
+    errs = [_image_error(lib, i, status[i]) if status[i] != 0 else None for i in range(n)]
     return gpu.DeviceArray(out, (n, *resize.slot_shape(desc, nc)), desc.c.dtype), errs

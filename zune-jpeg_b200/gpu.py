@@ -248,6 +248,10 @@ class OutputDesc:
     def np_dtype(self):
         return _NP_DTYPES[self.c.dtype]
 
+    def out_channels(self, nc: int) -> int:
+        """channels written per pixel of nc source bytes (channels=3 drops the fourth byte)"""
+        return 3 if (self.c.channels == 3 and nc == 4) else nc
+
     def shape_of(self, img: ZjImage):
         w, h, ch = C.c_uint32(), C.c_uint32(), C.c_uint32()
         _check(_ffi.load().zj_consumer_output_shape(C.byref(img), C.byref(self.c), C.byref(w), C.byref(h), C.byref(ch)), "zj_consumer_output_shape")
@@ -317,7 +321,7 @@ def convert_device(src: DeviceBuffer, width: int, height: int, nc: int, desc: Ou
     """zj_gpu_convert_device: the consumer alone over interleaved u8 pixels already in device memory."""
     lib = _ffi.load()
     ow, oh = width >> desc.c.scale_log2, height >> desc.c.scale_log2
-    oc = 3 if (desc.c.channels == 3 and nc == 4) else nc
+    oc = desc.out_channels(nc)
     sz = ow * oh * oc * np.dtype(desc.np_dtype).itemsize
     b = DeviceBuffer(max(sz, 1), device)
     _check(lib.zj_gpu_convert_device(device, stream, src.ptr, width, height, nc, C.byref(desc.c), b.ptr, sz), "zj_gpu_convert_device")
@@ -359,7 +363,7 @@ class Resize:
         return (self.c.out_h, self.c.out_w)
 
     def slot_shape(self, desc: OutputDesc, nc: int):
-        oc = 3 if (desc.c.channels == 3 and nc == 4) else nc
+        oc = desc.out_channels(nc)
         return (oc, self.c.out_h, self.c.out_w) if desc.chw else (self.c.out_h, self.c.out_w, oc)
 
     def slot_size(self, desc: OutputDesc, nc: int) -> int:
