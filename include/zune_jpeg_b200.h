@@ -52,7 +52,34 @@ typedef enum zj_colorspace {
  *          (src/upsampler/avx2.rs, scalar below 500 samples), AVX2 RGB (src/color_convert/avx.rs).
  * SCALAR = use_unsafe == false or `--no-default-features`: src/idct/scalar.rs, src/upsampler/scalar.rs,
  *          src/color_convert/scalar.rs. */
-typedef enum zj_variant { ZJ_VARIANT_X86 = 0, ZJ_VARIANT_SCALAR = 1 } zj_variant;
+typedef enum zj_variant { ZJ_VARIANT_X86 = 0, ZJ_VARIANT_SCALAR = 1, ZJ_VARIANT_SPEC = 2 } zj_variant;
+
+/* ZJ_VARIANT_SPEC -- not in the reference: spec-correct output, none of its pixel-path quirks (DESIGN.md section 4.6).  The
+ * output is a function of the coefficient planes, bit-exact:
+ *   1. Samples: every block of every component goes through the X86 IDCT above (dequantise, rows then columns, the DC-only
+ *      shortcut, clamp to [0, 255]); a component plane is the raster of its blocks.
+ *   2. Sizes: luma is width x height; chroma is cw = ceil(width / hs) by ch = ceil(height / vs), (hs, vs) = comp[0]'s factors.
+ *      Samples beyond these sizes (block padding) are never read: every neighbour index below is clamped to
+ *      [0, ch-1] x [0, cw-1].
+ *   3. Up-sampling (libjpeg jdsample.c, integer "fancy" forms), c[j][i] a chroma sample:
+ *        none  C(y, x) = c[y][x]
+ *        H     C(y, 2i) = (3c[y][i] + c[y][i-1] + 1) >> 2         C(y, 2i+1) = (3c[y][i] + c[y][i+1] + 2) >> 2
+ *        V     C(2j, x) = (3c[j][x] + c[j-1][x] + 1) >> 2         C(2j+1, x) = (3c[j][x] + c[j+1][x] + 2) >> 2
+ *        HV    s[i] = 3c[j][i] + c[j'][i], j' = j-1 for output row 2j and j+1 for row 2j+1 (indices of s clamped alike):
+ *              C(., 2i) = (3s[i] + s[i-1] + 8) >> 4                C(., 2i+1) = (3s[i] + s[i+1] + 7) >> 4
+ *      then cut to width x height.
+ *   4. Colour (libjpeg jdcolor.c, 16-bit fixed point, arithmetic shifts), cb' = Cb - 128, cr' = Cr - 128:
+ *        R = clamp(Y + ((91881 cr' + 32768) >> 16))
+ *        G = clamp(Y + ((-22554 cb' - 46802 cr' + 32768) >> 16))
+ *        B = clamp(Y + ((116130 cb' + 32768) >> 16))
+ *   5. Output: RGB = R, G, B; RGBA and RGBX = R, G, B, 255; YCBCR = Y, Cb, Cr; GRAYSCALE = Y.  One-component input: GRAYSCALE = Y,
+ *      RGB / RGBA / RGBX = Y, Y, Y (, 255).  Every other pair is ZJ_ERR_UNSUPPORTED.
+ * Every byte of the width*height*nc output is written.  Every strip of the image is reconstructed (4:2:2 and 4:2:0: ceil(mcu_y/2)
+ * strips), so the planes must cover them (ZJ_ERR_SHORT_PLANE otherwise, e.g. for planes of an as-written host stage that dropped
+ * an odd last MCU row); none of the reference's panic rules applies.  Such an image cannot be cut into strip ranges: the rows of a
+ * strip need chroma from its neighbours (zj_image_strip_range returns ZJ_ERR_UNSUPPORTED for any cut).  The host stage produces
+ * it with zj_options.use_unsafe = ZJ_USE_SPEC_OUTPUT. */
+enum { ZJ_USE_SPEC_OUTPUT = 2 };
 
 typedef enum zj_status {
     ZJ_OK = 0,
@@ -142,7 +169,7 @@ ZJ_API void zj_partition(size_t n_items, size_t n_parts, size_t part, size_t *be
  * *out_bytes = where its pixels live inside the whole image's output.  *n_strips = strips of the whole image (pass sub,
  * out_offset, out_bytes = NULL to query only that).  Reconstructing every range of a partition gives exactly the bytes of
  * reconstructing the whole image.  ZJ_ERR_UNSUPPORTED: this image cannot be cut (its strip count was limited by the
- * reference's output-capacity rule, mcu_prog.rs:206-209). */
+ * reference's output-capacity rule, mcu_prog.rs:206-209, or it is a ZJ_VARIANT_SPEC image). */
 ZJ_API int zj_image_strip_range(const zj_image *img, uint32_t strip_begin, uint32_t strip_end, zj_image *sub,
                                 size_t *out_offset, size_t *out_bytes, uint32_t *n_strips);
 
@@ -264,7 +291,8 @@ ZJ_API uint64_t zj_gpu_launch_count(void);
  * deployment these symbols are not needed (INTEGRATION.md). */
 
 typedef struct zj_options {       /* ZuneJpegOptions (src/options.rs:6-40), same defaults */
-    uint32_t use_unsafe;          /* 1                                                   */
+    uint32_t use_unsafe;          /* 1; ZJ_USE_SPEC_OUTPUT (not in the reference): ZJ_VARIANT_SPEC output, and the host stage
+                                     decodes every MCU row with Q9-Q11 off, whatever zj_host_set_quirks says              */
     uint32_t out_colorspace;      /* ZJ_CS_RGB                                           */
     uint32_t num_threads;         /* 4                                                   */
     uint32_t max_width;           /* 16384                                               */
@@ -389,8 +417,9 @@ ZJ_API int zj_decode_batch_gpu_device_resized(const zj_options *o, const uint8_t
  *   Q9  src/huffman.rs:249-252   fast-AC entry `(k << 10) + ...` is an i16: |k| >= 32 loses its top bits
  *   Q10 src/bitstream.rs:278-281 decode_dc refills only below 16 buffered bits but may consume 27: the reader under-runs
  *   Q11 src/mcu.rs:337-342       the MCU loop breaks on a PREFETCHED EOI: trailing components of the last MCU stay zero
- * Process-wide; takes effect for tables built / streams started afterwards.  With any bit cleared the GPU entropy route
- * (zj_decode_batch_gpu*) sends every image through the host stage.  tests/test_quirks.py is the only caller. */
+ * Process-wide; takes effect for decodes started afterwards (a ZJ_USE_SPEC_OUTPUT decode runs with every bit cleared, whatever
+ * is set here).  With any bit cleared the GPU entropy route (zj_decode_batch_gpu*) sends every image through the host stage.
+ * tests/test_quirks.py is the only caller. */
 enum { ZJ_QUIRK_Q9_FAST_AC_I16 = 1u, ZJ_QUIRK_Q10_DC_REFILL = 2u, ZJ_QUIRK_Q11_EOI_BREAK = 4u, ZJ_QUIRK_ALL = 7u };
 ZJ_API void zj_host_set_quirks(uint32_t mask);
 ZJ_API uint32_t zj_host_get_quirks(void);

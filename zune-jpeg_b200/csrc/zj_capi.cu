@@ -61,7 +61,8 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     if (img->width == 0 || img->height == 0 || img->width > 65535 || img->height > 65535) return ZJ_ERR_INVALID_ARG;
     const int nc = num_components(img->out_cs);
     if (nc == 0) return ZJ_ERR_INVALID_ARG;
-    if (img->variant != ZJ_VARIANT_X86 && img->variant != ZJ_VARIANT_SCALAR) return ZJ_ERR_INVALID_ARG;
+    if (img->variant != ZJ_VARIANT_X86 && img->variant != ZJ_VARIANT_SCALAR && img->variant != ZJ_VARIANT_SPEC) return ZJ_ERR_INVALID_ARG;
+    const bool spec = img->variant == ZJ_VARIANT_SPEC;
     const uint32_t h = img->comp[0].h_samp, v = img->comp[0].v_samp;
     if (img->n_comp == 1 && (h != 1 || v != 1)) return ZJ_ERR_UNSUPPORTED;  // mcu.rs:171-196 resets these before the path
     for (uint32_t z = 1; z < img->n_comp; z++)
@@ -90,12 +91,13 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     case MODE_V: n_strips = mcu_y; ybr = 2; cbr = 1; break;       // mcu.rs:160-163
     default: n_strips = (hh + 7) / 8; ybr = 1; cbr = 1; break;    // mcu.rs:164-169
     }
+    if (spec && (mode == MODE_H || mode == MODE_HV)) n_strips = (mcu_y + 1) / 2;   // every MCU row
     const uint32_t rows = 8 * h * v;
     const size_t out_chunk = (size_t)w * nc * rows;               // mcu.rs:226
     const size_t capacity = (size_t)(uint16_t)(w + 8) * (size_t)(uint16_t)(hh + 8);  // mcu.rs:198 (u16 add)
     const size_t extra = (mode != MODE_NONE ? 128u : 0u) * (size_t)hh * nc;           // mcu.rs:207
     const size_t avail = (capacity * nc + extra) / out_chunk;
-    if (n_strips > avail) {
+    if (n_strips > avail && !spec) {
         if (img->flags & ZJ_FLAG_PROGRESSIVE) n_strips = (uint32_t)avail;  // mcu_prog.rs:206-209, zip stops
         else return ZJ_ERR_REF_PANIC;                                      // mcu.rs:354, chunks.next().unwrap()
     }
@@ -113,9 +115,13 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     else if (in_cs == ZJ_CS_YCBCR && oc == ZJ_CS_YCBCR) kind = OUT_YCC;               // worker.rs:120-123
     else if (in_cs == ZJ_CS_YCBCR && (oc == ZJ_CS_RGB || oc == ZJ_CS_RGBA || oc == ZJ_CS_RGBX)) kind = OUT_RGB;  // :125-129
     else kind = OUT_ZERO;                                                             // worker.rs:131-132
+    if (spec && kind == OUT_ZERO) {   // one-component input keeps RGB / RGBA / RGBX; every other pair has no stated output
+        if (in_cs != ZJ_CS_GRAYSCALE || (oc != ZJ_CS_RGB && oc != ZJ_CS_RGBA && oc != ZJ_CS_RGBX)) return ZJ_ERR_UNSUPPORTED;
+        kind = OUT_RGB;
+    }
     pl->gray = kind == OUT_GRAY;
     pl->zero_only = kind == OUT_ZERO;
-    pl->ncomp_used = kind == OUT_GRAY ? 1u : (kind == OUT_ZERO ? 0u : 3u);  // min(in, out) comps are IDCT'd; unused results are dropped
+    pl->ncomp_used = kind == OUT_GRAY ? 1u : (kind == OUT_ZERO ? 0u : img->n_comp);  // min(in, out) comps are IDCT'd; unused results are dropped
 
     DevImage &d = pl->dev;
     d.width = w; d.height = hh; d.nc = (uint32_t)nc; d.out_kind = kind;
@@ -134,11 +140,12 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
         // ycbcr_to_grayscale (color_convert/scalar.rs:97-112): width_mcu = len / width must equal the strip's row
         // count, otherwise the chunking overruns the strip's output slice and the reference panics (Q7).
         const size_t len = (size_t)rows * d.Wp;
-        if (n_strips > 0 && len / w != rows) return ZJ_ERR_REF_PANIC;   // (no strip, no call, no panic: the output stays zero)
+        if (n_strips > 0 && len / w != rows && !spec) return ZJ_ERR_REF_PANIC;   // (no strip, no call, no panic: the output stays zero)
         d.gray_rows_ok = 1;
         d.gray_brows = n_strips * (rows / 8);
-        // X86 variant: producer / consumer kernel over pairs of block rows; SCALAR (unclamped DC-only samples): gray_kernel
-        pl->fast = img->variant == ZJ_VARIANT_X86 && !getenv("ZJ_NO_FAST");
+        // X86 variant (and SPEC, whose grey output is the X86 luma plane): producer / consumer kernel over pairs of block rows;
+        // SCALAR (unclamped DC-only samples): gray_kernel
+        pl->fast = img->variant != ZJ_VARIANT_SCALAR && !getenv("ZJ_NO_FAST");
         if (pl->fast) {
             const uint32_t ucols = (d.Wp + 15) / 16;
             d.n_tiles = (ucols + ZF_XU_GRAY - 1) / ZF_XU_GRAY;
@@ -149,6 +156,13 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
             d.n_tiles = (d.Wp / 8 + ZJ_THREADS - 1) / ZJ_THREADS;
         }
         pl->grid_tiles = d.n_tiles;
+    } else if (spec) {
+        // spec_kernel: tiles of exactly TM MCU columns, so that every tile starts on a 16-pixel boundary
+        const int tmv[4] = {TM_NONE, TM_H, TM_V, TM_HV};
+        d.n_tiles = (mcu_x + tmv[mode] - 1) / tmv[mode];
+        d.tile_q = tmv[mode];
+        pl->grid_tiles = d.n_tiles;
+        return ZJ_OK;
     } else if (kind == OUT_YCC) {
         d.n_norm = w; d.P = 3 * w;
     } else if (kind == OUT_RGB) {
@@ -336,7 +350,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         b->algo_bytes += plans[i].out_size;
         for (uint32_t z = 0; z < plans[i].ncomp_used; z++) b->algo_bytes += (uint64_t)plans[i].n_strips * plans[i].chunk[z] * 2;
     }
-    auto key = [&](size_t i) { return plans[i].gray * 32 + plans[i].fast * 16 + plans[i].mode * 2 + plans[i].variant; };
+    auto key = [&](size_t i) { return plans[i].gray * 32 + plans[i].fast * 16 + plans[i].mode * 4 + plans[i].variant; };
     std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t c) { return key(a) < key(c); });
     std::vector<DevImage> host(order.size());
     for (size_t k = 0; k < order.size(); k++) host[k] = plans[order[k]].dev;
@@ -1058,6 +1072,7 @@ int zj_image_strip_range(const zj_image *img, uint32_t strip_begin, uint32_t str
     if (rc) return rc;
     if (n_strips) *n_strips = pl.n_strips;
     if (!sub && !out_offset && !out_bytes) return ZJ_OK;           // a query for the strip count
+    if (img->variant == ZJ_VARIANT_SPEC) return ZJ_ERR_UNSUPPORTED;  // its rows need chroma context from neighbouring strips
     if (strip_begin > strip_end || strip_end > pl.n_strips) return ZJ_ERR_INVALID_ARG;
     const size_t row_bytes = (size_t)img->width * num_components(img->out_cs);
     // the range that holds the last strip also owns the rows below it; an image without strips is one (empty) range at 0

@@ -145,9 +145,9 @@ constexpr int HUFF_LOOKAHEAD = 9;  // src/huffman.rs:9
 
 // Host-stage quirks of the reference (DESIGN.md section 2), reproduced by default.  zj_host_set_quirks() clears bits for
 // TESTS ONLY: with a bit cleared the corresponding lines behave the way libjpeg does, which is how tests/test_quirks.py
-// shows that each deviation from libjpeg on the reference's own fixtures comes from exactly the cited lines.
+// shows that each deviation from libjpeg on the reference's own fixtures comes from exactly the cited lines.  Every decode takes
+// its mask from here when it starts (zj_decoder::quirks); a spec-output decode (ZJ_USE_SPEC_OUTPUT) runs with none of them.
 static std::atomic<uint32_t> g_quirks{ZJ_QUIRK_ALL};
-static inline bool quirk(uint32_t bit) { return (g_quirks.load(std::memory_order_relaxed) & bit) != 0; }
 
 struct HuffmanTable {  // src/huffman.rs:14-41
     int32_t maxcode[18];
@@ -161,7 +161,7 @@ struct HuffmanTable {  // src/huffman.rs:14-41
 };
 
 // HuffmanTable::new + make_derived_table, src/huffman.rs:45-276
-static void build_huffman(HuffmanTable &p, const uint8_t codes[17], const uint8_t values[256], bool is_dc, bool is_progressive)
+static void build_huffman(HuffmanTable &p, const uint8_t codes[17], const uint8_t values[256], bool is_dc, bool is_progressive, bool q9)
 {
     const int32_t too_long = (HUFF_LOOKAHEAD + 1) << HUFF_LOOKAHEAD;
     memset(p.maxcode, 0, sizeof(p.maxcode));
@@ -229,7 +229,7 @@ static void build_huffman(HuffmanTable &p, const uint8_t codes[17], const uint8_
                     if (kk < m) kk = (int16_t)(kk + (int16_t)((int16_t)(~0u << mag_bits) + 1));
                     // Q9 (huffman.rs:249-252): the entry is an i16, so `k << 10` keeps only 6 bits of k: |k| >= 32 decodes wrong.
                     // Quirk off: such values stay out of the fast table and take the general path below it.
-                    const int16_t lim = quirk(ZJ_QUIRK_Q9_FAST_AC_I16) ? 128 : 32;
+                    const int16_t lim = q9 ? 128 : 32;
                     if (kk >= -lim && kk <= lim - 1) p.ac_lookup[i] = (int16_t)((kk << 10) + (run << 4) + (len + mag_bits));
                 }
             }
@@ -249,7 +249,7 @@ struct BitStream {  // src/bitstream.rs:94-114
     Marker marker{};
     uint8_t successive_high = 0, successive_low = 0, spec_start = 0, spec_end = 0;
     int32_t eob_run = 0;
-    bool q10 = quirk(ZJ_QUIRK_Q10_DC_REFILL);   // decode_dc refills only below 16 buffered bits (bitstream.rs:278-281)
+    bool q10 = true;   // Q10: decode_dc refills only below 16 buffered bits (bitstream.rs:278-281); set from zj_decoder::quirks
 
     static bool has_byte_ff(uint32_t b)  // has_byte(b, 255), bitstream.rs:705-717
     {
@@ -602,6 +602,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
 
     void reset_state()  // a fresh Decoder::default(options) for every call, keeping the plane buffers
     {
+        quirks = spec() ? 0u : g_quirks.load();
         const uint32_t keep_cs = user_out_cs;
         options.out_colorspace = keep_cs;
         info = zj_image_info{};
@@ -621,6 +622,15 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         todo = 0x7fffffff;
     }
     uint32_t user_out_cs = ZJ_CS_RGB;
+    uint32_t quirks = ZJ_QUIRK_ALL;   // the host-stage quirks of this decode (g_quirks when it started; none for spec output)
+    bool quirk(uint32_t bit) const { return (quirks & bit) != 0; }
+    bool spec() const { return options.use_unsafe == ZJ_USE_SPEC_OUTPUT; }
+    // a one-component image: GRAYSCALE output (headers.rs:278-285, mcu.rs:171-196), except that spec output keeps RGB / RGBA / RGBX
+    void gray_input_out_cs()
+    {
+        const uint32_t cs = options.out_colorspace;
+        if (!(spec() && (cs == ZJ_CS_RGB || cs == ZJ_CS_RGBA || cs == ZJ_CS_RGBX))) options.out_colorspace = ZJ_CS_GRAYSCALE;
+    }
 
     static size_t out_components(uint32_t cs)
     {
@@ -657,8 +667,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             dht_length -= symbols_sum;
             uint8_t symbols[256] = {0};
             buf.read_exact(symbols, (size_t)symbols_sum, ZJ_DE_FORMAT, "Could not read symbols into the buffer\nfailed to fill whole buffer");
-            if (dc_or_ac == 0) build_huffman(dc_tables[index], num_symbols, symbols, true, is_progressive);
-            else build_huffman(ac_tables[index], num_symbols, symbols, false, is_progressive);
+            if (dc_or_ac == 0) build_huffman(dc_tables[index], num_symbols, symbols, true, is_progressive, quirk(ZJ_QUIRK_Q9_FAST_AC_I16));
+            else build_huffman(ac_tables[index], num_symbols, symbols, false, is_progressive, quirk(ZJ_QUIRK_Q9_FAST_AC_I16));
         }
         if (dht_length > 0) FAIL(ZJ_DE_HUFFMAN_DECODE, "Bogus Huffman table definition");
     }
@@ -714,7 +724,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         const uint16_t expected = (uint16_t)(8 + 3 * (uint16_t)num_components);
         if (length != expected)
             FAIL(ZJ_DE_SOF_ERROR, fmt("Length of start of frame differs from expected %u,value is %u", (unsigned)expected, (unsigned)length));
-        if (num_components == 1) { input_colorspace = ZJ_CS_GRAYSCALE; options.out_colorspace = ZJ_CS_GRAYSCALE; }
+        if (num_components == 1) { input_colorspace = ZJ_CS_GRAYSCALE; gray_input_out_cs(); }
         info.components = num_components;
         std::vector<Component> comps;
         for (int i = 0; i < num_components; i++) {
@@ -898,6 +908,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     };
     struct BaselineGeom {
         size_t mcu_w = 0, mcu_h = 0, bias = 1, width_stride = 0, hv_width_stride = 0, out_nc = 0, ncomp = 0;
+        size_t total = 0;   // MCUs the scan decodes
         bool is_hv = false, zero_per_strip = false;
         size_t strip_len[3] = {0, 0, 0};
     };
@@ -1011,7 +1022,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     // sequential loop would have gone through the very same states.  Anything else returns false with the planes dirty.
     bool baseline_parallel(const Cursor &reader0, const ScanState &st0, const BaselineGeom &g, size_t threads)
     {
-        const size_t total = g.mcu_h * g.bias * g.mcu_w;
+        const size_t total = g.total;
         // a conformant stream has DRI MCUs per interval = DRI * ncomp ticks of the countdown (Q8: it ticks once per
         // component), so it fires ncomp times per interval and only the last firing, at the interval's end, meets the marker
         const size_t per_seg = restart_interval;
@@ -1045,7 +1056,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
                 Cursor rd = reader0;
                 ScanState st;
                 if (k == 0) st = st0;
-                else { rd.pos = ends[k - 1]; st.todo = restart_interval; }
+                else { rd.pos = ends[k - 1]; st.todo = restart_interval; st.stream.q10 = quirk(ZJ_QUIRK_Q10_DC_REFILL); }
                 const size_t first = k * per_seg, last = std::min(total, first + per_seg);
                 const bool must_reset = k + 1 < n_seg;
                 try {
@@ -1074,8 +1085,10 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         size_t mcu_w, mcu_h, bias = 1;
         if (interleaved) {
             set_upsampling();
-            if (sub_sample_ratio == SS_H) { mcu_w = mcu_x * 2; mcu_h = mcu_y / 2; }
-            else if (sub_sample_ratio == SS_HV) { mcu_w = mcu_x; mcu_h = mcu_y / 2; bias = 2; }
+            // Q1: strips of two MCU rows, an odd last MCU row is dropped; spec output decodes it, in a half-empty last strip
+            const size_t strips2 = spec() ? (mcu_y + 1) / 2 : mcu_y / 2;
+            if (sub_sample_ratio == SS_H) { mcu_w = mcu_x * 2; mcu_h = strips2; }
+            else if (sub_sample_ratio == SS_HV) { mcu_w = mcu_x; mcu_h = strips2; bias = 2; }
             else { mcu_w = mcu_x; mcu_h = mcu_y; }
         } else {
             mcu_w = ((size_t)info.width + 7) / 8;
@@ -1085,7 +1098,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             if (options.strict_mode) FAIL(ZJ_DE_FORMAT_STATIC, "[strict-mode]: Grayscale image with down-sampled component.");
             mcu_w = ((size_t)info.width + 7) / 8;
             h_max = 1;
-            options.out_colorspace = ZJ_CS_GRAYSCALE;
+            gray_input_out_cs();
             v_max = 1;
             sub_sample_ratio = SS_NONE;
             components[0].vertical_sample = 1;
@@ -1096,13 +1109,15 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         }
         const size_t component_capacity = mcu_w * 64;
         g.mcu_w = mcu_w; g.mcu_h = mcu_h; g.bias = bias;
+        g.total = mcu_w * mcu_h * bias;
+        if (spec() && (sub_sample_ratio == SS_H || sub_sample_ratio == SS_HV)) g.total = mcu_x * mcu_y;
         g.is_hv = sub_sample_ratio == SS_HV;
         g.out_nc = out_components(options.out_colorspace);
         g.ncomp = in_components();
         g.width_stride = (component_capacity * components[0].vertical_sample * components[0].horizontal_sample * bias) >> 1;
         g.hv_width_stride = g.width_stride >> 1;
         // the reference's output Vec must have one chunk per strip, or chunks.next().unwrap() panics (mcu.rs:354)
-        {
+        if (!spec()) {
             const size_t capacity = (size_t)(uint16_t)(info.width + 8) * (size_t)(uint16_t)(info.height + 8);
             const size_t extra = (interleaved ? 128u : 0u) * (size_t)info.height * g.out_nc;
             const size_t chunk = (size_t)info.width * g.out_nc * 8 * h_max * v_max;
@@ -1125,7 +1140,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         last_entropy_segments = 0;
         size_t threads = entropy_threads ? entropy_threads : (options.num_threads ? options.num_threads : std::thread::hardware_concurrency());
         if (threads == 0) threads = 1;
-        const size_t total = g.mcu_w * g.mcu_h * g.bias;
+        const size_t total = g.total;
         plane_block.ensure(planes, plane_len, have_device, false);
         // zeroing all planes at once, for the interval-parallel form (whose intervals start anywhere inside a strip): split over
         // the threads too -- 200 MB of planes of an 8192^2 image take as long to clear as to entropy-decode on 8 threads
@@ -1147,6 +1162,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             sink->begin(img, g.mcu_h);
         }
         ScanState st;
+        st.stream.q10 = quirk(ZJ_QUIRK_Q10_DC_REFILL);
         for (size_t pos = 0; pos < g.ncomp && pos < 3; pos++) st.dc_pred[pos] = components[pos].dc_pred;
         st.todo = todo;
         // worth the thread start-up only for scans of some size (about 0.1 ms of Huffman work per 4096 blocks)
@@ -1175,7 +1191,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     bool gpu_entropy_prepare(const Cursor &reader, GpuPrep &pp)
     {
         if (is_progressive || restart_interval == 0 || todo != restart_interval) return false;
-        if (g_quirks.load() != ZJ_QUIRK_ALL) return false;   // the GPU form carries the quirks as written; test switches -> host stage
+        if (quirks != ZJ_QUIRK_ALL) return false;   // the GPU form carries the quirks as written; test switches and spec output -> host stage
         if (reader.len >= 0xFFFFFFF0ull) return false;
         try { baseline_setup(pp.g); } catch (DecodeError &) { return false; }
         const BaselineGeom &g = pp.g;
@@ -1184,7 +1200,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             if (c.dc_pred != 0 || !dc_tables[c.dc_huff_table & 3].present || !ac_tables[c.ac_huff_table & 3].present) return false;
             if (g.strip_len[pos] > 0x7FFFFFFFull || plane_len[pos] > ((size_t)1 << 40)) return false;
         }
-        pp.total = g.mcu_w * g.mcu_h * g.bias;
+        pp.total = g.total;
         if (pp.total <= restart_interval || pp.total > 0x7FFFFFFFull) return false;
         pp.n_seg = (pp.total + restart_interval - 1) / restart_interval;
         std::vector<size_t> ends;
@@ -1314,6 +1330,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         check_component_dimensions();
         size_t mw, mh;
         if (interleaved) { mw = mcu_x; mh = mcu_y; } else { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
+        if (spec() && interleaved && h_max == 2) mh += mh & 1;   // 4:2:2 / 4:2:0 spec output reads whole strips of two MCU rows
         mw *= 64;
         if (components.size() < in_components()) FAIL(ZJ_DE_FORMAT, "missing components");
         for (size_t i = 0; i < 3; i++) plane_len[i] = 0;
@@ -1321,6 +1338,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         plane_block.ensure(planes, plane_len, have_device, true);
         size_t seen_scans = 1;
         BitStream stream;
+        stream.q10 = quirk(ZJ_QUIRK_Q10_DC_REFILL);
         stream.update_progressive_params(succ_high, succ_low, spec_start, spec_end);
         parse_entropy_coded_data(reader, stream);
         if (!stream.has_marker) FAIL(ZJ_DE_FORMAT_STATIC, "Marker missing where expected");
@@ -1361,7 +1379,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         img->height = info.height;
         img->n_comp = (uint32_t)in_components();
         img->out_cs = options.out_colorspace;
-        img->variant = options.use_unsafe ? ZJ_VARIANT_X86 : ZJ_VARIANT_SCALAR;
+        img->variant = spec() ? ZJ_VARIANT_SPEC : (options.use_unsafe ? ZJ_VARIANT_X86 : ZJ_VARIANT_SCALAR);
         img->flags = is_progressive ? ZJ_FLAG_PROGRESSIVE : 0;
         for (size_t z = 0; z < in_components(); z++) {
             zj_component &c = img->comp[z];
@@ -1479,6 +1497,9 @@ struct PipeSink : StripSink {
         uint32_t plan_strips = 0;
         // only when the image plans, has as many strips as the host stage counts, and is worth cutting
         if (zj_image_strip_range(&img, 0, 0, nullptr, nullptr, nullptr, &plan_strips) != ZJ_OK || plan_strips != ns) return;
+        zj_image whole;
+        size_t off = 0, bytes = 0;
+        if (zj_image_strip_range(&img, 0, (uint32_t)ns, &whole, &off, &bytes, nullptr) != ZJ_OK) return;   // cannot be cut
         if (zj_output_size(&img) == 0 || zj_output_size(&img) > out_cap) return;
         // a pageable destination makes every download a blocking, staged copy on the thread that queues it (2 GB/s): such
         // callers get the one-shot path, whose single download at least waits for nothing else

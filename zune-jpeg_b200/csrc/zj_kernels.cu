@@ -1715,7 +1715,208 @@ gray_kernel(const DevImage *__restrict__ images, int rows_per_strip)
     }
 }
 
+// ------------------------------------------------------------------------------------- spec-correct kernel
+// ZJ_VARIANT_SPEC (the statement is in include/zune_jpeg_b200.h): every row of the image, libjpeg's integer "fancy"
+// up-sampling with every neighbour index clamped to the real chroma size, JFIF colour, opaque alpha.  No quirk of the reference
+// applies, so the rows of a strip need chroma from the strips above and below and the tiles are simply TM MCU columns wide.
+// grid = (tiles, strips, images); block = ZJ_THREADS.
+//   phase 1: X86 IDCT (idct_block<0>) of the tile's luma and chroma blocks and of the chroma context the filters reach -- one
+//            block column on each side (H, HV) and one block row above and below (V, HV), where it lies inside the real
+//            chroma size -- into shared sample planes;
+//   phase 2: one thread = 16 consecutive pixels of one row, stored as 16-byte words where the row's address allows it.
+__device__ __forceinline__ void jfif_rgb(int y, int cb, int cr, u32 &r, u32 &g, u32 &b)  // jdcolor.c, 16-bit fixed point
+{
+    cb -= 128;
+    cr -= 128;
+    r = clamp255((u32)(y + ((91881 * cr + 32768) >> 16)));
+    g = clamp255((u32)(y + ((-22554 * cb - 46802 * cr + 32768) >> 16)));
+    b = clamp255((u32)(y + ((116130 * cb + 32768) >> 16)));
+}
+
+// (two CTAs per SM: at three, the 80-register cap makes the 16-pixel units of phase 2 spill)
+template <int MODE>
+__global__ void __launch_bounds__(ZJ_THREADS, 2)
+spec_kernel(const DevImage *__restrict__ images)
+{
+    typedef ModeTraits<MODE> MT;
+    constexpr int ROWS = 8 * MT::H * MT::V;   // luma rows per strip
+    constexpr int CROWS = 8 * MT::CBR;        // chroma rows per strip
+    constexpr int TWY = 8 * MT::H * MT::TM;   // luma tile width
+    constexpr int PC = MT::H == 2 ? 8 : 0;    // context columns on each side of the chroma tile
+    constexpr int PR = MT::V == 2 ? 8 : 0;    // context rows above and below it
+    constexpr int CS = 8 * MT::TM + 2 * PC;   // chroma smem row
+    constexpr int UPR = TWY / 16;             // 16-pixel units per row
+    static_assert(TWY % 16 == 0 && CS % 16 == 0, "16-byte units");
+    __shared__ __align__(16) uint8_t sY[ROWS * TWY];
+    __shared__ __align__(16) uint8_t sC[2][(CROWS + 2 * PR) * CS];
+    __shared__ u32 sQ[3][32];
+
+    const DevImage &im = images[blockIdx.z];
+    const int tile = (int)blockIdx.x, strip = (int)blockIdx.y;
+    if (tile >= (int)im.n_tiles || strip >= (int)im.n_strips) return;
+    const int tid = threadIdx.x;
+    const int mcu_x = (int)im.mcu_x, width = (int)im.width, height = (int)im.height;
+    const int m0 = tile * MT::TM, m1 = min(m0 + MT::TM, mcu_x), tm = m1 - m0;
+    const bool color = im.W != 0;                                                  // 0: one-component input
+    const int cw = (width + MT::H - 1) / MT::H, ch = (height + MT::V - 1) / MT::V;  // real chroma size
+    // chroma block rows [rb0, rb1) and block columns [cb0, cb1) of this CTA, context included
+    const int rb0 = strip * MT::CBR - ((PR && strip > 0) ? 1 : 0);
+    const int rb1 = (strip + 1) * MT::CBR + ((PR && (strip + 1) * CROWS < ch) ? 1 : 0);
+    const int cb0 = m0 - ((PC && m0 > 0) ? 1 : 0);
+    const int cb1 = m1 + ((PC && m1 * 8 < cw) ? 1 : 0);
+    const int ccols = cb1 - cb0;
+    const int nY = MT::YBR * MT::H * tm, nC = color ? (rb1 - rb0) * ccols : 0;
+    const int total = nY + 2 * nC;
+    const int ybpr = MT::H * mcu_x;
+    const float r_htm = __frcp_rn((float)(MT::H * tm)), r_cc = __frcp_rn((float)ccols);
+    for (int k = tid; k < 96; k += ZJ_THREADS) sQ[k >> 5][k & 31] = im.qtw[k >> 5][k & 31];
+    __syncthreads();
+
+    // ---------------------------------------------------------------- phase 1
+    for (int b0 = 0; b0 < total; b0 += ZJ_THREADS) {   // CTA-uniform trip count: every lane takes part in the warp votes
+        const int b = b0 + tid;
+        const bool active = b < total;
+        const int16_t *src = nullptr;
+        const u32 *qt = sQ[0];
+        uint8_t *dst = sY;
+        int dstride = TWY;
+        if (!active) {
+        } else if (b < nY) {
+            const int br = div_small(b, r_htm), bc = b - br * (MT::H * tm);
+            src = im.coeff[0] + (((size_t)strip * MT::YBR + br) * ybpr + (size_t)MT::H * m0 + bc) * 64;
+            dst = sY + br * 8 * TWY + bc * 8;
+        } else {
+            int c = b - nY;
+            const int comp = c >= nC ? 1 : 0;
+            c -= comp * nC;
+            const int r = div_small(c, r_cc), k = c - r * ccols;
+            const int br = rb0 + r, bc = cb0 + k;
+            src = im.coeff[1 + comp] + ((size_t)br * mcu_x + bc) * 64;
+            qt = sQ[1 + comp];
+            dst = sC[comp] + ((br - strip * MT::CBR) * 8 + PR) * CS + (bc - m0) * 8 + PC;
+            dstride = CS;
+        }
+        int4 raw[8];
+        load_block(active, src, raw);
+        idct_block<0, uint8_t>(active, raw, qt, dst, dstride);
+    }
+    __syncthreads();
+
+    // ---------------------------------------------------------------- phase 2
+    const int nc = (int)im.nc;
+    const bool ycc = im.out_kind == OUT_YCC;
+    const int xt = 8 * MT::H * m0;              // first luma column of the tile
+    const int ct0 = 8 * m0 - PC;                // chroma column of smem column 0
+    const int cr0 = strip * CROWS - PR;         // chroma row of smem row 0
+    for (int u = tid; u < ROWS * UPR; u += ZJ_THREADS) {
+        const int yl = u / UPR, ux = u - yl * UPR;
+        const int y = strip * ROWS + yl, x0 = xt + 16 * ux;
+        if (y >= height || x0 >= width) continue;
+        const int npx = min(16, width - x0);
+        const uint4 yv = *reinterpret_cast<const uint4 *>(sY + yl * TWY + 16 * ux);
+        const u32 yw[4] = {yv.x, yv.y, yv.z, yv.w};
+        // chroma rows: j, and for V / HV the vertical neighbour jn (j - 1 for even rows, j + 1 for odd ones)
+        int j = y, jn = y;
+        if (MT::V == 2) { j = y >> 1; jn = (y & 1) ? min(j + 1, ch - 1) : max(j - 1, 0); }
+        // H / HV: s[t] = the (column-summed) chroma sample at column clamp(x0 / 2 - 1 + t), t = 0..9
+        int s[2][10];
+        u32 cv[2][4];
+        if (color) {
+#pragma unroll
+            for (int comp = 0; comp < 2; comp++) {
+                const uint8_t *ra = sC[comp] + (j - cr0) * CS - ct0, *rn = sC[comp] + (jn - cr0) * CS - ct0;
+                if (MT::H == 2) {
+#pragma unroll
+                    for (int t = 0; t < 10; t++) {
+                        const int ci = min(max((x0 >> 1) - 1 + t, 0), cw - 1);
+                        s[comp][t] = MT::V == 2 ? 3 * (int)ra[ci] + (int)rn[ci] : (int)ra[ci];
+                    }
+                } else {
+                    const uint4 a = *reinterpret_cast<const uint4 *>(ra + x0);
+                    cv[comp][0] = a.x; cv[comp][1] = a.y; cv[comp][2] = a.z; cv[comp][3] = a.w;
+                    if (MT::V == 2) {
+                        const uint4 n = *reinterpret_cast<const uint4 *>(rn + x0);
+                        const u32 nw[4] = {n.x, n.y, n.z, n.w};
+                        const u32 bias = (y & 1) ? 2u : 1u;
+#pragma unroll
+                        for (int q = 0; q < 4; q++) {
+                            u32 o = 0;
+#pragma unroll
+                            for (int e = 0; e < 4; e++) {
+                                const u32 av = (cv[comp][q] >> (8 * e)) & 0xffu, nv = (nw[q] >> (8 * e)) & 0xffu;
+                                o |= ((3u * av + nv + bias) >> 2) << (8 * e);
+                            }
+                            cv[comp][q] = o;
+                        }
+                    }
+                }
+            }
+        }
+        u32 w[16];
+#pragma unroll
+        for (int k = 0; k < 16; k++) w[k] = 0;
+#pragma unroll
+        for (int k = 0; k < 16; k++) {
+            const int yy = (int)((yw[k >> 2] >> (8 * (k & 3))) & 0xffu);
+            int cb = yy, cr = yy;
+            if (color) {
+                if (MT::H == 2) {
+                    const int t = (k >> 1) + 1;   // s index of this pixel's chroma column
+                    if (MT::V == 2) {
+                        cb = (k & 1) ? (3 * s[0][t] + s[0][t + 1] + 7) >> 4 : (3 * s[0][t] + s[0][t - 1] + 8) >> 4;
+                        cr = (k & 1) ? (3 * s[1][t] + s[1][t + 1] + 7) >> 4 : (3 * s[1][t] + s[1][t - 1] + 8) >> 4;
+                    } else {
+                        cb = (k & 1) ? (3 * s[0][t] + s[0][t + 1] + 2) >> 2 : (3 * s[0][t] + s[0][t - 1] + 1) >> 2;
+                        cr = (k & 1) ? (3 * s[1][t] + s[1][t + 1] + 2) >> 2 : (3 * s[1][t] + s[1][t - 1] + 1) >> 2;
+                    }
+                } else {
+                    cb = (int)((cv[0][k >> 2] >> (8 * (k & 3))) & 0xffu);
+                    cr = (int)((cv[1][k >> 2] >> (8 * (k & 3))) & 0xffu);
+                }
+            }
+            u32 p0 = (u32)yy, p1 = (u32)cb, p2 = (u32)cr;
+            if (color && !ycc) jfif_rgb(yy, cb, cr, p0, p1, p2);
+            if (nc == 4) {
+                w[k] = p0 | (p1 << 8) | (p2 << 16) | 0xff000000u;
+            } else {
+                const u32 px[3] = {p0, p1, p2};
+#pragma unroll
+                for (int c = 0; c < 3; c++) w[(3 * k + c) >> 2] |= px[c] << (8 * ((3 * k + c) & 3));
+            }
+        }
+        uint8_t *d = im.out + ((size_t)y * width + x0) * nc;
+        const int nbytes = npx * nc, nw = 4 * nc;   // bytes of this unit, words of a whole unit
+        const uintptr_t a = reinterpret_cast<uintptr_t>(d);
+        if (npx == 16 && (a & 15) == 0) {
+            uint4 *d4 = reinterpret_cast<uint4 *>(d);
+            d4[0] = make_uint4(w[0], w[1], w[2], w[3]);
+            d4[1] = make_uint4(w[4], w[5], w[6], w[7]);
+            d4[2] = make_uint4(w[8], w[9], w[10], w[11]);
+            if (nc == 4) d4[3] = make_uint4(w[12], w[13], w[14], w[15]);
+        } else if ((a & 3) == 0) {
+            u32 *dw = reinterpret_cast<u32 *>(d);
+#pragma unroll
+            for (int k = 0; k < 16; k++) if (k < nw && 4 * k + 4 <= nbytes) dw[k] = w[k];
+#pragma unroll
+            for (int k = 0; k < 16; k++)
+                if (k < nw && 4 * k < nbytes && 4 * k + 4 > nbytes)
+                    for (int e = 0; e < 3; e++) if (4 * k + e < nbytes) d[4 * k + e] = (uint8_t)(w[k] >> (8 * e));
+        } else {
+#pragma unroll
+            for (int k = 0; k < 64; k++) if (k < nbytes) d[k] = (uint8_t)(w[k >> 2] >> (8 * (k & 3)));
+        }
+    }
+}
+
 // ----------------------------------------------------------------------------------------- host launchers
+template <int MODE>
+static cudaError_t launch_spec(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
+{
+    dim3 grid(g.max_tiles, g.max_strips, g.count);
+    spec_kernel<MODE><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
+    return cudaGetLastError();
+}
+
 template <int MODE, int VARIANT>
 static cudaError_t launch_reconstruct(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
 {
@@ -1908,6 +2109,14 @@ static cudaError_t launch_gray_fast(const DevImage *d_images, const LaunchGroup 
 cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
 {
     if (g.gray && g.fast) return launch_gray_fast(d_images, g, stream);
+    if (g.variant == ZJ_VARIANT_SPEC && !g.gray) {
+        switch (g.mode) {
+        case MODE_NONE: return launch_spec<MODE_NONE>(d_images, g, stream);
+        case MODE_H: return launch_spec<MODE_H>(d_images, g, stream);
+        case MODE_V: return launch_spec<MODE_V>(d_images, g, stream);
+        default: return launch_spec<MODE_HV>(d_images, g, stream);
+        }
+    }
     if (g.fast) {
         switch (g.mode) {
         case MODE_NONE: return launch_fast<MODE_NONE>(d_images, g, stream);
@@ -1919,7 +2128,7 @@ cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStr
     if (g.gray) {
         const int rows = g.mode == MODE_NONE ? 8 : (g.mode == MODE_HV ? 32 : 16);
         dim3 grid(g.max_tiles, g.max_strips * (rows >> 3) + 1, g.count);
-        if (g.variant == 0) gray_kernel<0><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);
+        if (g.variant != ZJ_VARIANT_SCALAR) gray_kernel<0><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);   // X86 or SPEC
         else gray_kernel<1><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);
         return cudaGetLastError();
     }

@@ -85,6 +85,7 @@ class ZuneJpegOptions:
         self._max_scans = 64
         self._strict_mode = False
         self._device = 0
+        self._spec_output = False
 
     @staticmethod
     def new() -> "ZuneJpegOptions":
@@ -118,10 +119,14 @@ class ZuneJpegOptions:
     # not in the reference: which GPU runs the pixel path
     def get_device(self): return self._device
     def set_device(self, device: int): return self._with(_device=int(device))
+    # not in the reference: spec-correct output (every row decoded, libjpeg-style chroma up-sampling, JFIF colour, opaque
+    # alpha; the statement is in include/zune_jpeg_b200.h, ZJ_VARIANT_SPEC)
+    def get_spec_output(self): return self._spec_output
+    def set_spec_output(self, choice: bool): return self._with(_spec_output=bool(choice))
 
     def _raw(self) -> ZjOptions:
         o = ZjOptions()
-        o.use_unsafe = int(self._use_unsafe)
+        o.use_unsafe = _ffi.USE_SPEC_OUTPUT if self._spec_output else int(self._use_unsafe)
         o.out_colorspace = int(self._out_colorspace)
         o.num_threads = self._num_threads
         o.max_width, o.max_height = self._max_width, self._max_height
