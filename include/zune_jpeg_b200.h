@@ -81,6 +81,23 @@ typedef enum zj_variant { ZJ_VARIANT_X86 = 0, ZJ_VARIANT_SCALAR = 1, ZJ_VARIANT_
  * it with zj_options.use_unsafe = ZJ_USE_SPEC_OUTPUT. */
 enum { ZJ_USE_SPEC_OUTPUT = 2 };
 
+/* ZJ_VARIANT_SPEC with ZJ_FLAG_ISLOW in zj_image.flags -- libjpeg-turbo-exact output (DESIGN.md section 4.6.1).  The statement
+ * above with one alternative step 1; steps 2-5 stay as they are:
+ *   1'. Samples: every block of every component goes through jpeg_idct_islow of libjpeg-turbo's jidctint.c, in 32-bit
+ *       two's-complement arithmetic that wraps (as the X86 IDCT does), shifts arithmetic.  CONST_BITS 13, PASS1_BITS 2, the
+ *       FIX_* constants 2446 3196 4433 6270 7373 9633 12299 15137 16069 16819 20995 25172; dequantise (coefficient x table
+ *       entry); pass 1 down the columns, DESCALE(x, 11); pass 2 along the rows, DESCALE(x, 18); DESCALE(x, n) = (x + 2^(n-1)) >> n.
+ *       The sample is range_limit[v & 1023]: v + 128 for v in [0, 127], 255 for [128, 511], 0 for [512, 895], v - 896 for
+ *       [896, 1023].  A column whose coefficients in rows 1-7 are all zero takes jidctint.c's pass-1 shortcut: its 8 values are
+ *       (DC x table entry) << 2.  (That equals the full pass unless the dequantised DC is 2^18 or more in magnitude, where the
+ *       full pass would wrap.)  The pass-2 shortcut for rows whose AC is zero equals the full pass, so it is not part of the
+ *       statement.  Whenever no intermediate leaves 32 bits -- every block an 8-bit JPEG encoder produces -- this equals
+ *       jidctint.c with a 64-bit JLONG; with libjpeg-turbo's fancy up-sampling (step 3) and colour conversion (step 4) it is
+ *       then the decode of libjpeg-turbo's default settings (JDCT_ISLOW, do_fancy_upsampling), i.e. Pillow's.
+ * The flag is valid with ZJ_VARIANT_SPEC only (ZJ_ERR_INVALID_ARG otherwise).  The host stage produces such images with
+ * zj_options.use_unsafe = ZJ_USE_LIBJPEG_OUTPUT: it decodes exactly as for ZJ_USE_SPEC_OUTPUT and sets the flag. */
+enum { ZJ_USE_LIBJPEG_OUTPUT = 3 };
+
 typedef enum zj_status {
     ZJ_OK = 0,
     ZJ_ERR_INVALID_ARG = -1,     /* null pointer, bad enum, inconsistent descriptor                        */
@@ -115,6 +132,8 @@ typedef struct zj_component {
 #define ZJ_FLAG_PROGRESSIVE 1u /* strips come from mcu_prog.rs:188-233 (zip stops silently) instead of
                                   mcu.rs:225-369 (chunks.next().unwrap()) -- only matters when the
                                   over-allocated output runs out of strips, see DESIGN.md                   */
+#define ZJ_FLAG_ISLOW 2u       /* not in the reference: ZJ_VARIANT_SPEC with libjpeg-turbo's islow IDCT as step 1
+                                  (the statement is above, next to ZJ_VARIANT_SPEC's)                        */
 
 typedef struct zj_image {
     uint32_t width, height; /* ImageInfo::width/height (decoder.rs:652-668)                                 */
@@ -292,7 +311,8 @@ ZJ_API uint64_t zj_gpu_launch_count(void);
 
 typedef struct zj_options {       /* ZuneJpegOptions (src/options.rs:6-40), same defaults */
     uint32_t use_unsafe;          /* 1; ZJ_USE_SPEC_OUTPUT (not in the reference): ZJ_VARIANT_SPEC output, and the host stage
-                                     decodes every MCU row with Q9-Q11 off, whatever zj_host_set_quirks says              */
+                                     decodes every MCU row with Q9-Q11 off, whatever zj_host_set_quirks says;
+                                     ZJ_USE_LIBJPEG_OUTPUT: the same, and the images carry ZJ_FLAG_ISLOW                  */
     uint32_t out_colorspace;      /* ZJ_CS_RGB                                           */
     uint32_t num_threads;         /* 4                                                   */
     uint32_t max_width;           /* 16384                                               */

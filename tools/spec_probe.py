@@ -1,14 +1,15 @@
 #!/usr/bin/env python
-"""tools/spec_probe.py [n] -- spec-correct output (ZJ_VARIANT_SPEC) on the bench's workload: n (256) 3840x2160 4:2:0 images,
-resident coefficient planes (8 distinct images, as bench.py's pool), output RGB u8.  Prints the card and its power limit, then:
-  - zj_batch_run of the as-written plan and of the spec plan, alternating, timed with CUDA events (medians), in GP/s;
+"""tools/spec_probe.py [n] -- spec-correct output (ZJ_VARIANT_SPEC) and libjpeg-turbo-exact output (ZJ_VARIANT_SPEC with
+ZJ_FLAG_ISLOW) on the bench's workload: n (256) 3840x2160 4:2:0 images, resident coefficient planes (8 distinct images, as
+bench.py's pool), output RGB u8.  Prints the card and its power limit, then:
+  - zj_batch_run of the as-written plan, the spec plan and the islow plan, alternating, timed with CUDA events (medians), in GP/s;
   - a device-to-device copy in the same run, so that each rate can be stated as a share of the measured copy rate;
-  - the bytes each plan reads and writes: the algorithmic 6 B/px, and for the spec kernel the bytes it reads counting the
-    chroma context blocks it transforms again (computed from the shapes);
-  - JPEG bytes -> f16 CHW (ImageNet mean / std) through decode_batch(device_out, desc), as written and spec, alternating: spec
-    images take the host entropy route, so this shows what that costs.
-Before anything is timed, the spec outputs of the 8 distinct images are checked against the statement (tests/test_spec_output.py)
-and the as-written ones against the oracle."""
+  - the bytes each plan reads and writes: the algorithmic 6 B/px, and for the spec kernel (both IDCTs) the bytes it reads
+    counting the chroma context blocks it transforms again (computed from the shapes);
+  - JPEG bytes -> f16 CHW (ImageNet mean / std) through decode_batch(device_out, desc), as written, spec and libjpeg,
+    alternating: spec and libjpeg images take the host entropy route, so this shows what that costs.
+Before anything is timed, the spec and islow outputs of the 8 distinct images are checked against their statements
+(tests/test_spec_output.py, tests/test_libjpeg_output.py) and the as-written ones against the oracle."""
 import ctypes as C
 import json
 import os
@@ -23,6 +24,7 @@ import torch
 
 import jpeg_util
 import oracle
+from test_libjpeg_output import libjpeg_expected
 from test_spec_output import spec_expected
 from zune_jpeg_b200 import _ffi, gpu
 from zune_jpeg_b200.decoder import ColorSpace, Decoder, ZuneJpegOptions, decode_batch
@@ -72,14 +74,18 @@ def main():
     print(f"card: {card()}", flush=True)
     datas = [jpeg_util.synth_jpeg(i, W, H, "420", 90) for i in range(DISTINCT)]
     spec_opts = ZuneJpegOptions().set_out_colorspace(ColorSpace.RGB).set_spec_output(True)
+    islow_opts = ZuneJpegOptions().set_out_colorspace(ColorSpace.RGB).set_libjpeg_output(True)
+    all_opts = (("as_written", ZuneJpegOptions()), ("spec", spec_opts), ("islow", islow_opts))
+    statement = {"spec": spec_expected, "islow": libjpeg_expected,
+                 "as_written": lambda img, planes: oracle.reconstruct(img, threads=os.cpu_count() or 4)}
     plans = {}
     keep = []
-    wants = {"as_written": [], "spec": []}
-    for name, opts in (("as_written", ZuneJpegOptions()), ("spec", spec_opts)):
+    wants = {name: [] for name, _ in all_opts}
+    for name, opts in all_opts:
         pool = []
         for data in datas:
             img, planes = Decoder.new_with_options(opts).decode_coefficients(data)
-            wants[name].append(spec_expected(img, planes) if name == "spec" else oracle.reconstruct(img, threads=os.cpu_count() or 4))
+            wants[name].append(statement[name](img, planes))
             bufs = [gpu.DeviceBuffer(p.nbytes) for p in planes]
             for b_, p in zip(bufs, planes):
                 b_.upload(p)
@@ -101,7 +107,7 @@ def main():
         for i in range(DISTINCT):
             got = out.download(size, offset=i * size)
             assert np.array_equal(got, wants[name][i]), (name, i, int(np.count_nonzero(got != wants[name][i])))
-    print("outputs checked: spec = the statement, as written = the oracle (8 distinct images)", flush=True)
+    print("outputs checked: spec and islow = their statements, as written = the oracle (8 distinct images)", flush=True)
 
     copy_src = torch.empty(size * N // 2, dtype=torch.uint8, device="cuda")
     copy_dst = torch.empty_like(copy_src)
@@ -109,7 +115,7 @@ def main():
         b.run()
     copy_dst.copy_(copy_src)
     torch.cuda.synchronize()
-    t = {"as_written": [], "spec": [], "copy": []}
+    t = {"as_written": [], "spec": [], "islow": [], "copy": []}
     for _ in range(REPS):
         for name, b in batches.items():
             t[name].append(timed(b.run))
@@ -117,11 +123,11 @@ def main():
     med = {k: float(np.median(v)) for k, v in t.items()}
     copy_rate = 2 * copy_src.numel() / (med["copy"] * 1e-3)           # bytes read + written per second
     res = {"card": card(), "images": N, "width": W, "height": H, "copy_GBps": copy_rate / 1e9}
-    coef = {k: sum(2 * p.size for p in keep[i * DISTINCT][0]) for i, k in enumerate(("as_written", "spec"))}
-    for name in ("as_written", "spec"):
+    coef = {k: sum(2 * p.size for p in keep[i * DISTINCT][0]) for i, (k, _) in enumerate(all_opts)}
+    for name, _ in all_opts:
         ms = med[name]
         algo = N * (coef[name] + size)
-        moved = N * (spec_read_bytes(W, H) + size) if name == "spec" else algo
+        moved = N * (spec_read_bytes(W, H) + size) if name != "as_written" else algo
         res[name] = {"ms": ms, "GPps": N * W * H / (ms * 1e-3) / 1e9, "algo_B_per_px": algo / (N * W * H),
                      "moved_B_per_px": moved / (N * W * H), "share_of_copy_rate": algo / (ms * 1e-3) / copy_rate,
                      "moved_share_of_copy_rate": moved / (ms * 1e-3) / copy_rate, "spread_ms": [min(t[name]), max(t[name])]}
@@ -129,21 +135,21 @@ def main():
     for b in batches.values():
         b.destroy()
 
-    # ---- JPEG bytes -> f16 CHW in device memory, as written and spec
+    # ---- JPEG bytes -> f16 CHW in device memory, as written, spec and libjpeg
     desc = gpu.OutputDesc("CHW", "f16", False, 0, MEAN, INV)
     jdatas = [np.frombuffer(datas[i % DISTINCT], np.uint8) for i in range(JPEG_N)]
     dst = gpu.DeviceBuffer(W * H * 3 * 2 * JPEG_N)
     dev_out = [(dst.ptr + i * W * H * 6, W * H * 6) for i in range(JPEG_N)]
-    jt = {"as_written": [], "spec": []}
+    jt = {name: [] for name, _ in all_opts}
     for rep in range(4):
-        for name, opts in (("as_written", ZuneJpegOptions()), ("spec", spec_opts)):
+        for name, opts in all_opts:
             stats = {}
             t0 = time.perf_counter()
             r = decode_batch(jdatas, opts, threads=0, device_out=dev_out, desc=desc, stats=stats)
             dt = time.perf_counter() - t0
             assert all(x == W * H * 6 for x in r), r
-            if rep == 0 and name == "spec":
-                want = desc.expected(wants["spec"][1], W, H, 3)
+            if rep == 0 and name != "as_written":
+                want = desc.expected(wants[name][1], W, H, 3)
                 assert dst.download(W * H * 6, offset=W * H * 6).tobytes() == want.tobytes()
             if rep > 0:
                 jt[name].append(dt)

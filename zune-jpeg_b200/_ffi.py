@@ -15,7 +15,8 @@ LIB_PATH = os.environ.get("ZJ_LIB_PATH") or os.path.join(_HERE, "csrc", "libzune
 CS_RGB, CS_GRAYSCALE, CS_YCBCR, CS_CMYK, CS_YCCK, CS_RGBA, CS_RGBX = range(7)
 VARIANT_X86, VARIANT_SCALAR, VARIANT_SPEC = 0, 1, 2
 USE_SPEC_OUTPUT = 2   # zj_options.use_unsafe value that selects VARIANT_SPEC
-FLAG_PROGRESSIVE = 1
+USE_LIBJPEG_OUTPUT = 3   # zj_options.use_unsafe value that selects VARIANT_SPEC with FLAG_ISLOW
+FLAG_PROGRESSIVE, FLAG_ISLOW = 1, 2
 QUIRK_Q9, QUIRK_Q10, QUIRK_Q11, QUIRK_ALL = 1, 2, 4, 7   # zj_host_set_quirks (tests only)
 OK = 0
 ERR_INVALID_ARG, ERR_UNSUPPORTED, ERR_SHORT_PLANE, ERR_SHORT_OUTPUT = -1, -2, -3, -4

@@ -45,6 +45,7 @@ int zj::num_components(uint32_t cs)  // ColorSpace::num_components, reference sr
 // --------------------------------------------------------------------------------------------- planning
 struct Plan {
     int mode, variant, gray, zero_only, fast;
+    int islow;         // ZJ_FLAG_ISLOW: the kernels' IDCT is libjpeg-turbo's islow
     uint32_t n_strips, rows, ncomp_used;
     size_t chunk[3];   // i16 per strip per component
     size_t out_size;
@@ -63,6 +64,8 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     if (nc == 0) return ZJ_ERR_INVALID_ARG;
     if (img->variant != ZJ_VARIANT_X86 && img->variant != ZJ_VARIANT_SCALAR && img->variant != ZJ_VARIANT_SPEC) return ZJ_ERR_INVALID_ARG;
     const bool spec = img->variant == ZJ_VARIANT_SPEC;
+    const bool islow = (img->flags & ZJ_FLAG_ISLOW) != 0;   // spec output with libjpeg-turbo's IDCT: every rule below as for spec
+    if (islow && !spec) return ZJ_ERR_INVALID_ARG;
     const uint32_t h = img->comp[0].h_samp, v = img->comp[0].v_samp;
     if (img->n_comp == 1 && (h != 1 || v != 1)) return ZJ_ERR_UNSUPPORTED;  // mcu.rs:171-196 resets these before the path
     for (uint32_t z = 1; z < img->n_comp; z++)
@@ -84,6 +87,7 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     memset(pl, 0, sizeof(*pl));
     pl->mode = mode;
     pl->variant = (int)img->variant;
+    pl->islow = islow;
     uint32_t n_strips, ybr, cbr;
     switch (mode) {
     case MODE_H: n_strips = mcu_y / 2; ybr = 2; cbr = 2; break;   // mcu.rs:147-154 -- Q1: odd MCU row dropped
@@ -144,8 +148,8 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
         d.gray_rows_ok = 1;
         d.gray_brows = n_strips * (rows / 8);
         // X86 variant (and SPEC, whose grey output is the X86 luma plane): producer / consumer kernel over pairs of block rows;
-        // SCALAR (unclamped DC-only samples): gray_kernel
-        pl->fast = img->variant != ZJ_VARIANT_SCALAR && !getenv("ZJ_NO_FAST");
+        // SCALAR (unclamped DC-only samples) and SPEC | ISLOW (the islow luma plane): gray_kernel
+        pl->fast = img->variant != ZJ_VARIANT_SCALAR && !islow && !getenv("ZJ_NO_FAST");
         if (pl->fast) {
             const uint32_t ucols = (d.Wp + 15) / 16;
             d.n_tiles = (ucols + ZF_XU_GRAY - 1) / ZF_XU_GRAY;
@@ -342,7 +346,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
     b->d_images = nullptr;
     b->n_images = 0;
     b->algo_bytes = 0;
-    // group by kernel: (gray, mode, variant); stable so images keep their relative order
+    // group by kernel: (gray, fast, mode, variant, IDCT); stable so images keep their relative order
     std::vector<size_t> order;
     for (size_t i = 0; i < n; i++) {
         if (plans[i].zero_only) b->zero_only.push_back({out_dev[i], plans[i].out_size});
@@ -350,7 +354,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         b->algo_bytes += plans[i].out_size;
         for (uint32_t z = 0; z < plans[i].ncomp_used; z++) b->algo_bytes += (uint64_t)plans[i].n_strips * plans[i].chunk[z] * 2;
     }
-    auto key = [&](size_t i) { return plans[i].gray * 32 + plans[i].fast * 16 + plans[i].mode * 4 + plans[i].variant; };
+    auto key = [&](size_t i) { return plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 + plans[i].variant; };
     std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t c) { return key(a) < key(c); });
     std::vector<DevImage> host(order.size());
     for (size_t k = 0; k < order.size(); k++) host[k] = plans[order[k]].dev;
@@ -358,6 +362,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         size_t e = k;
         LaunchGroup g{};
         g.gray = plans[order[k]].gray; g.mode = plans[order[k]].mode; g.variant = plans[order[k]].variant; g.fast = plans[order[k]].fast;
+        g.islow = plans[order[k]].islow;
         g.first = (uint32_t)k;
         while (e < order.size() && key(order[e]) == key(order[k]) && e - k < 65535) {
             g.max_tiles = std::max(g.max_tiles, plans[order[e]].grid_tiles);

@@ -67,10 +67,11 @@ struct DevImage {
     uint64_t magic_w;         // ceil(2^40 / W): idx / W == (idx * magic_w) >> 40 for idx < 2^20
 };
 
-// Host-side launch plan entry: one kernel launch per (mode, variant, out-kind class) group.
+// Host-side launch plan entry: one kernel launch per (mode, variant, IDCT, out-kind class) group.
 struct LaunchGroup {
     int mode, variant, gray;  // gray = luma-only kernel
     int fast;                 // reconstruct_fast_kernel (X86 variant, aligned output)
+    int islow;                // ZJ_FLAG_ISLOW (SPEC variant only): libjpeg-turbo's islow IDCT
     uint32_t first, count;    // images [first, first+count) of the sorted device array
     uint32_t max_tiles, max_strips;
 };

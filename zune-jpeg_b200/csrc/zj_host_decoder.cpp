@@ -146,7 +146,8 @@ constexpr int HUFF_LOOKAHEAD = 9;  // src/huffman.rs:9
 // Host-stage quirks of the reference (DESIGN.md section 2), reproduced by default.  zj_host_set_quirks() clears bits for
 // TESTS ONLY: with a bit cleared the corresponding lines behave the way libjpeg does, which is how tests/test_quirks.py
 // shows that each deviation from libjpeg on the reference's own fixtures comes from exactly the cited lines.  Every decode takes
-// its mask from here when it starts (zj_decoder::quirks); a spec-output decode (ZJ_USE_SPEC_OUTPUT) runs with none of them.
+// its mask from here when it starts (zj_decoder::quirks); a spec-output decode (ZJ_USE_SPEC_OUTPUT or ZJ_USE_LIBJPEG_OUTPUT)
+// runs with none of them.
 static std::atomic<uint32_t> g_quirks{ZJ_QUIRK_ALL};
 
 struct HuffmanTable {  // src/huffman.rs:14-41
@@ -624,7 +625,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     uint32_t user_out_cs = ZJ_CS_RGB;
     uint32_t quirks = ZJ_QUIRK_ALL;   // the host-stage quirks of this decode (g_quirks when it started; none for spec output)
     bool quirk(uint32_t bit) const { return (quirks & bit) != 0; }
-    bool spec() const { return options.use_unsafe == ZJ_USE_SPEC_OUTPUT; }
+    // spec output, with either IDCT: the host stage is the same for both, only the descriptor's ZJ_FLAG_ISLOW differs
+    bool spec() const { return options.use_unsafe == ZJ_USE_SPEC_OUTPUT || options.use_unsafe == ZJ_USE_LIBJPEG_OUTPUT; }
     // a one-component image: GRAYSCALE output (headers.rs:278-285, mcu.rs:171-196), except that spec output keeps RGB / RGBA / RGBX
     void gray_input_out_cs()
     {
@@ -1380,7 +1382,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         img->n_comp = (uint32_t)in_components();
         img->out_cs = options.out_colorspace;
         img->variant = spec() ? ZJ_VARIANT_SPEC : (options.use_unsafe ? ZJ_VARIANT_X86 : ZJ_VARIANT_SCALAR);
-        img->flags = is_progressive ? ZJ_FLAG_PROGRESSIVE : 0;
+        img->flags = (is_progressive ? ZJ_FLAG_PROGRESSIVE : 0) | (options.use_unsafe == ZJ_USE_LIBJPEG_OUTPUT ? ZJ_FLAG_ISLOW : 0);
         for (size_t z = 0; z < in_components(); z++) {
             zj_component &c = img->comp[z];
             c.coeff = plane_len[z] ? planes[z].p : nullptr;

@@ -260,6 +260,148 @@ __device__ __forceinline__ void idct_block(const bool active, const int4 (&raw)[
     }
 }
 
+// ------------------------------------------------------------------------------------------------ islow IDCT
+constexpr int IDCT_X86 = 0, IDCT_ISLOW = 2;   // spec_kernel's IDCT parameter (gray_kernel's VARIANT: 1 is SCALAR's)
+// libjpeg-turbo's jpeg_idct_islow (jidctint.c): step 1 of ZJ_FLAG_ISLOW images (the statement is in include/zune_jpeg_b200.h).
+// All arithmetic is in Z/2^32, as in the X86 IDCT.  One 1-D pass: CONST_BITS 13, 12 multiplies; the DESCALE rounding comes in as
+// `bias`.  Pass 1 (columns) ends in DESCALE(x, 11).  Pass 2 (rows) ends in range_limit[v], v = DESCALE(x, 18) & 1023 = bits
+// 18-27 of x + 2^17: the table is v + 128 for v in [0, 511] and v - 896 for [512, 1023], each clamped to [0, 255], i.e. v read as
+// a signed 10-bit value, plus 128, clamped (store_row's saturating pack clamps).
+template <bool ROWS>
+__device__ __forceinline__ void islow8(u32 &s0, u32 &s1, u32 &s2, u32 &s3, u32 &s4, u32 &s5, u32 &s6, u32 &s7, const u32 bias)
+{
+    // even part
+    const u32 z1 = (s2 + s6) * 4433u;                                        // FIX_0_541196100
+    const u32 t2 = madk<-15137>(s6, z1), t3 = madk<6270>(s2, z1);           // FIX_1_847759065, FIX_0_765366865
+    const u32 t0 = madk<8192>(s0 + s4, bias), t1 = madk<8192>(s0 - s4, bias);
+    const u32 x0 = t0 + t3, x3 = t0 - t3, x1 = t1 + t2, x2 = t1 - t2;         // tmp10, tmp13, tmp11, tmp12
+    // odd part: z1 = s7 + s1, z2 = s5 + s3, z3 = s7 + s3, z4 = s5 + s1
+    const u32 z3 = s7 + s3, z4 = s5 + s1;
+    const u32 z5 = (z3 + z4) * 9633u;                                        // FIX_1_175875602
+    const u32 p1 = (s7 + s1) * (u32)-7373, p2 = (s5 + s3) * (u32)-20995;   // FIX_0_899976223, FIX_2_562915447
+    const u32 r3 = madk<-16069>(z3, z5), r4 = madk<-3196>(z4, z5);          // FIX_1_961570560, FIX_0_390180644
+    const u32 a = madk<2446>(s7, p1 + r3);                                   // tmp0, FIX_0_298631336
+    const u32 b = madk<16819>(s5, p2 + r4);                                  // tmp1, FIX_2_053119869
+    const u32 c = madk<25172>(s3, p2 + r3);                                  // tmp2, FIX_3_072711026
+    const u32 d = madk<12299>(s1, p1 + r4);                                  // tmp3, FIX_1_501321110
+    const u32 o[8] = {x0 + d, x1 + c, x2 + b, x3 + a, x3 - a, x2 - b, x1 - c, x0 - d};
+    u32 *const s[8] = {&s0, &s1, &s2, &s3, &s4, &s5, &s6, &s7};
+#pragma unroll
+    for (int k = 0; k < 8; k++) *s[k] = ROWS ? (u32)(((int)(o[k] << 4) >> 22) + 128) : (u32)((int)o[k] >> 11);
+}
+
+// Dequantise + islow IDCT of one block, u8 rows written to dst[r*dst_stride + 0..7]; fits load_block like idct_block, and every
+// lane of the warp must call it.  The zero-AC shortcuts of jidctint.c: a block whose AC is all zero has one sample value; the
+// row shortcut of pass 2 equals the full pass and is not taken; the column shortcut of pass 1 equals the full pass unless the
+// dequantised DC is 2^18 or more in magnitude, so it is applied after the full pass, only in warps where such a DC occurs.
+// Warp-uniform sparsity classes fold zero inputs out of the passes, as in idct_block: top-left 4x4 only, rows 6-7 zero, full.
+__device__ __forceinline__ void idct_islow_block(const bool active, const int4 (&raw)[8], const u32 *__restrict__ qtw, uint8_t *__restrict__ dst, int dst_stride)
+{
+    u32 rowor[8], col47 = 0, cor[4] = {0u, 0u, 0u, 0u};
+    rowor[0] = ((u32)raw[0].x & 0xffff0000u) | (u32)raw[0].y | (u32)raw[0].z | (u32)raw[0].w;
+#pragma unroll
+    for (int r = 1; r < 8; r++) {
+        rowor[r] = (u32)raw[r].x | (u32)raw[r].y | (u32)raw[r].z | (u32)raw[r].w;
+        cor[0] |= (u32)raw[r].x; cor[1] |= (u32)raw[r].y; cor[2] |= (u32)raw[r].z; cor[3] |= (u32)raw[r].w;
+    }
+#pragma unroll
+    for (int r = 0; r < 8; r++) col47 |= (u32)raw[r].z | (u32)raw[r].w;
+    u32 dcol = 0;   // bit c: column c has no coefficient in rows 1-7 (jidctint.c's pass-1 shortcut)
+#pragma unroll
+    for (int c = 0; c < 8; c++) dcol |= (((c & 1) ? cor[c >> 1] >> 16 : cor[c >> 1] & 0xffffu) == 0 ? 1u : 0u) << c;
+    const u32 r45 = rowor[4] | rowor[5], r67 = rowor[6] | rowor[7];
+    const u32 acc = rowor[0] | rowor[1] | rowor[2] | rowor[3] | r45 | r67;
+    const bool any_r67 = __any_sync(0xffffffffu, r67 != 0);
+    const bool any_r47 = __any_sync(0xffffffffu, (r45 | r67) != 0);
+    const bool any_c47 = __any_sync(0xffffffffu, col47 != 0);
+    if (!active) return;
+
+    if (acc == 0) {
+        // every column takes the pass-1 shortcut, every row the pass-2 one: range_limit[DESCALE(DC * q << 2, 5) & 1023]
+        const int z = (int)(int16_t)((u32)raw[0].x & 0xffffu) * (int)(qtw[0] & 0xffu);
+        const u32 v = (u32)(((int)((u32)((z * 4 + 16) >> 5) << 22) >> 22) + 128);
+        u32 vv[8];
+#pragma unroll
+        for (int k = 0; k < 8; k++) vv[k] = v;
+#pragma unroll
+        for (int r = 0; r < 8; r++) store_row(dst + r * dst_stride, vv);   // clamps
+        return;
+    }
+
+    u32 a[64];
+    auto dequant_row = [&](int r, int nwords) {
+        const u32 w[4] = {(u32)raw[r].x, (u32)raw[r].y, (u32)raw[r].z, (u32)raw[r].w};
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            if (k < nwords) {
+                const u32 q = qtw[r * 4 + k];
+                a[r * 8 + 2 * k] = dp2a_lo(w[k], q);
+                a[r * 8 + 2 * k + 1] = dp2a_hi(w[k], q);
+            } else {
+                a[r * 8 + 2 * k] = 0;
+                a[r * 8 + 2 * k + 1] = 0;
+            }
+        }
+    };
+    // pass 1 down columns [0, ncols); a column without AC whose DC wraps gets the shortcut value DC << 2 instead
+    auto pass1 = [&](int ncols, bool fix) {
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            if (c >= ncols) continue;
+            const u32 dc = a[c];
+            islow8<false>(a[c], a[8 + c], a[16 + c], a[24 + c], a[32 + c], a[40 + c], a[48 + c], a[56 + c], 1u << 10);
+            if (fix && ((dcol >> c) & 1u)) {
+#pragma unroll
+                for (int r = 0; r < 8; r++) a[r * 8 + c] = dc << 2;
+            }
+        }
+    };
+    // some dequantised DC of row 0 has |value| >= 2^18 (vote of the lanes still here: the outcome only decides who runs the
+    // exact per-lane fix-up of pass1)
+    auto big_dc = [&]() {
+        u32 o = 0;
+#pragma unroll
+        for (int c = 0; c < 8; c++) o |= a[c] + (1u << 18);
+        return __any_sync(__activemask(), dcol != 0 && o >= (1u << 19));
+    };
+    // pass 2 along the rows, and the stores
+    auto pass2 = [&]() {
+#pragma unroll
+        for (int r = 0; r < 8; r++) {
+            islow8<true>(a[r * 8], a[r * 8 + 1], a[r * 8 + 2], a[r * 8 + 3], a[r * 8 + 4], a[r * 8 + 5], a[r * 8 + 6], a[r * 8 + 7], 1u << 17);
+            u32 vv[8];
+#pragma unroll
+            for (int k = 0; k < 8; k++) vv[k] = a[r * 8 + k];
+            store_row(dst + r * dst_stride, vv);   // clamps: range_limit
+        }
+    };
+    // each class runs its own copy of the passes, so that the zeros it knows of fold away
+    if (!any_r47 && !any_c47) {
+#pragma unroll
+        for (int r = 0; r < 8; r++) dequant_row(r, r < 4 ? 2 : 0);
+        pass1(4, big_dc());
+#pragma unroll
+        for (int r = 0; r < 8; r++)
+#pragma unroll
+            for (int c = 4; c < 8; c++) a[r * 8 + c] = 0;   // all-zero columns: 0 by either form of pass 1
+        pass2();
+    } else {
+#pragma unroll
+        for (int r = 0; r < 6; r++) dequant_row(r, 4);
+        const bool fix = big_dc();
+        if (any_r67) {
+            dequant_row(6, 4);
+            dequant_row(7, 4);
+            pass1(8, fix);
+        } else {
+            dequant_row(6, 0);
+            dequant_row(7, 0);
+            pass1(8, fix);
+        }
+        pass2();
+    }
+}
+
 // The IDCT of the fast kernel's producers (X86 variant, u8 planes), written as two short loops instead of one long
 // unrolled body so that it stays resident in the instruction cache next to the consumers' code:
 //   row pass:    row r of the block is read from the thread's staging slot (16-byte chunk r at sl ^ (r << 4)),
@@ -1672,11 +1814,13 @@ reconstruct_fast_kernel(const DevImage *__restrict__ images, const int spc)
 // (YCbCr | GRAYSCALE) -> GRAYSCALE: IDCT of the Y plane only (worker.rs:59,115-118), `as u8` row copy
 // (color_convert/scalar.rs:91-114; Q7 is resolved on the host: geometries where the reference panics are
 // rejected before launch).  grid = (ceil(blocks per block-row / 128), block-rows + 1, images).
+// VARIANT: the IDCT -- 0 = X86, 1 = SCALAR, IDCT_ISLOW = the islow luma plane of ZJ_FLAG_ISLOW images (whose rows all lie in
+// the image's strips, so the reference's geometry rules are no-ops here).
 template <int VARIANT>
 __global__ void __launch_bounds__(ZJ_THREADS)
 gray_kernel(const DevImage *__restrict__ images, int rows_per_strip)
 {
-    typedef typename std::conditional<VARIANT == 0, uint8_t, int16_t>::type ST;
+    typedef typename std::conditional<VARIANT == 1, int16_t, uint8_t>::type ST;
     __shared__ __align__(16) ST sT[ZJ_THREADS][64 + 8];  // one block per thread, padded
     __shared__ u32 sQ[32];
     const DevImage &im = images[blockIdx.z];
@@ -1702,7 +1846,8 @@ gray_kernel(const DevImage *__restrict__ images, int rows_per_strip)
     const size_t blk = (size_t)br * ybpr + (active ? bc : 0);
     int4 raw[8];
     load_block(active, im.coeff[0] + blk * 64, raw);
-    idct_block<VARIANT, ST>(active, raw, sQ, &sT[tid][0], 8);
+    if constexpr (VARIANT == IDCT_ISLOW) idct_islow_block(active, raw, sQ, &sT[tid][0], 8);
+    else idct_block<VARIANT, ST>(active, raw, sQ, &sT[tid][0], 8);
     if (!active) return;
     const u32 x0 = (u32)bc * 8;
 #pragma unroll 1
@@ -1720,9 +1865,9 @@ gray_kernel(const DevImage *__restrict__ images, int rows_per_strip)
 // up-sampling with every neighbour index clamped to the real chroma size, JFIF colour, opaque alpha.  No quirk of the reference
 // applies, so the rows of a strip need chroma from the strips above and below and the tiles are simply TM MCU columns wide.
 // grid = (tiles, strips, images); block = ZJ_THREADS.
-//   phase 1: X86 IDCT (idct_block<0>) of the tile's luma and chroma blocks and of the chroma context the filters reach -- one
-//            block column on each side (H, HV) and one block row above and below (V, HV), where it lies inside the real
-//            chroma size -- into shared sample planes;
+//   phase 1: IDCT of the tile's luma and chroma blocks and of the chroma context the filters reach -- one block column on each
+//            side (H, HV) and one block row above and below (V, HV), where it lies inside the real chroma size -- into shared
+//            sample planes; IDCT_X86: the X86 IDCT (idct_block<0>), IDCT_ISLOW (ZJ_FLAG_ISLOW): idct_islow_block;
 //   phase 2: one thread = 16 consecutive pixels of one row, stored as 16-byte words where the row's address allows it.
 __device__ __forceinline__ void jfif_rgb(int y, int cb, int cr, u32 &r, u32 &g, u32 &b)  // jdcolor.c, 16-bit fixed point
 {
@@ -1734,7 +1879,7 @@ __device__ __forceinline__ void jfif_rgb(int y, int cb, int cr, u32 &r, u32 &g, 
 }
 
 // (two CTAs per SM: at three, the 80-register cap makes the 16-pixel units of phase 2 spill)
-template <int MODE>
+template <int MODE, int IDCT>
 __global__ void __launch_bounds__(ZJ_THREADS, 2)
 spec_kernel(const DevImage *__restrict__ images)
 {
@@ -1798,7 +1943,8 @@ spec_kernel(const DevImage *__restrict__ images)
         }
         int4 raw[8];
         load_block(active, src, raw);
-        idct_block<0, uint8_t>(active, raw, qt, dst, dstride);
+        if constexpr (IDCT == IDCT_ISLOW) idct_islow_block(active, raw, qt, dst, dstride);
+        else idct_block<0, uint8_t>(active, raw, qt, dst, dstride);
     }
     __syncthreads();
 
@@ -1913,7 +2059,8 @@ template <int MODE>
 static cudaError_t launch_spec(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
 {
     dim3 grid(g.max_tiles, g.max_strips, g.count);
-    spec_kernel<MODE><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
+    if (g.islow) spec_kernel<MODE, IDCT_ISLOW><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
+    else spec_kernel<MODE, IDCT_X86><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
     return cudaGetLastError();
 }
 
@@ -2128,7 +2275,8 @@ cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStr
     if (g.gray) {
         const int rows = g.mode == MODE_NONE ? 8 : (g.mode == MODE_HV ? 32 : 16);
         dim3 grid(g.max_tiles, g.max_strips * (rows >> 3) + 1, g.count);
-        if (g.variant != ZJ_VARIANT_SCALAR) gray_kernel<0><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);   // X86 or SPEC
+        if (g.islow) gray_kernel<IDCT_ISLOW><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);
+        else if (g.variant != ZJ_VARIANT_SCALAR) gray_kernel<0><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);   // X86 or SPEC
         else gray_kernel<1><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first, rows);
         return cudaGetLastError();
     }

@@ -86,6 +86,7 @@ class ZuneJpegOptions:
         self._strict_mode = False
         self._device = 0
         self._spec_output = False
+        self._libjpeg_output = False
 
     @staticmethod
     def new() -> "ZuneJpegOptions":
@@ -123,10 +124,17 @@ class ZuneJpegOptions:
     # alpha; the statement is in include/zune_jpeg_b200.h, ZJ_VARIANT_SPEC)
     def get_spec_output(self): return self._spec_output
     def set_spec_output(self, choice: bool): return self._with(_spec_output=bool(choice))
+    # not in the reference: libjpeg-turbo-exact output (spec output with libjpeg-turbo's islow IDCT: byte for byte what Pillow
+    # and other libjpeg-turbo decodes with default settings give; ZJ_FLAG_ISLOW).  Takes precedence over spec output.
+    def get_libjpeg_output(self): return self._libjpeg_output
+    def set_libjpeg_output(self, choice: bool): return self._with(_libjpeg_output=bool(choice))
 
     def _raw(self) -> ZjOptions:
         o = ZjOptions()
-        o.use_unsafe = _ffi.USE_SPEC_OUTPUT if self._spec_output else int(self._use_unsafe)
+        if self._libjpeg_output:
+            o.use_unsafe = _ffi.USE_LIBJPEG_OUTPUT
+        else:
+            o.use_unsafe = _ffi.USE_SPEC_OUTPUT if self._spec_output else int(self._use_unsafe)
         o.out_colorspace = int(self._out_colorspace)
         o.num_threads = self._num_threads
         o.max_width, o.max_height = self._max_width, self._max_height
