@@ -259,10 +259,33 @@ ZJ_API int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image
  *                       ax = fx - float(c0), bx = 1 - ax; rows alike (sy, r0, r1, ay, by).  top = bx*p[r0][c0] + ax*p[r0][c1],
  *                       bot = bx*p[r1][c0] + ax*p[r1][c1], v = by*top + ay*bot.  u8: v rounded to nearest even, clamped to [0, 255].
  *   float outputs       (v - mean[c]) * inv_std[c]; f16 = that value rounded to nearest even.
- * OC = nc, or 3 when channels = 3 and nc = 4; every image of a call must have the same OC. */
+ * OC = nc, or 3 when channels = 3 and nc = 4; every image of a call must have the same OC.
+ *
+ * Pillow's Image.resize (DESIGN.md section 4.5.2): ZJ_FILTER_PIL_BILINEAR and ZJ_FILTER_PIL_BICUBIC (16 + Pillow's Resampling
+ * number) give Pillow's bytes, and with short_side the result of torchvision's Resize(S) + CenterCrop on a PIL image.  Each
+ * channel is independent; for nc = 4 this is Pillow's "RGBX" result, and channels = 3 then gives Pillow's "RGB".
+ *   1. Resized size.  short_side = 0: (RW, RH) = (OW, OH), top = left = 0 (RandomResizedCrop, Resize((h, w))).  short_side =
+ *      S > 0: short = min(w, h), long = max(w, h), new_long = (int)((double)(S * long) / (double)short), (RW, RH) = (S,
+ *      new_long) if w <= h, else (new_long, S); top = round_half_even((RH - OH) / 2.0), left likewise.  RW < OW, RH < OH
+ *      (torchvision would pad), RW > 65535 or RH > 65535: ZJ_ERR_INVALID_ARG.
+ *   2. Coefficients per axis (in = crop size, out = RW or RH, i = index of the full resized axis), IEEE double in the order
+ *      written, no FMA: support0 = 1 (bilinear) or 2 (bicubic); scale = (double)in / out, fs = max(scale, 1.0),
+ *      support = support0 * fs, center = (i + 0.5) * scale, xmin = max((int)(center - support + 0.5), 0),
+ *      xmax = min((int)(center + support + 0.5), in) - xmin; for x < xmax: k[x] = f(((x + xmin) - center + 0.5) * (1.0 / fs)),
+ *      summed in order as ww; k[x] /= ww when ww != 0; kk[x] = (int)(k[x] * 2^22 + 0.5), or (int)(-0.5 + k[x] * 2^22) when
+ *      k[x] < 0.  f: bilinear 1 - |x| on |x| < 1; bicubic (a = -0.5) ((a + 2)|x| - (a + 3))x^2 + 1 on |x| < 1,
+ *      (((|x| - 5)|x| + 8)|x| - 4)a on |x| < 2; 0 elsewhere.
+ *   3. A horizontal pass, then a vertical pass over its u8 result: each value clip8(2^21 + sum(p * kk)) in int32, clip8(s) =
+ *      clamp(s >> 22, 0, 255).  (An axis that keeps its size has weights 1, 0, ...: running its pass equals skipping it.)
+ *   4. The slot holds rows [top, top + OH) x columns [left, left + OW) of that u8 result u; float outputs are
+ *      (float(u) - mean[c]) * inv_std[c]. */
 typedef struct zj_roi { uint32_t x, y, w, h; } zj_roi;                      /* w, h >= 1, x + w <= width, y + h <= height */
-typedef struct zj_resize { uint32_t out_w, out_h, filter, reserved; } zj_resize;   /* out_w, out_h 1..65535; reserved = 0 */
-enum { ZJ_FILTER_AREA = 0, ZJ_FILTER_BILINEAR = 1 };
+/* out_w, out_h 1..65535.  reserved = 0 for AREA and BILINEAR; short_side for the PIL filters (0 = resize straight to out_w x out_h) */
+typedef struct zj_resize {
+    uint32_t out_w, out_h, filter;
+    union { uint32_t reserved; uint32_t short_side; };
+} zj_resize;
+enum { ZJ_FILTER_AREA = 0, ZJ_FILTER_BILINEAR = 1, ZJ_FILTER_PIL_BILINEAR = 18, ZJ_FILTER_PIL_BICUBIC = 19 };
 /* bytes of one slot for images of nc bytes per pixel (0 on a bad descriptor) */
 ZJ_API size_t zj_resize_slot_size(const zj_output_desc *d, const zj_resize *r, uint32_t nc);
 /* The smallest strip range (zj_image_strip_range) whose rows cover [row_begin, row_end), as a virtual image *sub; *sub_row0 =

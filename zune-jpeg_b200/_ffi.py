@@ -62,15 +62,20 @@ class ZjOutputDesc(C.Structure):
     ]
 
 
-FILTER_AREA, FILTER_BILINEAR = 0, 1
+FILTER_AREA, FILTER_BILINEAR, FILTER_PIL_BILINEAR, FILTER_PIL_BICUBIC = 0, 1, 18, 19
 
 
 class ZjRoi(C.Structure):
     _fields_ = [("x", C.c_uint32), ("y", C.c_uint32), ("w", C.c_uint32), ("h", C.c_uint32)]
 
 
+class _ZjResizeLast(C.Union):
+    _fields_ = [("reserved", C.c_uint32), ("short_side", C.c_uint32)]
+
+
 class ZjResize(C.Structure):
-    _fields_ = [("out_w", C.c_uint32), ("out_h", C.c_uint32), ("filter", C.c_uint32), ("reserved", C.c_uint32)]
+    _anonymous_ = ("_u",)
+    _fields_ = [("out_w", C.c_uint32), ("out_h", C.c_uint32), ("filter", C.c_uint32), ("_u", _ZjResizeLast)]
 
 
 class ZjOptions(C.Structure):

@@ -499,6 +499,13 @@ static int launch_runs(const Img *dev, const Img *host, const uint32_t *nc, size
         if constexpr (convert) {
             if (!mw || !mh) continue;   // nothing to write (half size of images one pixel wide or high)
             e = launch_convert(dev + k, (uint32_t)(k1 - k), nc[k], mw, mh, d, s);
+        } else if (pil_filter(r->filter)) {
+            int device = 0, launches = 0;
+            e = cudaGetDevice(&device);
+            if (e == cudaSuccess) e = launch_pil_resize(host + k, (uint32_t)(k1 - k), nc[k], d, *r, device, s, &launches);
+            g_launches.fetch_add(launches);
+            if (e != cudaSuccess) return cuda_fail(e, "PIL resize launch");
+            continue;
         } else {
             e = launch_resize(dev + k, (uint32_t)(k1 - k), nc[k], d, *r, s);
         }
@@ -651,9 +658,9 @@ static int resize_check(const zj_output_desc *d, const zj_resize *r)
     int rc = desc_check(d);
     if (rc) return rc;
     // (sizes up to 65535, as for images: the kernels' window products fit 32 bits)
-    if (d->scale_log2 != 0 || !r || r->out_w == 0 || r->out_h == 0 || r->out_w > 65535 || r->out_h > 65535 || r->filter > ZJ_FILTER_BILINEAR ||
-        r->reserved != 0)
+    if (d->scale_log2 != 0 || !r || r->out_w == 0 || r->out_h == 0 || r->out_w > 65535 || r->out_h > 65535)
         return ZJ_ERR_INVALID_ARG;
+    if (!pil_filter(r->filter) && (r->filter > ZJ_FILTER_BILINEAR || r->reserved != 0)) return ZJ_ERR_INVALID_ARG;
     return ZJ_OK;
 }
 
@@ -672,13 +679,26 @@ static int roi_resolve(const zj_roi *roi, uint32_t width, uint32_t height, zj_ro
     return ZJ_OK;
 }
 
-int zj::resize_admit(const zj_output_desc *d, uint32_t slot_nc, const zj_roi *roi, uint32_t width, uint32_t height, uint32_t nc, zj_roi *crop)
+int zj::resize_admit(const zj_output_desc *d, const zj_resize *r, uint32_t slot_nc, const zj_roi *roi, uint32_t width, uint32_t height,
+                     uint32_t nc, zj_roi *crop)
 {
     if (out_channels(d, nc) != out_channels(d, slot_nc)) return ZJ_ERR_INVALID_ARG;   // one tensor: one channel count
-    return roi_resolve(roi, width, height, crop);
+    int rc = roi_resolve(roi, width, height, crop);
+    PilGeometry g;
+    if (rc == ZJ_OK && pil_filter(r->filter)) rc = pil_geometry(*r, crop->w, crop->h, &g);
+    return rc;
 }
 
-// src: the width x height (rows of it) u8 image the crop lies in, from its row `row0` on
+// The crop rows [*first, *end) the resize reads: all of them, or (PIL filters) the rows of the window's vertical taps
+static void crop_rows(const zj_resize &r, const zj_roi &crop, uint32_t *first, uint32_t *end)
+{
+    PilGeometry g;
+    if (pil_filter(r.filter) && pil_geometry(r, crop.w, crop.h, &g) == ZJ_OK) { *first = g.y0; *end = g.y1; }
+    else { *first = 0; *end = crop.h; }
+}
+
+// src: the width x height (rows of it) u8 image the crop lies in, from its row `row0` on; row0 is the row of the crop's first
+// row the resize reads (crop_rows)
 static ResizeImage resize_image(const uint8_t *src, uint32_t width, uint32_t height, uint32_t nc, uint32_t row0, const zj_roi &roi, void *dst,
                                 const zj_resize &r)
 {
@@ -724,12 +744,14 @@ int zj_gpu_resize_device(int device, void *stream, const uint8_t *src_dev, uint3
     const size_t slot = zj_resize_slot_size(d, r, nc);
     if (slot == 0 || width == 0 || height == 0 || width > 65535 || height > 65535 || !src_dev || !dst_dev) return ZJ_ERR_INVALID_ARG;
     zj_roi crop;
-    int rc = roi_resolve(roi, width, height, &crop);
+    int rc = resize_admit(d, r, nc, roi, width, height, nc, &crop);
     if (rc) return rc;
     if (dst_len < slot) return ZJ_ERR_SHORT_OUTPUT;
     rc = set_device(device);
     if (rc) return rc;
-    const ResizeImage ri = resize_image(src_dev, width, height, nc, crop.y, crop, dst_dev, *r);
+    uint32_t first, end;
+    crop_rows(*r, crop, &first, &end);
+    const ResizeImage ri = resize_image(src_dev, width, height, nc, crop.y + first, crop, dst_dev, *r);
     return run_pass(device, (cudaStream_t)stream, &ri, &nc, 1, *d, r);
 }
 
@@ -739,7 +761,7 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     int rc = resize_check(d, r);
     if (rc) return rc;
     if ((!imgs || !out_dev) && n) return ZJ_ERR_INVALID_ARG;
-    // per image: the crop, the strips that hold its rows and the size of their u8 pixels
+    // per image: the crop, the strips that hold the rows the resize reads and the size of their u8 pixels
     std::vector<zj_image> subs(n);
     std::vector<zj_roi> crops(n);
     std::vector<uint32_t> row0(n), nc(n);
@@ -747,9 +769,11 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     for (size_t i = 0; i < n; i++) {
         if (zj_output_size(&imgs[i]) == 0) { rc = zj_validate_image(&imgs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
         nc[i] = (uint32_t)num_components(imgs[i].out_cs);
-        rc = resize_admit(d, nc[0], rois ? &rois[i] : nullptr, imgs[i].width, imgs[i].height, nc[i], &crops[i]);
+        rc = resize_admit(d, r, nc[0], rois ? &rois[i] : nullptr, imgs[i].width, imgs[i].height, nc[i], &crops[i]);
         if (rc) return rc;
-        rc = zj_image_rows(&imgs[i], crops[i].y, crops[i].y + crops[i].h, &subs[i], &row0[i]);
+        uint32_t first, end;
+        crop_rows(*r, crops[i], &first, &end);
+        rc = zj_image_rows(&imgs[i], crops[i].y + first, crops[i].y + end, &subs[i], &row0[i]);
         if (rc) return rc;
         u8_size[i] = zj_output_size(&subs[i]);
         if (u8_size[i] == 0) { rc = zj_validate_image(&subs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
@@ -792,7 +816,7 @@ int zj::convert_many(int device, void *stream, const U8Image *imgs, size_t n, co
     return run_pass(device, (cudaStream_t)stream, conv.data(), nc.data(), n, *d, nullptr);
 }
 
-// (the crops and channel counts were admitted by the caller: resize_admit)
+// (the crops, channel counts and resized sizes were admitted by the caller: resize_admit)
 int zj::resize_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d, const zj_resize *r)
 {
     int rc = resize_check(d, r);
@@ -804,7 +828,9 @@ int zj::resize_many(int device, void *stream, const U8Image *imgs, size_t n, con
     std::vector<uint32_t> nc(n);
     for (size_t i = 0; i < n; i++) {
         nc[i] = imgs[i].nc;
-        ri[i] = resize_image(imgs[i].src, imgs[i].width, imgs[i].height, nc[i], imgs[i].crop.y, imgs[i].crop, imgs[i].dst, *r);
+        uint32_t first, end;
+        crop_rows(*r, imgs[i].crop, &first, &end);
+        ri[i] = resize_image(imgs[i].src, imgs[i].width, imgs[i].height, nc[i], imgs[i].crop.y + first, imgs[i].crop, imgs[i].dst, *r);
     }
     return run_pass(device, (cudaStream_t)stream, ri.data(), nc.data(), n, *d, r);
 }

@@ -19,6 +19,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstdlib>
 #include <vector>
 
@@ -463,6 +464,319 @@ cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t 
     default: launch_resize_t<float>(d_images, count, nc, oc, chw, area, prm, s); break;
     }
     return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------------ Pillow's resize
+// ZJ_FILTER_PIL_BILINEAR / _BICUBIC (the header's rules 1-4, DESIGN.md section 4.5.2), structured as Pillow's Resample.c: a
+// table kernel builds each image's integer weights for the window's columns and rows, a horizontal pass writes a u8
+// intermediate of the rows the vertical taps read x the window's columns, and a vertical pass writes the slot.
+
+// Double operations of the coefficient rule, each one IEEE round-to-nearest operation: on the device through the intrinsics
+// (nvcc contracts a * b + c into an FMA otherwise), on the host through a volatile product, which no compiler can fuse.
+__host__ __device__ __forceinline__ double pil_add(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+__host__ __device__ __forceinline__ double pil_mul(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    volatile double p = a * b;
+    return p;
+#endif
+}
+__host__ __device__ __forceinline__ double pil_div(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __ddiv_rn(a, b);
+#else
+    volatile double q = a / b;
+    return q;
+#endif
+}
+
+// One output index i of an axis resized from n_in to n_out: the first tap, the tap count, the centre and 1 / fs (rule 2)
+struct PilSpan { int xmin, count; double center, ss; };
+__host__ __device__ __forceinline__ PilSpan pil_span(uint32_t i, uint32_t n_in, uint32_t n_out, double support0)
+{
+    const double scale = pil_div((double)n_in, (double)n_out);
+    const double fs = scale > 1.0 ? scale : 1.0;
+    const double support = pil_mul(support0, fs);
+    PilSpan sp;
+    sp.center = pil_mul(pil_add((double)i, 0.5), scale);
+    sp.xmin = (int)pil_add(pil_add(sp.center, -support), 0.5);
+    if (sp.xmin < 0) sp.xmin = 0;
+    int xmax = (int)pil_add(pil_add(sp.center, support), 0.5);
+    if (xmax > (int)n_in) xmax = (int)n_in;
+    sp.count = xmax - sp.xmin;
+    sp.ss = pil_div(1.0, fs);
+    return sp;
+}
+
+static double pil_support0(uint32_t filter) { return filter == ZJ_FILTER_PIL_BICUBIC ? 2.0 : 1.0; }
+
+int pil_geometry(const zj_resize &r, uint32_t w, uint32_t h, PilGeometry *g)
+{
+    uint64_t rw = r.out_w, rh = r.out_h, left = 0, top = 0;
+    if (r.short_side) {
+        const uint64_t s = r.short_side, sh = std::min(w, h), lg = std::max(w, h);
+        const uint64_t nl = (uint64_t)((double)(s * lg) / (double)sh);   // (one IEEE division, then truncation)
+        rw = w <= h ? s : nl;
+        rh = w <= h ? nl : s;
+        if (rw < r.out_w || rh < r.out_h || rw > 65535 || rh > 65535) return ZJ_ERR_INVALID_ARG;
+        // round_half_even((R - out) / 2.0)
+        const uint64_t dx = rw - r.out_w, dy = rh - r.out_h;
+        left = dx / 2 + ((dx & 1) && ((dx / 2) & 1));
+        top = dy / 2 + ((dy & 1) && ((dy / 2) & 1));
+    }
+    g->rw = (uint32_t)rw; g->rh = (uint32_t)rh; g->left = (uint32_t)left; g->top = (uint32_t)top;
+    // the taps' first rows grow with the output row, and so do their ends: the window's first and last rows bound them
+    const double s0 = pil_support0(r.filter);
+    const PilSpan a = pil_span(g->top, h, g->rh, s0), b = pil_span(g->top + r.out_h - 1, h, g->rh, s0);
+    g->y0 = (uint32_t)a.xmin;
+    g->y1 = (uint32_t)(b.xmin + b.count);
+    return ZJ_OK;
+}
+
+// One image of the PIL launches.  tab: the horizontal table (n = out_w entries: xmin[n], count[n], then kk[x][n] for x < ksh),
+// then at tab_v the vertical one (n = out_h, ksv), xmin relative to the crop; tmp: rows x tpitch u8, crop rows [y0, y0 + rows)
+// x the window's columns, OC bytes per pixel.
+struct PilImage {
+    const uint8_t *src;           // byte 0 of the crop's pixel (0, y0)
+    uint8_t *tmp;
+    void *dst;
+    int *tab;
+    uint32_t pitch, w, h;         // source row bytes, crop size
+    uint32_t rw, rh, left, top;   // resized size, window offset
+    uint32_t y0, rows;
+    uint32_t ksh, ksv, tab_v;
+};
+struct PilParams {
+    uint32_t filter, tpitch;
+};
+
+__device__ __forceinline__ double pil_f(double x, bool bicubic)
+{
+    if (x < 0.0) x = -x;
+    if (!bicubic) return x < 1.0 ? __dadd_rn(1.0, -x) : 0.0;
+    const double a = -0.5;
+    if (x < 1.0) return __dadd_rn(__dmul_rn(__dmul_rn(__dadd_rn(__dmul_rn(a + 2.0, x), -(a + 3.0)), x), x), 1.0);
+    if (x < 2.0) return __dmul_rn(__dadd_rn(__dmul_rn(__dadd_rn(__dmul_rn(__dadd_rn(x, -5.0), x), 8.0), x), -4.0), a);
+    return 0.0;
+}
+
+// One thread per window index and axis (blockIdx.y: 0 = columns, 1 = rows): rule 2's weights, the filter evaluated twice (the
+// sum, then the normalised values) rather than stored
+__global__ void __launch_bounds__(256) pil_table_kernel(const PilImage *__restrict__ images, const ResizeParams prm, const PilParams pp)
+{
+    const PilImage im = images[blockIdx.z];
+    const bool vert = blockIdx.y == 1;
+    const u32 n = vert ? prm.oh : prm.ow;
+    const u32 i = blockIdx.x * 256u + threadIdx.x;
+    if (i >= n) return;
+    const bool bicubic = pp.filter == ZJ_FILTER_PIL_BICUBIC;
+    const PilSpan sp = pil_span(i + (vert ? im.top : im.left), vert ? im.h : im.w, vert ? im.rh : im.rw, bicubic ? 2.0 : 1.0);
+    int *tab = im.tab + (vert ? im.tab_v : 0u);
+    tab[i] = sp.xmin;
+    tab[n + i] = sp.count;
+    double ww = 0.0;
+    for (int x = 0; x < sp.count; x++) ww = __dadd_rn(ww, pil_f(__dmul_rn(__dadd_rn(__dadd_rn((double)(x + sp.xmin), -sp.center), 0.5), sp.ss), bicubic));
+    int *kk = tab + 2 * n + i;
+    for (int x = 0; x < sp.count; x++) {
+        double k = pil_f(__dmul_rn(__dadd_rn(__dadd_rn((double)(x + sp.xmin), -sp.center), 0.5), sp.ss), bicubic);
+        if (ww != 0.0) k = __ddiv_rn(k, ww);
+        kk[(size_t)x * n] = k < 0.0 ? (int)__dadd_rn(-0.5, __dmul_rn(k, 4194304.0)) : (int)__dadd_rn(0.5, __dmul_rn(k, 4194304.0));
+    }
+}
+
+__device__ __forceinline__ u32 clip8(int s) { return (u32)min(max(s >> 22, 0), 255); }
+
+constexpr int PIL_HROWS = 4;   // rows per thread of the horizontal pass: each weight is loaded once for them
+
+// Horizontal pass: a warp owns 32 consecutive window columns of PIL_HROWS intermediate rows (8 warps: 32 rows), a lane one
+// column: per tap one weight (the lanes' weights are consecutive words) and NC bytes per row.  Every byte read lies in the crop.
+template <int NC, int OC>
+__global__ void __launch_bounds__(256) pil_horizontal_kernel(const PilImage *__restrict__ images, const ResizeParams prm, const PilParams pp)
+{
+    const PilImage im = images[blockIdx.z];
+    const u32 j = blockIdx.x * 32u + (threadIdx.x & 31);
+    const u32 r0 = (blockIdx.y * 8u + (threadIdx.x >> 5)) * PIL_HROWS;
+    if (j >= prm.ow || r0 >= im.rows) return;
+    const int nr = (int)min((u32)PIL_HROWS, im.rows - r0);
+    const int xmin = im.tab[j], count = im.tab[prm.ow + j];
+    const int *kk = im.tab + 2 * prm.ow + j;
+    const uint8_t *row[PIL_HROWS];
+#pragma unroll
+    for (int r = 0; r < PIL_HROWS; r++) row[r] = im.src + (size_t)(r0 + min(r, nr - 1)) * im.pitch + (size_t)xmin * NC;   // (rows past the last repeat it)
+    int acc[PIL_HROWS][OC];
+#pragma unroll
+    for (int r = 0; r < PIL_HROWS; r++)
+#pragma unroll
+        for (int c = 0; c < OC; c++) acc[r][c] = 1 << 21;
+    const bool words = NC == 4 && (reinterpret_cast<uintptr_t>(im.src) & 3) == 0;   // (pitch = 4 * width: every pixel aligned)
+    for (int x = 0; x < count; x++) {
+        const int k = __ldg(kk + (size_t)x * prm.ow);
+#pragma unroll
+        for (int r = 0; r < PIL_HROWS; r++) {
+            const uint8_t *p = row[r] + x * NC;
+            if (NC == 4 && words) {
+                const u32 wd = __ldg(reinterpret_cast<const u32 *>(p));
+#pragma unroll
+                for (int c = 0; c < OC; c++) acc[r][c] += (int)((wd >> (8 * c)) & 0xffu) * k;
+            } else {
+#pragma unroll
+                for (int c = 0; c < OC; c++) acc[r][c] += (int)__ldg(p + c) * k;
+            }
+        }
+    }
+    uint8_t *t = im.tmp + (size_t)r0 * pp.tpitch + (size_t)j * OC;
+#pragma unroll
+    for (int r = 0; r < PIL_HROWS; r++)
+        if (r < nr)
+#pragma unroll
+            for (int c = 0; c < OC; c++) t[(size_t)r * pp.tpitch + c] = (uint8_t)clip8(acc[r][c]);
+}
+
+// Vertical pass: a thread produces 8 consecutive pixels of one slot row (8 warps: 8 rows), reading 8 * OC intermediate bytes
+// per tap as OC 8-byte words (tpitch and the window columns are multiples of 8 pixels), and stores them as the resize does.
+template <typename T, bool CHW, int OC>
+__global__ void __launch_bounds__(256) pil_vertical_kernel(const PilImage *__restrict__ images, const ResizeParams prm, const PilParams pp)
+{
+    const PilImage im = images[blockIdx.z];
+    const u32 i = blockIdx.y * RZ_ROWS + (threadIdx.x >> 5);
+    const u32 x0 = 8u * (blockIdx.x * 32u + (threadIdx.x & 31));
+    if (i >= prm.oh || x0 >= prm.ow) return;
+    const int *tv = im.tab + im.tab_v;
+    const int ymin = tv[i] - (int)im.y0, count = tv[prm.oh + i];
+    const int *kk = tv + 2 * prm.oh + i;
+    int acc[8][OC];
+#pragma unroll
+    for (int e = 0; e < 8; e++)
+#pragma unroll
+        for (int c = 0; c < OC; c++) acc[e][c] = 1 << 21;
+    const uint8_t *q = im.tmp + (size_t)ymin * pp.tpitch + (size_t)x0 * OC;
+    for (int y = 0; y < count; y++, q += pp.tpitch) {
+        const int k = __ldg(kk + (size_t)y * prm.oh);
+        uint2 wd[OC];
+#pragma unroll
+        for (int g = 0; g < OC; g++) wd[g] = __ldg(reinterpret_cast<const uint2 *>(q) + g);
+#pragma unroll
+        for (int b = 0; b < 8 * OC; b++) {
+            const u32 word = (b & 7) < 4 ? wd[b >> 3].x : wd[b >> 3].y;
+            acc[b / OC][b % OC] += (int)((word >> (8 * (b & 3))) & 0xffu) * k;
+        }
+    }
+    T v[8][OC];
+#pragma unroll
+    for (int e = 0; e < 8; e++)
+#pragma unroll
+        for (int c = 0; c < OC; c++) {
+            const u32 u = clip8(acc[e][c]);
+            v[e][c] = sizeof(T) == 1 ? (T)u : normalise<T>((float)u, prm.mean[c], prm.inv_std[c]);
+        }
+    store_px8<T, CHW, OC>(reinterpret_cast<T *>(im.dst), prm, i, x0, (int)min(8u, prm.ow - x0), v);
+}
+
+template <typename T, bool CHW>
+static void launch_pil_vertical(const PilImage *d, uint32_t count, uint32_t oc, const ResizeParams &prm, const PilParams &pp, cudaStream_t s)
+{
+    const dim3 grid((prm.ow + 255) / 256, (prm.oh + RZ_ROWS - 1) / RZ_ROWS, count);
+    if (oc == 1) pil_vertical_kernel<T, CHW, 1><<<grid, 256, 0, s>>>(d, prm, pp);
+    else if (oc == 3) pil_vertical_kernel<T, CHW, 3><<<grid, 256, 0, s>>>(d, prm, pp);
+    else pil_vertical_kernel<T, CHW, 4><<<grid, 256, 0, s>>>(d, prm, pp);
+}
+
+template <typename T>
+static void launch_pil_vertical_t(const PilImage *d, uint32_t count, uint32_t oc, bool chw, const ResizeParams &prm, const PilParams &pp, cudaStream_t s)
+{
+    if (chw) launch_pil_vertical<T, true>(d, count, oc, prm, pp, s);
+    else launch_pil_vertical<T, false>(d, count, oc, prm, pp, s);
+}
+
+// Intermediate and table bytes per launch of the passes: a run whose images need more is cut into sub-batches that take turns
+// in one scratch buffer (at least one image each)
+constexpr size_t PIL_CHUNK_BYTES = (size_t)1 << 30;
+
+cudaError_t launch_pil_resize(const ResizeImage *host, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r,
+                              int device, cudaStream_t s, int *launches)
+{
+    ResizeParams prm;
+    for (int c = 0; c < 4; c++) { prm.mean[c] = d.mean[c]; prm.inv_std[c] = d.inv_std[c]; }
+    prm.ow = r.out_w;
+    prm.oh = r.out_h;
+    const uint32_t oc = (d.channels == 3 && nc == 4) ? 3u : nc;
+    PilParams pp;
+    pp.filter = r.filter;
+    pp.tpitch = ((r.out_w + 7u) & ~7u) * oc;
+    const double s0 = pil_support0(r.filter);
+    auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    // per image: geometry, table strides (at most 2 * ceil(support) + 1 taps, as Pillow's), and its table + intermediate bytes
+    std::vector<PilImage> im(count);
+    std::vector<size_t> off(count);
+    struct Chunk { uint32_t first, count, max_rows; size_t bytes; };
+    std::vector<Chunk> chunks;
+    size_t scratch = 0;
+    for (uint32_t k = 0; k < count; k++) {
+        const ResizeImage &ri = host[k];
+        PilGeometry g;
+        if (pil_geometry(r, ri.w, ri.h, &g) != ZJ_OK) return cudaErrorInvalidValue;   // (never: the callers admitted the crops)
+        PilImage &p = im[k];
+        p.src = ri.src; p.dst = ri.dst; p.pitch = ri.pitch; p.w = ri.w; p.h = ri.h;
+        p.rw = g.rw; p.rh = g.rh; p.left = g.left; p.top = g.top; p.y0 = g.y0; p.rows = g.y1 - g.y0;
+        auto ksize = [&](uint32_t n_in, uint32_t n_out) {
+            const double sup = pil_mul(s0, std::max(pil_div((double)n_in, (double)n_out), 1.0));
+            return 2u * (uint32_t)std::ceil(sup) + 1u;
+        };
+        p.ksh = ksize(ri.w, g.rw);
+        p.ksv = ksize(ri.h, g.rh);
+        p.tab_v = (uint32_t)(align((size_t)r.out_w * (2 + p.ksh) * 4) / 4);
+        const size_t tab_bytes = align(((size_t)p.tab_v + (size_t)r.out_h * (2 + p.ksv)) * 4);
+        const size_t bytes = tab_bytes + align((size_t)p.rows * pp.tpitch);
+        if (chunks.empty() || chunks.back().bytes + bytes > PIL_CHUNK_BYTES) chunks.push_back({k, 0, 0, 0});
+        Chunk &ch = chunks.back();
+        off[k] = ch.bytes;
+        ch.bytes += bytes;
+        ch.count++;
+        ch.max_rows = std::max(ch.max_rows, p.rows);
+        scratch = std::max(scratch, ch.bytes);
+    }
+    const size_t desc_bytes = align(count * sizeof(PilImage));
+    uint8_t *buf = nullptr;
+    if (scratch_alloc((void **)&buf, desc_bytes + scratch, device, s) != ZJ_OK) return cudaErrorMemoryAllocation;
+    uint8_t *const work = buf + desc_bytes;
+    for (uint32_t k = 0; k < count; k++) {
+        im[k].tab = reinterpret_cast<int *>(work + off[k]);
+        im[k].tmp = work + off[k] + align(((size_t)im[k].tab_v + (size_t)r.out_h * (2 + im[k].ksv)) * 4);
+    }
+    PilImage *dev = reinterpret_cast<PilImage *>(buf);
+    // (pageable source: the async copy returns once the data sits in the driver's staging buffer)
+    cudaError_t e = cudaMemcpyAsync(dev, im.data(), count * sizeof(PilImage), cudaMemcpyHostToDevice, s);
+    // the sub-batches take turns in the scratch buffer, in the order of s
+    for (size_t c = 0; c < chunks.size() && e == cudaSuccess; c++) {
+        const Chunk &ch = chunks[c];
+        const PilImage *di = dev + ch.first;
+        pil_table_kernel<<<dim3((std::max(r.out_w, r.out_h) + 255) / 256, 2, ch.count), 256, 0, s>>>(di, prm, pp);
+        const dim3 gh((r.out_w + 31) / 32, (ch.max_rows + 8 * PIL_HROWS - 1) / (8 * PIL_HROWS), ch.count);
+        if (nc == 1) pil_horizontal_kernel<1, 1><<<gh, 256, 0, s>>>(di, prm, pp);
+        else if (nc == 3) pil_horizontal_kernel<3, 3><<<gh, 256, 0, s>>>(di, prm, pp);
+        else if (oc == 3) pil_horizontal_kernel<4, 3><<<gh, 256, 0, s>>>(di, prm, pp);
+        else pil_horizontal_kernel<4, 4><<<gh, 256, 0, s>>>(di, prm, pp);
+        const bool chw = d.layout == ZJ_LAYOUT_CHW;
+        switch (d.dtype) {
+        case ZJ_DTYPE_U8: launch_pil_vertical_t<uint8_t>(di, ch.count, oc, chw, prm, pp, s); break;
+        case ZJ_DTYPE_F16: launch_pil_vertical_t<__half>(di, ch.count, oc, chw, prm, pp, s); break;
+        default: launch_pil_vertical_t<float>(di, ch.count, oc, chw, prm, pp, s); break;
+        }
+        *launches += 3;
+        e = cudaGetLastError();
+    }
+    scratch_free(buf, s);
+    return e;
 }
 
 }  // namespace zj

@@ -87,7 +87,7 @@ struct ConvImage {
 // One image of a resize launch (zj_consumer.cu): a crop of interleaved u8 pixels in, one slot of the batch tensor out.  The
 // output size, layout, type and channels are the launch's.
 struct ResizeImage {
-    const uint8_t *src;           // byte 0 of the crop's pixel (0, 0)
+    const uint8_t *src;           // byte 0 of the crop's pixel (0, first): first = 0, or PilGeometry::y0 for the PIL filters
     const uint8_t *lo, *hi;       // the source image's bytes: no load reaches outside [lo, hi)
     void *dst;                    // the image's slot
     uint32_t pitch;               // bytes per source row (width * nc)
@@ -100,13 +100,25 @@ cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStr
 cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
 cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
 
+// The PIL filters (header rules 1 and 2) for a crop of w x h: the resized size, the window's offset in it, and the crop rows
+// [y0, y1) the window's vertical taps read.  ZJ_ERR_INVALID_ARG when the resized size breaks rule 1.
+inline bool pil_filter(uint32_t filter) { return filter == ZJ_FILTER_PIL_BILINEAR || filter == ZJ_FILTER_PIL_BICUBIC; }
+struct PilGeometry { uint32_t rw, rh, left, top, y0, y1; };
+int pil_geometry(const zj_resize &r, uint32_t w, uint32_t h, PilGeometry *g);
+// The PIL resize of images host[0, count) (count <= 65535, one nc): coefficient tables, horizontal and vertical passes, with
+// their scratch from the stream-ordered pool of `device`.  *launches += the kernels launched.  Asynchronous on `s`.
+cudaError_t launch_pil_resize(const ResizeImage *host, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r,
+                              int device, cudaStream_t s, int *launches);
+
 // ---- zj_capi.cu for zj_host_decoder.cpp (hidden symbols, not part of the C ABI)
 int num_components(uint32_t cs);   // output bytes per pixel of colourspace cs (ColorSpace::num_components); 0 = not a colourspace
 // bytes the consumer writes for a width x height image of nc bytes per pixel; 0 = a bad descriptor or nc
 size_t convert_size(uint32_t width, uint32_t height, uint32_t nc, const zj_output_desc *d);
 // *crop = the crop `roi` of a width x height image of nc bytes per pixel (NULL = the whole image), into a batch tensor of
-// slot_nc-byte source pixels; ZJ_ERR_INVALID_ARG when it does not fit the image or the image's channel count is not the slots'
-int resize_admit(const zj_output_desc *d, uint32_t slot_nc, const zj_roi *roi, uint32_t width, uint32_t height, uint32_t nc, zj_roi *crop);
+// slot_nc-byte source pixels; ZJ_ERR_INVALID_ARG when it does not fit the image, the image's channel count is not the slots' or
+// (PIL filters) its resized size breaks rule 1
+int resize_admit(const zj_output_desc *d, const zj_resize *r, uint32_t slot_nc, const zj_roi *roi, uint32_t width, uint32_t height,
+                 uint32_t nc, zj_roi *crop);
 // device memory from this library's stream-ordered pool of `device`, allocated / freed in the order of `stream`
 int scratch_alloc(void **p, size_t bytes, int device, void *stream);
 void scratch_free(void *p, void *stream);

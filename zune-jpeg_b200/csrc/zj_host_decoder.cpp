@@ -2289,7 +2289,7 @@ ZJ_API int zj_decode_batch_gpu_device_resized(const zj_options *o, const uint8_t
         std::vector<zj::U8Image> admitted;
         for (size_t i = 0; i < n; i++) {
             if (status[i] != ZJ_OK) continue;
-            if (zj::resize_admit(d, nc_opt, rois ? &rois[i] : nullptr, img[i].width, img[i].height, img[i].nc, &img[i].crop) != ZJ_OK) {
+            if (zj::resize_admit(d, r, nc_opt, rois ? &rois[i] : nullptr, img[i].width, img[i].height, img[i].nc, &img[i].crop) != ZJ_OK) {
                 status[i] = ZJ_ERR_INVALID_ARG; failed++; continue;
             }
             img[i].dst = static_cast<uint8_t *>(out_dev) + i * slot;

@@ -330,7 +330,54 @@ def convert_device(src: DeviceBuffer, width: int, height: int, nc: int, desc: Ou
 
 
 # ------------------------------------------------------------------ cropped, resized batch tensors (DESIGN.md section 4.5.1)
-_FILTERS = {"area": _ffi.FILTER_AREA, "bilinear": _ffi.FILTER_BILINEAR}
+_FILTERS = {"area": _ffi.FILTER_AREA, "bilinear": _ffi.FILTER_BILINEAR, "pil_bilinear": _ffi.FILTER_PIL_BILINEAR,
+            "pil_bicubic": _ffi.FILTER_PIL_BICUBIC}
+
+
+def _pil_filter(x: float, bicubic: bool) -> float:
+    x = -x if x < 0.0 else x
+    if not bicubic:
+        return 1.0 - x if x < 1.0 else 0.0
+    a = -0.5
+    if x < 1.0:
+        return ((a + 2.0) * x - (a + 3.0)) * x * x + 1
+    if x < 2.0:
+        return (((x - 5) * x + 8) * x - 4) * a
+    return 0.0
+
+
+def pil_coefficients(n_in: int, n_out: int, bicubic: bool, first: int = 0, count: int | None = None):
+    """Rule 2 of the PIL filters for indices [first, first + count) of an axis resized from n_in to n_out: per index (xmin,
+    int64 weights).  Python floats are IEEE doubles and Python evaluates in the order written, without FMA."""
+    scale = n_in / n_out
+    fs = max(scale, 1.0)
+    support = (2.0 if bicubic else 1.0) * fs
+    ss = 1.0 / fs
+    out = []
+    for i in range(first, first + (n_out - first if count is None else count)):
+        center = (i + 0.5) * scale
+        xmin = max(int(center - support + 0.5), 0)
+        xmax = min(int(center + support + 0.5), n_in) - xmin
+        k = [_pil_filter((x + xmin - center + 0.5) * ss, bicubic) for x in range(xmax)]
+        ww = 0.0
+        for w in k:
+            ww += w
+        if ww != 0.0:
+            k = [w / ww for w in k]
+        out.append((xmin, np.array([int(-0.5 + w * (1 << 22)) if w < 0 else int(0.5 + w * (1 << 22)) for w in k], np.int64)))
+    return out
+
+
+def pil_geometry(w: int, h: int, out_w: int, out_h: int, short_side: int = 0):
+    """Rule 1 of the PIL filters: (RW, RH, left, top) for a w x h crop, or None where the call is ZJ_ERR_INVALID_ARG"""
+    if not short_side:
+        return out_w, out_h, 0, 0
+    short, long = (w, h) if w <= h else (h, w)
+    new_long = int(short_side * long / short)
+    rw, rh = (short_side, new_long) if w <= h else (new_long, short_side)
+    if rw < out_w or rh < out_h or rw > 65535 or rh > 65535:
+        return None
+    return rw, rh, int(round((rw - out_w) / 2.0)), int(round((rh - out_h) / 2.0))      # (round: half to even)
 
 
 def _nc_of(img: ZjImage) -> int:
@@ -349,13 +396,19 @@ def _roi_array(rois, sizes):
 
 class Resize:
     """zj_resize: each image's crop resized to size = (OH, OW) with filter "area" (adaptive average pooling: the anti-aliased
-    choice for down-scales) or "bilinear" (torch interpolate, align_corners=False, antialias=False).  Every value is the
-    function of the crop's u8 bytes that expected() states."""
+    choice for down-scales), "bilinear" (torch interpolate, align_corners=False, antialias=False), or Pillow's Image.resize
+    with "pil_bilinear" / "pil_bicubic" (torchvision's resized_crop on a PIL image).  With a PIL filter, short_side = S is
+    torchvision's Resize(S) of the crop followed by CenterCrop(size).  Every value is the function of the crop's u8 bytes that
+    expected() states."""
 
-    def __init__(self, size, filter: str = "area"):
+    def __init__(self, size, filter: str = "area", short_side: int | None = None):
         oh, ow = size
         r = _ffi.ZjResize()
         r.out_w, r.out_h, r.filter = int(ow), int(oh), _FILTERS[filter]
+        if short_side is not None:
+            if filter not in ("pil_bilinear", "pil_bicubic"):
+                raise ValueError("short_side needs a PIL filter")
+            r.short_side = int(short_side)
         self.c = r
 
     @property
@@ -379,7 +432,29 @@ class Resize:
         p = np.asarray(u8, np.uint8).reshape(height, width, nc)[y:y + h, x:x + w, :oc]
         OH, OW = self.c.out_h, self.c.out_w
         u8_out = desc.c.dtype == _ffi.DTYPE_U8
-        if self.c.filter == _ffi.FILTER_AREA:
+        if self.c.filter in (_ffi.FILTER_PIL_BILINEAR, _ffi.FILTER_PIL_BICUBIC):
+            g = pil_geometry(w, h, OW, OH, self.c.short_side)
+            if g is None:
+                raise ValueError(f"a {w}x{h} crop resized to short side {self.c.short_side} does not cover {OW}x{OH}")
+            rw, rh, left, top = g
+            bicubic = self.c.filter == _ffi.FILTER_PIL_BICUBIC
+            cx = pil_coefficients(w, rw, bicubic, left, OW)
+            cy = pil_coefficients(h, rh, bicubic, top, OH)
+            y0, y1 = cy[0][0], cy[-1][0] + len(cy[-1][1])
+
+            def clip8(s):
+                return np.clip(s >> 22, 0, 255)
+            q = p[y0:y1].astype(np.int64)
+            tmp = np.empty((y1 - y0, OW, oc), np.int64)                 # the horizontal pass's u8 intermediate
+            for j, (xm, k) in enumerate(cx):
+                tmp[:, j] = clip8((1 << 21) + np.einsum("ywc,w->yc", q[:, xm:xm + len(k)], k))
+            v = np.empty((OH, OW, oc), np.int64)
+            for i, (ym, k) in enumerate(cy):
+                v[i] = clip8((1 << 21) + np.einsum("ywc,y->wc", tmp[ym - y0:ym - y0 + len(k)], k))
+            v = v.astype(np.uint8)
+            if not u8_out:
+                v = v.astype(f32)
+        elif self.c.filter == _ffi.FILTER_AREA:
             def windows(n_out, n_in):
                 i = np.arange(n_out, dtype=np.int64)
                 return (i * n_in) // n_out, ((i + 1) * n_in + n_out - 1) // n_out
