@@ -98,6 +98,40 @@ enum { ZJ_USE_SPEC_OUTPUT = 2 };
  * zj_options.use_unsafe = ZJ_USE_LIBJPEG_OUTPUT: it decodes exactly as for ZJ_USE_SPEC_OUTPUT and sets the flag. */
 enum { ZJ_USE_LIBJPEG_OUTPUT = 3 };
 
+/* ZJ_VARIANT_SPEC | ZJ_FLAG_ISLOW with a scale k = (flags & ZJ_FLAG_SCALE_MASK) >> ZJ_FLAG_SCALE_SHIFT in {1, 2, 3} -- libjpeg-turbo's
+ * DCT-scaled decode to 1/d, d = 2^k (DESIGN.md section 4.6.2): what Pillow's Image.draft(mode, size) gives.  s0 = 8 / d; (hmax, vmax)
+ * = comp[0]'s factors, (h_z, v_z) = component z's.
+ *   1''. Block size per component (jdmaster.c): ss_z = s0, doubled while ss_z < 8, (hmax s0) mod (2 h_z ss_z) = 0 and (vmax s0) mod
+ *       (2 v_z ss_z) = 0.  Luma gets s0; 4:2:0 chroma 2 s0; 4:4:4, 4:2:2 and 4:4:0 chroma s0.
+ *   2''. Samples: every block of component z becomes ss_z x ss_z samples.  ss = 8: step 1'.  Otherwise jidctred.c, in the
+ *       arithmetic of step 1' (32-bit two's complement that wraps, arithmetic shifts, CONST_BITS 13, PASS1_BITS 2, dequantise =
+ *       coefficient x table entry, DESCALE and range_limit[v & 1023] as there):
+ *       ss = 4 (jpeg_idct_4x4): pass 1 down columns 0-3 and 5-7 (column 4 is never used); a column whose coefficients in rows 1, 2,
+ *         3, 5, 6, 7 are all zero gives 4 values (DC x q) << 2; otherwise, with z_r the dequantised row r,
+ *           t0 = z_0 << 14, t2 = 15137 z_2 - 6270 z_6, t10 = t0 + t2, t12 = t0 - t2,
+ *           a = -1730 z_7 + 11893 z_5 - 17799 z_3 + 8697 z_1, b = -4176 z_7 - 4926 z_5 + 7373 z_3 + 20995 z_1,
+ *           values DESCALE(t10 + b, 12), DESCALE(t12 + a, 12), DESCALE(t12 - a, 12), DESCALE(t10 - b, 12).
+ *         Pass 2 along each of the 4 rows w: a row whose w_1, w_2, w_3, w_5, w_6, w_7 are all zero gives 4 samples
+ *         range_limit[DESCALE(w_0, 5)]; otherwise the same formulas on w (t0 = w_0 << 14) with DESCALE(., 19).
+ *       ss = 2 (jpeg_idct_2x2): only rows and columns 0, 1, 3, 5, 7 are read.  Pass 1 down columns 0, 1, 3, 5, 7: a column whose rows
+ *         1, 3, 5, 7 are zero gives 2 values (DC x q) << 2; otherwise t10 = z_0 << 15, t0 = -5906 z_7 + 6967 z_5 - 10426 z_3 +
+ *         29692 z_1, values DESCALE(t10 + t0, 13), DESCALE(t10 - t0, 13).  Pass 2 along each of the 2 rows w: w_1, w_3, w_5, w_7 all
+ *         zero gives range_limit[DESCALE(w_0, 5)] twice; otherwise the same formulas on w with DESCALE(., 20).
+ *       ss = 1 (jpeg_idct_1x1): range_limit[DESCALE(DC x q, 3)].
+ *       The zero tests read the coefficients (pass 1) and the pass-1 values (pass 2), as jidctred.c does.  Whenever no intermediate
+ *       leaves 32 bits -- every block an 8-bit JPEG encoder produces -- this equals jidctred.c with a 64-bit JLONG.
+ *   3''. Sizes: the output is W' x H' = ceil(width / d) x ceil(height / d); component z is dw_z = ceil(width h_z ss_z / (hmax 8)) by
+ *       dh_z = ceil(height v_z ss_z / (vmax 8)) samples, and samples beyond these sizes are never read.
+ *   4''. Up-sampling by (hmax s0 / (h_z ss_z), vmax s0 / (v_z ss_z)), fancy = (s0 > 1): (1, 1) none; (2, 1) step 3's H filter when
+ *       fancy and dw_z > 2, else each sample twice; (1, 2) step 3's V filter when fancy, else each row twice.  Neighbour indices are
+ *       clamped to [0, dh_z-1] x [0, dw_z-1]; the result is cut to W' x H'.
+ *   5''. Steps 4 and 5 as they are, over W' x H' pixels: GRAYSCALE output is the luma plane.
+ * A non-zero scale on any other image is ZJ_ERR_INVALID_ARG; k = 0 is the statement above.  Everything downstream of reconstruction
+ * (zj_output_size, the consumers' shapes, rois, resizes) sees the W' x H' image.  The host stage produces such images with
+ * zj_options.use_unsafe = ZJ_USE_LIBJPEG_OUTPUT | k << 4: it decodes exactly as for ZJ_USE_LIBJPEG_OUTPUT and sets the scale. */
+#define ZJ_FLAG_SCALE_SHIFT 2
+#define ZJ_FLAG_SCALE_MASK (3u << ZJ_FLAG_SCALE_SHIFT)
+
 typedef enum zj_status {
     ZJ_OK = 0,
     ZJ_ERR_INVALID_ARG = -1,     /* null pointer, bad enum, inconsistent descriptor                        */
@@ -150,7 +184,7 @@ typedef struct zj_image {
 ZJ_API int zj_gpu_device_count(void);
 
 /* Bytes the reference's decode_buffer returns for this image: width*height*out_components
- * (mcu.rs:375-379).  Returns 0 on a bad descriptor. */
+ * (mcu.rs:375-379); ceil(width / d) * ceil(height / d) * out_components for a DCT-scaled image.  Returns 0 on a bad descriptor. */
 ZJ_API size_t zj_output_size(const zj_image *img);
 
 /* Validate a descriptor exactly as the GPU entry points do, without touching a device. */
@@ -335,7 +369,8 @@ ZJ_API uint64_t zj_gpu_launch_count(void);
 typedef struct zj_options {       /* ZuneJpegOptions (src/options.rs:6-40), same defaults */
     uint32_t use_unsafe;          /* 1; ZJ_USE_SPEC_OUTPUT (not in the reference): ZJ_VARIANT_SPEC output, and the host stage
                                      decodes every MCU row with Q9-Q11 off, whatever zj_host_set_quirks says;
-                                     ZJ_USE_LIBJPEG_OUTPUT: the same, and the images carry ZJ_FLAG_ISLOW                  */
+                                     ZJ_USE_LIBJPEG_OUTPUT: the same, and the images carry ZJ_FLAG_ISLOW;
+                                     ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the same, decoded at 1/2^k (ZJ_FLAG_SCALE_*) */
     uint32_t out_colorspace;      /* ZJ_CS_RGB                                           */
     uint32_t num_threads;         /* 4                                                   */
     uint32_t max_width;           /* 16384                                               */

@@ -6,12 +6,12 @@ from ._ffi import (  # noqa: F401
 )
 
 __all__ = ["Decoder", "ZuneJpegOptions", "JpegDecoder", "DecoderOptions", "ColorSpace", "DecodeErrors", "ImageInfo", "reconstruct", "decode_batch",
-           "decode_batch_resized", "Resize"]
+           "decode_batch_resized", "Resize", "draft_scale"]
 
 
 def __getattr__(name):  # lazy: importing the package must not require the built library
     if name in ("Decoder", "ZuneJpegOptions", "ColorSpace", "DecodeErrors", "ImageInfo", "UnsupportedSchemes", "decode_batch",
-                "decode_batch_resized", "JpegDecoder", "DecoderOptions"):
+                "decode_batch_resized", "JpegDecoder", "DecoderOptions", "draft_scale"):
         from . import decoder as _d
         return getattr(_d, name)
     if name in ("reconstruct", "Batch", "DeviceBuffer", "PinnedBuffer", "make_image", "Resize"):

@@ -17,6 +17,18 @@ VARIANT_X86, VARIANT_SCALAR, VARIANT_SPEC = 0, 1, 2
 USE_SPEC_OUTPUT = 2   # zj_options.use_unsafe value that selects VARIANT_SPEC
 USE_LIBJPEG_OUTPUT = 3   # zj_options.use_unsafe value that selects VARIANT_SPEC with FLAG_ISLOW
 FLAG_PROGRESSIVE, FLAG_ISLOW = 1, 2
+FLAG_SCALE_SHIFT, FLAG_SCALE_MASK = 2, 3 << 2   # zj_image.flags bits 2-3: k of a DCT-scaled (1/2^k) image
+USE_SCALE_SHIFT = 4   # zj_options.use_unsafe = USE_LIBJPEG_OUTPUT | k << USE_SCALE_SHIFT, k = 1..3: libjpeg output at 1/2^k
+
+
+def scaled_size(width: int, height: int, denom: int):
+    """The output size of a DCT-scaled decode to 1/denom: (ceil(width / denom), ceil(height / denom))"""
+    return -(-width // denom), -(-height // denom)
+
+
+def image_size(img) -> tuple:
+    """(width, height) of a zj_image's output: its size, or the scaled size of a DCT-scaled image (ZJ_FLAG_SCALE_*)"""
+    return scaled_size(img.width, img.height, 1 << ((img.flags & FLAG_SCALE_MASK) >> FLAG_SCALE_SHIFT))
 QUIRK_Q9, QUIRK_Q10, QUIRK_Q11, QUIRK_ALL = 1, 2, 4, 7   # zj_host_set_quirks (tests only)
 OK = 0
 ERR_INVALID_ARG, ERR_UNSUPPORTED, ERR_SHORT_PLANE, ERR_SHORT_OUTPUT = -1, -2, -3, -4

@@ -46,6 +46,7 @@ int zj::num_components(uint32_t cs)  // ColorSpace::num_components, reference sr
 struct Plan {
     int mode, variant, gray, zero_only, fast;
     int islow;         // ZJ_FLAG_ISLOW: the kernels' IDCT is libjpeg-turbo's islow
+    int scale;         // ZJ_FLAG_SCALE_*: DCT-scaled decode to 1/2^scale (scaled_kernel)
     uint32_t n_strips, rows, ncomp_used;
     size_t chunk[3];   // i16 per strip per component
     size_t out_size;
@@ -66,6 +67,8 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     const bool spec = img->variant == ZJ_VARIANT_SPEC;
     const bool islow = (img->flags & ZJ_FLAG_ISLOW) != 0;   // spec output with libjpeg-turbo's IDCT: every rule below as for spec
     if (islow && !spec) return ZJ_ERR_INVALID_ARG;
+    const uint32_t scale = image_scale(img);                 // DCT-scaled: spec | islow planes, reconstructed by scaled_kernel
+    if (scale && !islow) return ZJ_ERR_INVALID_ARG;
     const uint32_t h = img->comp[0].h_samp, v = img->comp[0].v_samp;
     if (img->n_comp == 1 && (h != 1 || v != 1)) return ZJ_ERR_UNSUPPORTED;  // mcu.rs:171-196 resets these before the path
     for (uint32_t z = 1; z < img->n_comp; z++)
@@ -88,6 +91,7 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     pl->mode = mode;
     pl->variant = (int)img->variant;
     pl->islow = islow;
+    pl->scale = (int)scale;
     uint32_t n_strips, ybr, cbr;
     switch (mode) {
     case MODE_H: n_strips = mcu_y / 2; ybr = 2; cbr = 2; break;   // mcu.rs:147-154 -- Q1: odd MCU row dropped
@@ -108,7 +112,9 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     pl->n_strips = n_strips;
     pl->grid_strips = n_strips;
     pl->rows = rows;
-    pl->out_size = (size_t)w * hh * nc;
+    uint32_t ow, oh;
+    output_dims(img, &ow, &oh);
+    pl->out_size = (size_t)ow * oh * nc;
     pl->chunk[0] = (size_t)ybr * h * mcu_x * 64;
     pl->chunk[1] = pl->chunk[2] = (size_t)cbr * mcu_x * 64;
 
@@ -140,6 +146,19 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
         for (int k = 0; k < 32; k++)
             d.qtw[z][k] = (uint32_t)img->comp[z].qt[2 * k] | ((uint32_t)img->comp[z].qt[2 * k + 1] << 24);
 
+    if (scale) {
+        // scaled_kernel, for every output colourspace (GRAYSCALE: the luma plane): one MCU row x TS MCU columns per CTA
+        d.width = ow; d.height = oh; d.stride = ow * (uint32_t)nc;
+        d.n_strips = mcu_y;
+        // the real chroma size (rules 1'' and 3''): 4:2:0 chroma blocks are 2 s0 samples wide, every other chroma block s0
+        const uint64_t ss = (8u >> scale) * (mode == MODE_HV ? 2u : 1u);
+        d.chroma_wh = (uint32_t)((w * ss + 8 * h - 1) / (8 * h)) | (uint32_t)((hh * ss + 8 * v - 1) / (8 * v)) << 16;
+        const int tsv[4] = {TS_NONE, TS_H, TS_V, TS_HV};
+        d.n_tiles = (mcu_x + tsv[mode] - 1) / tsv[mode];
+        pl->grid_tiles = d.n_tiles;
+        pl->grid_strips = mcu_y;
+        return ZJ_OK;
+    }
     if (kind == OUT_GRAY) {
         // ycbcr_to_grayscale (color_convert/scalar.rs:97-112): width_mcu = len / width must equal the strip's row
         // count, otherwise the chunking overruns the strip's output slice and the reference panics (Q7).
@@ -299,7 +318,9 @@ size_t zj_output_size(const zj_image *img)
     Plan pl;
     int rc = plan_image(img, &pl);
     if (rc != ZJ_OK && rc != ZJ_ERR_REF_PANIC) return 0;
-    return img ? (size_t)img->width * img->height * num_components(img->out_cs) : 0;
+    uint32_t w, h;
+    output_dims(img, &w, &h);
+    return (size_t)w * h * num_components(img->out_cs);
 }
 
 int zj_validate_image(const zj_image *img)
@@ -346,7 +367,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
     b->d_images = nullptr;
     b->n_images = 0;
     b->algo_bytes = 0;
-    // group by kernel: (gray, fast, mode, variant, IDCT); stable so images keep their relative order
+    // group by kernel: (scale, gray, fast, mode, variant, IDCT); stable so images keep their relative order
     std::vector<size_t> order;
     for (size_t i = 0; i < n; i++) {
         if (plans[i].zero_only) b->zero_only.push_back({out_dev[i], plans[i].out_size});
@@ -354,7 +375,9 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         b->algo_bytes += plans[i].out_size;
         for (uint32_t z = 0; z < plans[i].ncomp_used; z++) b->algo_bytes += (uint64_t)plans[i].n_strips * plans[i].chunk[z] * 2;
     }
-    auto key = [&](size_t i) { return plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 + plans[i].variant; };
+    auto key = [&](size_t i) {
+        return plans[i].scale * 128 + plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 + plans[i].variant;
+    };
     std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t c) { return key(a) < key(c); });
     std::vector<DevImage> host(order.size());
     for (size_t k = 0; k < order.size(); k++) host[k] = plans[order[k]].dev;
@@ -363,6 +386,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         LaunchGroup g{};
         g.gray = plans[order[k]].gray; g.mode = plans[order[k]].mode; g.variant = plans[order[k]].variant; g.fast = plans[order[k]].fast;
         g.islow = plans[order[k]].islow;
+        g.scale = plans[order[k]].scale;
         g.first = (uint32_t)k;
         while (e < order.size() && key(order[e]) == key(order[k]) && e - k < 65535) {
             g.max_tiles = std::max(g.max_tiles, plans[order[e]].grid_tiles);
@@ -475,13 +499,17 @@ size_t zj::convert_size(uint32_t width, uint32_t height, uint32_t nc, const zj_o
 int zj_consumer_output_shape(const zj_image *img, const zj_output_desc *d, uint32_t *out_w, uint32_t *out_h, uint32_t *out_c)
 {
     if (!img || !out_w || !out_h || !out_c) return ZJ_ERR_INVALID_ARG;
-    return conv_shape(img->width, img->height, (uint32_t)num_components(img->out_cs), d, out_w, out_h, out_c);
+    uint32_t w, h;
+    output_dims(img, &w, &h);
+    return conv_shape(w, h, (uint32_t)num_components(img->out_cs), d, out_w, out_h, out_c);
 }
 
 size_t zj_consumer_output_size(const zj_image *img, const zj_output_desc *d)
 {
     if (!img || zj_output_size(img) == 0) return 0;
-    return convert_size(img->width, img->height, (uint32_t)num_components(img->out_cs), d);
+    uint32_t w, h;
+    output_dims(img, &w, &h);
+    return convert_size(w, h, (uint32_t)num_components(img->out_cs), d);
 }
 
 // One launch of the second pass (the consumer for ConvImage, the resize for ResizeImage) per run of consecutive images with the
@@ -638,7 +666,8 @@ int zj_gpu_reconstruct_device_ex(int device, void *stream, const zj_image *imgs,
         u8_size[i] = zj_output_size(&imgs[i]);
         if (u8_size[i] == 0) { rc = zj_validate_image(&imgs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
         ConvImage &ci = conv[i];
-        ci.width = imgs[i].width; ci.height = imgs[i].height; ci.nc = nc[i] = (uint32_t)num_components(imgs[i].out_cs);
+        output_dims(&imgs[i], &ci.width, &ci.height);
+        ci.nc = nc[i] = (uint32_t)num_components(imgs[i].out_cs);
         rc = conv_shape(ci.width, ci.height, ci.nc, d, &ci.ow, &ci.oh, &ci.oc);
         if (rc) return rc;
         if (!out_dev[i]) return ZJ_ERR_INVALID_ARG;
@@ -719,7 +748,9 @@ int zj_image_rows(const zj_image *img, uint32_t row_begin, uint32_t row_end, zj_
     Plan pl;
     int rc = plan_image(img, &pl);
     if (rc) return rc;
-    if (!sub || !sub_row0 || row_begin >= row_end || row_end > img->height) return ZJ_ERR_INVALID_ARG;
+    uint32_t w, h;
+    output_dims(img, &w, &h);
+    if (!sub || !sub_row0 || row_begin >= row_end || row_end > h) return ZJ_ERR_INVALID_ARG;
     // strips [s0, s1): the strips the rows fall in; rows at or below the last strip belong to the range that ends with it
     const uint32_t ns = pl.n_strips;
     const uint32_t s0 = ns ? std::min(row_begin / pl.rows, ns - 1) : 0;
@@ -764,12 +795,14 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     // per image: the crop, the strips that hold the rows the resize reads and the size of their u8 pixels
     std::vector<zj_image> subs(n);
     std::vector<zj_roi> crops(n);
-    std::vector<uint32_t> row0(n), nc(n);
+    std::vector<uint32_t> row0(n), nc(n), width(n);
     std::vector<size_t> u8_size(n);
     for (size_t i = 0; i < n; i++) {
         if (zj_output_size(&imgs[i]) == 0) { rc = zj_validate_image(&imgs[i]); return rc ? rc : (int)ZJ_ERR_INVALID_ARG; }
         nc[i] = (uint32_t)num_components(imgs[i].out_cs);
-        rc = resize_admit(d, r, nc[0], rois ? &rois[i] : nullptr, imgs[i].width, imgs[i].height, nc[i], &crops[i]);
+        uint32_t height;
+        output_dims(&imgs[i], &width[i], &height);
+        rc = resize_admit(d, r, nc[0], rois ? &rois[i] : nullptr, width[i], height, nc[i], &crops[i]);
         if (rc) return rc;
         uint32_t first, end;
         crop_rows(*r, crops[i], &first, &end);
@@ -784,7 +817,9 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     if (rc) return rc;
     if (n == 0) return ZJ_OK;
     return reconstruct_then(device, (cudaStream_t)stream, subs.data(), u8_size, nc.data(), *d, r, [&](size_t i, const uint8_t *u8) {
-        return resize_image(u8, imgs[i].width, subs[i].height, nc[i], row0[i], crops[i], static_cast<uint8_t *>(out_dev) + i * slot, *r);
+        uint32_t sub_w, sub_h;
+        output_dims(&subs[i], &sub_w, &sub_h);
+        return resize_image(u8, width[i], sub_h, nc[i], row0[i], crops[i], static_cast<uint8_t *>(out_dev) + i * slot, *r);
     });
 }
 

@@ -64,14 +64,29 @@ struct DevImage {
     uint32_t gray_rows_ok;    // Q7 resolved: 1 = plain row copy is what the reference does
     uint32_t gray_brows;      // luma-only output: block rows of the Y plane the reference processes
     uint32_t tile_q, tile_r;  // tile t covers MCU columns (fast kernel: 16-sample unit columns) [t*q + min(t,r), ...): the first r tiles are one wider
+    uint32_t chroma_wh;       // DCT-scaled images: the real chroma size dw | dh << 16 (width, height, stride: the scaled output's;
+                              // n_strips: MCU rows)
     uint64_t magic_w;         // ceil(2^40 / W): idx / W == (idx * magic_w) >> 40 for idx < 2^20
 };
+
+// MCU columns per tile of scaled_kernel (DCT-scaled images), by mode: about one block per thread in phase 1
+constexpr int TS_NONE = 80, TS_H = 60, TS_V = 32, TS_HV = 42;
+// The scale k of a zj_image (ZJ_FLAG_SCALE_*), and the size of its output: width x height, or ceil(width / 2^k) x ceil(height / 2^k)
+// for a DCT-scaled image.  Everything downstream of reconstruction sees this size.
+inline uint32_t image_scale(const zj_image *img) { return (img->flags & ZJ_FLAG_SCALE_MASK) >> ZJ_FLAG_SCALE_SHIFT; }
+inline void output_dims(const zj_image *img, uint32_t *w, uint32_t *h)
+{
+    const uint32_t k = image_scale(img), m = (1u << k) - 1;
+    *w = (uint32_t)(((uint64_t)img->width + m) >> k);
+    *h = (uint32_t)(((uint64_t)img->height + m) >> k);
+}
 
 // Host-side launch plan entry: one kernel launch per (mode, variant, IDCT, out-kind class) group.
 struct LaunchGroup {
     int mode, variant, gray;  // gray = luma-only kernel
     int fast;                 // reconstruct_fast_kernel (X86 variant, aligned output)
     int islow;                // ZJ_FLAG_ISLOW (SPEC variant only): libjpeg-turbo's islow IDCT
+    int scale;                // ZJ_FLAG_SCALE_* (SPEC | ISLOW only): 1/2^scale DCT-scaled decode, scaled_kernel
     uint32_t first, count;    // images [first, first+count) of the sorted device array
     uint32_t max_tiles, max_strips;
 };

@@ -625,8 +625,16 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     uint32_t user_out_cs = ZJ_CS_RGB;
     uint32_t quirks = ZJ_QUIRK_ALL;   // the host-stage quirks of this decode (g_quirks when it started; none for spec output)
     bool quirk(uint32_t bit) const { return (quirks & bit) != 0; }
-    // spec output, with either IDCT: the host stage is the same for both, only the descriptor's ZJ_FLAG_ISLOW differs
-    bool spec() const { return options.use_unsafe == ZJ_USE_SPEC_OUTPUT || options.use_unsafe == ZJ_USE_LIBJPEG_OUTPUT; }
+    // spec output, with either IDCT and at any scale: the host stage is the same for all, only the descriptor's ZJ_FLAG_ISLOW and
+    // ZJ_FLAG_SCALE_* differ
+    bool spec() const { return options.use_unsafe == ZJ_USE_SPEC_OUTPUT || libjpeg(); }
+    bool libjpeg() const { return options.use_unsafe == ZJ_USE_LIBJPEG_OUTPUT || scale() != 0; }
+    // ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the DCT-scaled decode to 1/2^k (every other value keeps its meaning)
+    uint32_t scale() const
+    {
+        const uint32_t k = options.use_unsafe >> 4;
+        return (options.use_unsafe & 15u) == ZJ_USE_LIBJPEG_OUTPUT && k >= 1 && k <= 3 ? k : 0;
+    }
     // a one-component image: GRAYSCALE output (headers.rs:278-285, mcu.rs:171-196), except that spec output keeps RGB / RGBA / RGBX
     void gray_input_out_cs()
     {
@@ -1382,7 +1390,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         img->n_comp = (uint32_t)in_components();
         img->out_cs = options.out_colorspace;
         img->variant = spec() ? ZJ_VARIANT_SPEC : (options.use_unsafe ? ZJ_VARIANT_X86 : ZJ_VARIANT_SCALAR);
-        img->flags = (is_progressive ? ZJ_FLAG_PROGRESSIVE : 0) | (options.use_unsafe == ZJ_USE_LIBJPEG_OUTPUT ? ZJ_FLAG_ISLOW : 0);
+        img->flags = (is_progressive ? ZJ_FLAG_PROGRESSIVE : 0) | (libjpeg() ? ZJ_FLAG_ISLOW : 0) | scale() << ZJ_FLAG_SCALE_SHIFT;
         for (size_t z = 0; z < in_components(); z++) {
             zj_component &c = img->comp[z];
             c.coeff = plane_len[z] ? planes[z].p : nullptr;
@@ -2218,7 +2226,9 @@ static int decode_then(const zj_options &opt, const uint8_t *const *bufs, const 
         zj_decoder *dd = zj_decoder_new(&opt);
         zj_image_info info;
         if (dd && zj_decoder_read_headers(dd, bufs[i], lens[i]) == ZJ_OK && zj_decoder_info(dd, &info) == ZJ_OK && info.valid) {
-            img[i].width = info.width; img[i].height = info.height;
+            // (the output's size: a DCT-scaled decode gives ceil(width / 2^k) x ceil(height / 2^k), as output_dims states)
+            const uint32_t k = dd->scale(), m = (1u << k) - 1;
+            img[i].width = (info.width + m) >> k; img[i].height = (info.height + m) >> k;
             img[i].nc = (uint32_t)zj::num_components(zj_decoder_out_colorspace(dd));
             len[i] = (size_t)img[i].width * img[i].height * img[i].nc;
             off[i] = total;

@@ -402,6 +402,121 @@ __device__ __forceinline__ void idct_islow_block(const bool active, const int4 (
     }
 }
 
+// ------------------------------------------------------------------------------------------------ reduced IDCTs
+// libjpeg-turbo's jidctred.c: step 2'' of DCT-scaled images (the statement is in include/zune_jpeg_b200.h), in Z/2^32 as islow8.
+// A block of S x S samples (S = 4: jpeg_idct_4x4, 2: jpeg_idct_2x2, 1: jpeg_idct_1x1) fits load_block's registers: load_rows<S>
+// reads only the rows the transform uses (S = 1: the DC's 32-byte sector), and idct_reduced<S> needs no warp vote.
+template <int S>
+__device__ __forceinline__ bool row_used(int r) { return S == 4 ? r != 4 : (S == 2 ? (r < 2 || (r & 1)) : r == 0); }
+
+template <int S>
+__device__ __forceinline__ void load_rows(const bool active, const int16_t *__restrict__ src, int4 (&raw)[8])
+{
+    const int4 *p = reinterpret_cast<const int4 *>(src);
+#pragma unroll
+    for (int r = 0; r < 8; r++) raw[r] = active && row_used<S>(r) ? __ldg(p + r) : make_int4(0, 0, 0, 0);
+}
+
+// coefficient and dequantised value at row r, column c (compile-time after unrolling)
+__device__ __forceinline__ int coef_at(const int4 (&raw)[8], int r, int c)
+{
+    const int k = c >> 1;
+    const u32 w = (u32)(k == 0 ? raw[r].x : k == 1 ? raw[r].y : k == 2 ? raw[r].z : raw[r].w);
+    return (c & 1) ? (int)w >> 16 : (int)(int16_t)(w & 0xffffu);
+}
+__device__ __forceinline__ u32 dequant_at(const int4 (&raw)[8], const u32 *__restrict__ qtw, int r, int c)
+{
+    const u32 w = qtw[(r * 8 + c) >> 1];
+    return (u32)coef_at(raw, r, c) * ((c & 1) ? w >> 24 : w & 0xffu);
+}
+// range_limit[DESCALE(x, N) & 1023]: bits N..N+9 of x + 2^(N-1) read as a signed 10-bit value, plus 128, clamped
+template <int N>
+__device__ __forceinline__ u32 descale_limit(u32 x) { return clamp255((u32)(((int)((x + (1u << (N - 1))) << (22 - N)) >> 22) + 128)); }
+
+// one 1-D pass of jpeg_idct_4x4 (inputs 0-3, 5-7) and of jpeg_idct_2x2 (inputs 0, 1, 3, 5, 7), before the DESCALE
+__device__ __forceinline__ void red4(u32 v0, u32 v1, u32 v2, u32 v3, u32 v5, u32 v6, u32 v7, u32 o[4])
+{
+    const u32 t0 = v0 << 14;                                                              // << (CONST_BITS + 1)
+    const u32 t2 = v2 * 15137u + v6 * (u32)-6270;                                         // FIX_1_847759065, -FIX_0_765366865
+    const u32 t10 = t0 + t2, t12 = t0 - t2;
+    const u32 a = v7 * (u32)-1730 + v5 * 11893u + v3 * (u32)-17799 + v1 * 8697u;         // tmp0
+    const u32 b = v7 * (u32)-4176 + v5 * (u32)-4926 + v3 * 7373u + v1 * 20995u;          // tmp2
+    o[0] = t10 + b; o[1] = t12 + a; o[2] = t12 - a; o[3] = t10 - b;
+}
+__device__ __forceinline__ void red2(u32 v0, u32 v1, u32 v3, u32 v5, u32 v7, u32 o[2])
+{
+    const u32 t10 = v0 << 15;                                                             // << (CONST_BITS + 2)
+    const u32 t0 = v7 * (u32)-5906 + v5 * 6967u + v3 * (u32)-10426 + v1 * 29692u;
+    o[0] = t10 + t0; o[1] = t10 - t0;
+}
+
+// Dequantise + reduced IDCT of one block into dst[r * dst_stride + c], r, c < S (S = 4, 2, 1); called by lanes that own a block
+template <int S>
+__device__ __forceinline__ void idct_reduced(const int4 (&raw)[8], const u32 *__restrict__ qtw, uint8_t *__restrict__ dst, int dst_stride)
+{
+    if constexpr (S == 1) {
+        dst[0] = (uint8_t)descale_limit<3>(dequant_at(raw, qtw, 0, 0));
+    } else if constexpr (S == 2) {
+        u32 ws[2][8];
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            if (!row_used<2>(c)) continue;   // columns 2, 4, 6: never read by pass 2
+            if ((coef_at(raw, 1, c) | coef_at(raw, 3, c) | coef_at(raw, 5, c) | coef_at(raw, 7, c)) == 0) {
+                ws[0][c] = ws[1][c] = dequant_at(raw, qtw, 0, c) << 2;
+            } else {
+                u32 o[2];
+                red2(dequant_at(raw, qtw, 0, c), dequant_at(raw, qtw, 1, c), dequant_at(raw, qtw, 3, c), dequant_at(raw, qtw, 5, c),
+                     dequant_at(raw, qtw, 7, c), o);
+                ws[0][c] = (u32)((int)(o[0] + (1u << 12)) >> 13);
+                ws[1][c] = (u32)((int)(o[1] + (1u << 12)) >> 13);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 2; r++) {
+            const u32 *w = ws[r];
+            uint8_t *d = dst + r * dst_stride;
+            if ((w[1] | w[3] | w[5] | w[7]) == 0) {
+                d[0] = d[1] = (uint8_t)descale_limit<5>(w[0]);
+            } else {
+                u32 o[2];
+                red2(w[0], w[1], w[3], w[5], w[7], o);
+                d[0] = (uint8_t)descale_limit<20>(o[0]);
+                d[1] = (uint8_t)descale_limit<20>(o[1]);
+            }
+        }
+    } else {
+        static_assert(S == 4, "reduced IDCT sizes: 4, 2, 1");
+        u32 ws[4][8];
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            if (c == 4) continue;            // column 4: never read by pass 2
+            if ((coef_at(raw, 1, c) | coef_at(raw, 2, c) | coef_at(raw, 3, c) | coef_at(raw, 5, c) | coef_at(raw, 6, c) | coef_at(raw, 7, c)) == 0) {
+                ws[0][c] = ws[1][c] = ws[2][c] = ws[3][c] = dequant_at(raw, qtw, 0, c) << 2;
+            } else {
+                u32 o[4];
+                red4(dequant_at(raw, qtw, 0, c), dequant_at(raw, qtw, 1, c), dequant_at(raw, qtw, 2, c), dequant_at(raw, qtw, 3, c),
+                     dequant_at(raw, qtw, 5, c), dequant_at(raw, qtw, 6, c), dequant_at(raw, qtw, 7, c), o);
+#pragma unroll
+                for (int r = 0; r < 4; r++) ws[r][c] = (u32)((int)(o[r] + (1u << 11)) >> 12);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 4; r++) {
+            const u32 *w = ws[r];
+            u32 v[4];
+            if ((w[1] | w[2] | w[3] | w[5] | w[6] | w[7]) == 0) {
+                v[0] = v[1] = v[2] = v[3] = descale_limit<5>(w[0]);
+            } else {
+                u32 o[4];
+                red4(w[0], w[1], w[2], w[3], w[5], w[6], w[7], o);
+#pragma unroll
+                for (int k = 0; k < 4; k++) v[k] = descale_limit<19>(o[k]);
+            }
+            *reinterpret_cast<u32 *>(dst + r * dst_stride) = v[0] | v[1] << 8 | v[2] << 16 | v[3] << 24;
+        }
+    }
+}
+
 // The IDCT of the fast kernel's producers (X86 variant, u8 planes), written as two short loops instead of one long
 // unrolled body so that it stays resident in the instruction cache next to the consumers' code:
 //   row pass:    row r of the block is read from the thread's staging slot (16-byte chunk r at sl ^ (r << 4)),
@@ -2054,6 +2169,121 @@ spec_kernel(const DevImage *__restrict__ images)
     }
 }
 
+// ------------------------------------------------------------------------------------- DCT-scaled kernel
+// ZJ_VARIANT_SPEC | ZJ_FLAG_ISLOW with ZJ_FLAG_SCALE_* = LOG2D (the statement is in include/zune_jpeg_b200.h): every block becomes
+// S0 = 8 >> LOG2D (luma) or SC (chroma: 2 S0 for 4:2:0, else S0) samples a side, so one MCU is H S0 x V S0 output pixels and carries
+// one SC x SC chroma block.  4:4:4 and 4:2:0 chroma then needs no up-sampling, 4:2:2 is up-sampled along rows and 4:4:0 down
+// columns -- with libjpeg's fancy filters when S0 > 1 (4:2:2: and the chroma is wider than 2), by repetition otherwise.
+// grid = (tiles of TS MCU columns, MCU rows, images); block = ZJ_THREADS; one kernel for every output colourspace.
+//   phase 1: the tile's luma blocks, then its chroma blocks and the context the fancy filters reach (one block column on each side
+//            for 4:2:2, one block row above and below for 4:4:0, where it holds real chroma samples), into shared sample planes;
+//            SC = 8 (4:2:0 at 1/2) is the islow IDCT of step 1', whose warp votes need the loop's CTA-uniform trip count;
+//   phase 2: one thread per output pixel: up-sampling, JFIF colour, alpha.
+template <int MODE, int LOG2D>
+__global__ void __launch_bounds__(ZJ_THREADS, ZJ_MINBLOCKS)
+scaled_kernel(const DevImage *__restrict__ images)
+{
+    static_assert(LOG2D >= 1 && LOG2D <= 3, "scales 1/2, 1/4, 1/8");
+    typedef ModeTraits<MODE> MT;
+    constexpr int S0 = 8 >> LOG2D;
+    constexpr int SC = MODE == MODE_HV ? 2 * S0 : S0;
+    constexpr int TS = MODE == MODE_NONE ? TS_NONE : (MODE == MODE_H ? TS_H : (MODE == MODE_V ? TS_V : TS_HV));
+    constexpr bool FANCY = S0 > 1;
+    constexpr int PC = MODE == MODE_H && FANCY ? SC : 0;   // context columns on each side of the chroma tile
+    constexpr int PR = MODE == MODE_V && FANCY ? SC : 0;   // context rows above and below it
+    constexpr int YW = TS * MT::H * S0, YR = MT::V * S0;   // luma tile
+    constexpr int CW = TS * SC + 2 * PC, CR = SC + 2 * PR; // chroma tile
+    __shared__ __align__(16) uint8_t sY[YR * YW];
+    __shared__ __align__(16) uint8_t sC[2][CR * CW];
+    __shared__ u32 sQ[3][32];
+
+    const DevImage &im = images[blockIdx.z];
+    const int tile = (int)blockIdx.x, my = (int)blockIdx.y;
+    if (tile >= (int)im.n_tiles || my >= (int)im.n_strips) return;
+    const int tid = threadIdx.x;
+    const int mcu_x = (int)im.mcu_x, width = (int)im.width, height = (int)im.height;
+    const int m0 = tile * TS, m1 = min(m0 + TS, mcu_x), tm = m1 - m0;
+    const bool color = im.W != 0 && im.out_kind != OUT_GRAY;          // luma only: one-component input or GRAYSCALE output
+    const int dw = (int)(im.chroma_wh & 0xffffu), dh = (int)(im.chroma_wh >> 16);
+    for (int k = tid; k < 96; k += ZJ_THREADS) sQ[k >> 5][k & 31] = im.qtw[k >> 5][k & 31];
+    __syncthreads();
+
+    // ---------------------------------------------------------------- phase 1
+    // S x S samples of the block at src into dst (S = 8: every lane of the warp must call it)
+    auto transform = [&](auto size, const bool active, const int16_t *src, const u32 *qt, uint8_t *dst, int dstride) {
+        constexpr int S = decltype(size)::value;
+        int4 raw[8];
+        if constexpr (S == 8) {
+            load_block(active, src, raw);
+            idct_islow_block(active, raw, qt, dst, dstride);
+        } else {
+            load_rows<S>(active, src, raw);
+            if (active) idct_reduced<S>(raw, qt, dst, dstride);
+        }
+    };
+    const int ybpr = MT::H * mcu_x, ycols = MT::H * tm, nY = MT::V * ycols;
+    for (int b = tid; b < nY; b += ZJ_THREADS) {
+        const int br = b / ycols, bc = b - br * ycols;
+        transform(std::integral_constant<int, S0>(), true, im.coeff[0] + ((size_t)(my * MT::V + br) * ybpr + MT::H * m0 + bc) * 64, sQ[0],
+                  sY + br * S0 * YW + bc * S0, YW);
+    }
+    if (color) {
+        // chroma block rows [rb0, rb1) and block columns [cb0, cb1), context included
+        const int rb0 = my - (PR && my > 0 ? 1 : 0), rb1 = my + 1 + (PR && (my + 1) * SC < dh ? 1 : 0);
+        const int cb0 = m0 - (PC && m0 > 0 ? 1 : 0), cb1 = m1 + (PC && m1 * SC < dw ? 1 : 0);
+        const int ccols = cb1 - cb0, nC = (rb1 - rb0) * ccols;
+        for (int b0 = 0; b0 < 2 * nC; b0 += ZJ_THREADS) {   // CTA-uniform trip count
+            const int b = b0 + tid;
+            const bool active = b < 2 * nC;
+            const int comp = active && b >= nC ? 1 : 0, c = active ? b - comp * nC : 0;
+            const int br = rb0 + c / ccols, bc = cb0 + c % ccols;
+            transform(std::integral_constant<int, SC>(), active, im.coeff[1 + comp] + ((size_t)br * mcu_x + bc) * 64, sQ[1 + comp],
+                      sC[comp] + ((br - my) * SC + PR) * CW + (bc - m0) * SC + PC, CW);
+        }
+    }
+    __syncthreads();
+
+    // ---------------------------------------------------------------- phase 2
+    const int nc = (int)im.nc;
+    const bool ycc = im.out_kind == OUT_YCC;
+    const int x_t = m0 * MT::H * S0, y_t = my * YR;   // first output column / row of the tile
+    for (int u = tid; u < YR * YW; u += ZJ_THREADS) {
+        const int yl = u / YW, xl = u - yl * YW;
+        const int y = y_t + yl, x = x_t + xl;
+        if (y >= height || x >= width) continue;
+        const int yy = sY[yl * YW + xl];
+        u32 p[3] = {(u32)yy, (u32)yy, (u32)yy};
+        if (color) {
+            int cc[2];
+#pragma unroll
+            for (int comp = 0; comp < 2; comp++) {
+                const uint8_t *s = sC[comp];
+                if (MODE == MODE_H) {
+                    // chroma column i of the image is smem column i - (m0 SC - PC); the row is the pixel's
+                    const uint8_t *row = s + yl * CW - (m0 * SC - PC);
+                    const int i = x >> 1;
+                    if (FANCY && dw > 2) cc[comp] = (x & 1) ? (3 * row[i] + row[min(i + 1, dw - 1)] + 2) >> 2 : (3 * row[i] + row[max(i - 1, 0)] + 1) >> 2;
+                    else cc[comp] = row[i];
+                } else if (MODE == MODE_V) {
+                    // chroma row j of the image is smem row j - (my SC - PR); the column is the pixel's
+                    const uint8_t *col = s + xl - (my * SC - PR) * CW;
+                    const int j = y >> 1;
+                    if (FANCY) cc[comp] = (y & 1) ? (3 * col[j * CW] + col[min(j + 1, dh - 1) * CW] + 2) >> 2 : (3 * col[j * CW] + col[max(j - 1, 0) * CW] + 1) >> 2;
+                    else cc[comp] = col[j * CW];
+                } else {
+                    cc[comp] = s[yl * CW + xl];
+                }
+            }
+            p[1] = (u32)cc[0]; p[2] = (u32)cc[1];
+            if (!ycc) jfif_rgb(yy, cc[0], cc[1], p[0], p[1], p[2]);
+        }
+        uint8_t *d = im.out + ((size_t)y * width + x) * nc;
+        d[0] = (uint8_t)p[0];
+        if (nc >= 3) { d[1] = (uint8_t)p[1]; d[2] = (uint8_t)p[2]; }
+        if (nc == 4) d[3] = 255;
+    }
+}
+
 // ----------------------------------------------------------------------------------------- host launchers
 template <int MODE>
 static cudaError_t launch_spec(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
@@ -2061,6 +2291,16 @@ static cudaError_t launch_spec(const DevImage *d_images, const LaunchGroup &g, c
     dim3 grid(g.max_tiles, g.max_strips, g.count);
     if (g.islow) spec_kernel<MODE, IDCT_ISLOW><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
     else spec_kernel<MODE, IDCT_X86><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
+    return cudaGetLastError();
+}
+
+template <int MODE>
+static cudaError_t launch_scaled(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
+{
+    dim3 grid(g.max_tiles, g.max_strips, g.count);   // max_strips: MCU rows
+    if (g.scale == 1) scaled_kernel<MODE, 1><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
+    else if (g.scale == 2) scaled_kernel<MODE, 2><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
+    else scaled_kernel<MODE, 3><<<grid, ZJ_THREADS, 0, stream>>>(d_images + g.first);
     return cudaGetLastError();
 }
 
@@ -2255,6 +2495,14 @@ static cudaError_t launch_gray_fast(const DevImage *d_images, const LaunchGroup 
 
 cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream)
 {
+    if (g.scale) {
+        switch (g.mode) {
+        case MODE_NONE: return launch_scaled<MODE_NONE>(d_images, g, stream);
+        case MODE_H: return launch_scaled<MODE_H>(d_images, g, stream);
+        case MODE_V: return launch_scaled<MODE_V>(d_images, g, stream);
+        default: return launch_scaled<MODE_HV>(d_images, g, stream);
+        }
+    }
     if (g.gray && g.fast) return launch_gray_fast(d_images, g, stream);
     if (g.variant == ZJ_VARIANT_SPEC && !g.gray) {
         switch (g.mode) {

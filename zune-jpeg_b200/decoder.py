@@ -87,6 +87,7 @@ class ZuneJpegOptions:
         self._device = 0
         self._spec_output = False
         self._libjpeg_output = False
+        self._scale_denom = 1
 
     @staticmethod
     def new() -> "ZuneJpegOptions":
@@ -128,11 +129,21 @@ class ZuneJpegOptions:
     # and other libjpeg-turbo decodes with default settings give; ZJ_FLAG_ISLOW).  Takes precedence over spec output.
     def get_libjpeg_output(self): return self._libjpeg_output
     def set_libjpeg_output(self, choice: bool): return self._with(_libjpeg_output=bool(choice))
+    # not in the reference: libjpeg-turbo's DCT-scaled decode of libjpeg output to ceil(width / d) x ceil(height / d), d = 1, 2, 4
+    # or 8 -- what Pillow's Image.draft gives (ZJ_FLAG_SCALE_*; draft_scale picks d as Pillow does).  d > 1 needs libjpeg output.
+    def get_scale_denom(self): return self._scale_denom
+
+    def set_scale_denom(self, d: int):
+        if d not in (1, 2, 4, 8):
+            raise ValueError(f"scale denominator must be 1, 2, 4 or 8, not {d!r}")
+        return self._with(_scale_denom=int(d))
 
     def _raw(self) -> ZjOptions:
         o = ZjOptions()
+        if self._scale_denom > 1 and not self._libjpeg_output:
+            raise ValueError("a scale denominator above 1 needs libjpeg output (set_libjpeg_output(True))")
         if self._libjpeg_output:
-            o.use_unsafe = _ffi.USE_LIBJPEG_OUTPUT
+            o.use_unsafe = _ffi.USE_LIBJPEG_OUTPUT | (self._scale_denom.bit_length() - 1) << _ffi.USE_SCALE_SHIFT
         else:
             o.use_unsafe = _ffi.USE_SPEC_OUTPUT if self._spec_output else int(self._use_unsafe)
         o.out_colorspace = int(self._out_colorspace)
@@ -187,7 +198,8 @@ class Decoder:
 
     # ---- decoding
     def decode_buffer(self, buf: bytes) -> bytes:
-        """Decoder::decode_buffer (decoder.rs:178): JPEG bytes -> width*height*components pixel bytes."""
+        """Decoder::decode_buffer (decoder.rs:178): JPEG bytes -> width*height*components pixel bytes (with a scale denominator
+        d: ceil(width / d) * ceil(height / d) * components)."""
         buf = bytes(buf)
         out = C.POINTER(C.c_uint8)()
         n = C.c_size_t()
@@ -203,8 +215,9 @@ class Decoder:
 
     def decode_into(self, buf, out) -> int:
         """JpegDecoder::decode_into of later zune-jpeg releases: the pixels go into `out` (a writable uint8 buffer, e.g. a
-        PinnedBuffer.array slice); returns the number of bytes written.  Baseline images of >= 4 MP run as a strip pipeline
-        (zj_decoder_decode_into): finished strip ranges are on their way through the GPU while the host still entropy-decodes."""
+        PinnedBuffer.array slice); returns the number of bytes written (the scaled size's with a scale denominator).  Baseline
+        images of >= 4 MP run as a strip pipeline (zj_decoder_decode_into): finished strip ranges are on their way through the GPU
+        while the host still entropy-decodes."""
         import numpy as np
         data = buf if isinstance(buf, np.ndarray) else bytes(buf)
         p = data.ctypes.data if isinstance(data, np.ndarray) else C.cast(C.c_char_p(data), C.c_void_p).value
@@ -309,6 +322,15 @@ JpegDecoder = Decoder
 DecoderOptions = ZuneJpegOptions
 
 
+def draft_scale(width: int, height: int, size):
+    """Pillow's Image.draft rule for a width x height JPEG drafted to size = (w, h): d = the largest of 8, 4, 2, 1 with
+    min(width // w, height // h) >= d.  Returns (d, (ceil(width / d), ceil(height / d))), the denominator for
+    ZuneJpegOptions.set_scale_denom and the size the decode then has."""
+    scale = min(width // size[0], height // size[1])
+    d = next(a for a in (8, 4, 2, 1) if scale >= a or a == 1)
+    return d, _ffi.scaled_size(width, height, d)
+
+
 def _input_arrays(buffers):
     """(keep, bufs, lens): the inputs as bytes or uint8 arrays (the caller keeps them alive during the call) and the pointer and
     length arrays the batch calls take"""
@@ -340,8 +362,9 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
 
     Returns a list with one entry per input: `bytes` (or, with `out` / `device_out`, the number of bytes written) for a decoded
     image, a `DecodeErrors` instance for a failed one.  `out`: optional list of writable buffers (e.g. PinnedBuffer.array
-    slices), one per image, large enough for width*height*components.  Inputs may be `bytes` or uint8 numpy arrays (e.g. views
-    of pinned memory, which upload at the full PCIe rate)."""
+    slices), one per image, large enough for width*height*components (ceil(width / d) * ceil(height / d) * components with the
+    options' scale denominator d).  Inputs may be `bytes` or uint8 numpy arrays (e.g. views of pinned memory, which upload at the
+    full PCIe rate)."""
     lib = _ffi.load()
     options = options if options is not None else ZuneJpegOptions()
     raw = options._raw()
@@ -393,7 +416,8 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
 def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpegOptions | None = None, threads: int = 0):
     """zj_decode_batch_gpu_device_resized: JPEG byte strings in, one batch tensor in device memory out -- every image decoded
     whole, its crop resized to `resize` (a gpu.Resize) in the layout / type / normalisation of `desc` (a gpu.OutputDesc, scale
-    must be full size; default HWC u8).  rois: None, or one (x, y, w, h) or None (= the whole image) per image.
+    must be full size; default HWC u8).  rois: None, or one (x, y, w, h) or None (= the whole image) per image, in the
+    coordinates of the decoded image (ceil(width / d) x ceil(height / d) with the options' scale denominator d).
 
     Returns (gpu.DeviceArray of shape (N, C, OH, OW) or (N, OH, OW, C), [None | DecodeErrors per image]).  The errors are the
     ones decode_batch reports for the same inputs; a crop that does not fit its image, or an image whose channel count is not
@@ -414,7 +438,7 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
                 d = Decoder(options)
                 try:
                     d.read_headers(keep[i])
-                    sizes[i] = (d.width(), d.height())
+                    sizes[i] = _ffi.scaled_size(d.width(), d.height(), options.get_scale_denom())
                 except DecodeErrors:
                     sizes[i] = (1, 1)
     nc = ColorSpace(options.get_out_colorspace()).num_components()

@@ -34,6 +34,7 @@ def launch_count() -> int:
 
 
 def output_size(img: ZjImage) -> int:
+    """zj_output_size: bytes of the image's output (width x height, or the scaled size of a DCT-scaled image, x components)"""
     return int(_ffi.load().zj_output_size(C.byref(img)))
 
 
@@ -507,8 +508,8 @@ def resize_device(src: DeviceBuffer, width: int, height: int, nc: int, resize: R
 
 def reconstruct_device_resized(images, resize: Resize, desc: OutputDesc | None = None, rois=None, device: int = 0, stream=None) -> DeviceArray:
     """zj_gpu_reconstruct_device_resized: `images` carry DEVICE coefficient planes; returns one (N, C, OH, OW) or (N, OH, OW, C)
-    DeviceArray.  rois: None, or one (x, y, w, h) or None (= the whole image) per image; only the strips that hold a crop's rows
-    are reconstructed."""
+    DeviceArray.  rois: None, or one (x, y, w, h) or None (= the whole image) per image, in the coordinates of the image's output
+    (the scaled size of a DCT-scaled image); only the strips that hold a crop's rows are reconstructed."""
     lib = _ffi.load()
     desc = desc if desc is not None else OutputDesc()
     n = len(images)
@@ -516,7 +517,7 @@ def reconstruct_device_resized(images, resize: Resize, desc: OutputDesc | None =
     slot = resize.slot_size(desc, nc)
     b = DeviceBuffer(max(slot * n, 1), device)
     arr = _img_array(images)
-    r = _roi_array(rois, [(im.width, im.height) for im in images])
+    r = _roi_array(rois, [_ffi.image_size(im) for im in images])
     _check(lib.zj_gpu_reconstruct_device_resized(device, stream, arr, n, r, C.byref(desc.c), C.byref(resize.c), b.ptr, slot * n),
            "zj_gpu_reconstruct_device_resized")
     return DeviceArray(b, (n, *resize.slot_shape(desc, nc)), desc.c.dtype)
