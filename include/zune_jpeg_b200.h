@@ -132,6 +132,40 @@ enum { ZJ_USE_LIBJPEG_OUTPUT = 3 };
 #define ZJ_FLAG_SCALE_SHIFT 2
 #define ZJ_FLAG_SCALE_MASK (3u << ZJ_FLAG_SCALE_SHIFT)
 
+/* ZJ_VARIANT_SPEC (with or without ZJ_FLAG_ISLOW and a scale) with an orientation o = ((flags & ZJ_FLAG_ORIENT_MASK) >>
+ * ZJ_FLAG_ORIENT_SHIFT) + 1 in {2, ..., 8} -- the EXIF orientation applied (DESIGN.md section 4.6.3): what Pillow 12.2's
+ * ImageOps.exif_transpose gives.  The W' x H' image the statements above give (after any DCT scaling, as draft then
+ * exif_transpose) goes through Pillow's Transpose for o, each pixel's nc bytes moving together:
+ *   o = 2 FLIP_LEFT_RIGHT  out(X, Y) = in(W'-1-X, Y)          o = 5 TRANSPOSE   out(X, Y) = in(Y, X)
+ *   o = 3 ROTATE_180       out(X, Y) = in(W'-1-X, H'-1-Y)     o = 6 ROTATE_270  out(X, Y) = in(Y, H'-1-X)
+ *   o = 4 FLIP_TOP_BOTTOM  out(X, Y) = in(X, H'-1-Y)          o = 7 TRANSVERSE  out(X, Y) = in(W'-1-Y, H'-1-X)
+ *                                                             o = 8 ROTATE_90   out(X, Y) = in(W'-1-Y, X)
+ * The output is W' x H' for o = 2-4 and H' x W' for o = 5-8 (the same byte count).  Everything downstream of reconstruction
+ * (zj_output_size, the consumers' shapes, rois -- given in the displayed frame -- and resizes) sees the oriented image.  The bits
+ * are valid with ZJ_VARIANT_SPEC only (ZJ_ERR_INVALID_ARG otherwise); 0 is no transform.
+ *
+ * The host stage finds o (zj_decoder_orientation) the way Pillow 12.2's Image.getexif() does (PIL/Image.py, JpegImagePlugin.py
+ * APP()), reading only the markers before the first SOS:
+ *   - EXIF: the APP1 segments that start with "Exif\0\0" -- the first one's payload, with each later one's bytes after its 6-byte
+ *     header appended, every leading "Exif\0\0" of the result stripped.  Nothing left: no EXIF.  Otherwise an 8-byte TIFF header
+ *     ("II*\0" or "MM\0*" and IFD0's offset); a shorter or other header gives o = 1 and the XMP is not read (Pillow raises there).
+ *   - IFD0: its entry count, then its 12-byte entries in order, up to the first one that cannot be read whole -- its 12 bytes, or
+ *     the data it points at when its count x type size (types 1-13: 1 1 2 4 8 1 1 2 4 8 4 8 4 bytes) exceeds 4.  Entries of another
+ *     type or of size 0 are skipped; a later entry of a tag replaces an earlier one.  IFD0's offset past the data: no entries.
+ *   - Tag 0x0112 of type SHORT, LONG, SSHORT or SLONG: its first value, whatever the count (Pillow keeps the first value when the
+ *     count is not 1).  Of any other type: a value that is not an orientation (Pillow compares a RATIONAL or FLOAT value with
+ *     2-8; this does not).
+ *   - XMP, only when IFD0 has no tag 0x0112: the last APP1 segment that starts with "http://ns.adobe.com/xap/1.0/\0"; the first
+ *     match of tiff:Orientation(="|>)([0-9]) in it.
+ *   Any value other than 2-8 means no transform, and so does a missing tag.  torchvision's decode_jpeg(apply_exif_orientation=True)
+ *   reads the EXIF only (and a single SHORT); an XMP-only orientation is applied here, as Pillow applies it, and not there.  A bad
+ *   EXIF never fails a decode.
+ * With zj_options.use_unsafe = ZJ_USE_SPEC_OUTPUT, ZJ_USE_LIBJPEG_OUTPUT or ZJ_USE_LIBJPEG_OUTPUT | k << 4, ORed with
+ * ZJ_USE_EXIF_ORIENTATION, the host stage decodes as without it and sets o in the images' flags. */
+#define ZJ_FLAG_ORIENT_SHIFT 4
+#define ZJ_FLAG_ORIENT_MASK (7u << ZJ_FLAG_ORIENT_SHIFT)
+enum { ZJ_USE_EXIF_ORIENTATION = 0x100 };
+
 typedef enum zj_status {
     ZJ_OK = 0,
     ZJ_ERR_INVALID_ARG = -1,     /* null pointer, bad enum, inconsistent descriptor                        */
@@ -370,7 +404,8 @@ typedef struct zj_options {       /* ZuneJpegOptions (src/options.rs:6-40), same
     uint32_t use_unsafe;          /* 1; ZJ_USE_SPEC_OUTPUT (not in the reference): ZJ_VARIANT_SPEC output, and the host stage
                                      decodes every MCU row with Q9-Q11 off, whatever zj_host_set_quirks says;
                                      ZJ_USE_LIBJPEG_OUTPUT: the same, and the images carry ZJ_FLAG_ISLOW;
-                                     ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the same, decoded at 1/2^k (ZJ_FLAG_SCALE_*) */
+                                     ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the same, decoded at 1/2^k (ZJ_FLAG_SCALE_*);
+                                     any of these three | ZJ_USE_EXIF_ORIENTATION: the same, oriented (ZJ_FLAG_ORIENT_*) */
     uint32_t out_colorspace;      /* ZJ_CS_RGB                                           */
     uint32_t num_threads;         /* 4                                                   */
     uint32_t max_width;           /* 16384                                               */
@@ -415,6 +450,9 @@ ZJ_API void zj_decoder_free(zj_decoder *d);
 ZJ_API int zj_decoder_read_headers(zj_decoder *d, const uint8_t *buf, size_t len); /* Decoder::read_headers  */
 ZJ_API int zj_decoder_info(const zj_decoder *d, zj_image_info *info);  /* Decoder::info                       */
 ZJ_API uint32_t zj_decoder_out_colorspace(const zj_decoder *d);        /* Decoder::get_output_colorspace      */
+/* The EXIF orientation o (1-8) of the last zj_decoder_read_headers / decode, whatever the options: 1 before headers were read
+ * or when the file has none (the rules are next to ZJ_FLAG_ORIENT_SHIFT).  Callers size outputs and draw crops with it. */
+ZJ_API uint32_t zj_decoder_orientation(const zj_decoder *d);
 /* Host stage only: headers + entropy decode into coefficient planes owned by the decoder (pinned when a
  * device is present).  `img` is filled with a descriptor pointing at them (valid until the next call). */
 ZJ_API int zj_decoder_decode_coefficients(zj_decoder *d, const uint8_t *buf, size_t len, zj_image *img);

@@ -26,9 +26,20 @@ def scaled_size(width: int, height: int, denom: int):
     return -(-width // denom), -(-height // denom)
 
 
+FLAG_ORIENT_SHIFT, FLAG_ORIENT_MASK = 4, 7 << 4   # zj_image.flags bits 4-6: EXIF orientation o - 1 (spec images only)
+USE_EXIF_ORIENTATION = 0x100   # ORed into a spec / libjpeg / scaled zj_options.use_unsafe value: the output is oriented
+
+
+def oriented_size(width: int, height: int, orientation: int):
+    """The size of a width x height image after EXIF orientation `orientation` (1-8): 5-8 swap the two"""
+    return (height, width) if orientation >= 5 else (width, height)
+
+
 def image_size(img) -> tuple:
-    """(width, height) of a zj_image's output: its size, or the scaled size of a DCT-scaled image (ZJ_FLAG_SCALE_*)"""
-    return scaled_size(img.width, img.height, 1 << ((img.flags & FLAG_SCALE_MASK) >> FLAG_SCALE_SHIFT))
+    """(width, height) of a zj_image's output: its size, or the scaled size of a DCT-scaled image (ZJ_FLAG_SCALE_*), oriented
+    (ZJ_FLAG_ORIENT_*)"""
+    w, h = scaled_size(img.width, img.height, 1 << ((img.flags & FLAG_SCALE_MASK) >> FLAG_SCALE_SHIFT))
+    return oriented_size(w, h, ((img.flags & FLAG_ORIENT_MASK) >> FLAG_ORIENT_SHIFT) + 1)
 QUIRK_Q9, QUIRK_Q10, QUIRK_Q11, QUIRK_ALL = 1, 2, 4, 7   # zj_host_set_quirks (tests only)
 OK = 0
 ERR_INVALID_ARG, ERR_UNSUPPORTED, ERR_SHORT_PLANE, ERR_SHORT_OUTPUT = -1, -2, -3, -4
@@ -177,6 +188,7 @@ SYMBOLS = {
     "zj_decoder_read_headers": (C.c_int, [_P, _P, C.c_size_t]),
     "zj_decoder_info": (C.c_int, [_P, C.POINTER(ZjImageInfo)]),
     "zj_decoder_out_colorspace": (C.c_uint32, [_P]),
+    "zj_decoder_orientation": (C.c_uint32, [_P]),
     "zj_decoder_decode_coefficients": (C.c_int, [_P, _P, C.c_size_t, C.POINTER(ZjImage)]),
     "zj_decoder_decode_buffer": (C.c_int, [_P, _P, C.c_size_t, C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(C.c_size_t)]),
     "zj_buffer_free": (None, [_P]),

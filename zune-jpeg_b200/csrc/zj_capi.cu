@@ -47,6 +47,7 @@ struct Plan {
     int mode, variant, gray, zero_only, fast;
     int islow;         // ZJ_FLAG_ISLOW: the kernels' IDCT is libjpeg-turbo's islow
     int scale;         // ZJ_FLAG_SCALE_*: DCT-scaled decode to 1/2^scale (scaled_kernel)
+    int orient;        // ZJ_FLAG_ORIENT_*: the orientation code o - 1 (0 = none), applied by a second pass (orient_kernel)
     uint32_t n_strips, rows, ncomp_used;
     size_t chunk[3];   // i16 per strip per component
     size_t out_size;
@@ -69,6 +70,8 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     if (islow && !spec) return ZJ_ERR_INVALID_ARG;
     const uint32_t scale = image_scale(img);                 // DCT-scaled: spec | islow planes, reconstructed by scaled_kernel
     if (scale && !islow) return ZJ_ERR_INVALID_ARG;
+    const uint32_t orient = image_orient(img);               // oriented: spec planes, reconstructed as such, then orient_kernel
+    if (orient && !spec) return ZJ_ERR_INVALID_ARG;
     const uint32_t h = img->comp[0].h_samp, v = img->comp[0].v_samp;
     if (img->n_comp == 1 && (h != 1 || v != 1)) return ZJ_ERR_UNSUPPORTED;  // mcu.rs:171-196 resets these before the path
     for (uint32_t z = 1; z < img->n_comp; z++)
@@ -92,6 +95,7 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     pl->variant = (int)img->variant;
     pl->islow = islow;
     pl->scale = (int)scale;
+    pl->orient = (int)orient;
     uint32_t n_strips, ybr, cbr;
     switch (mode) {
     case MODE_H: n_strips = mcu_y / 2; ybr = 2; cbr = 2; break;   // mcu.rs:147-154 -- Q1: odd MCU row dropped
@@ -112,8 +116,8 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     pl->n_strips = n_strips;
     pl->grid_strips = n_strips;
     pl->rows = rows;
-    uint32_t ow, oh;
-    output_dims(img, &ow, &oh);
+    uint32_t ow, oh;   // the kernels write the stored frame; the orient pass turns it into output_dims
+    stored_dims(img, &ow, &oh);
     pl->out_size = (size_t)ow * oh * nc;
     pl->chunk[0] = (size_t)ybr * h * mcu_x * 64;
     pl->chunk[1] = pl->chunk[2] = (size_t)cbr * mcu_x * 64;
@@ -245,12 +249,17 @@ static int check_device_alignment(const zj_image *img, const Plan &pl)
 }
 
 // ------------------------------------------------------------------------------------------------ batches
+struct OrientRun { uint32_t first, count, nc, max_w, max_h; };   // one orient_kernel launch over d_orient[first, first + count)
 struct zj_batch {
     int device;
     std::vector<LaunchGroup> groups;
     std::vector<std::pair<uint8_t *, size_t>> zero_only;  // outputs that are just memset (worker.rs:131-132)
     DevImage *d_images;
     size_t n_images;
+    // oriented images (ZJ_FLAG_ORIENT_*): reconstructed into `scratch`, owned by the batch, then oriented into their outputs
+    std::vector<OrientRun> orient_runs;
+    OrientImage *d_orient;
+    uint8_t *scratch;
     uint64_t algo_bytes;
     cudaStream_t pool_stream;   // non-null + pooled: descriptors come from the stream-ordered pool of this stream
     bool pooled;
@@ -335,16 +344,29 @@ int zj_validate_image(const zj_image *img)
 
 // `pooled`: allocate / upload the descriptors in stream order on `ps` (no device-wide synchronisation: cudaMalloc and
 // above all cudaFree serialise every thread that feeds the device, which is what zj_decode_batch's workers are)
+// `regions` (may be NULL): for an oriented image with regions[i].w != 0, only that rectangle of its stored frame is oriented, and
+// out_dev[i] receives it (regions[i].w * regions[i].h * nc bytes, in the displayed frame)
 static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t *const *out_dev, const size_t *out_len, zj_batch **plan,
-                             bool pooled, cudaStream_t ps);
+                             bool pooled, cudaStream_t ps, const zj_roi *regions = nullptr);
 
 int zj_batch_create(int device, const zj_image *imgs, size_t n, uint8_t *const *out_dev, const size_t *out_len, zj_batch **plan)
 {
     return batch_create_impl(device, imgs, n, out_dev, out_len, plan, false, nullptr);
 }
 
+// device memory for the batch's own arrays: from the stream-ordered pool on `ps` (pooled) or cudaMalloc
+static cudaError_t batch_alloc(void **p, size_t bytes, bool pooled, int device, cudaStream_t ps)
+{
+    return pooled ? pool_alloc(p, bytes, device, ps) : cudaMalloc(p, bytes);
+}
+static void batch_free(void *p, bool pooled, cudaStream_t ps)
+{
+    if (!p) return;
+    if (pooled) cudaFreeAsync(p, ps); else cudaFree(p);
+}
+
 static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t *const *out_dev, const size_t *out_len, zj_batch **plan,
-                             bool pooled, cudaStream_t ps)
+                             bool pooled, cudaStream_t ps, const zj_roi *regions)
 {
     if (!plan) return ZJ_ERR_INVALID_ARG;
     *plan = nullptr;
@@ -352,21 +374,55 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
     int rc = set_device(device);
     if (rc) return rc;
     std::vector<Plan> plans(n);
+    std::vector<OrientImage> orient;      // the oriented images' second pass, src = their offset into the scratch buffer for now
+    size_t scratch_bytes = 0;
     for (size_t i = 0; i < n; i++) {
         rc = plan_image(&imgs[i], &plans[i], out_dev[i]);
         if (rc) return rc;
-        rc = check_buffers(&imgs[i], plans[i], out_dev[i], out_len[i]);
+        const bool region = plans[i].orient && regions && regions[i].w;
+        rc = check_buffers(&imgs[i], plans[i], out_dev[i], region ? SIZE_MAX : out_len[i]);
         if (rc) return rc;
         rc = check_device_alignment(&imgs[i], plans[i]);
         if (rc) return rc;
         for (int z = 0; z < 3; z++) plans[i].dev.coeff[z] = (uint32_t)z < plans[i].ncomp_used ? imgs[i].comp[z].coeff : nullptr;
         plans[i].dev.out = out_dev[i];
+        if (plans[i].orient) {
+            OrientImage oi{};
+            const uint32_t nc = plans[i].dev.nc;
+            uint32_t w, h;
+            stored_dims(&imgs[i], &w, &h);
+            const zj_roi r = region ? regions[i] : zj_roi{0, 0, w, h};
+            if ((uint64_t)r.x + r.w > w || (uint64_t)r.y + r.h > h || r.h == 0) return ZJ_ERR_INVALID_ARG;
+            if (out_len[i] < (size_t)r.w * r.h * nc) return ZJ_ERR_SHORT_OUTPUT;
+            oi.src = reinterpret_cast<const uint8_t *>(scratch_bytes + (size_t)r.y * w * nc + (size_t)r.x * nc);
+            oi.dst = out_dev[i];
+            oi.pitch = w * nc;
+            oi.w = r.w; oi.h = r.h;
+            oi.orient = (uint32_t)plans[i].orient;
+            oi.nc = nc;
+            orient.push_back(oi);
+            plans[i].dev.out = reinterpret_cast<uint8_t *>(scratch_bytes);
+            scratch_bytes += (plans[i].out_size + 255) & ~(size_t)255;
+        }
     }
     zj_batch *b = new zj_batch();
     b->device = device;
     b->d_images = nullptr;
     b->n_images = 0;
     b->algo_bytes = 0;
+    b->d_orient = nullptr;
+    b->scratch = nullptr;
+    b->pooled = pooled;
+    b->pool_stream = ps;
+    if (scratch_bytes) {
+        cudaError_t e = batch_alloc((void **)&b->scratch, scratch_bytes, pooled, device, ps);
+        if (e != cudaSuccess) { delete b; return cuda_fail(e, "cudaMalloc(orientation scratch)"); }
+        for (size_t i = 0; i < n; i++)
+            if (plans[i].orient) plans[i].dev.out = b->scratch + reinterpret_cast<uintptr_t>(plans[i].dev.out);
+        for (OrientImage &oi : orient) oi.src = b->scratch + reinterpret_cast<uintptr_t>(oi.src);
+        // one launch per bytes-per-pixel class
+        std::stable_sort(orient.begin(), orient.end(), [](const OrientImage &a, const OrientImage &c) { return a.nc < c.nc; });
+    }
     // group by kernel: (scale, gray, fast, mode, variant, IDCT); stable so images keep their relative order
     std::vector<size_t> order;
     for (size_t i = 0; i < n; i++) {
@@ -397,18 +453,27 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         b->groups.push_back(g);
         k = e;
     }
+    for (size_t k = 0; k < orient.size();) {
+        OrientRun run{(uint32_t)k, 0, orient[k].nc, 0, 0};
+        for (; k < orient.size() && orient[k].nc == run.nc && run.count < 65535; k++, run.count++) {
+            run.max_w = std::max(run.max_w, orient[k].w);
+            run.max_h = std::max(run.max_h, orient[k].h);
+        }
+        b->orient_runs.push_back(run);
+    }
+    // (pageable sources: the async copies return once the data sits in the driver's staging buffer)
+    auto upload = [&](void **dst, const void *src, size_t bytes, const char *what) -> int {
+        cudaError_t e = batch_alloc(dst, bytes, pooled, device, ps);
+        if (e != cudaSuccess) { *dst = nullptr; return cuda_fail(e, what); }
+        e = pooled ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, ps) : cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
+        return e == cudaSuccess ? ZJ_OK : cuda_fail(e, what);
+    };
     if (!host.empty()) {
-        cudaError_t e = pooled ? pool_alloc((void **)&b->d_images, host.size() * sizeof(DevImage), device, ps)
-                               : cudaMalloc(&b->d_images, host.size() * sizeof(DevImage));
-        if (e != cudaSuccess) { delete b; return cuda_fail(e, "cudaMalloc(descriptors)"); }
-        // (pageable source: the async copy returns once the data sits in the driver's staging buffer)
-        e = pooled ? cudaMemcpyAsync(b->d_images, host.data(), host.size() * sizeof(DevImage), cudaMemcpyHostToDevice, ps)
-                   : cudaMemcpy(b->d_images, host.data(), host.size() * sizeof(DevImage), cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) { if (pooled) cudaFreeAsync(b->d_images, ps); else cudaFree(b->d_images); delete b; return cuda_fail(e, "cudaMemcpy(descriptors)"); }
+        rc = upload((void **)&b->d_images, host.data(), host.size() * sizeof(DevImage), "cudaMemcpy(descriptors)");
         b->n_images = host.size();
     }
-    b->pooled = pooled;
-    b->pool_stream = ps;
+    if (rc == ZJ_OK && !orient.empty()) rc = upload((void **)&b->d_orient, orient.data(), orient.size() * sizeof(OrientImage), "cudaMemcpy(orientation descriptors)");
+    if (rc != ZJ_OK) { zj_batch_destroy(b); return rc; }
     *plan = b;
     return ZJ_OK;
 }
@@ -424,18 +489,24 @@ int zj_batch_run(zj_batch *b, void *stream)
         CU(launch_group(b->d_images, g, s));
         g_launches.fetch_add(1);
     }
+    for (const OrientRun &r : b->orient_runs) {
+        CU(launch_orient(b->d_orient + r.first, r.count, r.nc, r.max_w, r.max_h, s));
+        g_launches.fetch_add(1);
+    }
     return ZJ_OK;
 }
 
-int zj_batch_launches(const zj_batch *b) { return b ? (int)b->groups.size() : 0; }
+int zj_batch_launches(const zj_batch *b) { return b ? (int)(b->groups.size() + b->orient_runs.size()) : 0; }
 uint64_t zj_batch_algorithmic_bytes(const zj_batch *b) { return b ? b->algo_bytes : 0; }
 
 void zj_batch_destroy(zj_batch *b)
 {
     if (!b) return;
-    if (b->d_images) {
+    if (b->d_images || b->d_orient || b->scratch) {
         cudaSetDevice(b->device);
-        if (b->pooled) cudaFreeAsync(b->d_images, b->pool_stream); else cudaFree(b->d_images);
+        batch_free(b->d_images, b->pooled, b->pool_stream);
+        batch_free(b->d_orient, b->pooled, b->pool_stream);
+        batch_free(b->scratch, b->pooled, b->pool_stream);
     }
     delete b;
 }
@@ -593,25 +664,36 @@ static size_t consumer_chunk_bytes()
     return v;
 }
 
-// Sub-batches of consecutive images whose u8 intermediates fit consumer_chunk_bytes() together (at least one image each)
-struct ConsumerChunk { size_t first, count, bytes; };
-// places image i's intermediate of `bytes` bytes in the last sub-batch or a new one; returns its offset in the scratch buffer
-static size_t chunk_place(std::vector<ConsumerChunk> &chunks, size_t i, size_t bytes)
+// Sub-batches of consecutive images whose u8 intermediates, and the scratch their zj_batch allocates for them (oriented images),
+// fit consumer_chunk_bytes() together (at least one image each)
+struct ConsumerChunk { size_t first, count, bytes, charged; };
+// places image i's intermediate of `bytes` bytes in the last sub-batch or a new one, charging `extra` more bytes to its budget;
+// returns its offset in the scratch buffer
+static size_t chunk_place(std::vector<ConsumerChunk> &chunks, size_t i, size_t bytes, size_t extra = 0)
 {
-    const size_t padded = (bytes + 255) & ~(size_t)255;
-    if (chunks.empty() || chunks.back().bytes + padded > consumer_chunk_bytes()) chunks.push_back({i, 0, 0});
+    const size_t padded = (bytes + 255) & ~(size_t)255, charge = padded + ((extra + 255) & ~(size_t)255);
+    if (chunks.empty() || chunks.back().charged + charge > consumer_chunk_bytes()) chunks.push_back({i, 0, 0, 0});
     const size_t off = chunks.back().bytes;
     chunks.back().bytes += padded;
+    chunks.back().charged += charge;
     chunks.back().count++;
     return off;
 }
 
+// Frees the scratch an oriented image's batch reconstructs into, in the order of the pooled batch's stream: once its launches
+// are queued, the next sub-batch may take its place
+static void batch_drop_scratch(zj_batch *b)
+{
+    if (b && b->scratch && b->pooled) { cudaFreeAsync(b->scratch, b->pool_stream); b->scratch = nullptr; }
+}
+
 // The planes route of the second pass: subs[i] is reconstructed into u8_size[i] bytes of a stream-ordered scratch buffer, in
 // sub-batches that take turns in it, and each sub-batch is followed by the pass over its images.  build(i, image i's u8
-// pixels) gives image i's descriptor; the descriptors are uploaded once.  Returns after `s` has drained.
+// pixels) gives image i's descriptor; the descriptors are uploaded once.  regions (may be NULL): the rectangles of oriented images
+// that are oriented into their u8_size[i] bytes (batch_create_impl).  Returns after `s` has drained.
 template <class Build>
 static int reconstruct_then(int device, cudaStream_t s, const zj_image *subs, const std::vector<size_t> &u8_size, const uint32_t *nc,
-                            const zj_output_desc &d, const zj_resize *r, Build build)
+                            const zj_output_desc &d, const zj_resize *r, Build build, const zj_roi *regions = nullptr)
 {
     using Img = decltype(build(0, nullptr));
     const size_t n = u8_size.size();
@@ -619,7 +701,8 @@ static int reconstruct_then(int device, cudaStream_t s, const zj_image *subs, co
     std::vector<size_t> u8_off(n);
     size_t scratch_bytes = 0;
     for (size_t i = 0; i < n; i++) {
-        u8_off[i] = chunk_place(chunks, i, u8_size[i]);
+        // (an oriented image is reconstructed whole into its batch's own scratch, then oriented into its u8_size[i] bytes)
+        u8_off[i] = chunk_place(chunks, i, u8_size[i], image_orient(&subs[i]) ? zj_output_size(&subs[i]) : 0);
         scratch_bytes = std::max(scratch_bytes, chunks.back().bytes);
     }
     uint8_t *scratch = nullptr;
@@ -634,10 +717,12 @@ static int reconstruct_then(int device, cudaStream_t s, const zj_image *subs, co
             std::vector<uint8_t *> outs(ch.count);
             for (size_t k = 0; k < ch.count; k++) outs[k] = scratch + u8_off[ch.first + k];
             zj_batch *b = nullptr;
-            rc = batch_create_impl(device, subs + ch.first, ch.count, outs.data(), u8_size.data() + ch.first, &b, true, s);
+            rc = batch_create_impl(device, subs + ch.first, ch.count, outs.data(), u8_size.data() + ch.first, &b, true, s,
+                                   regions ? regions + ch.first : nullptr);
             if (rc) break;
             batches.push_back(b);
             rc = zj_batch_run(b, s);
+            batch_drop_scratch(b);
             if (rc == ZJ_OK) rc = launch_runs(dev + ch.first, host.data() + ch.first, nc + ch.first, ch.count, d, r, s);
         }
         // the descriptor arrays and the scratch must outlive the kernels
@@ -792,9 +877,10 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     int rc = resize_check(d, r);
     if (rc) return rc;
     if ((!imgs || !out_dev) && n) return ZJ_ERR_INVALID_ARG;
-    // per image: the crop, the strips that hold the rows the resize reads and the size of their u8 pixels
+    // per image: the crop, the strips that hold the rows the resize reads and the size of their u8 pixels.  Of an oriented image
+    // only the rectangle that those rows and the crop's columns come from is oriented, into a buffer of its own: region[i].
     std::vector<zj_image> subs(n);
-    std::vector<zj_roi> crops(n);
+    std::vector<zj_roi> crops(n), region(n, zj_roi{0, 0, 0, 0});
     std::vector<uint32_t> row0(n), nc(n), width(n);
     std::vector<size_t> u8_size(n);
     for (size_t i = 0; i < n; i++) {
@@ -806,6 +892,22 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
         if (rc) return rc;
         uint32_t first, end;
         crop_rows(*r, crops[i], &first, &end);
+        if (const uint32_t t = image_orient(&imgs[i])) {
+            uint32_t sw, sh;
+            stored_dims(&imgs[i], &sw, &sh);
+            // displayed columns [crop.x, crop.x + crop.w) x rows [crop.y + first, crop.y + end): back through the swap and the mirrors
+            uint32_t xa = crops[i].x, xb = crops[i].x + crops[i].w, ya = crops[i].y + first, yb = crops[i].y + end;
+            if (orient_swap(t)) { std::swap(xa, ya); std::swap(xb, yb); }
+            if (orient_flip_x(t)) { const uint32_t a = sw - xb; xb = sw - xa; xa = a; }
+            if (orient_flip_y(t)) { const uint32_t a = sh - yb; yb = sh - ya; ya = a; }
+            region[i] = zj_roi{xa, ya, xb - xa, yb - ya};
+            subs[i] = imgs[i];
+            width[i] = crops[i].w;       // the buffer holds the crop's columns ...
+            row0[i] = 0;                 // ... and its rows [first, end)
+            crops[i].x = 0;
+            u8_size[i] = (size_t)region[i].w * region[i].h * nc[i];
+            continue;
+        }
         rc = zj_image_rows(&imgs[i], crops[i].y + first, crops[i].y + end, &subs[i], &row0[i]);
         if (rc) return rc;
         u8_size[i] = zj_output_size(&subs[i]);
@@ -819,8 +921,9 @@ int zj_gpu_reconstruct_device_resized(int device, void *stream, const zj_image *
     return reconstruct_then(device, (cudaStream_t)stream, subs.data(), u8_size, nc.data(), *d, r, [&](size_t i, const uint8_t *u8) {
         uint32_t sub_w, sub_h;
         output_dims(&subs[i], &sub_w, &sub_h);
+        if (region[i].w) sub_h = (uint32_t)(u8_size[i] / ((size_t)width[i] * nc[i]));
         return resize_image(u8, width[i], sub_h, nc[i], row0[i], crops[i], static_cast<uint8_t *>(out_dev) + i * slot, *r);
-    });
+    }, region.data());
 }
 
 // ------------------------------------------------------------------------------------- the JPEG-bytes route's second pass
@@ -1012,14 +1115,16 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
     int which = 0;
     rc = ZJ_OK;
     while (i < n && rc == ZJ_OK) {
-        size_t j = i, bytes = 0;
+        size_t j = i, bytes = 0, charged = 0;   // staging bytes; those plus the batch's own scratch for oriented images
         while (j < n) {
             size_t need = plans[j].out_size, coef = 0;
             for (uint32_t z = 0; z < plans[j].ncomp_used; z++) coef += (size_t)plans[j].n_strips * plans[j].chunk[z] * 2;
             need += coef + coef / 8 + 4096;      // (planes uploaded as one span may carry the gaps between them)
+            const size_t orient_scratch = plans[j].orient ? plans[j].out_size + 256 : 0;
             // (the first sub-batch is a small one: kernels and downloads start after 1/8 of the usual upload)
-            if (j > i && bytes + need > (i == 0 ? budget / 8 : budget)) break;
+            if (j > i && charged + need + orient_scratch > (i == 0 ? budget / 8 : budget)) break;
             bytes += need + 4 * 256;
+            charged += need + 4 * 256 + orient_scratch;
             j++;
         }
         const int slot = which;                   // stream s and its staging buffer
@@ -1090,6 +1195,7 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
         lap("descriptors + uploads");
         pd->batches.push_back(b);
         rc = zj_batch_run(b, s);
+        batch_drop_scratch(b);
         if (rc != ZJ_OK) break;
         for (size_t k = i; k < j; k++) {
             e = cudaMemcpyAsync(out[k], douts[k - i], plans[k].out_size, cudaMemcpyDeviceToHost, s);

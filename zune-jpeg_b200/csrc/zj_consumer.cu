@@ -779,4 +779,103 @@ cudaError_t launch_pil_resize(const ResizeImage *host, uint32_t count, uint32_t 
     return e;
 }
 
+// ------------------------------------------------------------------------------------------------------ orientation
+// The EXIF orientation pass (DESIGN.md section 4.6.3): Pillow's Transpose of a region of u8 pixels, each pixel's NC bytes moving
+// together.  One CTA moves one OT x OT source tile through shared memory, so that the loads run along source rows and the
+// stores along destination rows: aligned 32-bit words wherever the word lies inside the row segment, bytes at its unaligned
+// ends.  No byte outside the source region is read, none outside the destination written.  Each thread issues all its loads
+// before its first shared store, so that a CTA has its whole tile in flight.
+constexpr int OT = 64;   // tile side in pixels
+
+template <int NC>
+__global__ void __launch_bounds__(256) orient_kernel(const OrientImage *__restrict__ images)
+{
+    // words per shared row: a row segment of OT * NC bytes starting at any offset mod 4 (odd, so that the column reads of the
+    // transposing orientations spread over the banks)
+    constexpr int P = (OT * NC + 3) / 4 + 1;
+    constexpr int NW = (OT * P + 255) / 256;   // word slots per thread and phase
+    __shared__ u32 tile[OT * P];
+    const OrientImage im = images[blockIdx.z];
+    const u32 x0 = blockIdx.x * OT, y0 = blockIdx.y * OT;
+    if (x0 >= im.w || y0 >= im.h) return;
+    const u32 tw = min((u32)OT, im.w - x0), th = min((u32)OT, im.h - y0);
+    // tile row r holds source row y0 + r, pixels [x0, x0 + tw): its byte b at shared byte 4 P r + (offset of the row mod 4) + b
+    const uint8_t *const src = im.src + (size_t)y0 * im.pitch + (size_t)x0 * NC;
+    const u32 src_a = (u32)reinterpret_cast<uintptr_t>(src);
+    {
+        const int nb = (int)(tw * NC);
+        u32 v[NW];
+#pragma unroll
+        for (int q = 0; q < NW; q++) {
+            const u32 i = threadIdx.x + 256u * q, r = i / P, k = i - r * P;
+            v[q] = 0;
+            const int mis = (int)((src_a + r * im.pitch) & 3u), lo = 4 * (int)k - mis;   // the word's first byte in the row segment
+            if (r >= th || lo >= nb) continue;
+            const uint8_t *row = src + (size_t)r * im.pitch;
+            if (lo >= 0 && lo + 4 <= nb) {
+                v[q] = __ldg(reinterpret_cast<const u32 *>(row + lo));
+            } else {
+#pragma unroll
+                for (int j = 0; j < 4; j++)
+                    if (lo + j >= 0 && lo + j < nb) v[q] |= (u32)__ldg(row + lo + j) << (8 * j);
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < NW; q++) {
+            const u32 i = threadIdx.x + 256u * q;
+            if (i < th * P) tile[i] = v[q];
+        }
+    }
+    __syncthreads();
+    const uint8_t *const sb = reinterpret_cast<const uint8_t *>(tile);
+    const bool fx = orient_flip_x(im.orient), fy = orient_flip_y(im.orient), sw = orient_swap(im.orient);
+    // the tile's place in the destination: mirrored x' / y' ranges, axes swapped
+    const u32 xm0 = fx ? im.w - x0 - tw : x0, ym0 = fy ? im.h - y0 - th : y0;
+    const u32 dx0 = sw ? ym0 : xm0, dy0 = sw ? xm0 : ym0, dtw = sw ? th : tw, dth = sw ? tw : th;
+    const u32 dpitch = (sw ? im.h : im.w) * NC;
+    uint8_t *const dst = im.dst + (size_t)dy0 * dpitch + (size_t)dx0 * NC;
+    const u32 dst_a = (u32)reinterpret_cast<uintptr_t>(dst);
+    const int nb = (int)(dtw * NC);
+#pragma unroll
+    for (int q = 0; q < NW; q++) {
+        const u32 i = threadIdx.x + 256u * q, r = i / P, k = i - r * P;
+        const int mis = (int)((dst_a + r * dpitch) & 3u), lo = 4 * (int)k - mis;
+        if (r >= dth || lo >= nb) continue;
+        // the shared bytes of destination pixel p of row r: its local (x', y'), mirrored back to the source tile
+        auto pixel = [&](u32 p) {
+            const u32 xl = sw ? r : p, yl = sw ? p : r;
+            const u32 sx = fx ? tw - 1 - xl : xl, sy = fy ? th - 1 - yl : yl;
+            return sb + 4 * P * sy + ((src_a + sy * im.pitch) & 3u) + sx * NC;
+        };
+        const u32 b0 = (u32)max(lo, 0);
+        u32 p = b0 / NC, c = b0 - p * NC;   // the word's first byte in the row: pixel p, channel c
+        const uint8_t *px = pixel(p);
+        u32 v = 0;
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int b = lo + j;
+            if (b < 0 || b >= nb) continue;
+            v |= (u32)px[c] << (8 * j);
+            if (++c == NC && b + 1 < nb) { c = 0; px = pixel(++p); }
+        }
+        uint8_t *row = dst + (size_t)r * dpitch;
+        if (lo >= 0 && lo + 4 <= nb) {
+            *reinterpret_cast<u32 *>(row + lo) = v;
+        } else {
+#pragma unroll
+            for (int j = 0; j < 4; j++)
+                if (lo + j >= 0 && lo + j < nb) row[lo + j] = (uint8_t)(v >> (8 * j));
+        }
+    }
+}
+
+cudaError_t launch_orient(const OrientImage *d_images, uint32_t count, uint32_t nc, uint32_t max_w, uint32_t max_h, cudaStream_t s)
+{
+    const dim3 grid((max_w + OT - 1) / OT, (max_h + OT - 1) / OT, count);
+    if (nc == 1) orient_kernel<1><<<grid, 256, 0, s>>>(d_images);
+    else if (nc == 3) orient_kernel<3><<<grid, 256, 0, s>>>(d_images);
+    else orient_kernel<4><<<grid, 256, 0, s>>>(d_images);
+    return cudaGetLastError();
+}
+
 }  // namespace zj

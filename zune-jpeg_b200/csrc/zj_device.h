@@ -71,15 +71,41 @@ struct DevImage {
 
 // MCU columns per tile of scaled_kernel (DCT-scaled images), by mode: about one block per thread in phase 1
 constexpr int TS_NONE = 80, TS_H = 60, TS_V = 32, TS_HV = 42;
-// The scale k of a zj_image (ZJ_FLAG_SCALE_*), and the size of its output: width x height, or ceil(width / 2^k) x ceil(height / 2^k)
-// for a DCT-scaled image.  Everything downstream of reconstruction sees this size.
+// The scale k of a zj_image (ZJ_FLAG_SCALE_*), and the size of its output (output_dims): width x height, or ceil(width / 2^k) x
+// ceil(height / 2^k) for a DCT-scaled image, with the two swapped by orientations 5-8.  Everything downstream of reconstruction
+// sees this size.
 inline uint32_t image_scale(const zj_image *img) { return (img->flags & ZJ_FLAG_SCALE_MASK) >> ZJ_FLAG_SCALE_SHIFT; }
-inline void output_dims(const zj_image *img, uint32_t *w, uint32_t *h)
+// The EXIF orientation code o - 1 of a zj_image (ZJ_FLAG_ORIENT_*): 0 = none; 4-7 (o = 5-8) swap width and height
+inline uint32_t image_orient(const zj_image *img) { return (img->flags & ZJ_FLAG_ORIENT_MASK) >> ZJ_FLAG_ORIENT_SHIFT; }
+// The reconstructed image before orientation: the size the kernels write (and the oriented image's stored frame)
+inline void stored_dims(const zj_image *img, uint32_t *w, uint32_t *h)
 {
     const uint32_t k = image_scale(img), m = (1u << k) - 1;
     *w = (uint32_t)(((uint64_t)img->width + m) >> k);
     *h = (uint32_t)(((uint64_t)img->height + m) >> k);
 }
+inline void output_dims(const zj_image *img, uint32_t *w, uint32_t *h)
+{
+    if (image_orient(img) >= 4) stored_dims(img, h, w);
+    else stored_dims(img, w, h);
+}
+
+// Pillow's Transpose for orientation code t = o - 1 (ZJ_FLAG_ORIENT_*), as a map of stored pixel (x, y) of a w x h image to the
+// output: mirror x (x -> w-1-x), mirror y, then swap the axes.
+inline __host__ __device__ bool orient_flip_x(uint32_t t) { return t == 1 || t == 2 || t == 6 || t == 7; }
+inline __host__ __device__ bool orient_flip_y(uint32_t t) { return t == 2 || t == 3 || t == 5 || t == 6; }
+inline __host__ __device__ bool orient_swap(uint32_t t) { return t >= 4; }
+
+// One image of an orient launch (zj_consumer.cu): a w x h region of interleaved u8 pixels (row pitch `pitch` bytes, starting at
+// `src`) goes through the transform of orientation code `orient` into `dst`, a tightly packed image of w x h (or h x w) pixels.
+struct OrientImage {
+    const uint8_t *src;
+    uint8_t *dst;
+    uint32_t pitch;
+    uint32_t w, h;
+    uint32_t orient;
+    uint32_t nc;                  // bytes per pixel (the launch's)
+};
 
 // Host-side launch plan entry: one kernel launch per (mode, variant, IDCT, out-kind class) group.
 struct LaunchGroup {
@@ -114,6 +140,8 @@ struct ResizeImage {
 cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream);
 cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
 cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
+// images [0, count) (count <= 65535) of nc bytes per pixel; max_w x max_h covers every region
+cudaError_t launch_orient(const OrientImage *d_images, uint32_t count, uint32_t nc, uint32_t max_w, uint32_t max_h, cudaStream_t s);
 
 // The PIL filters (header rules 1 and 2) for a crop of w x h: the resized size, the window's offset in it, and the crop rows
 // [y0, y1) the window's vertical taps read.  ZJ_ERR_INVALID_ARG when the resized size breaks rule 1.

@@ -563,6 +563,95 @@ struct StripSink {
     virtual ~StripSink() {}
 };
 
+// ------------------------------------------------------------------------------------------------ EXIF orientation
+// The APP1 segments before the first SOS that carry metadata (the statement is next to ZJ_FLAG_ORIENT_SHIFT in the header).
+// They point into the caller's buffer, which outlives the header parse they are read in.
+struct OrientSource {
+    struct Span { const uint8_t *p; size_t n; };
+    std::vector<Span> exif;        // the EXIF bytes: the first Exif APP1 payload, then each later one's bytes after its header
+    size_t exif_len = 0;
+    Span xmp{nullptr, 0};          // the last XMP APP1 segment's bytes after its 29-byte header
+
+    void clear() { exif.clear(); exif_len = 0; xmp = {nullptr, 0}; }   // (keeps the span list's capacity for the next file)
+
+    // n bytes at offset `off` of the EXIF bytes; false when they are not all there
+    bool read(size_t off, size_t n, uint8_t *dst) const
+    {
+        if (off > exif_len || n > exif_len - off) return false;
+        for (size_t k = 0; k < exif.size() && n; k++) {
+            if (off >= exif[k].n) { off -= exif[k].n; continue; }
+            const size_t m = std::min(n, exif[k].n - off);
+            memcpy(dst, exif[k].p + off, m);
+            dst += m; n -= m; off = 0;
+        }
+        return n == 0;
+    }
+    // Pillow's Image.getexif() orientation, then exif_transpose's choice: 2-8, or 1 for no transform
+    uint32_t orientation() const
+    {
+        static const uint8_t EXIF_HDR[6] = {'E', 'x', 'i', 'f', 0, 0};
+        size_t base = 0;   // Exif.load strips every leading "Exif\0\0"
+        for (uint8_t h[6]; read(base, 6, h) && memcmp(h, EXIF_HDR, 6) == 0;) base += 6;
+        long v = -1;       // the tag's value; -1 = IFD0 has no tag 0x0112
+        if (base < exif_len) {
+            uint8_t hd[8];
+            if (!read(base, 8, hd)) return 1;   // (Pillow raises on a short or unknown TIFF header; its orientation is then 1)
+            const bool le = memcmp(hd, "II*\0", 4) == 0;
+            if (!le && memcmp(hd, "MM\0*", 4) != 0) return 1;
+            auto u16 = [le](const uint8_t *b) { return le ? (uint32_t)(b[0] | b[1] << 8) : (uint32_t)(b[0] << 8 | b[1]); };
+            auto u32 = [le](const uint8_t *b) { return le ? (uint32_t)b[0] | (uint32_t)b[1] << 8 | (uint32_t)b[2] << 16 | (uint32_t)b[3] << 24
+                                                          : (uint32_t)b[0] << 24 | (uint32_t)b[1] << 16 | (uint32_t)b[2] << 8 | (uint32_t)b[3]; };
+            const size_t tiff_len = exif_len - base;
+            const size_t ifd = u32(hd + 4);
+            uint8_t cnt[2];
+            // IFD0 as ImageFileDirectory_v2.load reads it: entries up to the first one that cannot be read whole (its bytes, or
+            // the data it points at), skipping unknown types and empty values; a later entry of a tag replaces an earlier one
+            if (ifd <= tiff_len && read(base + ifd, 2, cnt)) {
+                static const uint8_t unit[14] = {0, 1, 1, 2, 4, 8, 1, 1, 2, 4, 8, 4, 8, 4};   // TIFF type -> bytes per value
+                const uint32_t n = u16(cnt);
+                for (uint32_t k = 0; k < n; k++) {
+                    uint8_t e[12];
+                    if (!read(base + ifd + 2 + 12 * (size_t)k, 12, e)) break;
+                    const uint32_t typ = u16(e + 2), count = u32(e + 4);
+                    if (typ == 0 || typ >= 14) continue;
+                    const uint64_t size = (uint64_t)count * unit[typ];
+                    if (size == 0) continue;
+                    uint8_t val[4];
+                    const uint8_t *vp = e + 8;
+                    if (size > 4) {
+                        const uint64_t off = u32(e + 8);
+                        if (off + size > tiff_len) break;
+                        if (u16(e) == 0x0112 && !read(base + off, 4, val)) break;
+                        vp = val;
+                    }
+                    if (u16(e) != 0x0112) continue;
+                    // SHORT / LONG and their signed forms: the first value (Pillow keeps it when the count is not 1); any other
+                    // type: a value that is not an orientation
+                    if (typ == 3) v = u16(vp);
+                    else if (typ == 8) v = (int16_t)u16(vp);
+                    else if (typ == 4) v = u32(vp);
+                    else if (typ == 9) v = (int32_t)u32(vp);
+                    else v = 0;
+                }
+            }
+        }
+        if (v < 0 && xmp.p) {
+            // the first match of tiff:Orientation(="|>)([0-9])
+            static const char KEY[] = "tiff:Orientation";
+            const size_t kl = sizeof(KEY) - 1;
+            for (size_t at = 0; at + kl + 2 <= xmp.n;) {
+                const uint8_t *f = (const uint8_t *)memmem(xmp.p + at, xmp.n - at, KEY, kl);
+                if (!f) break;
+                const size_t q = (size_t)(f - xmp.p) + kl;
+                if (q + 1 < xmp.n && xmp.p[q] == '=' && xmp.p[q + 1] == '"' && q + 2 < xmp.n && xmp.p[q + 2] >= '0' && xmp.p[q + 2] <= '9') { v = xmp.p[q + 2] - '0'; break; }
+                if (q + 1 < xmp.n && xmp.p[q] == '>' && xmp.p[q + 1] >= '0' && xmp.p[q + 1] <= '9') { v = xmp.p[q + 1] - '0'; break; }
+                at = (size_t)(f - xmp.p) + 1;
+            }
+        }
+        return v >= 2 && v <= 8 ? (uint32_t)v : 1u;
+    }
+};
+
 struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     StripSink *sink = nullptr;   // set for the duration of one zj_decoder_decode_into call
     zj_options options;
@@ -590,6 +679,10 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     // restart-interval-parallel entropy decode: threads to use (0 = options.num_threads) and how many intervals the last
     // decode ran side by side (0 = the sequential loop)
     size_t entropy_threads = 0, last_entropy_segments = 0;
+    // EXIF orientation: the metadata segments met before the first SOS, and the orientation they give (1 until that SOS)
+    OrientSource orient_src;
+    bool before_sos = true;
+    uint32_t orientation = 1;
 
     explicit zj_decoder(const zj_options &o) : options(o)
     {
@@ -621,20 +714,31 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         for (auto &z : z_order) z = 0;
         restart_interval = 0;
         todo = 0x7fffffff;
+        orient_src.clear();
+        before_sos = true;
+        orientation = 1;
     }
     uint32_t user_out_cs = ZJ_CS_RGB;
     uint32_t quirks = ZJ_QUIRK_ALL;   // the host-stage quirks of this decode (g_quirks when it started; none for spec output)
     bool quirk(uint32_t bit) const { return (quirks & bit) != 0; }
     // spec output, with either IDCT and at any scale: the host stage is the same for all, only the descriptor's ZJ_FLAG_ISLOW and
     // ZJ_FLAG_SCALE_* differ
-    bool spec() const { return options.use_unsafe == ZJ_USE_SPEC_OUTPUT || libjpeg(); }
-    bool libjpeg() const { return options.use_unsafe == ZJ_USE_LIBJPEG_OUTPUT || scale() != 0; }
+    bool spec() const { return use() == ZJ_USE_SPEC_OUTPUT || libjpeg(); }
+    bool libjpeg() const { return use() == ZJ_USE_LIBJPEG_OUTPUT || scale() != 0; }
     // ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the DCT-scaled decode to 1/2^k (every other value keeps its meaning)
-    uint32_t scale() const
+    static uint32_t scale_of(uint32_t u)
     {
-        const uint32_t k = options.use_unsafe >> 4;
-        return (options.use_unsafe & 15u) == ZJ_USE_LIBJPEG_OUTPUT && k >= 1 && k <= 3 ? k : 0;
+        const uint32_t k = u >> 4;
+        return (u & 15u) == ZJ_USE_LIBJPEG_OUTPUT && k >= 1 && k <= 3 ? k : 0;
     }
+    uint32_t scale() const { return scale_of(use()); }
+    // ZJ_USE_EXIF_ORIENTATION ORed into a spec, libjpeg or scaled value: that value, oriented; every other value keeps its meaning
+    bool exif_orientation() const
+    {
+        const uint32_t u = options.use_unsafe & ~(uint32_t)ZJ_USE_EXIF_ORIENTATION;
+        return (options.use_unsafe & ZJ_USE_EXIF_ORIENTATION) && (u == ZJ_USE_SPEC_OUTPUT || u == ZJ_USE_LIBJPEG_OUTPUT || scale_of(u) != 0);
+    }
+    uint32_t use() const { return exif_orientation() ? options.use_unsafe & ~(uint32_t)ZJ_USE_EXIF_ORIENTATION : options.use_unsafe; }
     // a one-component image: GRAYSCALE output (headers.rs:278-285, mcu.rs:171-196), except that spec output keeps RGB / RGBA / RGBX
     void gray_input_out_cs()
     {
@@ -825,7 +929,10 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             break;
         case M_DQT: parse_dqt(buf); break;
         case M_DHT: parse_huffman(buf); break;
-        case M_SOS: parse_sos(buf); break;
+        case M_SOS:
+            if (before_sos) { before_sos = false; orientation = orient_src.orientation(); }
+            parse_sos(buf);
+            break;
         case M_EOI: FAIL(ZJ_DE_FORMAT, "Premature End of image");
         case M_DAC: case M_DNL:
             FAIL(ZJ_DE_FORMAT, fmt("Parsing of the following header `%s` is not supported,cannot continue", marker_debug(m).c_str()));
@@ -834,7 +941,29 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             restart_interval = buf.read_u16_be();
             todo = restart_interval;
             break;
+        case M_APP:
+            if (m.n == 1 && before_sos) {
+                const size_t start = buf.pos + 2;
+                skip_segment(buf, "Found a marker with invalid length:%u\n");
+                note_app1(buf.data + start, std::min(buf.pos, buf.len) - std::min(start, buf.len));
+                break;
+            }
+            skip_segment(buf, "Found a marker with invalid length:%u\n");
+            break;
         default: skip_segment(buf, "Found a marker with invalid length:%u\n"); break;
+        }
+    }
+    // an APP1 segment's payload before the first SOS: EXIF or XMP (JpegImagePlugin.py APP())
+    void note_app1(const uint8_t *p, size_t n)
+    {
+        static const char XMP[] = "http://ns.adobe.com/xap/1.0/";   // (29 bytes with its NUL)
+        OrientSource &o = orient_src;
+        if (n >= 6 && memcmp(p, "Exif\0\0", 6) == 0) {
+            const size_t skip = o.exif.empty() ? 0 : 6;
+            o.exif.push_back({p + skip, n - skip});
+            o.exif_len += n - skip;
+        } else if (n >= sizeof(XMP) && memcmp(p, XMP, sizeof(XMP)) == 0) {
+            o.xmp = {p + sizeof(XMP), n - sizeof(XMP)};
         }
     }
     void decode_headers_internal(Cursor &buf)  // decoder.rs:239-303
@@ -1390,7 +1519,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         img->n_comp = (uint32_t)in_components();
         img->out_cs = options.out_colorspace;
         img->variant = spec() ? ZJ_VARIANT_SPEC : (options.use_unsafe ? ZJ_VARIANT_X86 : ZJ_VARIANT_SCALAR);
-        img->flags = (is_progressive ? ZJ_FLAG_PROGRESSIVE : 0) | (libjpeg() ? ZJ_FLAG_ISLOW : 0) | scale() << ZJ_FLAG_SCALE_SHIFT;
+        img->flags = (is_progressive ? ZJ_FLAG_PROGRESSIVE : 0) | (libjpeg() ? ZJ_FLAG_ISLOW : 0) | scale() << ZJ_FLAG_SCALE_SHIFT |
+                     (exif_orientation() ? (orientation - 1) << ZJ_FLAG_ORIENT_SHIFT : 0);
         for (size_t z = 0; z < in_components(); z++) {
             zj_component &c = img->comp[z];
             c.coeff = plane_len[z] ? planes[z].p : nullptr;
@@ -1477,6 +1607,7 @@ ZJ_API int zj_decoder_info(const zj_decoder *d, zj_image_info *info)
     return ZJ_OK;
 }
 ZJ_API uint32_t zj_decoder_out_colorspace(const zj_decoder *d) { return d ? d->options.out_colorspace : 0; }
+ZJ_API uint32_t zj_decoder_orientation(const zj_decoder *d) { return d ? d->orientation : 1; }
 
 ZJ_API int zj_decoder_decode_coefficients(zj_decoder *d, const uint8_t *buf, size_t len, zj_image *img)
 {
@@ -2229,6 +2360,7 @@ static int decode_then(const zj_options &opt, const uint8_t *const *bufs, const 
             // (the output's size: a DCT-scaled decode gives ceil(width / 2^k) x ceil(height / 2^k), as output_dims states)
             const uint32_t k = dd->scale(), m = (1u << k) - 1;
             img[i].width = (info.width + m) >> k; img[i].height = (info.height + m) >> k;
+            if (dd->exif_orientation() && dd->orientation >= 5) std::swap(img[i].width, img[i].height);   // (orientations 5-8)
             img[i].nc = (uint32_t)zj::num_components(zj_decoder_out_colorspace(dd));
             len[i] = (size_t)img[i].width * img[i].height * img[i].nc;
             off[i] = total;

@@ -88,6 +88,7 @@ class ZuneJpegOptions:
         self._spec_output = False
         self._libjpeg_output = False
         self._scale_denom = 1
+        self._exif_orientation = False
 
     @staticmethod
     def new() -> "ZuneJpegOptions":
@@ -138,14 +139,23 @@ class ZuneJpegOptions:
             raise ValueError(f"scale denominator must be 1, 2, 4 or 8, not {d!r}")
         return self._with(_scale_denom=int(d))
 
+    # not in the reference: the EXIF orientation applied to spec or libjpeg output, as Pillow's ImageOps.exif_transpose does
+    # (ZJ_FLAG_ORIENT_*; sizes and rois are then those of the displayed image, oriented_size).  Needs spec or libjpeg output.
+    def get_exif_orientation(self): return self._exif_orientation
+    def set_exif_orientation(self, choice: bool): return self._with(_exif_orientation=bool(choice))
+
     def _raw(self) -> ZjOptions:
         o = ZjOptions()
         if self._scale_denom > 1 and not self._libjpeg_output:
             raise ValueError("a scale denominator above 1 needs libjpeg output (set_libjpeg_output(True))")
+        if self._exif_orientation and not (self._libjpeg_output or self._spec_output):
+            raise ValueError("EXIF orientation needs spec or libjpeg output (set_spec_output(True) or set_libjpeg_output(True))")
         if self._libjpeg_output:
             o.use_unsafe = _ffi.USE_LIBJPEG_OUTPUT | (self._scale_denom.bit_length() - 1) << _ffi.USE_SCALE_SHIFT
         else:
             o.use_unsafe = _ffi.USE_SPEC_OUTPUT if self._spec_output else int(self._use_unsafe)
+        if self._exif_orientation:
+            o.use_unsafe |= _ffi.USE_EXIF_ORIENTATION
         o.out_colorspace = int(self._out_colorspace)
         o.num_threads = self._num_threads
         o.max_width, o.max_height = self._max_width, self._max_height
@@ -292,6 +302,11 @@ class Decoder:
     def get_output_colorspace(self) -> ColorSpace:
         return ColorSpace(self._lib.zj_decoder_out_colorspace(self._h))
 
+    def exif_orientation(self) -> int:
+        """The EXIF orientation (1-8) of the file whose headers were read last, whatever the options: 1 before headers or when
+        the file has none.  Pillow's rule (getexif + exif_transpose; the header states it next to ZJ_FLAG_ORIENT_SHIFT)."""
+        return int(self._lib.zj_decoder_orientation(self._h))
+
     # ---- deprecated setters kept by the reference (decoder.rs:531-603)
     def rgba(self):
         self.set_output_colorspace(ColorSpace.RGBA)
@@ -417,7 +432,8 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
     """zj_decode_batch_gpu_device_resized: JPEG byte strings in, one batch tensor in device memory out -- every image decoded
     whole, its crop resized to `resize` (a gpu.Resize) in the layout / type / normalisation of `desc` (a gpu.OutputDesc, scale
     must be full size; default HWC u8).  rois: None, or one (x, y, w, h) or None (= the whole image) per image, in the
-    coordinates of the decoded image (ceil(width / d) x ceil(height / d) with the options' scale denominator d).
+    coordinates of the decoded image (ceil(width / d) x ceil(height / d) with the options' scale denominator d; with EXIF
+    orientation, of the displayed image: oriented_size).
 
     Returns (gpu.DeviceArray of shape (N, C, OH, OW) or (N, OH, OW, C), [None | DecodeErrors per image]).  The errors are the
     ones decode_batch reports for the same inputs; a crop that does not fit its image, or an image whose channel count is not
@@ -439,6 +455,8 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
                 try:
                     d.read_headers(keep[i])
                     sizes[i] = _ffi.scaled_size(d.width(), d.height(), options.get_scale_denom())
+                    if options.get_exif_orientation():
+                        sizes[i] = _ffi.oriented_size(*sizes[i], d.exif_orientation())
                 except DecodeErrors:
                     sizes[i] = (1, 1)
     nc = ColorSpace(options.get_out_colorspace()).num_components()
