@@ -205,7 +205,8 @@ typedef struct zj_component {
 
 typedef struct zj_image {
     uint32_t width, height; /* ImageInfo::width/height (decoder.rs:652-668)                                 */
-    uint32_t n_comp;        /* 1 (GRAYSCALE in) or 3 (YCbCr in) = input_colorspace.num_components()         */
+    uint32_t n_comp;        /* 1 (GRAYSCALE in) or 3 (YCbCr in) = input_colorspace.num_components(); 4 from the
+                               host stage for CMYK / YCCK (see zj_decoder_component)                          */
     uint32_t out_cs;        /* zj_colorspace: ZuneJpegOptions::out_colorspace                               */
     uint32_t variant;       /* zj_variant                                                                   */
     uint32_t flags;         /* ZJ_FLAG_*                                                                    */
@@ -453,6 +454,38 @@ ZJ_API uint32_t zj_decoder_out_colorspace(const zj_decoder *d);        /* Decode
 /* The EXIF orientation o (1-8) of the last zj_decoder_read_headers / decode, whatever the options: 1 before headers were read
  * or when the file has none (the rules are next to ZJ_FLAG_ORIENT_SHIFT).  Callers size outputs and draw crops with it. */
 ZJ_API uint32_t zj_decoder_orientation(const zj_decoder *d);
+/* Four-component JPEGs -- CMYK, and YCCK as Photoshop writes it (DESIGN.md section 4.6.4).  The host stage decodes them with
+ * zj_options.use_unsafe = ZJ_USE_SPEC_OUTPUT, ZJ_USE_LIBJPEG_OUTPUT or ZJ_USE_LIBJPEG_OUTPUT | k << 4 (with or without
+ * ZJ_USE_EXIF_ORIENTATION), baseline or progressive; every other use_unsafe value rejects them as the reference does.  The
+ * output is what Pillow 12.2's Image.open(f).convert(...) gives.  For components z = 0..3 in SOF order:
+ *   1. Colour model (libjpeg-turbo jdmarker.c examine_app14, jdapimin.c default_decompress_parms): an Adobe marker is an APP14
+ *      segment before the first SOS whose payload is at least 12 bytes long and starts with "Adobe"; its transform is payload
+ *      byte 11, and the last such segment wins.  Transform 0: CMYK; any other value: YCCK; no Adobe marker: CMYK.  JFIF markers
+ *      do not matter.  Component ids may be any distinct bytes; SOS selects components by id.
+ *   2. Samples: every component goes through step 1 (ZJ_USE_SPEC_OUTPUT), 1' (ZJ_FLAG_ISLOW) or 2'' (a scale), with rule 1'''s
+ *      block size ss_z and rule 3'''s size dw_z x dh_z per component, (hmax, vmax) = the largest factors over all four.  Sampling
+ *      factors are 1 or 2 (others: ZJ_ERR_UNSUPPORTED).  Component z is up-sampled on its own by (hmax s0 / (h_z ss_z),
+ *      vmax s0 / (v_z ss_z)), fancy = (s0 > 1): (1, 1) none; (2, 1) step 3's H filter when fancy and dw_z > 2, else each sample
+ *      twice; (1, 2) the V filter when fancy, else each row twice; (2, 2) the HV filter when fancy and dw_z > 2, else 2x2
+ *      repetition (libjpeg-turbo jdsample.c jinit_upsampler).  Neighbours are clamped to [0, dh_z-1] x [0, dw_z-1].
+ *   3. YCCK -> CMYK (jdcolor.c ycck_cmyk_convert), cb' = Cb - 128, cr' = Cr - 128:
+ *        C0 = clamp(255 - (Y + ((91881 cr' + 32768) >> 16)))     M0 = clamp(255 - (Y + ((-22554 cb' - 46802 cr' + 32768) >> 16)))
+ *        Y0 = clamp(255 - (Y + ((116130 cb' + 32768) >> 16)))   K0 = K
+ *      CMYK: (C0, M0, Y0, K0) = the samples.
+ *   4. Pillow reads every CMYK JPEG as "CMYK;I": (c, m, y, k) = 255 - (C0, M0, Y0, K0).  Convert.c cmyk2rgb, nk = 255 - k,
+ *      t = x nk + 128: R = clamp(nk - (((t >> 8) + t) >> 8)) from x = c, G likewise from m, B from y.
+ *   5. Output: RGB = R, G, B (convert("RGB")); RGBA / RGBX = R, G, B, 255 (convert("RGBA")); GRAYSCALE = (19595 R + 38470 G +
+ *      7471 B + 32768) >> 16 (convert("L")); CMYK = c, m, y, k (the pixels of Image.open(f)).  YCBCR and YCCK output:
+ *      ZJ_ERR_UNSUPPORTED.  Orientation (ZJ_FLAG_ORIENT_*) and the consumers apply to this output unchanged.
+ * zj_image has room for three components, so zj_decoder_decode_coefficients fills `img` with n_comp = 4 and comp[0..2], and
+ * zj_decoder_component gives any component of the last decode, the fourth included.  The planes-in entry points
+ * (zj_gpu_reconstruct*, zj_batch_create, ...) refuse n_comp = 4 (ZJ_ERR_INVALID_ARG); the JPEG-bytes entry points decode these
+ * files. */
+/* The colour model of the last headers read: ZJ_CS_GRAYSCALE, ZJ_CS_YCBCR, or for four components ZJ_CS_CMYK / ZJ_CS_YCCK. */
+ZJ_API uint32_t zj_decoder_jpeg_colorspace(const zj_decoder *d);
+/* *c = component z (SOF order) of the last zj_decoder_decode_coefficients, pointing at the decoder's planes (valid until the
+ * next call); ZJ_ERR_INVALID_ARG when the image has no component z. */
+ZJ_API int zj_decoder_component(const zj_decoder *d, uint32_t z, zj_component *c);
 /* Host stage only: headers + entropy decode into coefficient planes owned by the decoder (pinned when a
  * device is present).  `img` is filled with a descriptor pointing at them (valid until the next call). */
 ZJ_API int zj_decoder_decode_coefficients(zj_decoder *d, const uint8_t *buf, size_t len, zj_image *img);

@@ -189,6 +189,8 @@ SYMBOLS = {
     "zj_decoder_info": (C.c_int, [_P, C.POINTER(ZjImageInfo)]),
     "zj_decoder_out_colorspace": (C.c_uint32, [_P]),
     "zj_decoder_orientation": (C.c_uint32, [_P]),
+    "zj_decoder_jpeg_colorspace": (C.c_uint32, [_P]),
+    "zj_decoder_component": (C.c_int, [_P, C.c_uint32, C.POINTER(ZjComponent)]),
     "zj_decoder_decode_coefficients": (C.c_int, [_P, _P, C.c_size_t, C.POINTER(ZjImage)]),
     "zj_decoder_decode_buffer": (C.c_int, [_P, _P, C.c_size_t, C.POINTER(C.POINTER(C.c_uint8)), C.POINTER(C.c_size_t)]),
     "zj_buffer_free": (None, [_P]),

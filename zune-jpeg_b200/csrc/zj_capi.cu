@@ -48,18 +48,89 @@ struct Plan {
     int islow;         // ZJ_FLAG_ISLOW: the kernels' IDCT is libjpeg-turbo's islow
     int scale;         // ZJ_FLAG_SCALE_*: DCT-scaled decode to 1/2^scale (scaled_kernel)
     int orient;        // ZJ_FLAG_ORIENT_*: the orientation code o - 1 (0 = none), applied by a second pass (orient_kernel)
+    int cmyk;          // four-component input: `cm` instead of `dev`, cmyk_kernel
     uint32_t n_strips, rows, ncomp_used;
-    size_t chunk[3];   // i16 per strip per component
+    size_t chunk[4];   // i16 per strip per component
     size_t out_size;
     DevImage dev;      // pointers filled by the caller
+    CmykImage cm;
     uint32_t grid_tiles, grid_strips;   // launch extents (grid_strips: strips as the kernel counts them)
+    uint8_t *&out_ptr() { return cmyk ? cm.out : dev.out; }
 };
+
+// component z of an image: comp[z], and for four-component images the Extra4's as z = 3
+static const zj_component &component(const zj_image *img, const Extra4 *ext, uint32_t z) { return z < 3 ? img->comp[z] : ext->k; }
+
+// A four-component image (the statement is in include/zune_jpeg_b200.h next to zj_decoder_jpeg_colorspace): spec output only.
+// Strips are MCU rows; the planes are raster planes of mcu_x h_z x mcu_y v_z blocks.
+static int plan_cmyk(const zj_image *img, const Extra4 *ext, Plan *pl)
+{
+    if (!ext || (ext->jpeg_cs != ZJ_CS_CMYK && ext->jpeg_cs != ZJ_CS_YCCK)) return ZJ_ERR_INVALID_ARG;
+    if (img->width == 0 || img->height == 0 || img->width > 65535 || img->height > 65535) return ZJ_ERR_INVALID_ARG;
+    const int nc = num_components(img->out_cs);
+    if (nc == 0 || img->variant != ZJ_VARIANT_SPEC) return ZJ_ERR_INVALID_ARG;
+    const bool islow = (img->flags & ZJ_FLAG_ISLOW) != 0;
+    const uint32_t scale = image_scale(img), orient = image_orient(img);
+    if (scale && !islow) return ZJ_ERR_INVALID_ARG;
+    uint32_t kind;
+    switch (img->out_cs) {
+    case ZJ_CS_RGB: case ZJ_CS_RGBA: case ZJ_CS_RGBX: kind = CMYK_OUT_RGB; break;
+    case ZJ_CS_GRAYSCALE: kind = CMYK_OUT_GRAY; break;
+    case ZJ_CS_CMYK: kind = CMYK_OUT_CMYK; break;
+    default: return ZJ_ERR_UNSUPPORTED;   // YCBCR, YCCK
+    }
+    uint32_t hmax = 1, vmax = 1;
+    for (uint32_t z = 0; z < 4; z++) {
+        const zj_component &c = component(img, ext, z);
+        if (c.h_samp < 1 || c.h_samp > 2 || c.v_samp < 1 || c.v_samp > 2) return ZJ_ERR_UNSUPPORTED;   // up-sampling by 1 or 2 only
+        hmax = std::max(hmax, c.h_samp);
+        vmax = std::max(vmax, c.v_samp);
+    }
+    const uint32_t w = img->width, hh = img->height, s0 = 8u >> scale;
+    const uint32_t mcu_x = (w + 8 * hmax - 1) / (8 * hmax), mcu_y = (hh + 8 * vmax - 1) / (8 * vmax);
+    memset(pl, 0, sizeof(*pl));
+    CmykImage &m = pl->cm;
+    for (uint32_t z = 0; z < 4; z++) {
+        const zj_component &c = component(img, ext, z);
+        if (c.width_stride != c.h_samp * mcu_x * 8) return ZJ_ERR_INVALID_ARG;
+        for (int k = 0; k < 64; k++)
+            if (c.qt[k] < 0 || c.qt[k] > 255) return ZJ_ERR_INVALID_ARG;
+        uint32_t ss = s0;   // rule 1'' (jdmaster.c)
+        while (ss < 8 && (hmax * s0) % (2 * c.h_samp * ss) == 0 && (vmax * s0) % (2 * c.v_samp * ss) == 0) ss *= 2;
+        m.h[z] = c.h_samp; m.v[z] = c.v_samp; m.ss[z] = ss;
+        m.bpr[z] = c.width_stride / 8;
+        m.dw[z] = (uint32_t)(((uint64_t)w * c.h_samp * ss + 8 * hmax - 1) / (8 * hmax));
+        m.dh[z] = (uint32_t)(((uint64_t)hh * c.v_samp * ss + 8 * vmax - 1) / (8 * vmax));
+        for (int k = 0; k < 32; k++) m.qtw[z][k] = (uint32_t)c.qt[2 * k] | ((uint32_t)c.qt[2 * k + 1] << 24);
+        pl->chunk[z] = (size_t)c.v_samp * 8 * c.width_stride;
+    }
+    uint32_t ow, oh;
+    stored_dims(img, &ow, &oh);
+    m.width = ow; m.height = oh; m.nc = (uint32_t)nc; m.kind = kind; m.ycck = ext->jpeg_cs == ZJ_CS_YCCK;
+    m.hmax = hmax; m.vmax = vmax; m.mcu_x = mcu_x; m.mcu_y = mcu_y;
+    m.tile_mcus = TC_PIXELS / (hmax * s0);
+    m.n_tiles = (mcu_x + m.tile_mcus - 1) / m.tile_mcus;
+    pl->cmyk = 1;
+    pl->variant = ZJ_VARIANT_SPEC;
+    pl->islow = islow;
+    pl->scale = (int)scale;
+    pl->orient = (int)orient;
+    pl->n_strips = mcu_y;
+    pl->rows = 8 * vmax;
+    pl->ncomp_used = 4;
+    pl->out_size = (size_t)ow * oh * nc;
+    pl->dev.nc = (uint32_t)nc;
+    pl->grid_tiles = m.n_tiles;
+    pl->grid_strips = mcu_y;
+    return ZJ_OK;
+}
 
 // Strip geometry of reference src/mcu.rs:139-226 (baseline) / src/mcu_prog.rs:132-203 (progressive) and the
 // colour-writer constants of src/worker.rs:143-251.
-static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
+static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr, const Extra4 *ext = nullptr)
 {
     if (!img) return ZJ_ERR_INVALID_ARG;
+    if (img->n_comp == 4) return plan_cmyk(img, ext, pl);   // (no Extra4: ZJ_ERR_INVALID_ARG, as for any other count)
     if (img->n_comp != 1 && img->n_comp != 3) return ZJ_ERR_INVALID_ARG;
     if (img->width == 0 || img->height == 0 || img->width > 65535 || img->height > 65535) return ZJ_ERR_INVALID_ARG;
     const int nc = num_components(img->out_cs);
@@ -229,11 +300,12 @@ static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr)
     return ZJ_OK;
 }
 
-static int check_buffers(const zj_image *img, const Plan &pl, const void *out, size_t out_len)
+static int check_buffers(const zj_image *img, const Plan &pl, const void *out, size_t out_len, const Extra4 *ext = nullptr)
 {
     for (uint32_t z = 0; z < pl.ncomp_used; z++) {
-        if (!img->comp[z].coeff) return ZJ_ERR_INVALID_ARG;
-        if (img->comp[z].n_i16 < (uint64_t)pl.n_strips * pl.chunk[z]) return ZJ_ERR_SHORT_PLANE;
+        const zj_component &c = component(img, ext, z);
+        if (!c.coeff) return ZJ_ERR_INVALID_ARG;
+        if (c.n_i16 < (uint64_t)pl.n_strips * pl.chunk[z]) return ZJ_ERR_SHORT_PLANE;
     }
     if (!out) return ZJ_ERR_INVALID_ARG;
     if (out_len < pl.out_size) return ZJ_ERR_SHORT_OUTPUT;
@@ -241,10 +313,27 @@ static int check_buffers(const zj_image *img, const Plan &pl, const void *out, s
 }
 
 // device-resident planes are read with 128-bit accesses: every plane must start on a 16-byte boundary
-static int check_device_alignment(const zj_image *img, const Plan &pl)
+static int check_device_alignment(const zj_image *img, const Plan &pl, const Extra4 *ext = nullptr)
 {
     for (uint32_t z = 0; z < pl.ncomp_used; z++)
-        if (reinterpret_cast<uintptr_t>(img->comp[z].coeff) & 15) return ZJ_ERR_INVALID_ARG;
+        if (reinterpret_cast<uintptr_t>(component(img, ext, z).coeff) & 15) return ZJ_ERR_INVALID_ARG;
+    return ZJ_OK;
+}
+
+// zj_validate_image and zj_output_size of an image that may have four components (the JPEG-bytes routes)
+int zj::validate_image4(const zj_image *img, const Extra4 *ext, size_t *out_size)
+{
+    *out_size = 0;
+    if (!img || img->n_comp != 4) {
+        *out_size = zj_output_size(img);
+        return zj_validate_image(img);
+    }
+    Plan pl;
+    int rc = plan_image(img, &pl, nullptr, ext);
+    if (rc) return rc;
+    for (uint32_t z = 0; z < 4; z++)
+        if (component(img, ext, z).n_i16 < (uint64_t)pl.n_strips * pl.chunk[z]) return ZJ_ERR_SHORT_PLANE;
+    *out_size = pl.out_size;
     return ZJ_OK;
 }
 
@@ -256,6 +345,7 @@ struct zj_batch {
     std::vector<std::pair<uint8_t *, size_t>> zero_only;  // outputs that are just memset (worker.rs:131-132)
     DevImage *d_images;
     size_t n_images;
+    CmykImage *d_cmyk;            // the four-component images' records (LaunchGroup::cmyk)
     // oriented images (ZJ_FLAG_ORIENT_*): reconstructed into `scratch`, owned by the batch, then oriented into their outputs
     std::vector<OrientRun> orient_runs;
     OrientImage *d_orient;
@@ -346,8 +436,9 @@ int zj_validate_image(const zj_image *img)
 // above all cudaFree serialise every thread that feeds the device, which is what zj_decode_batch's workers are)
 // `regions` (may be NULL): for an oriented image with regions[i].w != 0, only that rectangle of its stored frame is oriented, and
 // out_dev[i] receives it (regions[i].w * regions[i].h * nc bytes, in the displayed frame)
+// `ext` (may be NULL): the Extra4 of the four-component images
 static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t *const *out_dev, const size_t *out_len, zj_batch **plan,
-                             bool pooled, cudaStream_t ps, const zj_roi *regions = nullptr);
+                             bool pooled, cudaStream_t ps, const zj_roi *regions = nullptr, const Extra4 *ext = nullptr);
 
 int zj_batch_create(int device, const zj_image *imgs, size_t n, uint8_t *const *out_dev, const size_t *out_len, zj_batch **plan)
 {
@@ -366,7 +457,7 @@ static void batch_free(void *p, bool pooled, cudaStream_t ps)
 }
 
 static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t *const *out_dev, const size_t *out_len, zj_batch **plan,
-                             bool pooled, cudaStream_t ps, const zj_roi *regions)
+                             bool pooled, cudaStream_t ps, const zj_roi *regions, const Extra4 *ext)
 {
     if (!plan) return ZJ_ERR_INVALID_ARG;
     *plan = nullptr;
@@ -377,15 +468,17 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
     std::vector<OrientImage> orient;      // the oriented images' second pass, src = their offset into the scratch buffer for now
     size_t scratch_bytes = 0;
     for (size_t i = 0; i < n; i++) {
-        rc = plan_image(&imgs[i], &plans[i], out_dev[i]);
+        const Extra4 *e = ext ? &ext[i] : nullptr;
+        rc = plan_image(&imgs[i], &plans[i], out_dev[i], e);
         if (rc) return rc;
         const bool region = plans[i].orient && regions && regions[i].w;
-        rc = check_buffers(&imgs[i], plans[i], out_dev[i], region ? SIZE_MAX : out_len[i]);
+        rc = check_buffers(&imgs[i], plans[i], out_dev[i], region ? SIZE_MAX : out_len[i], e);
         if (rc) return rc;
-        rc = check_device_alignment(&imgs[i], plans[i]);
+        rc = check_device_alignment(&imgs[i], plans[i], e);
         if (rc) return rc;
-        for (int z = 0; z < 3; z++) plans[i].dev.coeff[z] = (uint32_t)z < plans[i].ncomp_used ? imgs[i].comp[z].coeff : nullptr;
-        plans[i].dev.out = out_dev[i];
+        if (plans[i].cmyk) for (uint32_t z = 0; z < 4; z++) plans[i].cm.coeff[z] = component(&imgs[i], e, z).coeff;
+        else for (int z = 0; z < 3; z++) plans[i].dev.coeff[z] = (uint32_t)z < plans[i].ncomp_used ? imgs[i].comp[z].coeff : nullptr;
+        plans[i].out_ptr() = out_dev[i];
         if (plans[i].orient) {
             OrientImage oi{};
             const uint32_t nc = plans[i].dev.nc;
@@ -401,7 +494,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
             oi.orient = (uint32_t)plans[i].orient;
             oi.nc = nc;
             orient.push_back(oi);
-            plans[i].dev.out = reinterpret_cast<uint8_t *>(scratch_bytes);
+            plans[i].out_ptr() = reinterpret_cast<uint8_t *>(scratch_bytes);
             scratch_bytes += (plans[i].out_size + 255) & ~(size_t)255;
         }
     }
@@ -409,6 +502,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
     b->device = device;
     b->d_images = nullptr;
     b->n_images = 0;
+    b->d_cmyk = nullptr;
     b->algo_bytes = 0;
     b->d_orient = nullptr;
     b->scratch = nullptr;
@@ -418,7 +512,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         cudaError_t e = batch_alloc((void **)&b->scratch, scratch_bytes, pooled, device, ps);
         if (e != cudaSuccess) { delete b; return cuda_fail(e, "cudaMalloc(orientation scratch)"); }
         for (size_t i = 0; i < n; i++)
-            if (plans[i].orient) plans[i].dev.out = b->scratch + reinterpret_cast<uintptr_t>(plans[i].dev.out);
+            if (plans[i].orient) plans[i].out_ptr() = b->scratch + reinterpret_cast<uintptr_t>(plans[i].out_ptr());
         for (OrientImage &oi : orient) oi.src = b->scratch + reinterpret_cast<uintptr_t>(oi.src);
         // one launch per bytes-per-pixel class
         std::stable_sort(orient.begin(), orient.end(), [](const OrientImage &a, const OrientImage &c) { return a.nc < c.nc; });
@@ -431,19 +525,26 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         b->algo_bytes += plans[i].out_size;
         for (uint32_t z = 0; z < plans[i].ncomp_used; z++) b->algo_bytes += (uint64_t)plans[i].n_strips * plans[i].chunk[z] * 2;
     }
+    // (four-component images sort last and index an array of their own)
     auto key = [&](size_t i) {
-        return plans[i].scale * 128 + plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 + plans[i].variant;
+        return plans[i].cmyk * 1024 + plans[i].scale * 128 + plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 +
+               plans[i].variant;
     };
     std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t c) { return key(a) < key(c); });
-    std::vector<DevImage> host(order.size());
-    for (size_t k = 0; k < order.size(); k++) host[k] = plans[order[k]].dev;
+    std::vector<DevImage> host;
+    std::vector<CmykImage> host_cmyk;
+    for (size_t k = 0; k < order.size(); k++) {
+        if (plans[order[k]].cmyk) host_cmyk.push_back(plans[order[k]].cm);
+        else host.push_back(plans[order[k]].dev);
+    }
     for (size_t k = 0; k < order.size();) {
         size_t e = k;
         LaunchGroup g{};
         g.gray = plans[order[k]].gray; g.mode = plans[order[k]].mode; g.variant = plans[order[k]].variant; g.fast = plans[order[k]].fast;
         g.islow = plans[order[k]].islow;
         g.scale = plans[order[k]].scale;
-        g.first = (uint32_t)k;
+        g.cmyk = plans[order[k]].cmyk;
+        g.first = (uint32_t)(g.cmyk ? k - host.size() : k);
         while (e < order.size() && key(order[e]) == key(order[k]) && e - k < 65535) {
             g.max_tiles = std::max(g.max_tiles, plans[order[e]].grid_tiles);
             g.max_strips = std::max(g.max_strips, plans[order[e]].grid_strips);
@@ -472,6 +573,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         rc = upload((void **)&b->d_images, host.data(), host.size() * sizeof(DevImage), "cudaMemcpy(descriptors)");
         b->n_images = host.size();
     }
+    if (rc == ZJ_OK && !host_cmyk.empty()) rc = upload((void **)&b->d_cmyk, host_cmyk.data(), host_cmyk.size() * sizeof(CmykImage), "cudaMemcpy(descriptors)");
     if (rc == ZJ_OK && !orient.empty()) rc = upload((void **)&b->d_orient, orient.data(), orient.size() * sizeof(OrientImage), "cudaMemcpy(orientation descriptors)");
     if (rc != ZJ_OK) { zj_batch_destroy(b); return rc; }
     *plan = b;
@@ -486,7 +588,7 @@ int zj_batch_run(zj_batch *b, void *stream)
     cudaStream_t s = (cudaStream_t)stream;
     for (auto &z : b->zero_only) CU(cudaMemsetAsync(z.first, 0, z.second, s));
     for (auto &g : b->groups) {
-        CU(launch_group(b->d_images, g, s));
+        CU(g.cmyk ? launch_cmyk(b->d_cmyk, g, s) : launch_group(b->d_images, g, s));
         g_launches.fetch_add(1);
     }
     for (const OrientRun &r : b->orient_runs) {
@@ -502,9 +604,10 @@ uint64_t zj_batch_algorithmic_bytes(const zj_batch *b) { return b ? b->algo_byte
 void zj_batch_destroy(zj_batch *b)
 {
     if (!b) return;
-    if (b->d_images || b->d_orient || b->scratch) {
+    if (b->d_images || b->d_cmyk || b->d_orient || b->scratch) {
         cudaSetDevice(b->device);
         batch_free(b->d_images, b->pooled, b->pool_stream);
+        batch_free(b->d_cmyk, b->pooled, b->pool_stream);
         batch_free(b->d_orient, b->pooled, b->pool_stream);
         batch_free(b->scratch, b->pooled, b->pool_stream);
     }
@@ -1050,16 +1153,25 @@ int zj_gpu_reconstruct_finish(zj_pending *p)
 
 int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, size_t n, uint8_t *const *out, const size_t *out_len, zj_pending **pending)
 {
+    return zj::reconstruct_submit4(device, stream, imgs, nullptr, n, out, out_len, pending);
+}
+
+}  // extern "C"
+
+int zj::reconstruct_submit4(int device, void *stream, const zj_image *imgs, const Extra4 *ext, size_t n, uint8_t *const *out,
+                            const size_t *out_len, zj_pending **pending)
+{
     if (!pending) return ZJ_ERR_INVALID_ARG;
     *pending = nullptr;
     if ((!imgs || !out || !out_len) && n) return ZJ_ERR_INVALID_ARG;
     int rc = set_device(device);
     if (rc) return rc;
     std::vector<Plan> plans(n);
+    auto ext_of = [&](size_t i) { return ext ? &ext[i] : nullptr; };
     for (size_t i = 0; i < n; i++) {
-        rc = plan_image(&imgs[i], &plans[i]);
+        rc = plan_image(&imgs[i], &plans[i], nullptr, ext_of(i));
         if (rc) return rc;
-        rc = check_buffers(&imgs[i], plans[i], out[i], out_len[i]);
+        rc = check_buffers(&imgs[i], plans[i], out[i], out_len[i], ext_of(i));
         if (rc) return rc;
     }
     static const bool trace = getenv("ZJ_SUBMIT_TRACE") != nullptr;
@@ -1143,6 +1255,10 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
         lap("staging buffer");
         uint8_t *pool = cache.buf[device][slot];
         std::vector<zj_image> dimgs(imgs + i, imgs + j);
+        std::vector<Extra4> dext(ext ? ext + i : nullptr, ext ? ext + j : nullptr);
+        // component z's plane pointer of sub-batch image t (the device copy) and of image k (the caller's)
+        auto dcoeff = [&](size_t t, uint32_t z) -> const int16_t *& { return z < 3 ? dimgs[t].comp[z].coeff : dext[t].k.coeff; };
+        auto hcoeff = [&](size_t k, uint32_t z) { return component(&imgs[k], ext_of(k), z).coeff; };
         std::vector<uint8_t *> douts(j - i);
         std::vector<size_t> dlens(j - i);
         size_t off = 0;
@@ -1156,11 +1272,11 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
         std::vector<size_t> span(j - i, 0);     // bytes of the merged copy (0 = one copy per plane)
         for (size_t k = i; k < j; k++) {
             const uint32_t nz = plans[k].ncomp_used;
-            size_t nbz[3] = {0, 0, 0}, rel[3] = {0, 0, 0}, sum = 0;
+            size_t nbz[4] = {0, 0, 0, 0}, rel[4] = {0, 0, 0, 0}, sum = 0;
             bool merge = nz > 1;
             for (uint32_t z = 0; z < nz; z++) { nbz[z] = (size_t)plans[k].n_strips * plans[k].chunk[z] * 2; sum += nbz[z]; }
             for (uint32_t z = 0; z < nz; z++) {
-                const uintptr_t a0 = reinterpret_cast<uintptr_t>(imgs[k].comp[0].coeff), az = reinterpret_cast<uintptr_t>(imgs[k].comp[z].coeff);
+                const uintptr_t a0 = reinterpret_cast<uintptr_t>(hcoeff(k, 0)), az = reinterpret_cast<uintptr_t>(hcoeff(k, z));
                 if (az < a0) { merge = false; break; }
                 rel[z] = az - a0;
                 if ((rel[z] & 15) || (z > 0 && rel[z] < rel[z - 1] + nbz[z - 1])) { merge = false; break; }
@@ -1168,26 +1284,26 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
             const size_t total = merge ? rel[nz - 1] + nbz[nz - 1] : 0;
             if (merge && total <= sum + sum / 8 + 4096) {
                 uint8_t *base = take(total);
-                for (uint32_t z = 0; z < nz; z++) dimgs[k - i].comp[z].coeff = (const int16_t *)(base + rel[z]);
+                for (uint32_t z = 0; z < nz; z++) dcoeff(k - i, z) = (const int16_t *)(base + rel[z]);
                 span[k - i] = total;
             } else {
-                for (uint32_t z = 0; z < nz; z++) dimgs[k - i].comp[z].coeff = (const int16_t *)take(nbz[z]);
+                for (uint32_t z = 0; z < nz; z++) dcoeff(k - i, z) = (const int16_t *)take(nbz[z]);
             }
             douts[k - i] = take(plans[k].out_size);
             dlens[k - i] = plans[k].out_size;
         }
         zj_batch *b = nullptr;
-        rc = batch_create_impl(device, dimgs.data(), dimgs.size(), douts.data(), dlens.data(), &b, true, s);
+        rc = batch_create_impl(device, dimgs.data(), dimgs.size(), douts.data(), dlens.data(), &b, true, s, nullptr, ext ? dext.data() : nullptr);
         if (rc != ZJ_OK) break;
         for (size_t k = i; k < j && rc == ZJ_OK; k++) {
             if (span[k - i]) {
-                e = cudaMemcpyAsync((void *)dimgs[k - i].comp[0].coeff, imgs[k].comp[0].coeff, span[k - i], cudaMemcpyHostToDevice, s);
+                e = cudaMemcpyAsync((void *)dcoeff(k - i, 0), hcoeff(k, 0), span[k - i], cudaMemcpyHostToDevice, s);
                 if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(H2D)");
                 continue;
             }
             for (uint32_t z = 0; z < plans[k].ncomp_used; z++) {
                 const size_t nb = (size_t)plans[k].n_strips * plans[k].chunk[z] * 2;
-                e = cudaMemcpyAsync((void *)dimgs[k - i].comp[z].coeff, imgs[k].comp[z].coeff, nb, cudaMemcpyHostToDevice, s);
+                e = cudaMemcpyAsync((void *)dcoeff(k - i, z), hcoeff(k, z), nb, cudaMemcpyHostToDevice, s);
                 if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemcpyAsync(H2D)"); break; }
             }
         }
@@ -1216,6 +1332,8 @@ int zj_gpu_reconstruct_submit(int device, void *stream, const zj_image *imgs, si
     zj_gpu_reconstruct_finish(pd);   // waits for what was queued, releases the descriptors
     return rc_submit;
 }
+
+extern "C" {
 
 // ------------------------------------------------------------------------------------------ several devices
 // The path shards with no exchange step (SURVEY.md 8(e)): images are independent, and so are the strips of one image --

@@ -107,12 +107,37 @@ struct OrientImage {
     uint32_t nc;                  // bytes per pixel (the launch's)
 };
 
+// A four-component (CMYK / YCCK) image: what zj_image cannot carry -- the fourth component and the colour model the host stage
+// decided (DESIGN.md section 4.6.4).  Passed next to a zj_image with n_comp = 4; not part of the C ABI.
+struct Extra4 {
+    zj_component k;           // the fourth component in SOF order
+    uint32_t jpeg_cs;         // ZJ_CS_CMYK or ZJ_CS_YCCK
+};
+
+// One image of a cmyk_kernel launch (4-component input, ZJ_VARIANT_SPEC).  Only that kernel reads it, so DevImage -- and the
+// code of every other kernel -- stays as it is.
+enum CmykKind : uint32_t { CMYK_OUT_RGB = 0, CMYK_OUT_GRAY = 1, CMYK_OUT_CMYK = 2 };
+constexpr int TC_PIXELS = 128;   // output columns per cmyk_kernel tile
+struct CmykImage {
+    const int16_t *coeff[4];  // device pointers, whole-image planes in SOF order
+    uint8_t *out;             // W' x H' x nc bytes (the stored frame)
+    uint32_t qtw[4][32];      // as DevImage::qtw
+    uint32_t bpr[4];          // blocks per plane row (width_stride / 8)
+    uint32_t h[4], v[4];      // sampling factors (1 or 2)
+    uint32_t ss[4];           // block size in samples (rule 1'')
+    uint32_t dw[4], dh[4];    // real component sizes (rule 3'')
+    uint32_t width, height;   // W' x H'
+    uint32_t nc, kind, ycck;  // output bytes per pixel, CmykKind, 1 = YCCK colour model
+    uint32_t hmax, vmax, mcu_x, mcu_y, tile_mcus, n_tiles;
+};
+
 // Host-side launch plan entry: one kernel launch per (mode, variant, IDCT, out-kind class) group.
 struct LaunchGroup {
     int mode, variant, gray;  // gray = luma-only kernel
     int fast;                 // reconstruct_fast_kernel (X86 variant, aligned output)
     int islow;                // ZJ_FLAG_ISLOW (SPEC variant only): libjpeg-turbo's islow IDCT
     int scale;                // ZJ_FLAG_SCALE_* (SPEC | ISLOW only): 1/2^scale DCT-scaled decode, scaled_kernel
+    int cmyk;                 // four-component input: cmyk_kernel over CmykImage records (first / count index those)
     uint32_t first, count;    // images [first, first+count) of the sorted device array
     uint32_t max_tiles, max_strips;
 };
@@ -138,6 +163,7 @@ struct ResizeImage {
 
 // Kernel launches: zj_kernels.cu (reconstruction), zj_consumer.cu (consumer, resize)
 cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream);
+cudaError_t launch_cmyk(const CmykImage *d_images, const LaunchGroup &g, cudaStream_t stream);
 cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
 cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
 // images [0, count) (count <= 65535) of nc bytes per pixel; max_w x max_h covers every region
@@ -176,6 +202,14 @@ struct U8Image {
 // the consumer / the resize over n decoded images, one launch per run of equal pixel formats; asynchronous on `stream`
 int convert_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d);
 int resize_many(int device, void *stream, const U8Image *imgs, size_t n, const zj_output_desc *d, const zj_resize *r);
+
+// zj_gpu_reconstruct_submit with an optional Extra4 per image (ext = NULL, or ext[i] read only where imgs[i].n_comp = 4): the
+// JPEG-bytes routes reach four-component images through it.  zj_gpu_reconstruct_submit passes NULL, so the planes-in entry
+// points keep refusing n_comp = 4.
+int reconstruct_submit4(int device, void *stream, const zj_image *imgs, const Extra4 *ext, size_t n, uint8_t *const *out,
+                        const size_t *out_len, zj_pending **pending);
+// zj_validate_image of such an image, *out_size = zj_output_size (ext is read only when img->n_comp = 4)
+int validate_image4(const zj_image *img, const Extra4 *ext, size_t *out_size);
 
 void release_stream_caches();   // the idle staging streams and buffers of zj_gpu_reconstruct_submit
 void trim_pools();              // the stream-ordered pools' cached memory back to the driver

@@ -516,9 +516,9 @@ struct Component {  // src/components.rs:18-43
     uint8_t id;
 };
 
-// The three coefficient planes of an image live in ONE block (pinned when a device is present), each plane on a 256-byte
-// boundary: zj_gpu_reconstruct uploads planes that follow each other in host memory with a single copy (three copies of
-// 16.6 + 4.1 + 4.1 MB for a 4K 4:2:0 image run at 44 GB/s over PCIe, one of 24.9 MB at 49).
+// The coefficient planes of an image (three, or four for CMYK / YCCK) live in ONE block (pinned when a device is present), each
+// plane on a 256-byte boundary: zj_gpu_reconstruct uploads planes that follow each other in host memory with a single copy (three
+// copies of 16.6 + 4.1 + 4.1 MB for a 4K 4:2:0 image run at 44 GB/s over PCIe, one of 24.9 MB at 49).
 struct PlaneBuf { int16_t *p = nullptr; };
 struct PlaneBlock {
     int16_t *base = nullptr;
@@ -531,10 +531,10 @@ struct PlaneBlock {
         base = nullptr; cap = 0;
     }
     // planes[z].p for plane_len[z] i16 each (0 = no plane); zeroed on request
-    void ensure(PlaneBuf (&planes)[3], const size_t (&plane_len)[3], bool want_pinned, bool zero)
+    void ensure(PlaneBuf (&planes)[4], const size_t (&plane_len)[4], bool want_pinned, bool zero)
     {
-        size_t off[3], total = 0;
-        for (int z = 0; z < 3; z++) { off[z] = total; total += (plane_len[z] + 127) & ~(size_t)127; }
+        size_t off[4], total = 0;
+        for (int z = 0; z < 4; z++) { off[z] = total; total += (plane_len[z] + 127) & ~(size_t)127; }
         if (total > cap) {
             release();
             const size_t want = total + total / 8 + 128;
@@ -543,7 +543,7 @@ struct PlaneBlock {
             if (!base) { cap = 0; FAIL(ZJ_DE_FORMAT, "out of memory for coefficient planes"); }
             cap = want;
         }
-        for (int z = 0; z < 3; z++) {
+        for (int z = 0; z < 4; z++) {
             planes[z].p = plane_len[z] ? base + off[z] : nullptr;
             if (zero && plane_len[z]) memset(planes[z].p, 0, plane_len[z] * 2);
         }
@@ -672,9 +672,9 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     int err_kind = ZJ_DE_NONE;
     std::string err_msg, err_display;
     // coefficient planes (reused across calls)
-    PlaneBuf planes[3];
+    PlaneBuf planes[4];
     PlaneBlock plane_block;
-    size_t plane_len[3] = {0, 0, 0};
+    size_t plane_len[4] = {0, 0, 0, 0};
     bool have_device = false;
     // restart-interval-parallel entropy decode: threads to use (0 = options.num_threads) and how many intervals the last
     // decode ran side by side (0 = the sequential loop)
@@ -683,6 +683,10 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     OrientSource orient_src;
     bool before_sos = true;
     uint32_t orientation = 1;
+    // four-component images (spec output only): the transform of the last Adobe APP14 segment before the first SOS (-1: none),
+    // and the colour model it gives (ZJ_CS_CMYK or ZJ_CS_YCCK, decided at that SOS)
+    int adobe_transform = -1;
+    uint32_t jpeg_cs4 = ZJ_CS_CMYK;
 
     explicit zj_decoder(const zj_options &o) : options(o)
     {
@@ -717,6 +721,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         orient_src.clear();
         before_sos = true;
         orientation = 1;
+        adobe_transform = -1;
+        jpeg_cs4 = ZJ_CS_CMYK;
     }
     uint32_t user_out_cs = ZJ_CS_RGB;
     uint32_t quirks = ZJ_QUIRK_ALL;   // the host-stage quirks of this decode (g_quirks when it started; none for spec output)
@@ -754,7 +760,11 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         default: return 4;
         }
     }
-    size_t in_components() const { return input_colorspace == ZJ_CS_GRAYSCALE ? 1 : 3; }
+    size_t in_components() const { return input_colorspace == ZJ_CS_GRAYSCALE ? 1 : (four() ? 4 : 3); }
+    // a four-component frame, accepted by spec output only (input_colorspace is ZJ_CS_CMYK for these until the first SOS decides)
+    bool four() const { return input_colorspace == ZJ_CS_CMYK; }
+    // the colour model of the last headers read (zj_decoder_jpeg_colorspace)
+    uint32_t jpeg_colorspace() const { return four() ? jpeg_cs4 : input_colorspace; }
 
     // ---------------------------------------------------------------- headers (src/headers.rs)
     void parse_huffman(Cursor &buf)  // headers.rs:18-121
@@ -839,13 +849,20 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         if (length != expected)
             FAIL(ZJ_DE_SOF_ERROR, fmt("Length of start of frame differs from expected %u,value is %u", (unsigned)expected, (unsigned)length));
         if (num_components == 1) { input_colorspace = ZJ_CS_GRAYSCALE; gray_input_out_cs(); }
+        // CMYK / YCCK: spec output only, any distinct component ids (the as-written host stage rejects them below, as the reference does)
+        const bool four_in = spec() && num_components == 4;
+        if (four_in) input_colorspace = ZJ_CS_CMYK;
         info.components = num_components;
         std::vector<Component> comps;
         for (int i = 0; i < num_components; i++) {
             uint8_t a[3];
             buf.read_exact(a, 3, ZJ_DE_FORMAT, "Could not read component data\nfailed to fill whole buffer");
             Component c{};  // Components::from, components.rs:49-114
-            if (a[0] == 1) c.component_id = ID_Y;
+            if (four_in) {
+                for (const Component &o : comps)
+                    if (o.id == a[0]) FAIL(ZJ_DE_SOF_ERROR, fmt("Duplicate component id %u", (unsigned)a[0]));
+                c.component_id = std::min(i, (int)ID_CR);
+            } else if (a[0] == 1) c.component_id = ID_Y;
             else if (a[0] == 2) c.component_id = ID_CB;
             else if (a[0] == 3) c.component_id = ID_CR;
             else FAIL(ZJ_DE_FORMAT, fmt("Unknown component id found,%u, expected value between 1 and 3\nNote I and Q components are not supported yet", (unsigned)a[0]));
@@ -875,6 +892,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             c.width_stride *= mcu_x * 8;
         }
         for (bool &b : qt_present) b = false;  // headers.rs:343
+        if (four_in)   // raster planes of the final MCU grid: mcu_x h_z blocks per row
+            for (auto &c : comps) c.width_stride = c.horizontal_sample * mcu_x * 8;
         components = comps;
     }
     void parse_sos(Cursor &buf)  // headers.rs:350-463
@@ -884,6 +903,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         bool seen[4] = {false, false, false, false};
         num_scans = ns;
         if (ls != 6 + 2 * (uint16_t)ns) FAIL(ZJ_DE_SOS_ERROR, "Bad SOS length,corrupt jpeg");
+        if (four()) { parse_sos4(buf, ns); return; }
         if (!(ns >= 1 && ns < 4))
             FAIL(ZJ_DE_SOS_ERROR, fmt("Number of components in start of scan should be less than 3 but more than 0. Found %u", (unsigned)ns));
         if (info.components == 0) FAIL(ZJ_DE_SOF_ERROR, "Number of components cannot be zero.");
@@ -914,6 +934,29 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         succ_low = bit_approx & 0xF;
         if (succ_low > 13) FAIL(ZJ_DE_SOF_ERROR, fmt("Invalid Al parameter %u, range should be 0-13", (unsigned)succ_low));
     }
+    // SOS of a four-component frame: 1-4 components, selected by id (jdmarker.c get_sos)
+    void parse_sos4(Cursor &buf, uint8_t ns)
+    {
+        if (ns < 1 || ns > 4) FAIL(ZJ_DE_SOS_ERROR, fmt("Number of components in start of scan should be between 1 and 4. Found %u", (unsigned)ns));
+        bool seen[4] = {false, false, false, false};
+        for (int i = 0; i < ns; i++) {
+            const uint8_t id = buf.read_byte(), y = buf.read_byte();
+            size_t j = 0;
+            while (j < components.size() && components[j].id != id) j++;
+            if (j == components.size()) FAIL(ZJ_DE_SOS_ERROR, fmt("Invalid component id %u", (unsigned)id));
+            if (seen[j]) FAIL(ZJ_DE_SOS_ERROR, fmt("Duplicate ID %u seen twice in the same component", (unsigned)id));
+            seen[j] = true;
+            components[j].dc_huff_table = (y >> 4) & 0xF;
+            components[j].ac_huff_table = y & 0xF;
+            z_order[i] = j;
+        }
+        spec_start = buf.read_byte() & 63;
+        spec_end = buf.read_byte() & 63;
+        const uint8_t bit_approx = buf.read_byte();
+        succ_high = bit_approx >> 4;
+        succ_low = bit_approx & 0xF;
+        if (succ_high > 13 || succ_low > 13) FAIL(ZJ_DE_SOS_ERROR, fmt("Invalid Ah / Al parameters %u / %u", (unsigned)succ_high, (unsigned)succ_low));
+    }
     void skip_segment(Cursor &buf, const char *msg_fmt)
     {
         const uint16_t length = buf.read_u16_be();
@@ -930,7 +973,12 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         case M_DQT: parse_dqt(buf); break;
         case M_DHT: parse_huffman(buf); break;
         case M_SOS:
-            if (before_sos) { before_sos = false; orientation = orient_src.orientation(); }
+            if (before_sos) {
+                before_sos = false;
+                orientation = orient_src.orientation();
+                // jdapimin.c default_decompress_parms: Adobe transform 0 -> CMYK, any other -> YCCK, no Adobe marker -> CMYK
+                jpeg_cs4 = adobe_transform > 0 ? ZJ_CS_YCCK : ZJ_CS_CMYK;
+            }
             parse_sos(buf);
             break;
         case M_EOI: FAIL(ZJ_DE_FORMAT, "Premature End of image");
@@ -942,10 +990,13 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             todo = restart_interval;
             break;
         case M_APP:
-            if (m.n == 1 && before_sos) {
+            if ((m.n == 1 || m.n == 14) && before_sos) {
                 const size_t start = buf.pos + 2;
                 skip_segment(buf, "Found a marker with invalid length:%u\n");
-                note_app1(buf.data + start, std::min(buf.pos, buf.len) - std::min(start, buf.len));
+                const uint8_t *p = buf.data + start;
+                const size_t n = std::min(buf.pos, buf.len) - std::min(start, buf.len);
+                if (m.n == 1) note_app1(p, n);
+                else if (n >= 12 && memcmp(p, "Adobe", 5) == 0) adobe_transform = p[11];   // jdmarker.c examine_app14
                 break;
             }
             skip_segment(buf, "Found a marker with invalid length:%u\n");
@@ -1388,7 +1439,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     }
     void parse_entropy_coded_data(Cursor &reader, BitStream &stream)  // mcu_prog.rs:249-430
     {
-        check_component_dimensions();
+        if (!four()) check_component_dimensions();
         stream.reset();
         for (auto &c : components) c.dc_pred = 0;
         if ((size_t)num_scans > in_components())
@@ -1398,14 +1449,15 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             const size_t k = z_order[0];
             if (k >= components.size()) FAIL(ZJ_DE_FORMAT, fmt("Cannot find component %zu, corrupt image", k));
             size_t mw, mh;
-            if (components[k].component_id == ID_Y || !interleaved) { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
+            if (four()) blocks4(components[k], &mw, &mh);
+            else if (components[k].component_id == ID_Y || !interleaved) { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
             else { mw = mcu_x; mh = mcu_y; }
             size_t i = 0, j = 0;
             while (i < mh) {
                 while (j < mw) {
                     const size_t start = 64 * (j + i * (components[k].width_stride / 8));
                     if (i >= mh) break;
-                    if (k >= 3 || start + 64 > plane_len[k]) FAIL(ZJ_DE_GPU, "the reference decoder panics here (block index out of range, mcu_prog.rs:304)");
+                    if (k >= 4 || start + 64 > plane_len[k]) FAIL(ZJ_DE_GPU, "the reference decoder panics here (block index out of range, mcu_prog.rs:304)");
                     int16_t *data = planes[k].p + start;
                     if (spec_start == 0) {
                         const size_t pos = components[k].dc_huff_table & 3;
@@ -1451,7 +1503,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
                                 const size_t x2 = j * component.horizontal_sample + h_samp;
                                 const size_t y2 = i * component.vertical_sample + v_samp;
                                 const size_t position = 64 * (x2 + y2 * component.width_stride / 8);
-                                if (n >= 3 || position >= plane_len[n]) FAIL(ZJ_DE_GPU, "the reference decoder panics here (block index out of range, mcu_prog.rs:408)");
+                                if (n >= 4 || position >= plane_len[n]) FAIL(ZJ_DE_GPU, "the reference decoder panics here (block index out of range, mcu_prog.rs:408)");
                                 int16_t *data = planes[n].p + position;
                                 if (succ_high == 0) stream.decode_prog_dc_first(reader, huff_table, data, component.dc_pred);
                                 else stream.decode_prog_dc_refine(reader, data);
@@ -1466,15 +1518,18 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     }
     void decode_progressive(Cursor &reader)  // mcu_prog.rs:49-129 (+ the geometry half of finish_progressive_decoding)
     {
-        check_component_dimensions();
-        size_t mw, mh;
-        if (interleaved) { mw = mcu_x; mh = mcu_y; } else { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
-        if (spec() && interleaved && h_max == 2) mh += mh & 1;   // 4:2:2 / 4:2:0 spec output reads whole strips of two MCU rows
-        mw *= 64;
-        if (components.size() < in_components()) FAIL(ZJ_DE_FORMAT, "missing components");
-        for (size_t i = 0; i < 3; i++) plane_len[i] = 0;
-        for (size_t i = 0; i < in_components(); i++) plane_len[i] = mw * components[i].vertical_sample * components[i].horizontal_sample * mh;
-        plane_block.ensure(planes, plane_len, have_device, true);
+        if (four()) { planes4(); }
+        else {
+            check_component_dimensions();
+            size_t mw, mh;
+            if (interleaved) { mw = mcu_x; mh = mcu_y; } else { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
+            if (spec() && interleaved && h_max == 2) mh += mh & 1;   // 4:2:2 / 4:2:0 spec output reads whole strips of two MCU rows
+            mw *= 64;
+            if (components.size() < in_components()) FAIL(ZJ_DE_FORMAT, "missing components");
+            for (size_t i = 0; i < 4; i++) plane_len[i] = 0;
+            for (size_t i = 0; i < in_components(); i++) plane_len[i] = mw * components[i].vertical_sample * components[i].horizontal_sample * mh;
+            plane_block.ensure(planes, plane_len, have_device, true);
+        }
         size_t seen_scans = 1;
         BitStream stream;
         stream.q10 = quirk(ZJ_QUIRK_Q10_DC_REFILL);
@@ -1510,6 +1565,104 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         }
     }
 
+    // ---------------------------------------------------------------- four-component frames (spec output only)
+    // Blocks a non-interleaved scan of component c covers: ceil(ceil(width h / hmax) / 8) x ceil(ceil(height v / vmax) / 8)
+    void blocks4(const Component &c, size_t *bw, size_t *bh) const
+    {
+        *bw = (((size_t)info.width * c.horizontal_sample + h_max - 1) / h_max + 7) / 8;
+        *bh = (((size_t)info.height * c.vertical_sample + v_max - 1) / v_max + 7) / 8;
+    }
+    // raster planes of mcu_x h_z x mcu_y v_z blocks, zeroed (blocks no scan reaches stay zero)
+    void planes4()
+    {
+        if (h_max > 2 || v_max > 2) FAIL(ZJ_DE_FORMAT, "Unknown down-sampling method, cannot continue");
+        for (size_t z = 0; z < 4; z++)
+            plane_len[z] = (size_t)components[z].width_stride * 8 * components[z].vertical_sample * mcu_y;
+        plane_block.ensure(planes, plane_len, have_device, true);
+    }
+    // One sequential scan: MCUs of every component of the scan (one block per MCU when it has one component), restart
+    // markers every restart_interval MCUs (jdhuff.c process_restart).
+    void decode_scan4(Cursor &reader, BitStream &stream)
+    {
+        const size_t ns = num_scans;
+        for (size_t k = 0; k < ns; k++) {
+            const Component &c = components[z_order[k]];
+            if (c.dc_huff_table >= 4 || !dc_tables[c.dc_huff_table].present) FAIL(ZJ_DE_HUFFMAN_DECODE, fmt("No DC table for component %u", (unsigned)c.id));
+            if (c.ac_huff_table >= 4 || !ac_tables[c.ac_huff_table].present) FAIL(ZJ_DE_HUFFMAN_DECODE, fmt("No AC table for component %u", (unsigned)c.id));
+        }
+        int32_t pred[4] = {0, 0, 0, 0};
+        size_t bw = mcu_x, bh = mcu_y;
+        if (ns == 1) blocks4(components[z_order[0]], &bw, &bh);
+        const size_t total = bw * bh;
+        size_t todo_mcus = restart_interval;
+        for (size_t m = 0; m < total; m++) {
+            if (restart_interval && m > 0 && todo_mcus == 0) {
+                if (!stream.has_marker) {   // the RSTn is still ahead of the reader: only padding bits are left before it
+                    size_t p = reader.pos;
+                    while (p + 1 < reader.len && !(reader.data[p] == 0xFF && reader.data[p + 1] >= 0xD0 && reader.data[p + 1] <= 0xD7)) p++;
+                    reader.pos = std::min(p + 2, reader.len);
+                }
+                if (!stream.has_marker || stream.marker.kind == M_RST) {
+                    stream.reset();
+                    for (int32_t &v : pred) v = 0;
+                }
+                todo_mcus = restart_interval;
+            }
+            const size_t my = m / bw, mx = m - my * bw;
+            for (size_t k = 0; k < ns; k++) {
+                const size_t z = z_order[k];
+                const Component &c = components[z];
+                const size_t bh_ = ns == 1 ? 1 : c.vertical_sample, bw_ = ns == 1 ? 1 : c.horizontal_sample;
+                for (size_t v = 0; v < bh_; v++)
+                    for (size_t h = 0; h < bw_; h++) {
+                        const size_t by = my * bh_ + v, bx = mx * bw_ + h;
+                        const size_t at = 64 * (by * (c.width_stride / 8) + bx);
+                        if (at + 64 > plane_len[z]) FAIL(ZJ_DE_FORMAT, "block outside the coefficient plane");
+                        stream.decode_mcu_block(reader, dc_tables[c.dc_huff_table], ac_tables[c.ac_huff_table], planes[z].p + at, pred[k]);
+                    }
+            }
+            if (restart_interval) todo_mcus--;
+        }
+    }
+    // Every sequential scan of the frame, up to EOI or the end of the data
+    void decode_baseline4(Cursor &reader)
+    {
+        planes4();
+        BitStream stream;
+        stream.q10 = false;
+        decode_scan4(reader, stream);
+        Marker m;
+        while (get_marker(reader, stream, &m)) {
+            if (m.kind == M_EOI) break;
+            if (m.kind == M_RST) continue;
+            if (m.kind == M_SOS) {
+                parse_sos(reader);
+                stream.reset();
+                decode_scan4(reader, stream);
+                continue;
+            }
+            parse_marker_inner(m, reader);
+        }
+    }
+    // The fourth component of the last decode (zj_decoder_component, the routes' Extra4)
+    void extra4(zj::Extra4 *e) const
+    {
+        memset(e, 0, sizeof(*e));
+        e->jpeg_cs = jpeg_cs4;
+        if (!four() || components.size() < 4) return;
+        component_desc(3, &e->k);
+    }
+    void component_desc(size_t z, zj_component *c) const
+    {
+        memset(c, 0, sizeof(*c));
+        c->coeff = plane_len[z] ? planes[z].p : nullptr;
+        c->n_i16 = plane_len[z];
+        memcpy(c->qt, components[z].quantization_table, sizeof(c->qt));
+        c->h_samp = (uint32_t)components[z].horizontal_sample;
+        c->v_samp = (uint32_t)components[z].vertical_sample;
+        c->width_stride = (uint32_t)components[z].width_stride;
+    }
+
     // ---------------------------------------------------------------- host stage driver
     void fill_descriptor(zj_image *img)
     {
@@ -1521,22 +1674,16 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         img->variant = spec() ? ZJ_VARIANT_SPEC : (options.use_unsafe ? ZJ_VARIANT_X86 : ZJ_VARIANT_SCALAR);
         img->flags = (is_progressive ? ZJ_FLAG_PROGRESSIVE : 0) | (libjpeg() ? ZJ_FLAG_ISLOW : 0) | scale() << ZJ_FLAG_SCALE_SHIFT |
                      (exif_orientation() ? (orientation - 1) << ZJ_FLAG_ORIENT_SHIFT : 0);
-        for (size_t z = 0; z < in_components(); z++) {
-            zj_component &c = img->comp[z];
-            c.coeff = plane_len[z] ? planes[z].p : nullptr;
-            c.n_i16 = plane_len[z];
-            memcpy(c.qt, components[z].quantization_table, sizeof(c.qt));
-            c.h_samp = (uint32_t)components[z].horizontal_sample;
-            c.v_samp = (uint32_t)components[z].vertical_sample;
-            c.width_stride = (uint32_t)components[z].width_stride;
-        }
+        for (size_t z = 0; z < in_components() && z < 3; z++) component_desc(z, &img->comp[z]);   // (four components: K is extra4's)
     }
     void host_stage(const uint8_t *buf, size_t len, zj_image *img)  // decode_internal, decoder.rs:420-434
     {
         reset_state();
         Cursor cur{buf, len, 0};
         decode_headers_internal(cur);
+        if (four() && components.size() != 4) FAIL(ZJ_DE_FORMAT, "missing components");
         if (is_progressive) decode_progressive(cur);
+        else if (four()) decode_baseline4(cur);
         else decode_baseline(cur);
         fill_descriptor(img);
     }
@@ -1608,6 +1755,13 @@ ZJ_API int zj_decoder_info(const zj_decoder *d, zj_image_info *info)
 }
 ZJ_API uint32_t zj_decoder_out_colorspace(const zj_decoder *d) { return d ? d->options.out_colorspace : 0; }
 ZJ_API uint32_t zj_decoder_orientation(const zj_decoder *d) { return d ? d->orientation : 1; }
+ZJ_API uint32_t zj_decoder_jpeg_colorspace(const zj_decoder *d) { return d ? d->jpeg_colorspace() : (uint32_t)ZJ_CS_YCBCR; }
+ZJ_API int zj_decoder_component(const zj_decoder *d, uint32_t z, zj_component *c)
+{
+    if (!d || !c || z >= d->in_components() || z >= d->components.size()) return ZJ_ERR_INVALID_ARG;
+    d->component_desc(z, c);
+    return ZJ_OK;
+}
 
 ZJ_API int zj_decoder_decode_coefficients(zj_decoder *d, const uint8_t *buf, size_t len, zj_image *img)
 {
@@ -1617,6 +1771,22 @@ ZJ_API int zj_decoder_decode_coefficients(zj_decoder *d, const uint8_t *buf, siz
     catch (const std::bad_alloc &) { return ZJ_ERR_OOM; }
     catch (...) { return ZJ_ERR_DECODE; }
     return ZJ_OK;
+}
+
+// zj_gpu_reconstruct_submit of one decoded image, with its fourth component when it has one
+static int submit_decoded(const zj_decoder *d, int device, const zj_image *img, uint8_t *out, size_t n, zj_pending **pd)
+{
+    if (img->n_comp != 4) return zj_gpu_reconstruct_submit(device, nullptr, img, 1, &out, &n, pd);
+    zj::Extra4 ext;
+    d->extra4(&ext);
+    return zj::reconstruct_submit4(device, nullptr, img, &ext, 1, &out, &n, pd);
+}
+// zj_validate_image and zj_output_size of one decoded image
+static int validate_decoded(const zj_decoder *d, const zj_image *img, size_t *n)
+{
+    zj::Extra4 ext;
+    d->extra4(&ext);
+    return zj::validate_image4(img, &ext, n);
 }
 
 // Strip pipeline of ONE image (SURVEY 8(f).2, mcu.rs:230-369): finished strip ranges are uploaded, reconstructed and downloaded
@@ -1727,11 +1897,16 @@ ZJ_API int zj_decoder_decode_into(zj_decoder *d, const uint8_t *buf, size_t len,
     d->sink = nullptr;
     if (trace) fprintf(stderr, "[zj pipe] host stage returned after %.2f ms (begin was at +%.2f ms)\n", PipeSink::now_ms() - t_call, ps.t_begin - t_call);
     if (rc) return rc;          // (~PipeSink waits for whatever was queued)
-    const size_t n = zj_output_size(&img);
-    rc = zj_validate_image(&img);
+    size_t n = 0;
+    rc = validate_decoded(d, &img, &n);
     if (rc == ZJ_OK && n == 0) rc = ZJ_ERR_INVALID_ARG;
     if (rc == ZJ_OK && n > out_cap) rc = ZJ_ERR_SHORT_OUTPUT;
-    if (rc == ZJ_OK) rc = ps.active ? ps.finish() : zj_gpu_reconstruct(d->options.device, nullptr, &img, 1, &out, &n);
+    if (rc == ZJ_OK && ps.active) rc = ps.finish();
+    else if (rc == ZJ_OK) {
+        zj_pending *pd = nullptr;
+        rc = submit_decoded(d, d->options.device, &img, out, n, &pd);
+        if (rc == ZJ_OK) rc = zj_gpu_reconstruct_finish(pd);
+    }
     if (rc != ZJ_OK) {
         std::string m = zj_gpu_strerror(rc);
         if (rc == ZJ_ERR_CUDA || rc == ZJ_ERR_OOM) m += std::string(" -- ") + zj_gpu_last_cuda_error();
@@ -1862,8 +2037,7 @@ static int decode_batch_impl(const zj_options *o, const uint8_t *const *bufs, co
             if (rc == ZJ_ERR_DECODE && errs) { errs[i].kind = d->err_kind; errs[i].msg = d->err_display; }   // the reference's DecodeErrors
             size_t need = 0;
             if (rc == ZJ_OK) {
-                need = zj_output_size(&img);
-                rc = zj_validate_image(&img);
+                rc = validate_decoded(d, &img, &need);
                 if (rc == ZJ_OK && need == 0) rc = ZJ_ERR_INVALID_ARG;
             }
             uint8_t *dst = out[i];
@@ -1874,7 +2048,7 @@ static int decode_batch_impl(const zj_options *o, const uint8_t *const *bufs, co
             }
             settle();   // the previous image (its planes are the ones this thread decodes into next)
             zj_pending *pd = nullptr;
-            if (rc == ZJ_OK) rc = zj_gpu_reconstruct_submit(opt.device, nullptr, &img, 1, &dst, &need, &pd);
+            if (rc == ZJ_OK) rc = submit_decoded(d, opt.device, &img, dst, need, &pd);
             if (rc == ZJ_OK) {
                 fl.pd = pd; fl.i = i; fl.dst = dst; fl.need = need; fl.mine = mine;
                 cur ^= 1;
@@ -1937,14 +2111,19 @@ ZJ_API int zj_decode_batch_multi(const zj_options *o, const int *devices, size_t
         zj_image img;
         int rc = !d ? (int)ZJ_ERR_OOM : ((!bufs[i] && lens[i]) ? (int)ZJ_ERR_INVALID_ARG : zj_decoder_decode_coefficients(d, bufs[i], lens[i], &img));
         size_t need = 0;
-        if (rc == ZJ_OK) { need = zj_output_size(&img); rc = zj_validate_image(&img); if (rc == ZJ_OK && need == 0) rc = ZJ_ERR_INVALID_ARG; }
+        if (rc == ZJ_OK) { rc = validate_decoded(d, &img, &need); if (rc == ZJ_OK && need == 0) rc = ZJ_ERR_INVALID_ARG; }
         uint8_t *dst = out[i];
         bool mine = false;
         if (rc == ZJ_OK) {
             if (dst) { if (out_len[i] < need) rc = ZJ_ERR_SHORT_OUTPUT; }
             else { dst = (uint8_t *)malloc(need); mine = true; if (!dst) rc = ZJ_ERR_OOM; }
         }
-        if (rc == ZJ_OK) rc = zj_gpu_reconstruct_multi(devices, n_dev, &img, 1, &dst, &need);
+        // (a four-component image is a spec image: it cannot be cut into strips, zj_gpu_reconstruct_multi would run it on devices[0])
+        if (rc == ZJ_OK && img.n_comp == 4) {
+            zj_pending *pd = nullptr;
+            rc = submit_decoded(d, devices[0], &img, dst, need, &pd);
+            if (rc == ZJ_OK) rc = zj_gpu_reconstruct_finish(pd);
+        } else if (rc == ZJ_OK) rc = zj_gpu_reconstruct_multi(devices, n_dev, &img, 1, &dst, &need);
         if (rc == ZJ_OK) { out[i] = dst; out_len[i] = need; }
         else { if (mine) free(dst); if (mine || !out[i]) out[i] = nullptr; out_len[i] = 0; failed++; }
         status[i] = rc;

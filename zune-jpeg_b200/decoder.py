@@ -265,7 +265,7 @@ class Decoder:
             self._raise(rc)
         planes = []
         for z in range(img.n_comp):
-            c = img.comp[z]
+            c = img.comp[z] if z < 3 else self.component(z)
             if c.coeff and c.n_i16:
                 a = np.ctypeslib.as_array((C.c_int16 * c.n_i16).from_address(c.coeff)).copy()
             else:
@@ -276,6 +276,15 @@ class Decoder:
             c.coeff = a.ctypes.data if a.size else None
         img._planes = planes
         return img, planes
+
+    def component(self, z: int):
+        """Component z (SOF order) of the last decode_coefficients as a zj_component pointing at the decoder's planes: the way to
+        the fourth component of a CMYK / YCCK image, which the zj_image descriptor has no room for."""
+        c = _ffi.ZjComponent()
+        rc = self._lib.zj_decoder_component(self._h, z, C.byref(c))
+        if rc != 0:
+            raise IndexError(f"the last decode has no component {z}")
+        return c
 
     def entropy_segments(self) -> int:
         """Restart intervals the last decode entropy-decoded side by side on `num_threads` host threads (0 = the
@@ -301,6 +310,11 @@ class Decoder:
 
     def get_output_colorspace(self) -> ColorSpace:
         return ColorSpace(self._lib.zj_decoder_out_colorspace(self._h))
+
+    def jpeg_colorspace(self) -> ColorSpace:
+        """The colour model of the file whose headers were read last: GRAYSCALE, YCBCR, or for four components CMYK or YCCK (the
+        Adobe APP14 rule the header states next to zj_decoder_jpeg_colorspace)."""
+        return ColorSpace(self._lib.zj_decoder_jpeg_colorspace(self._h))
 
     def exif_orientation(self) -> int:
         """The EXIF orientation (1-8) of the file whose headers were read last, whatever the options: 1 before headers or when
