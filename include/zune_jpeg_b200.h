@@ -210,7 +210,9 @@ typedef struct zj_image {
     uint32_t out_cs;        /* zj_colorspace: ZuneJpegOptions::out_colorspace                               */
     uint32_t variant;       /* zj_variant                                                                   */
     uint32_t flags;         /* ZJ_FLAG_*                                                                    */
-    zj_component comp[3];   /* comp[0] = Y and carries the maximum sampling factors (decoder.rs:609-646)    */
+    zj_component comp[3];   /* comp[0] = Y and carries the maximum sampling factors (decoder.rs:609-646),
+                               except for the frames of the any-factor statement (next to
+                               zj_decoder_jpeg_colorspace), whose maxima may be any component's                */
 } zj_image;
 
 /* ------------------------------------------------------------- GPU path  */
@@ -464,10 +466,14 @@ ZJ_API uint32_t zj_decoder_orientation(const zj_decoder *d);
  *      do not matter.  Component ids may be any distinct bytes; SOS selects components by id.
  *   2. Samples: every component goes through step 1 (ZJ_USE_SPEC_OUTPUT), 1' (ZJ_FLAG_ISLOW) or 2'' (a scale), with rule 1'''s
  *      block size ss_z and rule 3'''s size dw_z x dh_z per component, (hmax, vmax) = the largest factors over all four.  Sampling
- *      factors are 1 or 2 (others: ZJ_ERR_UNSUPPORTED).  Component z is up-sampled on its own by (hmax s0 / (h_z ss_z),
+ *      factors are 1..4 (others: ZJ_ERR_UNSUPPORTED).  Component z is up-sampled on its own by (rh, rv) = (hmax s0 / (h_z ss_z),
  *      vmax s0 / (v_z ss_z)), fancy = (s0 > 1): (1, 1) none; (2, 1) step 3's H filter when fancy and dw_z > 2, else each sample
  *      twice; (1, 2) the V filter when fancy, else each row twice; (2, 2) the HV filter when fancy and dw_z > 2, else 2x2
- *      repetition (libjpeg-turbo jdsample.c jinit_upsampler).  Neighbours are clamped to [0, dh_z-1] x [0, dw_z-1].
+ *      repetition; any other integer pair: each sample repeated rh x rv times (libjpeg-turbo jdsample.c jinit_upsampler,
+ *      int_upsample).  Neighbours are clamped to [0, dh_z-1] x [0, dw_z-1].  A ratio that is not an integer is libjpeg's
+ *      JERR_FRACT_SAMPLE_NOTIMPL: the host stage fails with ZJ_DE_FORMAT, the planner returns ZJ_ERR_UNSUPPORTED.  Frames with a
+ *      factor above 2 also fail, as in libjpeg (jdinput.c per_scan_setup), when an interleaved scan has more than 10 blocks in its
+ *      MCU; frames with factors 1 and 2 decode as they always did.
  *   3. YCCK -> CMYK (jdcolor.c ycck_cmyk_convert), cb' = Cb - 128, cr' = Cr - 128:
  *        C0 = clamp(255 - (Y + ((91881 cr' + 32768) >> 16)))     M0 = clamp(255 - (Y + ((-22554 cb' - 46802 cr' + 32768) >> 16)))
  *        Y0 = clamp(255 - (Y + ((116130 cb' + 32768) >> 16)))   K0 = K
@@ -480,7 +486,24 @@ ZJ_API uint32_t zj_decoder_orientation(const zj_decoder *d);
  * zj_image has room for three components, so zj_decoder_decode_coefficients fills `img` with n_comp = 4 and comp[0..2], and
  * zj_decoder_component gives any component of the last decode, the fourth included.  The planes-in entry points
  * (zj_gpu_reconstruct*, zj_batch_create, ...) refuse n_comp = 4 (ZJ_ERR_INVALID_ARG); the JPEG-bytes entry points decode these
- * files. */
+ * files.
+ *
+ * Three-component JPEGs with any sampling factors libjpeg accepts -- 4:1:1, 4:1:0, factors of 3, chroma above luma, chroma
+ * factors that differ (DESIGN.md section 4.6.5).  This statement covers ZJ_VARIANT_SPEC images (with or without ZJ_FLAG_ISLOW,
+ * a scale and an orientation) of three components when their factors are all 1..4 and are not luma (1|2) x (1|2) with both
+ * chroma components 1 x 1; those sets keep the statements above, byte for byte.  The output is what Pillow 12.2's
+ * Image.open(f).convert(...) gives (with draft for a scale).  For components z = 0..2 in SOF order (ids 1, 2, 3):
+ *   1. Geometry: (hmax, vmax) = the largest factors over all three, whichever component has them; mcu_x x mcu_y MCUs of
+ *      8 hmax x 8 vmax pixels; comp[z] is a raster plane of mcu_x h_z x mcu_y v_z blocks, width_stride = h_z mcu_x 8.
+ *   2. Samples and up-sampling: step 2 of the four-component statement above, over three components: the same block sizes,
+ *      ratios, filters and failures, the 10-block rule included whatever the factors (all three at 2 x 2 fails, as in libjpeg).
+ *   3. Colour: steps 4 and 5 of the spec statement: RGB / RGBA / RGBX = the JFIF RGB of the up-sampled (Y, Cb, Cr), with alpha
+ *      255; GRAYSCALE = the up-sampled Y plane; YCBCR = the three up-sampled planes.  CMYK and YCCK output: ZJ_ERR_UNSUPPORTED.
+ * The host stage decodes them with the spec use_unsafe values above, baseline (restart markers and later scans included) or
+ * progressive; every other use_unsafe value keeps the reference's errors.  zj_decoder_decode_coefficients fills n_comp = 3 and
+ * comp[0..2] with each component's own factors.  Every entry point takes them: the planes-in ones as ZJ_VARIANT_SPEC descriptors
+ * (X86 and SCALAR descriptors with these factors: ZJ_ERR_UNSUPPORTED), and, as for every spec image, zj_image_strip_range
+ * refuses cuts and zj_image_rows returns the image whole. */
 /* The colour model of the last headers read: ZJ_CS_GRAYSCALE, ZJ_CS_YCBCR, or for four components ZJ_CS_CMYK / ZJ_CS_YCCK. */
 ZJ_API uint32_t zj_decoder_jpeg_colorspace(const zj_decoder *d);
 /* *c = component z (SOF order) of the last zj_decoder_decode_coefficients, pointing at the decoder's planes (valid until the

@@ -48,24 +48,26 @@ struct Plan {
     int islow;         // ZJ_FLAG_ISLOW: the kernels' IDCT is libjpeg-turbo's islow
     int scale;         // ZJ_FLAG_SCALE_*: DCT-scaled decode to 1/2^scale (scaled_kernel)
     int orient;        // ZJ_FLAG_ORIENT_*: the orientation code o - 1 (0 = none), applied by a second pass (orient_kernel)
-    int cmyk;          // four-component input: `cm` instead of `dev`, cmyk_kernel
+    int raster;        // 3 or 4: the components of an image raster_kernel reconstructs (`rm` instead of `dev`); 0 = none
     uint32_t n_strips, rows, ncomp_used;
     size_t chunk[4];   // i16 per strip per component
     size_t out_size;
     DevImage dev;      // pointers filled by the caller
-    CmykImage cm;
+    RasterImage rm;
     uint32_t grid_tiles, grid_strips;   // launch extents (grid_strips: strips as the kernel counts them)
-    uint8_t *&out_ptr() { return cmyk ? cm.out : dev.out; }
+    uint8_t *&out_ptr() { return raster ? rm.out : dev.out; }
 };
 
 // component z of an image: comp[z], and for four-component images the Extra4's as z = 3
 static const zj_component &component(const zj_image *img, const Extra4 *ext, uint32_t z) { return z < 3 ? img->comp[z] : ext->k; }
 
-// A four-component image (the statement is in include/zune_jpeg_b200.h next to zj_decoder_jpeg_colorspace): spec output only.
-// Strips are MCU rows; the planes are raster planes of mcu_x h_z x mcu_y v_z blocks.
-static int plan_cmyk(const zj_image *img, const Extra4 *ext, Plan *pl)
+// An image of raster_kernel (the statements are in include/zune_jpeg_b200.h next to zj_decoder_jpeg_colorspace): spec output only,
+// four components, or three with factors raster_factors() takes.  Strips are MCU rows; the planes are raster planes of
+// mcu_x h_z x mcu_y v_z blocks.
+static int plan_raster(const zj_image *img, const Extra4 *ext, Plan *pl)
 {
-    if (!ext || (ext->jpeg_cs != ZJ_CS_CMYK && ext->jpeg_cs != ZJ_CS_YCCK)) return ZJ_ERR_INVALID_ARG;
+    const uint32_t nz = img->n_comp;
+    if (nz == 4 && (!ext || (ext->jpeg_cs != ZJ_CS_CMYK && ext->jpeg_cs != ZJ_CS_YCCK))) return ZJ_ERR_INVALID_ARG;
     if (img->width == 0 || img->height == 0 || img->width > 65535 || img->height > 65535) return ZJ_ERR_INVALID_ARG;
     const int nc = num_components(img->out_cs);
     if (nc == 0 || img->variant != ZJ_VARIANT_SPEC) return ZJ_ERR_INVALID_ARG;
@@ -74,30 +76,33 @@ static int plan_cmyk(const zj_image *img, const Extra4 *ext, Plan *pl)
     if (scale && !islow) return ZJ_ERR_INVALID_ARG;
     uint32_t kind;
     switch (img->out_cs) {
-    case ZJ_CS_RGB: case ZJ_CS_RGBA: case ZJ_CS_RGBX: kind = CMYK_OUT_RGB; break;
-    case ZJ_CS_GRAYSCALE: kind = CMYK_OUT_GRAY; break;
-    case ZJ_CS_CMYK: kind = CMYK_OUT_CMYK; break;
-    default: return ZJ_ERR_UNSUPPORTED;   // YCBCR, YCCK
+    case ZJ_CS_RGB: case ZJ_CS_RGBA: case ZJ_CS_RGBX: kind = RASTER_OUT_RGB; break;
+    case ZJ_CS_GRAYSCALE: kind = RASTER_OUT_GRAY; break;
+    case ZJ_CS_CMYK: if (nz != 4) return ZJ_ERR_UNSUPPORTED; kind = RASTER_OUT_RAW; break;
+    case ZJ_CS_YCBCR: if (nz != 3) return ZJ_ERR_UNSUPPORTED; kind = RASTER_OUT_RAW; break;
+    default: return ZJ_ERR_UNSUPPORTED;   // YCCK
     }
     uint32_t hmax = 1, vmax = 1;
-    for (uint32_t z = 0; z < 4; z++) {
+    for (uint32_t z = 0; z < nz; z++) {
         const zj_component &c = component(img, ext, z);
-        if (c.h_samp < 1 || c.h_samp > 2 || c.v_samp < 1 || c.v_samp > 2) return ZJ_ERR_UNSUPPORTED;   // up-sampling by 1 or 2 only
+        if (c.h_samp < 1 || c.h_samp > 4 || c.v_samp < 1 || c.v_samp > 4) return ZJ_ERR_UNSUPPORTED;
         hmax = std::max(hmax, c.h_samp);
         vmax = std::max(vmax, c.v_samp);
     }
     const uint32_t w = img->width, hh = img->height, s0 = 8u >> scale;
     const uint32_t mcu_x = (w + 8 * hmax - 1) / (8 * hmax), mcu_y = (hh + 8 * vmax - 1) / (8 * vmax);
     memset(pl, 0, sizeof(*pl));
-    CmykImage &m = pl->cm;
-    for (uint32_t z = 0; z < 4; z++) {
+    RasterImage &m = pl->rm;
+    for (uint32_t z = 0; z < nz; z++) {
         const zj_component &c = component(img, ext, z);
         if (c.width_stride != c.h_samp * mcu_x * 8) return ZJ_ERR_INVALID_ARG;
         for (int k = 0; k < 64; k++)
             if (c.qt[k] < 0 || c.qt[k] > 255) return ZJ_ERR_INVALID_ARG;
-        uint32_t ss = s0;   // rule 1'' (jdmaster.c)
-        while (ss < 8 && (hmax * s0) % (2 * c.h_samp * ss) == 0 && (vmax * s0) % (2 * c.v_samp * ss) == 0) ss *= 2;
+        const uint32_t ss = block_size(hmax, vmax, c.h_samp, c.v_samp, s0);
+        // libjpeg-turbo jdsample.c jinit_upsampler: integer ratios only (JERR_FRACT_SAMPLE_NOTIMPL)
+        if ((hmax * s0) % (c.h_samp * ss) || (vmax * s0) % (c.v_samp * ss)) return ZJ_ERR_UNSUPPORTED;
         m.h[z] = c.h_samp; m.v[z] = c.v_samp; m.ss[z] = ss;
+        m.ratio[z] = hmax * s0 / (c.h_samp * ss) | (vmax * s0 / (c.v_samp * ss)) << 8;
         m.bpr[z] = c.width_stride / 8;
         m.dw[z] = (uint32_t)(((uint64_t)w * c.h_samp * ss + 8 * hmax - 1) / (8 * hmax));
         m.dh[z] = (uint32_t)(((uint64_t)hh * c.v_samp * ss + 8 * vmax - 1) / (8 * vmax));
@@ -106,18 +111,19 @@ static int plan_cmyk(const zj_image *img, const Extra4 *ext, Plan *pl)
     }
     uint32_t ow, oh;
     stored_dims(img, &ow, &oh);
-    m.width = ow; m.height = oh; m.nc = (uint32_t)nc; m.kind = kind; m.ycck = ext->jpeg_cs == ZJ_CS_YCCK;
+    m.width = ow; m.height = oh; m.nc = (uint32_t)nc; m.kind = kind;
+    m.model = nz == 3 ? RASTER_YCC : (ext->jpeg_cs == ZJ_CS_YCCK ? RASTER_YCCK : RASTER_CMYK);
     m.hmax = hmax; m.vmax = vmax; m.mcu_x = mcu_x; m.mcu_y = mcu_y;
     m.tile_mcus = TC_PIXELS / (hmax * s0);
     m.n_tiles = (mcu_x + m.tile_mcus - 1) / m.tile_mcus;
-    pl->cmyk = 1;
+    pl->raster = (int)nz;
     pl->variant = ZJ_VARIANT_SPEC;
     pl->islow = islow;
     pl->scale = (int)scale;
     pl->orient = (int)orient;
     pl->n_strips = mcu_y;
     pl->rows = 8 * vmax;
-    pl->ncomp_used = 4;
+    pl->ncomp_used = nz;
     pl->out_size = (size_t)ow * oh * nc;
     pl->dev.nc = (uint32_t)nc;
     pl->grid_tiles = m.n_tiles;
@@ -130,7 +136,8 @@ static int plan_cmyk(const zj_image *img, const Extra4 *ext, Plan *pl)
 static int plan_image(const zj_image *img, Plan *pl, const void *out = nullptr, const Extra4 *ext = nullptr)
 {
     if (!img) return ZJ_ERR_INVALID_ARG;
-    if (img->n_comp == 4) return plan_cmyk(img, ext, pl);   // (no Extra4: ZJ_ERR_INVALID_ARG, as for any other count)
+    if (img->n_comp == 4) return plan_raster(img, ext, pl);   // (no Extra4: ZJ_ERR_INVALID_ARG, as for any other count)
+    if (img->n_comp == 3 && img->variant == ZJ_VARIANT_SPEC && raster_factors(img->comp)) return plan_raster(img, nullptr, pl);
     if (img->n_comp != 1 && img->n_comp != 3) return ZJ_ERR_INVALID_ARG;
     if (img->width == 0 || img->height == 0 || img->width > 65535 || img->height > 65535) return ZJ_ERR_INVALID_ARG;
     const int nc = num_components(img->out_cs);
@@ -345,7 +352,7 @@ struct zj_batch {
     std::vector<std::pair<uint8_t *, size_t>> zero_only;  // outputs that are just memset (worker.rs:131-132)
     DevImage *d_images;
     size_t n_images;
-    CmykImage *d_cmyk;            // the four-component images' records (LaunchGroup::cmyk)
+    RasterImage *d_raster;        // the raster_kernel images' records (LaunchGroup::raster)
     // oriented images (ZJ_FLAG_ORIENT_*): reconstructed into `scratch`, owned by the batch, then oriented into their outputs
     std::vector<OrientRun> orient_runs;
     OrientImage *d_orient;
@@ -476,7 +483,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         if (rc) return rc;
         rc = check_device_alignment(&imgs[i], plans[i], e);
         if (rc) return rc;
-        if (plans[i].cmyk) for (uint32_t z = 0; z < 4; z++) plans[i].cm.coeff[z] = component(&imgs[i], e, z).coeff;
+        if (plans[i].raster) for (uint32_t z = 0; z < plans[i].ncomp_used; z++) plans[i].rm.coeff[z] = component(&imgs[i], e, z).coeff;
         else for (int z = 0; z < 3; z++) plans[i].dev.coeff[z] = (uint32_t)z < plans[i].ncomp_used ? imgs[i].comp[z].coeff : nullptr;
         plans[i].out_ptr() = out_dev[i];
         if (plans[i].orient) {
@@ -502,7 +509,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
     b->device = device;
     b->d_images = nullptr;
     b->n_images = 0;
-    b->d_cmyk = nullptr;
+    b->d_raster = nullptr;
     b->algo_bytes = 0;
     b->d_orient = nullptr;
     b->scratch = nullptr;
@@ -525,16 +532,16 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         b->algo_bytes += plans[i].out_size;
         for (uint32_t z = 0; z < plans[i].ncomp_used; z++) b->algo_bytes += (uint64_t)plans[i].n_strips * plans[i].chunk[z] * 2;
     }
-    // (four-component images sort last and index an array of their own)
+    // (raster_kernel images sort last and index an array of their own)
     auto key = [&](size_t i) {
-        return plans[i].cmyk * 1024 + plans[i].scale * 128 + plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 +
+        return plans[i].raster * 1024 + plans[i].scale * 128 + plans[i].gray * 64 + plans[i].fast * 32 + plans[i].mode * 8 + plans[i].islow * 4 +
                plans[i].variant;
     };
     std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t c) { return key(a) < key(c); });
     std::vector<DevImage> host;
-    std::vector<CmykImage> host_cmyk;
+    std::vector<RasterImage> host_raster;
     for (size_t k = 0; k < order.size(); k++) {
-        if (plans[order[k]].cmyk) host_cmyk.push_back(plans[order[k]].cm);
+        if (plans[order[k]].raster) host_raster.push_back(plans[order[k]].rm);
         else host.push_back(plans[order[k]].dev);
     }
     for (size_t k = 0; k < order.size();) {
@@ -543,8 +550,8 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         g.gray = plans[order[k]].gray; g.mode = plans[order[k]].mode; g.variant = plans[order[k]].variant; g.fast = plans[order[k]].fast;
         g.islow = plans[order[k]].islow;
         g.scale = plans[order[k]].scale;
-        g.cmyk = plans[order[k]].cmyk;
-        g.first = (uint32_t)(g.cmyk ? k - host.size() : k);
+        g.raster = plans[order[k]].raster;
+        g.first = (uint32_t)(g.raster ? k - host.size() : k);
         while (e < order.size() && key(order[e]) == key(order[k]) && e - k < 65535) {
             g.max_tiles = std::max(g.max_tiles, plans[order[e]].grid_tiles);
             g.max_strips = std::max(g.max_strips, plans[order[e]].grid_strips);
@@ -573,7 +580,7 @@ static int batch_create_impl(int device, const zj_image *imgs, size_t n, uint8_t
         rc = upload((void **)&b->d_images, host.data(), host.size() * sizeof(DevImage), "cudaMemcpy(descriptors)");
         b->n_images = host.size();
     }
-    if (rc == ZJ_OK && !host_cmyk.empty()) rc = upload((void **)&b->d_cmyk, host_cmyk.data(), host_cmyk.size() * sizeof(CmykImage), "cudaMemcpy(descriptors)");
+    if (rc == ZJ_OK && !host_raster.empty()) rc = upload((void **)&b->d_raster, host_raster.data(), host_raster.size() * sizeof(RasterImage), "cudaMemcpy(descriptors)");
     if (rc == ZJ_OK && !orient.empty()) rc = upload((void **)&b->d_orient, orient.data(), orient.size() * sizeof(OrientImage), "cudaMemcpy(orientation descriptors)");
     if (rc != ZJ_OK) { zj_batch_destroy(b); return rc; }
     *plan = b;
@@ -588,7 +595,7 @@ int zj_batch_run(zj_batch *b, void *stream)
     cudaStream_t s = (cudaStream_t)stream;
     for (auto &z : b->zero_only) CU(cudaMemsetAsync(z.first, 0, z.second, s));
     for (auto &g : b->groups) {
-        CU(g.cmyk ? launch_cmyk(b->d_cmyk, g, s) : launch_group(b->d_images, g, s));
+        CU(g.raster ? launch_raster(b->d_raster, g, s) : launch_group(b->d_images, g, s));
         g_launches.fetch_add(1);
     }
     for (const OrientRun &r : b->orient_runs) {
@@ -604,10 +611,10 @@ uint64_t zj_batch_algorithmic_bytes(const zj_batch *b) { return b ? b->algo_byte
 void zj_batch_destroy(zj_batch *b)
 {
     if (!b) return;
-    if (b->d_images || b->d_cmyk || b->d_orient || b->scratch) {
+    if (b->d_images || b->d_raster || b->d_orient || b->scratch) {
         cudaSetDevice(b->device);
         batch_free(b->d_images, b->pooled, b->pool_stream);
-        batch_free(b->d_cmyk, b->pooled, b->pool_stream);
+        batch_free(b->d_raster, b->pooled, b->pool_stream);
         batch_free(b->d_orient, b->pooled, b->pool_stream);
         batch_free(b->scratch, b->pooled, b->pool_stream);
     }

@@ -114,22 +114,46 @@ struct Extra4 {
     uint32_t jpeg_cs;         // ZJ_CS_CMYK or ZJ_CS_YCCK
 };
 
-// One image of a cmyk_kernel launch (4-component input, ZJ_VARIANT_SPEC).  Only that kernel reads it, so DevImage -- and the
-// code of every other kernel -- stays as it is.
-enum CmykKind : uint32_t { CMYK_OUT_RGB = 0, CMYK_OUT_GRAY = 1, CMYK_OUT_CMYK = 2 };
-constexpr int TC_PIXELS = 128;   // output columns per cmyk_kernel tile
-struct CmykImage {
+// One image of a raster_kernel launch (ZJ_VARIANT_SPEC): four-component input, or three components with sampling factors other
+// than luma (1|2) x (1|2) and chroma 1 x 1.  The planes are raster planes of mcu_x h_z x mcu_y v_z blocks.  Only that kernel reads
+// it, so DevImage -- and the code of every other kernel -- stays as it is.
+enum RasterKind : uint32_t {
+    RASTER_OUT_RGB = 0,    // RGB, RGBA, RGBX
+    RASTER_OUT_GRAY = 1,   // GRAYSCALE
+    RASTER_OUT_RAW = 2     // the colour model's own samples: CMYK (four components), YCbCr (three)
+};
+enum RasterModel : uint32_t { RASTER_YCC = 0, RASTER_CMYK = 1, RASTER_YCCK = 2 };   // the colour model of the components
+constexpr int TC_PIXELS = 128;   // output columns per raster_kernel tile (at most)
+struct RasterImage {
     const int16_t *coeff[4];  // device pointers, whole-image planes in SOF order
     uint8_t *out;             // W' x H' x nc bytes (the stored frame)
     uint32_t qtw[4][32];      // as DevImage::qtw
     uint32_t bpr[4];          // blocks per plane row (width_stride / 8)
-    uint32_t h[4], v[4];      // sampling factors (1 or 2)
+    uint32_t h[4], v[4];      // sampling factors (1..4)
     uint32_t ss[4];           // block size in samples (rule 1'')
     uint32_t dw[4], dh[4];    // real component sizes (rule 3'')
+    uint32_t ratio[4];        // up-sampling ratios rh | rv << 8: rh = hmax s0 / (h ss), rv = vmax s0 / (v ss) (1..4 each)
     uint32_t width, height;   // W' x H'
-    uint32_t nc, kind, ycck;  // output bytes per pixel, CmykKind, 1 = YCCK colour model
+    uint32_t nc, kind, model; // output bytes per pixel, RasterKind, RasterModel
     uint32_t hmax, vmax, mcu_x, mcu_y, tile_mcus, n_tiles;
 };
+// Three-component factors that take raster_kernel (spec output): every factor 1..4, and not luma (1|2) x (1|2) with chroma 1 x 1,
+// which the fused kernels take
+inline bool raster_factors(const zj_component (&c)[3])
+{
+    for (int z = 0; z < 3; z++)
+        if (c[z].h_samp < 1 || c[z].h_samp > 4 || c[z].v_samp < 1 || c[z].v_samp > 4) return false;
+    const bool luma = c[0].h_samp <= 2 && c[0].v_samp <= 2;
+    return !(luma && c[1].h_samp == 1 && c[1].v_samp == 1 && c[2].h_samp == 1 && c[2].v_samp == 1);
+}
+// Block size in samples of a component with factors (h, v) when the largest are (hmax, vmax) and the smallest block is s0 (rule
+// 1'', libjpeg-turbo jdmaster.c jpeg_core_output_dimensions)
+inline uint32_t block_size(uint32_t hmax, uint32_t vmax, uint32_t h, uint32_t v, uint32_t s0)
+{
+    uint32_t ss = s0;
+    while (ss < 8 && (hmax * s0) % (2 * h * ss) == 0 && (vmax * s0) % (2 * v * ss) == 0) ss *= 2;
+    return ss;
+}
 
 // Host-side launch plan entry: one kernel launch per (mode, variant, IDCT, out-kind class) group.
 struct LaunchGroup {
@@ -137,7 +161,7 @@ struct LaunchGroup {
     int fast;                 // reconstruct_fast_kernel (X86 variant, aligned output)
     int islow;                // ZJ_FLAG_ISLOW (SPEC variant only): libjpeg-turbo's islow IDCT
     int scale;                // ZJ_FLAG_SCALE_* (SPEC | ISLOW only): 1/2^scale DCT-scaled decode, scaled_kernel
-    int cmyk;                 // four-component input: cmyk_kernel over CmykImage records (first / count index those)
+    int raster;               // 3 or 4: raster_kernel over RasterImage records of that many components (first / count index those)
     uint32_t first, count;    // images [first, first+count) of the sorted device array
     uint32_t max_tiles, max_strips;
 };
@@ -163,7 +187,7 @@ struct ResizeImage {
 
 // Kernel launches: zj_kernels.cu (reconstruction), zj_consumer.cu (consumer, resize)
 cudaError_t launch_group(const DevImage *d_images, const LaunchGroup &g, cudaStream_t stream);
-cudaError_t launch_cmyk(const CmykImage *d_images, const LaunchGroup &g, cudaStream_t stream);
+cudaError_t launch_raster(const RasterImage *d_images, const LaunchGroup &g, cudaStream_t stream);
 cudaError_t launch_convert(const ConvImage *d_images, uint32_t count, uint32_t nc, uint32_t max_ow, uint32_t max_oh, const zj_output_desc &d, cudaStream_t s);
 cudaError_t launch_resize(const ResizeImage *d_images, uint32_t count, uint32_t nc, const zj_output_desc &d, const zj_resize &r, cudaStream_t s);
 // images [0, count) (count <= 65535) of nc bytes per pixel; max_w x max_h covers every region

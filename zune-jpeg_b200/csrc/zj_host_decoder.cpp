@@ -687,6 +687,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     // and the colour model it gives (ZJ_CS_CMYK or ZJ_CS_YCCK, decided at that SOS)
     int adobe_transform = -1;
     uint32_t jpeg_cs4 = ZJ_CS_CMYK;
+    // a three-component frame whose sampling factors the fused kernels do not take (spec output only, raster_factors)
+    bool raster3 = false;
 
     explicit zj_decoder(const zj_options &o) : options(o)
     {
@@ -723,6 +725,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         orientation = 1;
         adobe_transform = -1;
         jpeg_cs4 = ZJ_CS_CMYK;
+        raster3 = false;
     }
     uint32_t user_out_cs = ZJ_CS_RGB;
     uint32_t quirks = ZJ_QUIRK_ALL;   // the host-stage quirks of this decode (g_quirks when it started; none for spec output)
@@ -765,6 +768,9 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     bool four() const { return input_colorspace == ZJ_CS_CMYK; }
     // the colour model of the last headers read (zj_decoder_jpeg_colorspace)
     uint32_t jpeg_colorspace() const { return four() ? jpeg_cs4 : input_colorspace; }
+    // a frame decoded into raster planes, one plane of mcu_x h_z x mcu_y v_z blocks per component, with libjpeg's rules (spec
+    // output only): four components, or three with sampling factors other than luma (1|2) x (1|2) and chroma 1 x 1
+    bool raster() const { return four() || raster3; }
 
     // ---------------------------------------------------------------- headers (src/headers.rs)
     void parse_huffman(Cursor &buf)  // headers.rs:18-121
@@ -852,6 +858,13 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         // CMYK / YCCK: spec output only, any distinct component ids (the as-written host stage rejects them below, as the reference does)
         const bool four_in = spec() && num_components == 4;
         if (four_in) input_colorspace = ZJ_CS_CMYK;
+        // three components with factors 1..4 outside the fused kernels' sets: spec output only (the as-written host stage keeps
+        // the reference's power-of-two rule and errors)
+        if (spec() && num_components == 3 && buf.pos + 9 <= buf.len) {
+            zj_component f[3] = {};
+            for (int i = 0; i < 3; i++) { f[i].h_samp = buf.data[buf.pos + 3 * i + 1] >> 4; f[i].v_samp = buf.data[buf.pos + 3 * i + 1] & 15; }
+            raster3 = zj::raster_factors(f);
+        }
         info.components = num_components;
         std::vector<Component> comps;
         for (int i = 0; i < num_components; i++) {
@@ -870,7 +883,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             c.vertical_sample = a[1] & 0x0f;
             c.quantization_table_number = a[2];
             if (a[2] >= 4) FAIL(ZJ_DE_FORMAT, fmt("Too large quantization number :%u, expected value between 0 and 4", (unsigned)a[2]));
-            auto pow2 = [](size_t x) { return x != 0 && (x & (x - 1)) == 0; };
+            // (raster frames take any factor 1..4; planes_raster refuses larger ones)
+            auto pow2 = [&](size_t x) { return ((raster3 || four_in) && x >= 1 && x <= 4) || (x != 0 && (x & (x - 1)) == 0); };
             if (!pow2(c.horizontal_sample)) FAIL(ZJ_DE_FORMAT, fmt("Horizontal sample is not a power of two(%zu) cannot decode", c.horizontal_sample));
             if (!pow2(c.vertical_sample)) FAIL(ZJ_DE_FORMAT, fmt("Vertical sub-sample is not power of two(%zu) cannot decode", c.vertical_sample));
             c.width_stride = c.horizontal_sample;
@@ -892,7 +906,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             c.width_stride *= mcu_x * 8;
         }
         for (bool &b : qt_present) b = false;  // headers.rs:343
-        if (four_in)   // raster planes of the final MCU grid: mcu_x h_z blocks per row
+        if (raster())   // raster planes of the final MCU grid: mcu_x h_z blocks per row
             for (auto &c : comps) c.width_stride = c.horizontal_sample * mcu_x * 8;
         components = comps;
     }
@@ -1439,7 +1453,8 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     }
     void parse_entropy_coded_data(Cursor &reader, BitStream &stream)  // mcu_prog.rs:249-430
     {
-        if (!four()) check_component_dimensions();
+        if (raster()) check_scan_raster();
+        else check_component_dimensions();
         stream.reset();
         for (auto &c : components) c.dc_pred = 0;
         if ((size_t)num_scans > in_components())
@@ -1449,7 +1464,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             const size_t k = z_order[0];
             if (k >= components.size()) FAIL(ZJ_DE_FORMAT, fmt("Cannot find component %zu, corrupt image", k));
             size_t mw, mh;
-            if (four()) blocks4(components[k], &mw, &mh);
+            if (raster()) blocks_raster(components[k], &mw, &mh);
             else if (components[k].component_id == ID_Y || !interleaved) { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
             else { mw = mcu_x; mh = mcu_y; }
             size_t i = 0, j = 0;
@@ -1518,7 +1533,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     }
     void decode_progressive(Cursor &reader)  // mcu_prog.rs:49-129 (+ the geometry half of finish_progressive_decoding)
     {
-        if (four()) { planes4(); }
+        if (raster()) { planes_raster(); }
         else {
             check_component_dimensions();
             size_t mw, mh;
@@ -1556,6 +1571,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             if (!get_marker(reader, stream, &marker)) FAIL(ZJ_DE_FORMAT_STATIC, "Marker missing where expected");
         }
         // finish_progressive_decoding, mcu_prog.rs:132-168
+        if (raster()) return;
         set_upsampling();
         if (input_colorspace == ZJ_CS_GRAYSCALE && interleaved) {
             if (options.strict_mode) FAIL(ZJ_DE_FORMAT_STATIC, "[strict-mode]: Grayscale image with down-sampled component.");
@@ -1565,25 +1581,43 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         }
     }
 
-    // ---------------------------------------------------------------- four-component frames (spec output only)
+    // ---------------------------------------------------------------- raster frames (spec output only, raster())
     // Blocks a non-interleaved scan of component c covers: ceil(ceil(width h / hmax) / 8) x ceil(ceil(height v / vmax) / 8)
-    void blocks4(const Component &c, size_t *bw, size_t *bh) const
+    void blocks_raster(const Component &c, size_t *bw, size_t *bh) const
     {
         *bw = (((size_t)info.width * c.horizontal_sample + h_max - 1) / h_max + 7) / 8;
         *bh = (((size_t)info.height * c.vertical_sample + v_max - 1) / v_max + 7) / 8;
     }
-    // raster planes of mcu_x h_z x mcu_y v_z blocks, zeroed (blocks no scan reaches stay zero)
-    void planes4()
+    // raster planes of mcu_x h_z x mcu_y v_z blocks, zeroed (blocks no scan reaches stay zero), after libjpeg's check of the
+    // up-sampling ratios (jdsample.c jinit_upsampler)
+    void planes_raster()
     {
-        if (h_max > 2 || v_max > 2) FAIL(ZJ_DE_FORMAT, "Unknown down-sampling method, cannot continue");
+        const size_t s0 = (size_t)8 >> scale(), n = in_components();
+        for (size_t z = 0; z < n; z++) {
+            const Component &c = components[z];
+            if (c.horizontal_sample > 4 || c.vertical_sample > 4) FAIL(ZJ_DE_FORMAT, "Unknown down-sampling method, cannot continue");
+            const size_t ss = zj::block_size((uint32_t)h_max, (uint32_t)v_max, (uint32_t)c.horizontal_sample, (uint32_t)c.vertical_sample, (uint32_t)s0);
+            if ((h_max * s0) % (c.horizontal_sample * ss) || (v_max * s0) % (c.vertical_sample * ss))
+                FAIL(ZJ_DE_FORMAT, "Sampling factors need a non-integer up-sampling ratio (libjpeg: Fractional sampling not implemented yet)");
+        }
         for (size_t z = 0; z < 4; z++)
-            plane_len[z] = (size_t)components[z].width_stride * 8 * components[z].vertical_sample * mcu_y;
+            plane_len[z] = z < n ? (size_t)components[z].width_stride * 8 * components[z].vertical_sample * mcu_y : 0;
         plane_block.ensure(planes, plane_len, have_device, true);
+    }
+    // libjpeg's limit on the blocks of an interleaved scan's MCU (jdinput.c per_scan_setup, JERR_BAD_MCU_SIZE), for the frames whose
+    // factors only this statement takes (four-component frames with factors 1 and 2 keep decoding as they did)
+    void check_scan_raster() const
+    {
+        if (num_scans < 2 || (!raster3 && h_max <= 2 && v_max <= 2)) return;
+        size_t blocks = 0;
+        for (size_t k = 0; k < num_scans; k++) blocks += components[z_order[k]].horizontal_sample * components[z_order[k]].vertical_sample;
+        if (blocks > 10) FAIL(ZJ_DE_FORMAT, fmt("Sampling factors give %zu blocks in an MCU of an interleaved scan, more than 10 (libjpeg: Sampling factors too large for interleaved scan)", blocks));
     }
     // One sequential scan: MCUs of every component of the scan (one block per MCU when it has one component), restart
     // markers every restart_interval MCUs (jdhuff.c process_restart).
-    void decode_scan4(Cursor &reader, BitStream &stream)
+    void decode_scan_raster(Cursor &reader, BitStream &stream)
     {
+        check_scan_raster();
         const size_t ns = num_scans;
         for (size_t k = 0; k < ns; k++) {
             const Component &c = components[z_order[k]];
@@ -1592,7 +1626,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         }
         int32_t pred[4] = {0, 0, 0, 0};
         size_t bw = mcu_x, bh = mcu_y;
-        if (ns == 1) blocks4(components[z_order[0]], &bw, &bh);
+        if (ns == 1) blocks_raster(components[z_order[0]], &bw, &bh);
         const size_t total = bw * bh;
         size_t todo_mcus = restart_interval;
         for (size_t m = 0; m < total; m++) {
@@ -1625,12 +1659,12 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         }
     }
     // Every sequential scan of the frame, up to EOI or the end of the data
-    void decode_baseline4(Cursor &reader)
+    void decode_baseline_raster(Cursor &reader)
     {
-        planes4();
+        planes_raster();
         BitStream stream;
         stream.q10 = false;
-        decode_scan4(reader, stream);
+        decode_scan_raster(reader, stream);
         Marker m;
         while (get_marker(reader, stream, &m)) {
             if (m.kind == M_EOI) break;
@@ -1638,7 +1672,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             if (m.kind == M_SOS) {
                 parse_sos(reader);
                 stream.reset();
-                decode_scan4(reader, stream);
+                decode_scan_raster(reader, stream);
                 continue;
             }
             parse_marker_inner(m, reader);
@@ -1683,7 +1717,7 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         decode_headers_internal(cur);
         if (four() && components.size() != 4) FAIL(ZJ_DE_FORMAT, "missing components");
         if (is_progressive) decode_progressive(cur);
-        else if (four()) decode_baseline4(cur);
+        else if (raster()) decode_baseline_raster(cur);
         else decode_baseline(cur);
         fill_descriptor(img);
     }

@@ -2284,44 +2284,51 @@ scaled_kernel(const DevImage *__restrict__ images)
     }
 }
 
-// ------------------------------------------------------------------------------------- four-component kernel
-// CMYK / YCCK input (the statement is in include/zune_jpeg_b200.h next to zj_decoder_jpeg_colorspace).  Each of the four
-// components has its own factors (1 or 2), block size ss_z (S0 = 8 >> LOG2D, or 2 S0) and up-sampling ratio (1 or 2 per axis).
-// grid = (tiles of tile_mcus MCU columns = TC_PIXELS output columns, MCU rows, images); block = ZJ_THREADS.
+// ------------------------------------------------------------------------------------- per-component kernel
+// Images whose components each take their own way (the statements are in include/zune_jpeg_b200.h next to
+// zj_decoder_jpeg_colorspace): CMYK / YCCK input (NC = 4), and YCbCr input with sampling factors outside the fused kernels'
+// sets (NC = 3).  Each component has its own factors (1..4), block size ss_z (S0 = 8 >> LOG2D, 2 S0 or 4 S0) and integer
+// up-sampling ratio (rh_z, rv_z), each 1..4.
+// grid = (tiles of tile_mcus MCU columns = at most TC_PIXELS output columns, MCU rows, images); block = ZJ_THREADS.
 //   phase 1: every component's blocks of the tile, plus one context block on each side along an axis it is up-sampled on, into a
 //            shared plane per component whose sample (j, i) sits at row j - (first row - 8), column i - (first column - 8);
 //            blocks of ss = 8 (IDCT: X86 or islow, with warp votes) run in a CTA-uniform loop of their own, reduced ones after;
-//   phase 2: one thread per output pixel: up-sampling per component, YCCK -> CMYK, Pillow's CMYK;I -> RGB, output.
+//   phase 2: one thread per output pixel: up-sampling per component, then JFIF colour (NC = 3) or YCCK -> CMYK and Pillow's
+//            CMYK;I -> RGB (NC = 4), output.
 __device__ __forceinline__ u32 cmyk_channel(u32 x, u32 nk)   // Convert.c cmyk2rgb: nk - MULDIV255(x, nk)
 {
     const u32 t = x * nk + 128;
     return nk - (((t >> 8) + t) >> 8);
 }
+__device__ __forceinline__ int div_ratio(int x, int r) { return r == 3 ? x / 3 : x >> (r >> 1); }   // x / r, r = 1..4
 
-template <int IDCT, int LOG2D>
+template <int IDCT, int LOG2D, int NC>
 __global__ void __launch_bounds__(ZJ_THREADS, 2)
-cmyk_kernel(const CmykImage *__restrict__ images)
+raster_kernel(const RasterImage *__restrict__ images)
 {
     static_assert(LOG2D == 0 || IDCT == IDCT_ISLOW, "DCT scaling is libjpeg output only");
+    static_assert(NC == 3 || NC == 4, "three or four components");
     constexpr int S0 = 8 >> LOG2D;
     constexpr bool FANCY = S0 > 1;
-    constexpr int PS = 144, PR = 32;   // shared plane: 8 + TC_PIXELS + 8 columns, 8 + 16 + 8 rows
-    __shared__ __align__(16) uint8_t sP[4][PR * PS];
-    __shared__ u32 sQ[4][32];
+    // shared plane: 8 + TC_PIXELS + 8 columns; 8 rows above, then an MCU row of up to 32 rows (ratio 1), or up to 16 rows and 8 of
+    // context below (ratio 2; ratios 3 and 4 need less)
+    constexpr int PS = 144, PR = 40;
+    __shared__ __align__(16) uint8_t sP[NC][PR * PS];
+    __shared__ u32 sQ[NC][32];
 
-    const CmykImage &im = images[blockIdx.z];
+    const RasterImage &im = images[blockIdx.z];
     const int tile = (int)blockIdx.x, my = (int)blockIdx.y;
     if (tile >= (int)im.n_tiles || my >= (int)im.mcu_y) return;
     const int tid = threadIdx.x;
     const int m0 = tile * (int)im.tile_mcus, m1 = min(m0 + (int)im.tile_mcus, (int)im.mcu_x);
-    for (int k = tid; k < 128; k += ZJ_THREADS) sQ[k >> 5][k & 31] = im.qtw[k >> 5][k & 31];
+    for (int k = tid; k < 32 * NC; k += ZJ_THREADS) sQ[k >> 5][k & 31] = im.qtw[k >> 5][k & 31];
 
     // block rows [rb0, rb1) x columns [cb0, cb1) of each component, context included; its plane origin (c0, r0) in samples
-    int rb0[4], cb0[4], ncol[4], nblk[4], c0[4], r0[4];
+    int rb0[NC], cb0[NC], ncol[NC], nblk[NC], c0[NC], r0[NC];
 #pragma unroll
-    for (int z = 0; z < 4; z++) {
+    for (int z = 0; z < NC; z++) {
         const int h = (int)im.h[z], v = (int)im.v[z], ss = (int)im.ss[z];
-        const bool uh = h * ss < (int)im.hmax * S0, uv = v * ss < (int)im.vmax * S0;   // up-sampled along x / y
+        const bool uh = (im.ratio[z] & 255u) > 1, uv = im.ratio[z] > 255u;   // up-sampled along x / y
         const int a0 = m0 * h, a1 = m1 * h, b0 = my * v, b1 = (my + 1) * v;
         cb0[z] = a0 - (uh && a0 > 0 ? 1 : 0);
         const int cb1 = a1 + (uh && a1 * ss < (int)im.dw[z] ? 1 : 0);
@@ -2339,7 +2346,7 @@ cmyk_kernel(const CmykImage *__restrict__ images)
     // NULL past the last block)
     auto locate = [&](const bool full, int b, int &z, const int16_t *&src, uint8_t *&dst) {
 #pragma unroll
-        for (int k = 0; k < 4; k++) {
+        for (int k = 0; k < NC; k++) {
             if (src || ((int)im.ss[k] == 8) != full) continue;
             if (b >= nblk[k]) { b -= nblk[k]; continue; }
             const int ss = (int)im.ss[k];
@@ -2351,7 +2358,7 @@ cmyk_kernel(const CmykImage *__restrict__ images)
     };
     int n_full = 0, n_red = 0;
 #pragma unroll
-    for (int k = 0; k < 4; k++) (im.ss[k] == 8 ? n_full : n_red) += nblk[k];
+    for (int k = 0; k < NC; k++) (im.ss[k] == 8 ? n_full : n_red) += nblk[k];
     for (int b0 = 0; b0 < n_full; b0 += ZJ_THREADS) {   // CTA-uniform trip count: every lane takes part in the warp votes
         int z = 0;
         const int16_t *src = nullptr;
@@ -2370,12 +2377,18 @@ cmyk_kernel(const CmykImage *__restrict__ images)
             uint8_t *dst = nullptr;
             locate(false, b, z, src, dst);
             int4 raw[8];
-            if (im.ss[z] == S0) {
+            const int ss = (int)im.ss[z];   // S0, 2 S0 or 4 S0, below 8
+            if (ss == S0) {
                 load_rows<S0>(true, src, raw);
                 idct_reduced<S0>(raw, sQ[z], dst, PS);
             } else if constexpr (2 * S0 < 8) {
-                load_rows<2 * S0>(true, src, raw);
-                idct_reduced<2 * S0>(raw, sQ[z], dst, PS);
+                if (ss == 2 * S0) {
+                    load_rows<2 * S0>(true, src, raw);
+                    idct_reduced<2 * S0>(raw, sQ[z], dst, PS);
+                } else if constexpr (4 * S0 < 8) {
+                    load_rows<4 * S0>(true, src, raw);
+                    idct_reduced<4 * S0>(raw, sQ[z], dst, PS);
+                }
             }
         }
     }
@@ -2389,60 +2402,81 @@ cmyk_kernel(const CmykImage *__restrict__ images)
         const int yl = u / tw, xl = u - yl * tw;
         const int x = m0 * mw + xl, y = my * mh + yl;
         if (x >= width || y >= height) continue;
-        u32 s[4];
+        u32 s[NC];
 #pragma unroll
-        for (int z = 0; z < 4; z++) {
-            const int ss = (int)im.ss[z], dw = (int)im.dw[z], dh = (int)im.dh[z];
-            const bool uh = (int)im.h[z] * ss < mw, uv = (int)im.v[z] * ss < mh;
+        for (int z = 0; z < NC; z++) {
+            const int dw = (int)im.dw[z], dh = (int)im.dh[z], rh = (int)(im.ratio[z] & 255u), rv = (int)(im.ratio[z] >> 8);
             const uint8_t *p = sP[z];
-            const int i = uh ? x >> 1 : x, j = uv ? y >> 1 : y;
+            const int i = div_ratio(x, rh), j = div_ratio(y, rv);
             auto at = [&](int jj, int ii) { return (int)p[(jj - r0[z]) * PS + (ii - c0[z])]; };
             int val;
-            if (uh && uv && FANCY && dw > 2) {         // HV: s[i] = 3 c[j][i] + c[j'][i]
+            if (rh == 2 && rv == 2 && FANCY && dw > 2) {         // HV: s[i] = 3 c[j][i] + c[j'][i]
                 const int jn = (y & 1) ? min(j + 1, dh - 1) : max(j - 1, 0);
                 const int in = (x & 1) ? min(i + 1, dw - 1) : max(i - 1, 0);
                 const int si = 3 * at(j, i) + at(jn, i), sn = 3 * at(j, in) + at(jn, in);
                 val = (x & 1) ? (3 * si + sn + 7) >> 4 : (3 * si + sn + 8) >> 4;
-            } else if (uh && !uv && FANCY && dw > 2) {  // H
+            } else if (rh == 2 && rv == 1 && FANCY && dw > 2) {  // H
                 const int in = (x & 1) ? min(i + 1, dw - 1) : max(i - 1, 0);
                 val = (3 * at(j, i) + at(j, in) + 1 + (x & 1)) >> 2;
-            } else if (uv && !uh && FANCY) {            // V
+            } else if (rh == 1 && rv == 2 && FANCY) {            // V
                 const int jn = (y & 1) ? min(j + 1, dh - 1) : max(j - 1, 0);
                 val = (3 * at(j, i) + at(jn, i) + 1 + (y & 1)) >> 2;
-            } else {                                    // no up-sampling, or repetition
+            } else {                                             // no up-sampling, or rh x rv repetition
                 val = at(j, i);
             }
             s[z] = (u32)val;
         }
-        // Pillow's CMYK;I bytes: YCCK -> libjpeg's CMYK (255 - (Y + chroma term), clamped) inverted is the JFIF RGB of (Y, Cb, Cr)
-        u32 c, m, ye;
-        if (im.ycck) jfif_rgb((int)s[0], (int)s[1], (int)s[2], c, m, ye);
-        else { c = 255 - s[0]; m = 255 - s[1]; ye = 255 - s[2]; }
-        const u32 nk = s[3];
         uint8_t *d = im.out + ((size_t)y * width + x) * nc;
-        if (im.kind == CMYK_OUT_CMYK) {
-            d[0] = (uint8_t)c; d[1] = (uint8_t)m; d[2] = (uint8_t)ye; d[3] = (uint8_t)(255 - nk);
-            continue;
+        if constexpr (NC == 3) {
+            if (im.kind == RASTER_OUT_GRAY) {   // the Y plane
+                d[0] = (uint8_t)s[0];
+                continue;
+            }
+            if (im.kind == RASTER_OUT_RAW) {    // YCbCr
+                d[0] = (uint8_t)s[0]; d[1] = (uint8_t)s[1]; d[2] = (uint8_t)s[2];
+                continue;
+            }
+            u32 r, g, b;
+            jfif_rgb((int)s[0], (int)s[1], (int)s[2], r, g, b);
+            d[0] = (uint8_t)r; d[1] = (uint8_t)g; d[2] = (uint8_t)b;
+            if (nc == 4) d[3] = 255;
+        } else {
+            // Pillow's CMYK;I bytes: YCCK -> libjpeg's CMYK (255 - (Y + chroma term), clamped) inverted is the JFIF RGB of (Y, Cb, Cr)
+            u32 c, m, ye;
+            if (im.model == RASTER_YCCK) jfif_rgb((int)s[0], (int)s[1], (int)s[2], c, m, ye);
+            else { c = 255 - s[0]; m = 255 - s[1]; ye = 255 - s[2]; }
+            const u32 nk = s[3];
+            if (im.kind == RASTER_OUT_RAW) {    // CMYK
+                d[0] = (uint8_t)c; d[1] = (uint8_t)m; d[2] = (uint8_t)ye; d[3] = (uint8_t)(255 - nk);
+                continue;
+            }
+            const u32 r = cmyk_channel(c, nk), g = cmyk_channel(m, nk), b = cmyk_channel(ye, nk);
+            if (im.kind == RASTER_OUT_GRAY) {
+                d[0] = (uint8_t)((19595 * r + 38470 * g + 7471 * b + 32768) >> 16);
+                continue;
+            }
+            d[0] = (uint8_t)r; d[1] = (uint8_t)g; d[2] = (uint8_t)b;
+            if (nc == 4) d[3] = 255;
         }
-        const u32 r = cmyk_channel(c, nk), g = cmyk_channel(m, nk), b = cmyk_channel(ye, nk);
-        if (im.kind == CMYK_OUT_GRAY) {
-            d[0] = (uint8_t)((19595 * r + 38470 * g + 7471 * b + 32768) >> 16);
-            continue;
-        }
-        d[0] = (uint8_t)r; d[1] = (uint8_t)g; d[2] = (uint8_t)b;
-        if (nc == 4) d[3] = 255;
     }
 }
 
-cudaError_t launch_cmyk(const CmykImage *d_images, const LaunchGroup &g, cudaStream_t stream)
+template <int NC>
+static void launch_raster_nc(dim3 grid, const RasterImage *p, const LaunchGroup &g, cudaStream_t stream)
+{
+    if (!g.islow) raster_kernel<IDCT_X86, 0, NC><<<grid, ZJ_THREADS, 0, stream>>>(p);
+    else if (g.scale == 0) raster_kernel<IDCT_ISLOW, 0, NC><<<grid, ZJ_THREADS, 0, stream>>>(p);
+    else if (g.scale == 1) raster_kernel<IDCT_ISLOW, 1, NC><<<grid, ZJ_THREADS, 0, stream>>>(p);
+    else if (g.scale == 2) raster_kernel<IDCT_ISLOW, 2, NC><<<grid, ZJ_THREADS, 0, stream>>>(p);
+    else raster_kernel<IDCT_ISLOW, 3, NC><<<grid, ZJ_THREADS, 0, stream>>>(p);
+}
+
+cudaError_t launch_raster(const RasterImage *d_images, const LaunchGroup &g, cudaStream_t stream)
 {
     dim3 grid(g.max_tiles, g.max_strips, g.count);   // max_strips: MCU rows
-    const CmykImage *p = d_images + g.first;
-    if (!g.islow) cmyk_kernel<IDCT_X86, 0><<<grid, ZJ_THREADS, 0, stream>>>(p);
-    else if (g.scale == 0) cmyk_kernel<IDCT_ISLOW, 0><<<grid, ZJ_THREADS, 0, stream>>>(p);
-    else if (g.scale == 1) cmyk_kernel<IDCT_ISLOW, 1><<<grid, ZJ_THREADS, 0, stream>>>(p);
-    else if (g.scale == 2) cmyk_kernel<IDCT_ISLOW, 2><<<grid, ZJ_THREADS, 0, stream>>>(p);
-    else cmyk_kernel<IDCT_ISLOW, 3><<<grid, ZJ_THREADS, 0, stream>>>(p);
+    const RasterImage *p = d_images + g.first;
+    if (g.raster == 4) launch_raster_nc<4>(grid, p, g, stream);
+    else launch_raster_nc<3>(grid, p, g, stream);
     return cudaGetLastError();
 }
 
