@@ -165,6 +165,12 @@ enum { ZJ_USE_LIBJPEG_OUTPUT = 3 };
 #define ZJ_FLAG_ORIENT_SHIFT 4
 #define ZJ_FLAG_ORIENT_MASK (7u << ZJ_FLAG_ORIENT_SHIFT)
 enum { ZJ_USE_EXIF_ORIENTATION = 0x100 };
+/* GPU entropy decoding of spec and libjpeg output (opt-in).  ZJ_USE_GPU_ENTROPY ORed into ZJ_USE_SPEC_OUTPUT,
+ * ZJ_USE_LIBJPEG_OUTPUT or ZJ_USE_LIBJPEG_OUTPUT | k << 4 (with or without ZJ_USE_EXIF_ORIENTATION) lets the
+ * zj_decode_batch_gpu* front doors (_gpu, _gpu_device, _gpu_device_ex, _gpu_device_resized) entropy-decode those images on the
+ * GPU (see zj_decode_batch_gpu).  Every other entry point decodes exactly as without the bit; every value without it keeps its
+ * meaning. */
+enum { ZJ_USE_GPU_ENTROPY = 0x200 };
 
 typedef enum zj_status {
     ZJ_OK = 0,
@@ -408,7 +414,8 @@ typedef struct zj_options {       /* ZuneJpegOptions (src/options.rs:6-40), same
                                      decodes every MCU row with Q9-Q11 off, whatever zj_host_set_quirks says;
                                      ZJ_USE_LIBJPEG_OUTPUT: the same, and the images carry ZJ_FLAG_ISLOW;
                                      ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the same, decoded at 1/2^k (ZJ_FLAG_SCALE_*);
-                                     any of these three | ZJ_USE_EXIF_ORIENTATION: the same, oriented (ZJ_FLAG_ORIENT_*) */
+                                     any of these three | ZJ_USE_EXIF_ORIENTATION: the same, oriented (ZJ_FLAG_ORIENT_*);
+                                     | ZJ_USE_GPU_ENTROPY: the same, and zj_decode_batch_gpu* may entropy-decode on the GPU */
     uint32_t out_colorspace;      /* ZJ_CS_RGB                                           */
     uint32_t num_threads;         /* 4                                                   */
     uint32_t max_width;           /* 16384                                               */
@@ -563,7 +570,16 @@ ZJ_API void zj_release_device_caches(void);
  * uploaded instead of their coefficient planes, one GPU thread per restart interval runs the reference's bit reader and MCU
  * loop (src/bitstream.rs:159-402) into device planes, which are reconstructed in place.  All other images (no DRI,
  * progressive, header errors, an interval that ends differently) take the zj_decode_batch route, so pixels, statuses and
- * errors are those of zj_decode_batch.  *n_gpu_entropy (may be NULL) = images whose entropy stage ran on the GPU. */
+ * errors are those of zj_decode_batch.  *n_gpu_entropy (may be NULL) = images whose entropy stage ran on the GPU.
+ * Spec form (use_unsafe a spec, libjpeg or scaled value | ZJ_USE_GPU_ENTROPY; without the bit spec images take the host route):
+ * the host stage's loop with Q9-Q11 off.  An image takes it when it is a baseline frame whose first scan covers every frame
+ * component (or has one component), with factors the fused kernels take (not four components, not the raster-plane factor
+ * sets), in its scan-start state, and the first marker behind its entropy-coded data that is not RSTn is EOI.  With DRI one
+ * thread per restart interval decodes as above; without DRI (or with one interval) the scan is de-stuffed and decoded by a
+ * self-synchronising decode (DESIGN.md section 5.5).  That decode turns the image down -- it takes the host route -- when a
+ * code is invalid, a non-zero coefficient lands past index 63, a symbol needs bits beyond the scan's data, fewer blocks than
+ * the frame holds are decoded, a block falls outside its strip, or the subsequences do not settle within the sync rounds.
+ * Scaled and oriented images take these forms too. */
 ZJ_API int zj_decode_batch_gpu(const zj_options *o, const uint8_t *const *bufs, const size_t *lens, size_t n,
                                uint8_t **out, size_t *out_len, int *status, size_t *n_gpu_entropy);
 /* ... and with the pixels left in device memory (no PCIe download at all: what is uploaded is the JPEG file): out_dev[i] is a
@@ -590,7 +606,8 @@ ZJ_API int zj_decode_batch_gpu_device_resized(const zj_options *o, const uint8_t
  *   Q10 src/bitstream.rs:278-281 decode_dc refills only below 16 buffered bits but may consume 27: the reader under-runs
  *   Q11 src/mcu.rs:337-342       the MCU loop breaks on a PREFETCHED EOI: trailing components of the last MCU stay zero
  * Process-wide; takes effect for decodes started afterwards (a ZJ_USE_SPEC_OUTPUT decode runs with every bit cleared, whatever
- * is set here).  With any bit cleared the GPU entropy route (zj_decode_batch_gpu*) sends every image through the host stage.
+ * is set here).  With any bit cleared the GPU entropy route (zj_decode_batch_gpu*) sends every as-written image through the host
+ * stage; spec decodes ignore these switches.
  * tests/test_quirks.py is the only caller. */
 enum { ZJ_QUIRK_Q9_FAST_AC_I16 = 1u, ZJ_QUIRK_Q10_DC_REFILL = 2u, ZJ_QUIRK_Q11_EOI_BREAK = 4u, ZJ_QUIRK_ALL = 7u };
 ZJ_API void zj_host_set_quirks(uint32_t mask);

@@ -130,11 +130,13 @@ __device__ __forceinline__ void decode_huff(Reader &r, int &symbol, const EntTab
     r.drop_bits((u32)code_length);
 }
 
-// decode_mcu_block, bitstream.rs:314-373; block == nullptr: the component is not output, its coefficients are dropped
+// decode_mcu_block, bitstream.rs:314-373; block == nullptr: the component is not output, its coefficients are dropped.
+// SPEC: Q10 off (the DC refill happens whenever <= 32 bits are buffered, as before every AC symbol)
+template <bool SPEC>
 __device__ __forceinline__ void decode_block(Reader &r, const EntTable &dc, const EntTable &ac, const uint8_t *__restrict__ unzigzag, int16_t *__restrict__ block, int &pred)
 {
     // decode_dc, :272-297 (refills only below 16 buffered bits, Q10)
-    if (r.bits_left < 16) r.refill();
+    if (SPEC || r.bits_left < 16) r.refill();
     int symbol = dc.lookup[r.peek9()];
     decode_huff(r, symbol, dc);
     if (r.bad) return;
@@ -173,7 +175,8 @@ __device__ __forceinline__ void decode_block(Reader &r, const EntTable &dc, cons
     }
 }
 
-template <int ENT_LANES>
+// SPEC: the loop of a spec decode (Q10 and Q11 off); the acceptance rule and the Q8 bookkeeping are the same
+template <int ENT_LANES, bool SPEC>
 __global__ void __launch_bounds__(ENT_THREADS) entropy_kernel(const EntImage *__restrict__ images)
 {
     __shared__ EntTable sT[6];
@@ -222,7 +225,7 @@ __global__ void __launch_bounds__(ENT_THREADS) entropy_kernel(const EntImage *__
                         block = plane + (size_t)strip * im.strip_len[pos] + start;
                     }
                     int pred = pos == 0 ? dc0 : (pos == 1 ? dc1 : dc2);
-                    decode_block(r, dc, ac, sZ, block, pred);
+                    decode_block<SPEC>(r, dc, ac, sZ, block, pred);
                     if (pos == 0) dc0 = pred; else if (pos == 1) dc1 = pred; else dc2 = pred;
                     if (r.bad) ok = false;
                 }
@@ -242,7 +245,8 @@ __global__ void __launch_bounds__(ENT_THREADS) entropy_kernel(const EntImage *__
             if (r.marker != MK_NONE) {   // mcu.rs:337-348
                 if (r.marker == MK_EOI) {
                     if (must_reset) ok = false;
-                    break;
+                    if (!SPEC) break;      // Q11; spec: finish the MCU on the bits already buffered
+                    continue;
                 }
                 continue;                // RSTn met ahead of the countdown: keep going on faked zero bits
             }
@@ -253,22 +257,330 @@ __global__ void __launch_bounds__(ENT_THREADS) entropy_kernel(const EntImage *__
 }
 
 template <int LANES>
-static int launch_lanes(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, cudaStream_t s)
+static int launch_lanes(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, cudaStream_t s, bool spec)
 {
     constexpr uint32_t SEGS = ENT_THREADS / 32 * LANES;
     dim3 grid((max_seg + SEGS - 1) / SEGS, n_images);
-    entropy_kernel<LANES><<<grid, ENT_THREADS, 0, s>>>(d_images);
+    if (spec) entropy_kernel<LANES, true><<<grid, ENT_THREADS, 0, s>>>(d_images);
+    else entropy_kernel<LANES, false><<<grid, ENT_THREADS, 0, s>>>(d_images);
     return (int)cudaGetLastError();
 }
 
-int launch_entropy(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, void *stream)
+int launch_entropy(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, void *stream, bool spec)
 {
     if (n_images == 0 || max_seg == 0) return 0;
     const uint64_t intervals = (uint64_t)n_images * max_seg;          // (an upper bound: images of one launch may differ)
     cudaStream_t s = (cudaStream_t)stream;
-    if (intervals < 12000) return launch_lanes<8>(d_images, n_images, max_seg, s);
-    if (intervals < 24000) return launch_lanes<16>(d_images, n_images, max_seg, s);
-    return launch_lanes<32>(d_images, n_images, max_seg, s);
+    if (intervals < 12000) return launch_lanes<8>(d_images, n_images, max_seg, s, spec);
+    if (intervals < 24000) return launch_lanes<16>(d_images, n_images, max_seg, s, spec);
+    return launch_lanes<32>(d_images, n_images, max_seg, s, spec);
+}
+
+// ================================================================ scans without restart markers (spec and libjpeg output)
+// Phases per sub-batch, all on one stream: SYNC_ROUNDS launches of sync_round_kernel, then accept_kernel, write_kernel and
+// dc_kernel.  The de-stuffing (FF 00 -> FF, fill bytes dropped) is done by the host stage while it looks for the scan's end.
+//
+// Bounds: a decode runs only while its position is below its end (<= nbits) and refills only when <= 32 bits are buffered, so
+// the highest word it loads is (pos + 32) / 32 <= nbits / 32 + 1, inside the >= 8 zero bytes after the data.  Table reads are
+// indexed by 9-bit peeks, code lengths 1..17 and `& 0xFF`; coefficient positions are checked <= 63 before a store.  Stores
+// happen only in write_kernel and dc_kernel, from the states accept_kernel verified, at block indices below the total, after
+// the addressing check of mcu.rs:293-312 (start + 64 <= strip_len).  State words and counters are indexed by the thread's own
+// subsequence k < n_sub, its predecessor k - 1, or the round r < SYNC_ROUNDS.
+
+struct SyncBits {          // a bit reader over the de-stuffed scan: the next nb (>= 33 after refill) bits sit at the top of buf
+    const uint32_t *w;
+    u64 buf, pos;
+    u32 nb, wi;
+    __device__ __forceinline__ u32 word(u32 i) const { return __byte_perm(__ldg(w + i), 0, 0x0123); }
+    __device__ __forceinline__ void init(const uint32_t *words, u64 p)
+    {
+        w = words; pos = p;
+        wi = (u32)(p >> 5);
+        buf = ((u64)word(wi) << 32) | word(wi + 1);
+        wi += 2;
+        const u32 s = (u32)(p & 31);
+        buf <<= s;
+        nb = 64 - s;
+    }
+    __device__ __forceinline__ void refill() { if (nb <= 32) { buf |= (u64)word(wi++) << (32 - nb); nb += 32; } }
+    __device__ __forceinline__ u32 peek(u32 n) const { return (u32)(buf >> (64 - n)); }
+    __device__ __forceinline__ void drop(u32 n) { buf <<= n; nb -= n; pos += n; }
+    __device__ __forceinline__ int get(u32 n) { const int v = (int)peek(n); drop(n); return v; }
+};
+
+// decode_huff! (bitstream.rs:49-90) on SyncBits: the symbol, or -1 for a code the table does not hold
+__device__ __forceinline__ int sync_huff(SyncBits &b, const EntTable &t, int symbol)
+{
+    int code_length = symbol >> 9;
+    symbol &= 511;
+    if (code_length > 9) {
+        symbol = (int)b.peek(16);
+        while (code_length < 17) {
+            if (symbol < t.maxcode[code_length]) break;
+            code_length++;
+        }
+        if (code_length == 17) return -1;
+        symbol >>= (16 - code_length);
+        symbol = t.values[(symbol + t.offset[code_length]) & 0xFF];
+    }
+    b.drop((u32)code_length);
+    return symbol;
+}
+
+__device__ __forceinline__ u64 sync_state(u64 pos, u32 slot, u32 coef) { return pos << 16 | slot << 8 | coef; }
+
+// mcu.rs:293-312 for global block g: its coefficients, nullptr when its component is not output; ok = false when the
+// reference would index outside the strip
+__device__ __forceinline__ int16_t *sync_block(const SyncImage &im, u32 g, bool &ok)
+{
+    const u32 m = g / im.bpm, slot = g - m * im.bpm;
+    const u32 pos = im.slot_comp[slot], v_samp = im.slot_v[slot], h_samp = im.slot_h[slot];
+    int16_t *plane = im.plane[pos];
+    if (!plane) return nullptr;
+    const u32 per_strip = im.bias * im.mcu_w;
+    const u32 strip = m / per_strip, v = (m - strip * per_strip) / im.mcu_w, j = m - strip * per_strip - v * im.mcu_w;
+    const u32 hs = im.h_samp[pos], vs = im.v_samp[pos], is_y = im.is_y[pos];
+    const u32 y_offset = is_y * v * (im.hv_width_stride + (im.hv_width_stride * (vs - 1)));
+    const u32 another_stride = im.is_hv ? im.hv_width_stride * v_samp : im.width_stride * v_samp;
+    const u32 yet_another_stride = (im.is_hv && !is_y) ? (im.width_stride >> 2) * v : 0u;
+    const u32 start = (j * 64 * hs) + (h_samp * 64) + another_stride + y_offset + yet_another_stride;
+    if (start + 64 > im.strip_len[pos]) { ok = false; return nullptr; }
+    return plane + (size_t)strip * im.strip_len[pos] + start;
+}
+
+// The host stage's decode_mcu_block (bitstream.rs:314-373 with Q9-Q11 off), one symbol at a time, from state (pos, slot,
+// coef) over the symbols that start below `end`.  Returns the exit state, or SYNC_INVALID on a code the table does not hold,
+// a non-zero coefficient past index 63 or a symbol that ends beyond nbits; `blocks` = blocks completed before that.
+// WRITE: g0 = global index of the block in progress at the entry; coefficients and DC differences are stored for blocks
+// below `total`, and the decode stops at block `total`; ok = false when an addressing check fails.
+template <bool WRITE>
+__device__ u64 sync_decode(const SyncImage &im, const EntTable *T, const uint8_t *Z, u64 pos, u32 slot, u32 coef, u64 end,
+                           u32 &blocks, u32 g0, u32 total, bool &ok)
+{
+    blocks = 0;
+    if (pos >= end) return sync_state(pos, slot, coef);
+    SyncBits b;
+    b.init(im.bits, pos);
+    int16_t *blk = nullptr;
+    if (WRITE) { if (g0 >= total) return sync_state(pos, slot, coef); blk = sync_block(im, g0, ok); }
+    while (b.pos < end) {
+        if (WRITE && !ok) break;
+        const u32 comp = im.slot_comp[slot];
+        const EntTable &dc = T[2 * comp], &ac = T[2 * comp + 1];
+        b.refill();
+        if (coef == 0) {
+            int s = sync_huff(b, dc, dc.lookup[b.peek(9)]);
+            if (s < 0) return SYNC_INVALID;
+            int v = 0;
+            if (s != 0) v = huff_extend(b.get((u32)s), s);
+            if (WRITE) im.dc[g0 + blocks] = (int16_t)v;
+            coef = 1;
+        } else {
+            const int fast_ac = (int)ac.ac_lookup[b.peek(9)];
+            if (fast_ac != 0) {
+                coef += (u32)((fast_ac >> 4) & 63);
+                const int v = fast_ac >> 10;
+                if (v != 0) {
+                    if (coef > 63) return SYNC_INVALID;
+                    if (WRITE && blk) blk[Z[coef] & 63] = (int16_t)v;
+                }
+                b.drop((u32)(fast_ac & 15));
+                coef += 1;
+            } else {
+                int s = sync_huff(b, ac, ac.lookup[b.peek(9)]);
+                if (s < 0) return SYNC_INVALID;
+                const u32 rr = (u32)s >> 4;
+                s &= 15;
+                if (s != 0) {
+                    coef += rr;
+                    if (coef > 63) return SYNC_INVALID;
+                    const int v = huff_extend(b.get((u32)s), s);
+                    if (WRITE && blk) blk[Z[coef] & 63] = (int16_t)v;
+                    coef += 1;
+                } else if (rr != 15) {
+                    coef = 64;
+                } else {
+                    coef += 16;
+                }
+            }
+        }
+        if (b.pos > im.nbits) return SYNC_INVALID;
+        if (coef >= 64) {
+            blocks++;
+            coef = 0;
+            slot = slot + 1 == im.bpm ? 0 : slot + 1;
+            if (WRITE) {
+                if (g0 + blocks >= total) break;
+                blk = sync_block(im, g0 + blocks, ok);
+            }
+        }
+    }
+    return sync_state(b.pos, slot, coef);
+}
+
+__device__ __forceinline__ void sync_tables(const SyncImage &im, EntTable *sT, uint8_t *sZ)
+{
+    const u32 words = (u32)(sizeof(EntTable) / 4) * 2u * (u32)(im.slot_comp[im.bpm - 1] + 1);
+    const u32 *src = reinterpret_cast<const u32 *>(im.tables);
+    u32 *dst = reinterpret_cast<u32 *>(sT);
+    for (u32 i = threadIdx.x; i < words; i += SYNC_THREADS) dst[i] = src[i];
+    for (u32 i = threadIdx.x; i < 80; i += SYNC_THREADS) sZ[i] = c_unzigzag[i];
+    __syncthreads();
+}
+
+__device__ __forceinline__ u64 sync_end(const SyncImage &im, u32 k)
+{
+    return k + 1 == im.n_sub ? im.nbits : (u64)(k + 1) * SYNC_BITS;
+}
+
+// Round r: subsequence k's entry is its predecessor's exit of round r - 1 (round 0, or an invalid exit: the guess
+// (k * SYNC_BITS, slot 0, coefficient 0)); subsequence 0 always starts at the scan start.  A subsequence decodes only when its
+// entry differs from the one its last decode used.  A round in which no subsequence decodes is the fixpoint: both exit
+// buffers then hold the same states, and later rounds return at once.
+__global__ void __launch_bounds__(SYNC_THREADS) sync_round_kernel(const SyncImage *__restrict__ images, u32 r)
+{
+    __shared__ EntTable sT[6];
+    __shared__ uint8_t sZ[80];
+    const SyncImage &im = images[blockIdx.y];
+    if (blockIdx.x * SYNC_THREADS >= im.n_sub) return;
+    if (r >= 2 && im.changed[r - 1] == 0) return;
+    sync_tables(im, sT, sZ);
+    const u32 k = blockIdx.x * SYNC_THREADS + threadIdx.x;
+    if (k >= im.n_sub) return;
+    u64 entry = sync_state((u64)k * SYNC_BITS, 0, 0);
+    if (k > 0 && r > 0) {
+        const u64 e = im.exit[(r - 1) & 1][k - 1];
+        if (e != SYNC_INVALID) entry = e;
+    }
+    if (r > 0 && entry == im.used[k]) { im.exit[r & 1][k] = im.exit[(r - 1) & 1][k]; return; }
+    im.used[k] = entry;
+    u32 blocks;
+    bool ok = true;
+    im.exit[r & 1][k] = sync_decode<false>(im, sT, sZ, entry >> 16, (u32)(entry >> 8) & 255, (u32)entry & 255, sync_end(im, k), blocks, 0, 0, ok);
+    im.count[k] = blocks;
+    atomicAdd(&im.changed[r], 1u);
+}
+
+// One CTA per image: takes the image when the rounds reached the fixpoint and the decode from the true entries completes
+// total_mcus * bpm blocks before its first error (or without one); count[k] becomes subsequence k's first global block index.
+__global__ void __launch_bounds__(1024) accept_kernel(const SyncImage *__restrict__ images)
+{
+    __shared__ u32 s_sum[1024];
+    __shared__ u32 s_err;
+    const SyncImage &im = images[blockIdx.x];
+    bool settled = false;
+    for (u32 r = 1; r < SYNC_ROUNDS; r++) settled = settled || im.changed[r] == 0;
+    if (!settled) { if (threadIdx.x == 0) *im.status = 1; return; }
+    if (threadIdx.x == 0) s_err = 0xFFFFFFFFu;
+    const u32 n = im.n_sub, per = (n + 1023) / 1024;
+    const u32 k0 = min(n, threadIdx.x * per), k1 = min(n, k0 + per);
+    u32 sum = 0;
+    for (u32 k = k0; k < k1; k++) sum += im.count[k];
+    s_sum[threadIdx.x] = sum;
+    __syncthreads();
+    for (u32 d = 1; d < 1024; d <<= 1) {          // inclusive scan of the chunk sums
+        const u32 v = threadIdx.x >= d ? s_sum[threadIdx.x - d] : 0u;
+        __syncthreads();
+        s_sum[threadIdx.x] += v;
+        __syncthreads();
+    }
+    u32 base = s_sum[threadIdx.x] - sum;
+    for (u32 k = k0; k < k1; k++) {
+        const u32 c = im.count[k];
+        im.count[k] = base;
+        if (im.exit[0][k] == SYNC_INVALID) atomicMin(&s_err, k);
+        base += c;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const u32 total = im.total_mcus * im.bpm;
+        u64 reached;
+        if (s_err != 0xFFFFFFFFu) {
+            // the block in progress at the first error: the next subsequence's base (the scan total behind the last one)
+            const u32 kb = s_err;
+            reached = kb + 1 < n ? (u64)im.count[kb + 1] : (u64)s_sum[1023];
+        } else {
+            reached = s_sum[1023];
+        }
+        *im.status = reached >= total ? 0 : 1;
+    }
+}
+
+// Subsequence k decodes again from its verified entry and stores the AC coefficients and DC differences of its blocks
+__global__ void __launch_bounds__(SYNC_THREADS) write_kernel(const SyncImage *__restrict__ images)
+{
+    __shared__ EntTable sT[6];
+    __shared__ uint8_t sZ[80];
+    __shared__ uint8_t s_status;
+    const SyncImage &im = images[blockIdx.y];
+    if (blockIdx.x * SYNC_THREADS >= im.n_sub) return;
+    // (other CTAs of the image may set the status while this one runs: one read per CTA, published by the barrier)
+    if (threadIdx.x == 0) s_status = *im.status;
+    sync_tables(im, sT, sZ);
+    if (s_status != 0) return;
+    const u32 k = blockIdx.x * SYNC_THREADS + threadIdx.x;
+    if (k >= im.n_sub) return;
+    const u32 total = im.total_mcus * im.bpm, g0 = im.count[k];
+    if (g0 >= total) return;
+    const u64 entry = k == 0 ? 0ull : im.exit[0][k - 1];
+    if (entry == SYNC_INVALID) return;   // (not reached: subsequences behind an error start at or past block total)
+    u32 blocks;
+    bool ok = true;
+    sync_decode<true>(im, sT, sZ, entry >> 16, (u32)(entry >> 8) & 255, (u32)entry & 255, sync_end(im, k), blocks, g0, total, ok);
+    if (!ok) *im.status = 1;
+}
+
+// One CTA per image: the DC predictors, a wrapping 32-bit prefix sum of the differences per component in block order,
+// stored as (int16_t)pred the way decode_dc does
+__global__ void __launch_bounds__(1024) dc_kernel(const SyncImage *__restrict__ images)
+{
+    __shared__ u32 s_sum[3][1024];
+    const SyncImage &im = images[blockIdx.x];
+    if (*im.status != 0) return;
+    const u32 mcus = im.total_mcus, per = (mcus + 1023) / 1024, bpm = im.bpm;
+    const u32 m0 = min(mcus, threadIdx.x * per), m1 = min(mcus, m0 + per);
+    u32 sum[3] = {0, 0, 0};
+    for (u32 m = m0; m < m1; m++)
+        for (u32 s = 0; s < bpm; s++) {
+            const u32 c = im.slot_comp[s];
+            const u32 d = (u32)(int)im.dc[m * bpm + s];
+            sum[0] += c == 0 ? d : 0u; sum[1] += c == 1 ? d : 0u; sum[2] += c == 2 ? d : 0u;
+        }
+    for (int c = 0; c < 3; c++) s_sum[c][threadIdx.x] = sum[c];
+    __syncthreads();
+    for (u32 d = 1; d < 1024; d <<= 1) {
+        u32 v[3];
+        for (int c = 0; c < 3; c++) v[c] = threadIdx.x >= d ? s_sum[c][threadIdx.x - d] : 0u;
+        __syncthreads();
+        for (int c = 0; c < 3; c++) s_sum[c][threadIdx.x] += v[c];
+        __syncthreads();
+    }
+    u32 pred[3];
+    for (int c = 0; c < 3; c++) pred[c] = s_sum[c][threadIdx.x] - sum[c];
+    for (u32 m = m0; m < m1; m++)
+        for (u32 s = 0; s < bpm; s++) {
+            const u32 c = im.slot_comp[s];
+            const u32 d = (u32)(int)im.dc[m * bpm + s];
+            u32 p = c == 0 ? pred[0] : (c == 1 ? pred[1] : pred[2]);
+            p += d;
+            if (c == 0) pred[0] = p; else if (c == 1) pred[1] = p; else pred[2] = p;
+            bool ok = true;
+            int16_t *blk = sync_block(im, m * bpm + s, ok);   // (checked by write_kernel: every block below the total was visited)
+            if (blk) blk[0] = (int16_t)p;
+        }
+}
+
+int launch_sync_phase(const SyncImage *d_images, uint32_t n_images, uint32_t max_sub, void *stream, int phase)
+{
+    if (n_images == 0 || max_sub == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    const dim3 grid((max_sub + SYNC_THREADS - 1) / SYNC_THREADS, n_images);
+    if (phase == SYNC_PHASE_ROUNDS)
+        for (u32 r = 0; r < SYNC_ROUNDS; r++) sync_round_kernel<<<grid, SYNC_THREADS, 0, s>>>(d_images, r);
+    else if (phase == SYNC_PHASE_ACCEPT) accept_kernel<<<n_images, 1024, 0, s>>>(d_images);
+    else if (phase == SYNC_PHASE_WRITE) write_kernel<<<grid, SYNC_THREADS, 0, s>>>(d_images);
+    else dc_kernel<<<n_images, 1024, 0, s>>>(d_images);
+    return (int)cudaGetLastError();
 }
 
 }  // namespace zj

@@ -1,7 +1,8 @@
 // zj_entropy.h -- descriptors of the GPU form of the baseline entropy stage (zj_entropy.cu), filled by the host
 // front-end (zj_host_decoder.cpp).
 //
-// Scope: baseline scans with restart markers (DRI).  Every restart interval starts from a known state (fresh bit
+// Scope: baseline scans with restart markers (DRI), and (spec and libjpeg output only) baseline scans without them, below.
+// Every restart interval starts from a known state (fresh bit
 // reader right behind its RSTn, predictors 0, countdown = DRI), so one GPU thread per interval runs the reference's MCU
 // loop (src/mcu.rs:253-351, handle_rst :386-418) with the reference's bit reader (src/bitstream.rs:159-402) and writes
 // coefficients straight into the device planes the reconstruction kernels read.  An interval that does not end exactly
@@ -40,6 +41,40 @@ struct EntImage {
 // with 32 / 16 / 8 / 4 lanes, 256 images 27.2 / 30.1 / 30.7 / 33.4 ms: launch_entropy picks 8, 16 or 32 by the number of
 // intervals of the launch.  grid = (ceil(max n_seg / intervals per CTA), images)
 constexpr int ENT_THREADS = 256;                         // threads per CTA
-int launch_entropy(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, void *stream);
+// spec: the libjpeg form of the loop (spec and libjpeg output, zj_decoder::quirks == 0): the DC refill whenever <= 32 bits are
+// buffered (Q10 off) and no break on a prefetched EOI (Q11 off); the tables come without Q9 from the host stage
+int launch_entropy(const EntImage *d_images, uint32_t n_images, uint32_t max_seg, void *stream, bool spec = false);
+
+// ---- scans without restart markers, spec and libjpeg output only (zj_entropy.cu, DESIGN.md section 5.5)
+// With Q9-Q11 off the host stage's symbols are a pure function of the de-stuffed bit sequence, so a decode that starts at a
+// code boundary in the right (block slot, coefficient index) state goes on exactly as the sequential loop does.  The bits are
+// cut into subsequences of SYNC_BITS; each thread decodes one from an entry state and records its exit state (the state at the
+// first symbol that starts at or beyond the subsequence's end), rounds take the predecessor's exit as the next entry until a
+// round changes nothing; at that fixpoint every entry is the sequential decoder's state at that bit.
+constexpr uint32_t SYNC_BITS = 1024;       // bits per subsequence
+constexpr uint32_t SYNC_ROUNDS = 24;       // sync rounds launched per sub-batch; an image not settled by then is turned down
+constexpr int SYNC_THREADS = 256;
+constexpr uint64_t SYNC_INVALID = ~0ull;   // exit state of a decode that met an error (its count says how many blocks it completed)
+
+struct SyncImage {
+    const uint32_t *bits;         // de-stuffed scan, big-endian bytes, followed by >= 8 zero bytes (reads past nbits stay inside)
+    uint64_t nbits;
+    const EntTable *tables;       // 2 * ncomp entries: [dc, ac] of component 0, 1, 2
+    int16_t *plane[3];            // zeroed whole-image planes; nullptr = component not output
+    uint64_t *exit[2];            // n_sub states each (pos << 16 | slot << 8 | coef), by round parity
+    uint64_t *used;               // n_sub: the entry state the subsequence's last decode started from
+    uint32_t *count;              // n_sub: blocks that decode completed; then (accept kernel) the first global block index
+    uint32_t *changed;            // SYNC_ROUNDS counters, zeroed: decodes run in round r
+    int16_t *dc;                  // total blocks: DC differences in block order
+    uint8_t *status;              // one byte, written by the accept kernel: 0 = take the planes, 1 = host stage
+    uint32_t n_sub, total_mcus, bpm;
+    uint32_t mcu_w, bias, is_hv, width_stride, hv_width_stride;
+    uint32_t strip_len[3], h_samp[3], v_samp[3], is_y[3];
+    uint8_t slot_comp[8], slot_v[8], slot_h[8];   // block slot of the MCU -> component, v_samp, h_samp (bpm <= 6)
+};
+// Queues one phase of the decode of n_images images on `stream` (the phases in this order: SYNC_ROUNDS round launches, accept,
+// write, DC); returns a cudaError_t.
+enum { SYNC_PHASE_ROUNDS = 0, SYNC_PHASE_ACCEPT = 1, SYNC_PHASE_WRITE = 2, SYNC_PHASE_DC = 3 };
+int launch_sync_phase(const SyncImage *d_images, uint32_t n_images, uint32_t max_sub, void *stream, int phase);
 
 }  // namespace zj

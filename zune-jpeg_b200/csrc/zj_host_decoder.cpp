@@ -741,13 +741,20 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         return (u & 15u) == ZJ_USE_LIBJPEG_OUTPUT && k >= 1 && k <= 3 ? k : 0;
     }
     uint32_t scale() const { return scale_of(use()); }
-    // ZJ_USE_EXIF_ORIENTATION ORed into a spec, libjpeg or scaled value: that value, oriented; every other value keeps its meaning
-    bool exif_orientation() const
+    // ZJ_USE_EXIF_ORIENTATION and ZJ_USE_GPU_ENTROPY ORed into a spec, libjpeg or scaled value: that value, oriented / with the
+    // GPU entropy route of zj_decode_batch_gpu*; every other value keeps its meaning
+    static bool spec_value(uint32_t u) { return u == ZJ_USE_SPEC_OUTPUT || u == ZJ_USE_LIBJPEG_OUTPUT || scale_of(u) != 0; }
+    bool spec_bit(uint32_t bit) const
     {
-        const uint32_t u = options.use_unsafe & ~(uint32_t)ZJ_USE_EXIF_ORIENTATION;
-        return (options.use_unsafe & ZJ_USE_EXIF_ORIENTATION) && (u == ZJ_USE_SPEC_OUTPUT || u == ZJ_USE_LIBJPEG_OUTPUT || scale_of(u) != 0);
+        return (options.use_unsafe & bit) && spec_value(options.use_unsafe & ~(uint32_t)(ZJ_USE_EXIF_ORIENTATION | ZJ_USE_GPU_ENTROPY));
     }
-    uint32_t use() const { return exif_orientation() ? options.use_unsafe & ~(uint32_t)ZJ_USE_EXIF_ORIENTATION : options.use_unsafe; }
+    bool exif_orientation() const { return spec_bit(ZJ_USE_EXIF_ORIENTATION); }
+    bool gpu_entropy() const { return spec_bit(ZJ_USE_GPU_ENTROPY); }
+    uint32_t use() const
+    {
+        const uint32_t u = options.use_unsafe & ~(uint32_t)(ZJ_USE_EXIF_ORIENTATION | ZJ_USE_GPU_ENTROPY);
+        return spec_value(u) ? u : options.use_unsafe;
+    }
     // a one-component image: GRAYSCALE output (headers.rs:278-285, mcu.rs:171-196), except that spec output keeps RGB / RGBA / RGBX
     void gray_input_out_cs()
     {
@@ -1388,12 +1395,18 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         BaselineGeom g;
         std::vector<uint32_t> seg_start;   // reader position at the start of every restart interval (+ one unused entry)
         size_t n_seg = 0, total = 0;
+        // a spec scan without restart markers (zj_entropy.h, SyncImage): its de-stuffed bytes, zero-padded; n_seg is 1 (its status)
+        bool sync = false;
+        std::vector<uint8_t> bits;
+        uint64_t nbits = 0;
+        size_t n_sub = 0, bpm = 0;
     };
     // Headers are parsed (reader stands at the first entropy-coded byte).  True when the scan can be handed to the GPU: a
     // baseline scan with restart markers in the state the interval-parallel forms start from.  Everything else -- and every
     // error -- is left to the host stage, which then reports exactly what the reference reports.
     bool gpu_entropy_prepare(const Cursor &reader, GpuPrep &pp)
     {
+        if (spec()) return gpu_entropy() && gpu_entropy_prepare_spec(reader, pp);
         if (is_progressive || restart_interval == 0 || todo != restart_interval) return false;
         if (quirks != ZJ_QUIRK_ALL) return false;   // the GPU form carries the quirks as written; test switches and spec output -> host stage
         if (reader.len >= 0xFFFFFFF0ull) return false;
@@ -1415,6 +1428,88 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         pp.seg_start[0] = (uint32_t)reader.pos;
         for (size_t k = 1; k < pp.n_seg; k++) pp.seg_start[k] = (uint32_t)ends[k - 1];
         pp.seg_start[pp.n_seg] = 0;
+        return true;
+    }
+    // Code of the first marker at or after `from` that is not RSTn (FF 00 is data), -1 when the data ends first
+    static int first_marker_after(const Cursor &reader, size_t from)
+    {
+        const uint8_t *d = reader.data;
+        const size_t n = reader.len;
+        for (size_t p = from; p < n;) {
+            const uint8_t *f = (const uint8_t *)memchr(d + p, 0xFF, n - p);
+            if (!f) return -1;
+            p = (size_t)(f - d) + 1;
+            while (p < n && d[p] == 0xFF) p++;
+            if (p >= n) return -1;
+            const uint8_t b = d[p++];
+            if (b != 0x00 && !(b >= 0xD0 && b <= 0xD7)) return b;
+        }
+        return -1;
+    }
+    // The scan's entropy-coded data as the bit reader sees it (bitstream.rs:200-215): FF [FF..] 00 -> FF, and the FF [FF..] of
+    // the marker that ends it dropped.  True when that marker is EOI; RSTn (without DRI), DNL, a later scan, any other marker
+    // and data without an end marker are left to the host stage.
+    static bool destuff_scan(const Cursor &reader, std::vector<uint8_t> &out)
+    {
+        const uint8_t *d = reader.data;
+        const size_t n = reader.len;
+        size_t p = reader.pos;
+        out.clear();
+        out.reserve(n - std::min(n, p) + 16);
+        while (p < n) {
+            const uint8_t *f = (const uint8_t *)memchr(d + p, 0xFF, n - p);
+            if (!f) return false;
+            const size_t q = (size_t)(f - d);
+            out.insert(out.end(), d + p, d + q + 1);
+            p = q + 1;
+            while (p < n && d[p] == 0xFF) p++;
+            if (p >= n) return false;
+            const uint8_t b = d[p++];
+            if (b == 0x00) continue;
+            out.pop_back();
+            return b == 0xD9;
+        }
+        return false;
+    }
+    // The spec branch (ZJ_USE_GPU_ENTROPY with spec or libjpeg output, quirks off): a baseline frame whose first scan covers
+    // every frame component, with factors the fused and spec kernels take, in its scan-start state, whose entropy-coded data
+    // is followed by EOI.  With DRI it takes the interval kernel's spec form, without DRI the self-synchronising decode.
+    bool gpu_entropy_prepare_spec(const Cursor &reader, GpuPrep &pp)
+    {
+        if (is_progressive || raster() || four() || (size_t)num_scans != components.size()) return false;
+        if (restart_interval ? todo != restart_interval : todo != 0x7fffffff) return false;
+        if (reader.len >= ((size_t)1 << 28)) return false;   // (bit positions stay below 2^31)
+        try { baseline_setup(pp.g); } catch (DecodeError &) { return false; }
+        const BaselineGeom &g = pp.g;
+        pp.bpm = 0;
+        for (size_t pos = 0; pos < g.ncomp; pos++) {
+            const Component &c = components[pos];
+            if (c.dc_pred != 0 || !dc_tables[c.dc_huff_table & 3].present || !ac_tables[c.ac_huff_table & 3].present) return false;
+            if (g.strip_len[pos] > 0x7FFFFFFFull || plane_len[pos] > ((size_t)1 << 40)) return false;
+            pp.bpm += c.horizontal_sample * c.vertical_sample;
+        }
+        pp.total = g.total;
+        if (pp.total == 0 || pp.bpm == 0 || pp.bpm > 6 || pp.total * pp.bpm > 0x7FFFFFFFull) return false;
+        if (restart_interval && pp.total > restart_interval) {
+            pp.n_seg = (pp.total + restart_interval - 1) / restart_interval;
+            std::vector<size_t> ends;
+            ends.reserve(pp.n_seg);
+            find_restart_markers(reader, reader.pos, pp.n_seg - 1, ends);
+            if (ends.size() < pp.n_seg - 1 || first_marker_after(reader, ends.back()) != 0xD9) return false;
+            pp.seg_start.resize(pp.n_seg + 1);
+            pp.seg_start[0] = (uint32_t)reader.pos;
+            for (size_t k = 1; k < pp.n_seg; k++) pp.seg_start[k] = (uint32_t)ends[k - 1];
+            pp.seg_start[pp.n_seg] = 0;
+            return true;
+        }
+        // no DRI, or a scan of a single interval (no RSTn to meet): the self-synchronising decode
+        if (!destuff_scan(reader, pp.bits) || pp.bits.empty()) return false;
+        pp.nbits = (uint64_t)pp.bits.size() * 8;
+        pp.bits.resize(((pp.bits.size() + 3) & ~(size_t)3) + 16, 0);
+        pp.n_sub = (size_t)((pp.nbits + zj::SYNC_BITS - 1) / zj::SYNC_BITS);
+        pp.n_seg = 1;
+        pp.seg_start.assign(2, 0);
+        pp.sync = true;
         return true;
     }
     void gpu_entropy_tables(zj::EntTable *t) const   // [dc, ac] per component
@@ -2174,6 +2269,8 @@ struct GpuSlot {
     std::vector<zj_batch *> batches;          // reconstruction launch plans whose kernels may still be running
     std::vector<size_t> take, idx;            // images of the sub-batch in stage 1 / images whose pixels are on their way
     std::vector<zj::EntImage> eimg;
+    std::vector<zj::SyncImage> simg;
+    std::vector<int16_t *> planes;            // 3 per image of the sub-batch: its device planes
     std::vector<uint8_t *> pix;
     std::vector<size_t> st_off;
     uint8_t *meta_host = nullptr, *st_host = nullptr;   // pinned: descriptors + tables + interval starts up, statuses down
@@ -2324,7 +2421,11 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
     std::vector<char> on_gpu(n, 0);
     auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
     auto footprint = [&](const Item &it, size_t len) {
-        size_t b = al(len + 8) + al(sizeof(zj::EntImage)) + al(6 * sizeof(zj::EntTable)) + al((it.pp.n_seg + 1) * 4) + al(it.pp.n_seg) + 1024 + (dev_out ? 0 : al(it.need));
+        size_t b = al(sizeof(zj::EntImage)) + al(6 * sizeof(zj::EntTable)) + al((it.pp.n_seg + 1) * 4) + al(it.pp.n_seg) + 1024 + (dev_out ? 0 : al(it.need));
+        if (!it.pp.sync) b += al(len + 8);
+        else   // de-stuffed bits, subsequence states (2 exits, entry, count) and DC differences
+            b += al(sizeof(zj::SyncImage)) + al(it.pp.bits.size()) + 3 * al(it.pp.n_sub * 8) + al(it.pp.n_sub * 4) +
+                 al(it.pp.total * it.pp.bpm * 2) + al(zj::SYNC_ROUNDS * 4);
         for (int z = 0; z < 3; z++) b += al(it.d->plane_len[z] * 2);
         return b;
     };
@@ -2396,12 +2497,21 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
         const std::vector<size_t> &take = sl.take;
         size_t off = 0;
         auto carve = [&](size_t nb) { uint8_t *p = sl.mem + off; off += al(nb); return p; };
-        // planes of the whole sub-batch first, contiguous: one memset
-        sl.eimg.assign(take.size(), zj::EntImage{});
+        // planes of the whole sub-batch first, contiguous, and the sync round counters behind them: one memset.  Images of the
+        // interval form get an EntImage, those of the self-synchronising form a SyncImage (slot[t] indexes its array)
+        size_t n_int = 0, n_sync = 0;
+        std::vector<size_t> slot_of(take.size());
+        for (size_t t = 0; t < take.size(); t++) slot_of[t] = items[take[t]].pp.sync ? n_sync++ : n_int++;
+        sl.eimg.assign(n_int, zj::EntImage{});
+        sl.simg.assign(n_sync, zj::SyncImage{});
+        std::vector<int16_t *> &planes = sl.planes;
+        planes.assign(3 * take.size(), nullptr);
         for (size_t t = 0; t < take.size(); t++) {
             const Item &it = items[take[t]];
-            for (int z = 0; z < 3; z++) sl.eimg[t].plane[z] = it.d->plane_len[z] ? (int16_t *)carve(it.d->plane_len[z] * 2) : nullptr;
+            for (int z = 0; z < 3; z++) planes[3 * t + z] = it.d->plane_len[z] ? (int16_t *)carve(it.d->plane_len[z] * 2) : nullptr;
         }
+        for (size_t t = 0; t < take.size(); t++)
+            if (items[take[t]].pp.sync) sl.simg[slot_of[t]].changed = (uint32_t *)carve(zj::SYNC_ROUNDS * 4);
         bool ok = cudaMemsetAsync(sl.mem, 0, off, sl.s) == cudaSuccess;
         lap("memset planes", sl.s);
         // descriptors, Huffman tables and interval starts of the sub-batch travel as ONE pinned block, the statuses come back as one
@@ -2409,22 +2519,57 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
         sl.st_off.assign(take.size(), 0);
         size_t st_total = 0, seg_words = 0;
         for (size_t t = 0; t < take.size(); t++) { sl.st_off[t] = st_total; st_total += items[take[t]].pp.n_seg; seg_words += items[take[t]].pp.n_seg + 1; }
-        const size_t off_tab = al(take.size() * sizeof(zj::EntImage)), off_seg = off_tab + al(6 * take.size() * sizeof(zj::EntTable));
+        const size_t off_sync = al(n_int * sizeof(zj::EntImage)), off_tab = off_sync + al(n_sync * sizeof(zj::SyncImage));
+        const size_t off_seg = off_tab + al(6 * take.size() * sizeof(zj::EntTable));
         const size_t meta_bytes = off_seg + al(seg_words * 4);
         ok = ok && pinned_grow(sl.meta_host, sl.meta_cap, meta_bytes) && pinned_grow(sl.st_host, sl.st_cap, st_total);
         uint8_t *d_meta = carve(meta_bytes), *d_status = carve(st_total);
-        uint32_t max_seg = 0;
+        uint32_t max_seg = 0, max_sub = 0;
         size_t seg_at = 0;
+        std::vector<std::pair<uint8_t *, size_t>> uploads;   // (device destination, image): the file, or its de-stuffed scan
         for (size_t t = 0; t < take.size() && ok; t++) {
             const size_t i = take[t];
             Item &it = items[i];
-            zj::EntImage &e = sl.eimg[t];
             const zj_decoder::BaselineGeom &g = it.pp.g;
-            uint8_t *d_data = carve(lens[i] + 8);
             it.d->gpu_entropy_tables(reinterpret_cast<zj::EntTable *>(sl.meta_host + off_tab) + 6 * t);
             memcpy(sl.meta_host + off_seg + seg_at * 4, it.pp.seg_start.data(), (it.pp.n_seg + 1) * 4);
             sl.pix[t] = dev_out ? out[i] : carve(it.need);
+            if (it.pp.sync) {
+                zj::SyncImage &e = sl.simg[slot_of[t]];
+                const size_t n_sub = it.pp.n_sub, blocks = it.pp.total * it.pp.bpm;
+                uint8_t *d_bits = carve(it.pp.bits.size());
+                uploads.emplace_back(d_bits, i);
+                e.bits = reinterpret_cast<const uint32_t *>(d_bits);
+                e.nbits = it.pp.nbits;
+                e.tables = reinterpret_cast<const zj::EntTable *>(d_meta + off_tab) + 6 * t;
+                for (int z = 0; z < 3; z++) e.plane[z] = planes[3 * t + z];
+                e.exit[0] = (uint64_t *)carve(n_sub * 8); e.exit[1] = (uint64_t *)carve(n_sub * 8);
+                e.used = (uint64_t *)carve(n_sub * 8);
+                e.count = (uint32_t *)carve(n_sub * 4);
+                e.dc = (int16_t *)carve(blocks * 2);
+                e.status = d_status + sl.st_off[t];
+                e.n_sub = (uint32_t)n_sub; e.total_mcus = (uint32_t)it.pp.total; e.bpm = (uint32_t)it.pp.bpm;
+                e.mcu_w = (uint32_t)g.mcu_w; e.bias = (uint32_t)g.bias; e.is_hv = g.is_hv ? 1u : 0u;
+                e.width_stride = (uint32_t)g.width_stride; e.hv_width_stride = (uint32_t)g.hv_width_stride;
+                uint32_t slot = 0;
+                for (int z = 0; z < 3; z++) {
+                    e.strip_len[z] = (uint32_t)g.strip_len[z];
+                    const bool have = (size_t)z < g.ncomp;
+                    e.h_samp[z] = have ? (uint32_t)it.d->components[z].horizontal_sample : 0u;
+                    e.v_samp[z] = have ? (uint32_t)it.d->components[z].vertical_sample : 0u;
+                    e.is_y[z] = have && it.d->components[z].component_id == ID_Y ? 1u : 0u;
+                    for (uint32_t v = 0; v < e.v_samp[z]; v++)
+                        for (uint32_t h = 0; h < e.h_samp[z]; h++, slot++) { e.slot_comp[slot] = (uint8_t)z; e.slot_v[slot] = (uint8_t)v; e.slot_h[slot] = (uint8_t)h; }
+                }
+                seg_at += it.pp.n_seg + 1;
+                max_sub = std::max(max_sub, e.n_sub);
+                continue;
+            }
+            zj::EntImage &e = sl.eimg[slot_of[t]];
+            uint8_t *d_data = carve(lens[i] + 8);
+            uploads.emplace_back(d_data, i);
             e.data = d_data; e.len = (uint32_t)lens[i];
+            for (int z = 0; z < 3; z++) e.plane[z] = planes[3 * t + z];
             e.seg_start = reinterpret_cast<const uint32_t *>(d_meta + off_seg) + seg_at;
             e.status = d_status + sl.st_off[t];
             e.tables = reinterpret_cast<const zj::EntTable *>(d_meta + off_tab) + 6 * t;
@@ -2442,14 +2587,44 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
             }
             max_seg = std::max(max_seg, e.n_seg);
         }
-        if (ok) memcpy(sl.meta_host, sl.eimg.data(), take.size() * sizeof(zj::EntImage));
+        if (ok) {
+            memcpy(sl.meta_host, sl.eimg.data(), n_int * sizeof(zj::EntImage));
+            memcpy(sl.meta_host + off_sync, sl.simg.data(), n_sync * sizeof(zj::SyncImage));
+        }
         ok = ok && off <= sl.cap && cudaMemcpyAsync(d_meta, sl.meta_host, meta_bytes, cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
-        // files + entropy kernel (behind the cleared planes and the descriptors), then the statuses come back
-        for (size_t t = 0; t < take.size() && ok; t++)
-            ok = cudaMemcpyAsync(const_cast<uint8_t *>(sl.eimg[t].data), bufs[take[t]], lens[take[t]], cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
-        ok = ok && zj::launch_entropy(reinterpret_cast<const zj::EntImage *>(d_meta), (uint32_t)take.size(), max_seg, sl.s) == 0;
+        // files (de-stuffed scans) + entropy kernels (behind the cleared planes and the descriptors), then the statuses come back
+        for (size_t u = 0; u < uploads.size() && ok; u++) {
+            const size_t i = uploads[u].second;
+            const bool sync = items[i].pp.sync;
+            ok = cudaMemcpyAsync(uploads[u].first, sync ? items[i].pp.bits.data() : bufs[i], sync ? items[i].pp.bits.size() : lens[i], cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
+        }
+        const bool spec = items[take[0]].d->spec();
+        ok = ok && zj::launch_entropy(reinterpret_cast<const zj::EntImage *>(d_meta), (uint32_t)n_int, max_seg, sl.s, spec) == 0;
+        lap("files + interval kernels", sl.s);
+        static const char *const phase_name[4] = {"sync rounds", "sync accept", "sync write", "sync DC"};
+        const zj::SyncImage *d_simg = reinterpret_cast<const zj::SyncImage *>(d_meta + off_sync);
+        for (int ph = 0; ph < 4; ph++) {
+            ok = ok && zj::launch_sync_phase(d_simg, (uint32_t)n_sync, max_sub, sl.s, ph) == 0;
+            if (n_sync) lap(phase_name[ph], sl.s);
+        }
+        if (trace && ok && n_sync) {   // rounds each image took to reach the fixpoint (SYNC_ROUNDS: not reached), and turn-downs
+            uint32_t rmax = 0, down = 0;
+            double rsum = 0;
+            for (size_t t = 0; t < take.size(); t++) {
+                if (!items[take[t]].pp.sync) continue;
+                uint32_t ch[zj::SYNC_ROUNDS];
+                uint8_t st = 1;
+                cudaMemcpy(ch, sl.simg[slot_of[t]].changed, sizeof(ch), cudaMemcpyDeviceToHost);
+                cudaMemcpy(&st, d_status + sl.st_off[t], 1, cudaMemcpyDeviceToHost);
+                uint32_t r = 1;
+                while (r < zj::SYNC_ROUNDS && ch[r] != 0) r++;
+                rmax = std::max(rmax, r);
+                rsum += r;
+                down += st != 0;
+            }
+            fprintf(stderr, "[zj_decode_batch_gpu] sync rounds: images %zu, max %u, mean %.2f, turned down %u\n", n_sync, rmax, rsum / n_sync, down);
+        }
         ok = ok && (st_total == 0 || cudaMemcpyAsync(sl.st_host, d_status, st_total, cudaMemcpyDeviceToHost, sl.s) == cudaSuccess);
-        lap("files + entropy kernels", sl.s);
         if (!ok) cudaGetLastError();
         sl.staged = ok;   // (not staged: nothing is published, these images go through the host path)
         return true;
@@ -2469,7 +2644,7 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
             for (size_t k = 0; k < it.pp.n_seg; k++) all = all && sl.st_host[sl.st_off[t] + k] == 0;
             if (!all) continue;
             zj_image di = it.img;
-            for (uint32_t z = 0; z < di.n_comp; z++) di.comp[z].coeff = sl.eimg[t].plane[z];
+            for (uint32_t z = 0; z < di.n_comp; z++) di.comp[z].coeff = sl.planes[3 * t + z];
             dimgs.push_back(di); douts.push_back(sl.pix[t]); dlens.push_back(it.need); who.push_back(i);
         }
         if (dimgs.empty()) return;

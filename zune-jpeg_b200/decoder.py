@@ -89,6 +89,7 @@ class ZuneJpegOptions:
         self._libjpeg_output = False
         self._scale_denom = 1
         self._exif_orientation = False
+        self._gpu_entropy = False
 
     @staticmethod
     def new() -> "ZuneJpegOptions":
@@ -143,6 +144,10 @@ class ZuneJpegOptions:
     # (ZJ_FLAG_ORIENT_*; sizes and rois are then those of the displayed image, oriented_size).  Needs spec or libjpeg output.
     def get_exif_orientation(self): return self._exif_orientation
     def set_exif_orientation(self, choice: bool): return self._with(_exif_orientation=bool(choice))
+    # not in the reference: lets decode_batch(gpu_entropy=True), device_out and decode_batch_resized entropy-decode spec and
+    # libjpeg output on the GPU, with or without restart markers (ZJ_USE_GPU_ENTROPY); same results.  Needs spec or libjpeg output.
+    def get_gpu_entropy(self): return self._gpu_entropy
+    def set_gpu_entropy(self, choice: bool): return self._with(_gpu_entropy=bool(choice))
 
     def _raw(self) -> ZjOptions:
         o = ZjOptions()
@@ -150,12 +155,16 @@ class ZuneJpegOptions:
             raise ValueError("a scale denominator above 1 needs libjpeg output (set_libjpeg_output(True))")
         if self._exif_orientation and not (self._libjpeg_output or self._spec_output):
             raise ValueError("EXIF orientation needs spec or libjpeg output (set_spec_output(True) or set_libjpeg_output(True))")
+        if self._gpu_entropy and not (self._libjpeg_output or self._spec_output):
+            raise ValueError("GPU entropy decoding of spec output needs spec or libjpeg output (set_spec_output(True) or set_libjpeg_output(True))")
         if self._libjpeg_output:
             o.use_unsafe = _ffi.USE_LIBJPEG_OUTPUT | (self._scale_denom.bit_length() - 1) << _ffi.USE_SCALE_SHIFT
         else:
             o.use_unsafe = _ffi.USE_SPEC_OUTPUT if self._spec_output else int(self._use_unsafe)
         if self._exif_orientation:
             o.use_unsafe |= _ffi.USE_EXIF_ORIENTATION
+        if self._gpu_entropy:
+            o.use_unsafe |= _ffi.USE_GPU_ENTROPY
         o.out_colorspace = int(self._out_colorspace)
         o.num_threads = self._num_threads
         o.max_width, o.max_height = self._max_width, self._max_height
@@ -383,7 +392,9 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
     """zj_decode_batch: JPEG byte strings in, pixel bytes out, `threads` host threads (0 = one per hardware thread)
     running the host stage of different images side by side while the GPU reconstructs the finished ones.
     `gpu_entropy=True` (zj_decode_batch_gpu): baseline JPEGs with restart markers are entropy-decoded on the GPU as well, one
-    restart interval per thread; same results, `stats["gpu_entropy"]` = how many images took that route.
+    restart interval per thread; same results, `stats["gpu_entropy"]` = how many images took that route.  With spec or libjpeg
+    output, `options.set_gpu_entropy(True)` lets this route (and `device_out`) take those images too, with or without restart
+    markers (self-synchronising decode); without it they take the host route.
     `device_out=[(device_ptr, nbytes), ...]` (zj_decode_batch_gpu_device): the pixels stay in device memory; with
     `desc=gpu.OutputDesc(...)` (zj_decode_batch_gpu_device_ex) in the layout / type / scale a GPU consumer wants.
     `devices=[0, 1, ...]` (zj_decode_batch_multi): the batch is cut into contiguous image ranges, one per device of the box
@@ -442,7 +453,8 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
     return res
 
 
-def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpegOptions | None = None, threads: int = 0):
+def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpegOptions | None = None, threads: int = 0,
+                         stats: dict | None = None):
     """zj_decode_batch_gpu_device_resized: JPEG byte strings in, one batch tensor in device memory out -- every image decoded
     whole, its crop resized to `resize` (a gpu.Resize) in the layout / type / normalisation of `desc` (a gpu.OutputDesc, scale
     must be full size; default HWC u8).  rois: None, or one (x, y, w, h) or None (= the whole image) per image, in the
@@ -451,7 +463,9 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
 
     Returns (gpu.DeviceArray of shape (N, C, OH, OW) or (N, OH, OW, C), [None | DecodeErrors per image]).  The errors are the
     ones decode_batch reports for the same inputs; a crop that does not fit its image, or an image whose channel count is not
-    the one the options' colourspace gives, fails with status ZJ_ERR_INVALID_ARG.  The slot of a failed image is not written."""
+    the one the options' colourspace gives, fails with status ZJ_ERR_INVALID_ARG.  The slot of a failed image is not written.
+    With spec or libjpeg output and `options.set_gpu_entropy(True)` the entropy stage of baseline images runs on the GPU too
+    (same results); `stats["gpu_entropy"]` = how many images took that route."""
     from . import gpu
     lib = _ffi.load()
     options = options if options is not None else ZuneJpegOptions()
@@ -482,5 +496,7 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
                                                 out.ptr, slot * n, status, C.byref(n_gpu))
     if rc < 0:
         raise DecodeErrors(13, lib.zj_gpu_strerror(rc).decode(), rc)
+    if stats is not None:
+        stats["gpu_entropy"] = int(n_gpu.value)
     errs = [_image_error(lib, i, status[i]) if status[i] != 0 else None for i in range(n)]
     return gpu.DeviceArray(out, (n, *resize.slot_shape(desc, nc)), desc.c.dtype), errs
