@@ -171,6 +171,11 @@ enum { ZJ_USE_EXIF_ORIENTATION = 0x100 };
  * GPU (see zj_decode_batch_gpu).  Every other entry point decodes exactly as without the bit; every value without it keeps its
  * meaning. */
 enum { ZJ_USE_GPU_ENTROPY = 0x200 };
+/* GPU entropy decoding of progressive spec and libjpeg output (opt-in).  ZJ_USE_GPU_PROGRESSIVE is valid only together with
+ * ZJ_USE_GPU_ENTROPY and a spec, libjpeg or scaled value (with or without ZJ_USE_EXIF_ORIENTATION); it lets the
+ * zj_decode_batch_gpu* front doors entropy-decode progressive images of these modes on the GPU as well (see
+ * zj_decode_batch_gpu, DESIGN.md section 5.6).  Every other entry point decodes exactly as without it. */
+enum { ZJ_USE_GPU_PROGRESSIVE = 0x400 };
 
 typedef enum zj_status {
     ZJ_OK = 0,
@@ -415,7 +420,8 @@ typedef struct zj_options {       /* ZuneJpegOptions (src/options.rs:6-40), same
                                      ZJ_USE_LIBJPEG_OUTPUT: the same, and the images carry ZJ_FLAG_ISLOW;
                                      ZJ_USE_LIBJPEG_OUTPUT | k << 4, k = 1..3: the same, decoded at 1/2^k (ZJ_FLAG_SCALE_*);
                                      any of these three | ZJ_USE_EXIF_ORIENTATION: the same, oriented (ZJ_FLAG_ORIENT_*);
-                                     | ZJ_USE_GPU_ENTROPY: the same, and zj_decode_batch_gpu* may entropy-decode on the GPU */
+                                     | ZJ_USE_GPU_ENTROPY: the same, and zj_decode_batch_gpu* may entropy-decode on the GPU;
+                                     | ZJ_USE_GPU_ENTROPY | ZJ_USE_GPU_PROGRESSIVE: progressive images too */
     uint32_t out_colorspace;      /* ZJ_CS_RGB                                           */
     uint32_t num_threads;         /* 4                                                   */
     uint32_t max_width;           /* 16384                                               */
@@ -579,7 +585,15 @@ ZJ_API void zj_release_device_caches(void);
  * self-synchronising decode (DESIGN.md section 5.5).  That decode turns the image down -- it takes the host route -- when a
  * code is invalid, a non-zero coefficient lands past index 63, a symbol needs bits beyond the scan's data, fewer blocks than
  * the frame holds are decoded, a block falls outside its strip, or the subsequences do not settle within the sync rounds.
- * Scaled and oriented images take these forms too. */
+ * Scaled and oriented images take these forms too.
+ * Progressive form (| ZJ_USE_GPU_PROGRESSIVE as well): a progressive frame of one or three components with factors the fused
+ * kernels take, without DRI, whose scans are followed by DHT, SOS or EOI only, that ends with EOI within max_scans scans, whose
+ * every scan passes the host stage's checks, whose first scan is a first scan (not a refinement), and whose scan script puts
+ * every first scan of a component before that component's refinements of the same kind (DC / AC) and gives its first scans
+ * disjoint coefficients.  Every scan is de-stuffed and decoded into the host stage's progressive planes (DESIGN.md section
+ * 5.6).  Turned down, besides the causes above, are a refinement symbol with a magnitude other than 1, a zero run past the
+ * band of a refinement scan, a non-zero coefficient past the band of a first scan, a DC refinement scan with fewer bits than
+ * blocks, and a first scan whose bit reader would not have met the marker behind it. */
 ZJ_API int zj_decode_batch_gpu(const zj_options *o, const uint8_t *const *bufs, const size_t *lens, size_t n,
                                uint8_t **out, size_t *out_len, int *status, size_t *n_gpu_entropy);
 /* ... and with the pixels left in device memory (no PCIe download at all: what is uploaded is the JPEG file): out_dev[i] is a

@@ -29,6 +29,7 @@ def scaled_size(width: int, height: int, denom: int):
 FLAG_ORIENT_SHIFT, FLAG_ORIENT_MASK = 4, 7 << 4   # zj_image.flags bits 4-6: EXIF orientation o - 1 (spec images only)
 USE_EXIF_ORIENTATION = 0x100   # ORed into a spec / libjpeg / scaled zj_options.use_unsafe value: the output is oriented
 USE_GPU_ENTROPY = 0x200        # ORed into a spec / libjpeg / scaled value: zj_decode_batch_gpu* may entropy-decode on the GPU
+USE_GPU_PROGRESSIVE = 0x400    # ... next to USE_GPU_ENTROPY: progressive images too
 
 
 def oriented_size(width: int, height: int, orientation: int):

@@ -583,4 +583,474 @@ int launch_sync_phase(const SyncImage *d_images, uint32_t n_images, uint32_t max
     return (int)cudaGetLastError();
 }
 
+// ================================================================ progressive scans (spec and libjpeg output)
+// DESIGN.md section 5.6.  Reads are bounded as in the baseline decode: a decode stops once a read ends beyond nbits and loads at
+// most one word past (pos + 32) / 32 <= nbits / 32 + 1, inside the >= 8 zero bytes behind the scan.  Stores go to blocks
+// whose addressing check passed (prog_block), at zig-zag positions <= se <= 63, from verified states only: first scans store in
+// their write pass once the accept kernel set `ok`, refinements store as they go and turn the image down on any error, so
+// whatever they stored is never used.
+
+// the host stage's block of scan block g (mcu_prog.rs:304 / :408 address rules), nullptr when that check fails
+__device__ __forceinline__ int16_t *prog_block(const ProgScan &sc, u32 g)
+{
+    u32 z, x, y;
+    if (sc.nslot > 1) {
+        const u32 m = g / sc.nslot, s = g - m * sc.nslot, i = m / sc.mcu_x, j = m - i * sc.mcu_x;
+        z = sc.slot_z[s];
+        x = j * sc.hs[z] + sc.slot_h[s];
+        y = i * sc.vs[z] + sc.slot_v[s];
+    } else {
+        z = sc.slot_z[0];
+        y = g / sc.mw;
+        x = g - y * sc.mw;
+    }
+    const u64 at = 64ull * ((u64)y * sc.bw[z] + x);
+    if (at + 64 > sc.plane_len[z]) return nullptr;
+    return sc.plane[z] + at;
+}
+
+// One symbol at a time of a first scan (DC first: decode_prog_dc_first, AC first: decode_mcu_ac_first with the host loop's
+// EOB-run skip), from state (pos, slot, coef) over the symbols that start below `end`, as sync_decode does.  An EOB symbol
+// completes its block and EOBRUN - 1 more.  SYNC_INVALID additionally on a non-zero coefficient past se.
+// WRITE: stores DC differences / AC values (value << al) of blocks below total and stops there; *last = the start of the
+// symbol that reached total; ok = false on a failed addressing check.
+template <bool WRITE>
+__device__ u64 prog_decode(const ProgScan &sc, const EntTable *T, const uint8_t *Z, u64 pos, u32 slot, u32 coef, u64 end,
+                           u32 &blocks, u32 g0, bool &ok, u64 *last)
+{
+    blocks = 0;
+    if (pos >= end) return sync_state(pos, slot, coef);
+    SyncBits b;
+    b.init(sc.bits, pos);
+    const bool dc = sc.kind == PROG_DC_FIRST;
+    const u32 ss = sc.ss, se = sc.se, al = sc.al;
+    int16_t *blk = nullptr;
+    if (WRITE) {
+        if (g0 >= sc.total) return sync_state(pos, slot, coef);
+        blk = prog_block(sc, g0);
+        if (!blk) { ok = false; return sync_state(pos, slot, coef); }
+    }
+    while (b.pos < end) {
+        const u64 start = b.pos;
+        b.refill();
+        u32 done = 0;
+        if (dc) {
+            const EntTable &t = T[sc.slot_t[slot]];
+            const int s = sync_huff(b, t, t.lookup[b.peek(9)]);
+            if (s < 0) return SYNC_INVALID;
+            int v = 0;
+            if (s != 0) v = huff_extend(b.get((u32)s), s);
+            if (WRITE) sc.dc[g0 + blocks] = (int16_t)v;
+            done = 1;
+        } else {
+            const EntTable &t = T[0];
+            const int fast_ac = (int)t.ac_lookup[b.peek(9)];
+            if (fast_ac != 0) {   // (progressive tables: only entries with a value)
+                coef += (u32)((fast_ac >> 4) & 63);
+                if (coef > se) return SYNC_INVALID;
+                if (WRITE) blk[Z[coef] & 63] = (int16_t)((u32)(fast_ac >> 10) << al);
+                b.drop((u32)(fast_ac & 15));
+                coef += 1;
+            } else {
+                int s = sync_huff(b, t, t.lookup[b.peek(9)]);
+                if (s < 0) return SYNC_INVALID;
+                const u32 rr = (u32)s >> 4;
+                s &= 15;
+                if (s != 0) {
+                    coef += rr;
+                    if (coef > se) return SYNC_INVALID;
+                    const int v = huff_extend(b.get((u32)s), s);
+                    if (WRITE) blk[Z[coef] & 63] = (int16_t)((u32)v << al);
+                    coef += 1;
+                } else if (rr != 15) {
+                    done = (1u << rr) + (rr ? (u32)b.get(rr) : 0u);   // EOBRUN blocks, this one included
+                } else {
+                    coef += 16;
+                }
+            }
+            if (done == 0 && coef > se) done = 1;
+        }
+        if (b.pos > sc.nbits) return SYNC_INVALID;
+        if (done) {
+            blocks += done;
+            coef = dc ? 0 : ss;
+            slot = dc && slot + 1 < sc.nslot ? slot + 1 : 0;
+            if (WRITE) {
+                if (g0 + blocks >= sc.total) { *last = start; break; }
+                blk = prog_block(sc, g0 + blocks);
+                if (!blk) { ok = false; break; }
+            }
+        }
+    }
+    return sync_state(b.pos, slot, coef);
+}
+
+__device__ __forceinline__ void prog_tables(const ProgScan &sc, EntTable *sT, uint8_t *sZ, u32 nthreads)
+{
+    const u32 words = (u32)(sizeof(EntTable) / 4) * (sc.kind == PROG_DC_FIRST ? (u32)sc.slot_t[sc.nslot - 1] + 1 : 1u);
+    const u32 *src = reinterpret_cast<const u32 *>(sc.tables);
+    u32 *dst = reinterpret_cast<u32 *>(sT);
+    for (u32 i = threadIdx.x; i < words; i += nthreads) dst[i] = src[i];
+    for (u32 i = threadIdx.x; i < 80; i += nthreads) sZ[i] = c_unzigzag[i];
+    __syncthreads();
+}
+
+__device__ __forceinline__ u64 prog_end(const ProgScan &sc, u32 k) { return k + 1 == sc.n_sub ? sc.nbits : (u64)(k + 1) * SYNC_BITS; }
+__device__ __forceinline__ u32 prog_coef0(const ProgScan &sc) { return sc.kind == PROG_DC_FIRST ? 0u : sc.ss; }
+
+// sync_round_kernel over first scans: blockIdx.y = scan; the guess of subsequence k is (k * SYNC_BITS, slot 0, first coefficient)
+__global__ void __launch_bounds__(SYNC_THREADS) prog_round_kernel(const ProgScan *__restrict__ scans, u32 r)
+{
+    __shared__ EntTable sT[3];
+    __shared__ uint8_t sZ[80];
+    const ProgScan &sc = scans[blockIdx.y];
+    if (blockIdx.x * SYNC_THREADS >= sc.n_sub) return;
+    if (r >= 2 && sc.changed[r - 1] == 0) return;
+    prog_tables(sc, sT, sZ, SYNC_THREADS);
+    const u32 k = blockIdx.x * SYNC_THREADS + threadIdx.x;
+    if (k >= sc.n_sub) return;
+    u64 entry = sync_state((u64)k * SYNC_BITS, 0, prog_coef0(sc));
+    if (k > 0 && r > 0) {
+        const u64 e = sc.exit[(r - 1) & 1][k - 1];
+        if (e != SYNC_INVALID) entry = e;
+    }
+    if (r > 0 && entry == sc.used[k]) { sc.exit[r & 1][k] = sc.exit[(r - 1) & 1][k]; return; }
+    sc.used[k] = entry;
+    u32 blocks;
+    bool ok = true;
+    sc.exit[r & 1][k] = prog_decode<false>(sc, sT, sZ, entry >> 16, (u32)(entry >> 8) & 255, (u32)entry & 255, prog_end(sc, k), blocks, 0, ok, nullptr);
+    sc.count[k] = blocks;
+    atomicAdd(&sc.changed[r], 1u);
+}
+
+// accept_kernel over first scans (one CTA per scan): ok = settled and total blocks reached before the first error
+__global__ void __launch_bounds__(1024) prog_accept_kernel(const ProgScan *__restrict__ scans)
+{
+    __shared__ u32 s_sum[1024];
+    __shared__ u32 s_err;
+    const ProgScan &sc = scans[blockIdx.x];
+    bool settled = false;
+    for (u32 r = 1; r < PROG_ROUNDS; r++) settled = settled || sc.changed[r] == 0;
+    if (!settled) { if (threadIdx.x == 0) { *sc.ok = 0; *sc.status |= PROG_DOWN_FIRST; } return; }
+    if (threadIdx.x == 0) s_err = 0xFFFFFFFFu;
+    // (EOB runs let counts grow past any bound: sums saturate at total, an associative operation, so every base below the
+    // total is exact and the others say "at or past the total")
+    const u32 n = sc.n_sub, per = (n + 1023) / 1024, total = sc.total;
+    const u32 k0 = min(n, threadIdx.x * per), k1 = min(n, k0 + per);
+    u32 sum = 0;
+    for (u32 k = k0; k < k1; k++) sum = min(total, sum + min(total, sc.count[k]));
+    s_sum[threadIdx.x] = sum;
+    __syncthreads();
+    for (u32 d = 1; d < 1024; d <<= 1) {
+        const u32 v = threadIdx.x >= d ? s_sum[threadIdx.x - d] : 0u;
+        __syncthreads();
+        s_sum[threadIdx.x] = min(total, s_sum[threadIdx.x] + v);
+        __syncthreads();
+    }
+    u32 base = threadIdx.x ? s_sum[threadIdx.x - 1] : 0u;
+    for (u32 k = k0; k < k1; k++) {
+        const u32 c = min(total, sc.count[k]);
+        sc.count[k] = base;
+        if (sc.exit[0][k] == SYNC_INVALID) atomicMin(&s_err, k);
+        base = min(total, base + c);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const u64 reached = s_err != 0xFFFFFFFFu ? (s_err + 1 < n ? (u64)sc.count[s_err + 1] : (u64)s_sum[1023]) : (u64)s_sum[1023];
+        const bool ok = reached >= sc.total;
+        *sc.ok = ok ? 1 : 0;
+        if (!ok) *sc.status |= PROG_DOWN_FIRST;
+    }
+}
+
+// write_kernel over first scans; the thread that reaches the last block checks the file's first scan for the marker rule
+__global__ void __launch_bounds__(SYNC_THREADS) prog_write_kernel(const ProgScan *__restrict__ scans)
+{
+    __shared__ EntTable sT[3];
+    __shared__ uint8_t sZ[80];
+    __shared__ uint8_t s_ok;
+    const ProgScan &sc = scans[blockIdx.y];
+    if (blockIdx.x * SYNC_THREADS >= sc.n_sub) return;
+    if (threadIdx.x == 0) s_ok = *sc.ok;
+    prog_tables(sc, sT, sZ, SYNC_THREADS);
+    if (s_ok == 0) return;
+    const u32 k = blockIdx.x * SYNC_THREADS + threadIdx.x;
+    if (k >= sc.n_sub) return;
+    const u32 g0 = sc.count[k];
+    if (g0 >= sc.total) return;
+    const u64 entry = k == 0 ? sync_state(0, 0, prog_coef0(sc)) : sc.exit[0][k - 1];
+    if (entry == SYNC_INVALID) return;   // (not reached: subsequences behind an error start at or past block total)
+    u32 blocks;
+    bool ok = true;
+    u64 last = ~0ull;
+    prog_decode<true>(sc, sT, sZ, entry >> 16, (u32)(entry >> 8) & 255, (u32)entry & 255, prog_end(sc, k), blocks, g0, ok, &last);
+    if (!ok) *sc.status |= PROG_DOWN_ADDRESS;
+    if (sc.marker_check && last != ~0ull) {
+        // decode_progressive wants the marker behind the first scan met by its bit reader (has_marker): the reader fetches 32
+        // bits when <= 32 are buffered, before every symbol, so at the last symbol (start c) it has fetched 32 bits (c = 0) or
+        // the least multiple of 32 >= c + 33 -- and it met the marker when that is more than the scan holds
+        const u64 fetched = last == 0 ? 32 : (last + 33 + 31) / 32 * 32;
+        if (fetched <= sc.nbits) *sc.status |= PROG_DOWN_MARKER;
+    }
+}
+
+// dc_kernel over DC first scans: the predictor of each scan component, a wrapping 32-bit prefix sum in block order, stored
+// as decode_prog_dc_first stores it, (int16)((uint16)pred << al)
+__global__ void __launch_bounds__(1024) prog_dc_kernel(const ProgScan *__restrict__ scans)
+{
+    __shared__ u32 s_sum[3][1024];
+    const ProgScan &sc = scans[blockIdx.x];
+    if (sc.kind != PROG_DC_FIRST || *sc.ok == 0) return;
+    const u32 bpm = sc.nslot, mcus = sc.total / bpm, per = (mcus + 1023) / 1024;
+    const u32 m0 = min(mcus, threadIdx.x * per), m1 = min(mcus, m0 + per);
+    u32 sum[3] = {0, 0, 0};
+    for (u32 m = m0; m < m1; m++)
+        for (u32 s = 0; s < bpm; s++) {
+            const u32 c = sc.slot_t[s], d = (u32)(int)sc.dc[m * bpm + s];
+            sum[0] += c == 0 ? d : 0u; sum[1] += c == 1 ? d : 0u; sum[2] += c == 2 ? d : 0u;
+        }
+    for (int c = 0; c < 3; c++) s_sum[c][threadIdx.x] = sum[c];
+    __syncthreads();
+    for (u32 d = 1; d < 1024; d <<= 1) {
+        u32 v[3];
+        for (int c = 0; c < 3; c++) v[c] = threadIdx.x >= d ? s_sum[c][threadIdx.x - d] : 0u;
+        __syncthreads();
+        for (int c = 0; c < 3; c++) s_sum[c][threadIdx.x] += v[c];
+        __syncthreads();
+    }
+    u32 pred[3];
+    for (int c = 0; c < 3; c++) pred[c] = s_sum[c][threadIdx.x] - sum[c];
+    for (u32 m = m0; m < m1; m++)
+        for (u32 s = 0; s < bpm; s++) {
+            const u32 c = sc.slot_t[s];
+            u32 p = (c == 0 ? pred[0] : (c == 1 ? pred[1] : pred[2])) + (u32)(int)sc.dc[m * bpm + s];
+            if (c == 0) pred[0] = p; else if (c == 1) pred[1] = p; else pred[2] = p;
+            int16_t *blk = prog_block(sc, m * bpm + s);   // (checked by the write kernel: every block below the total was visited)
+            if (blk) blk[0] = (int16_t)(p << sc.al);
+        }
+}
+
+// DC refinement (decode_prog_dc_refine): bit g of the scan belongs to block g; blockIdx.y = scan of the launch's ordinal, so
+// no two threads of a launch touch one coefficient
+__global__ void __launch_bounds__(256) prog_dc_refine_kernel(const ProgScan *__restrict__ scans)
+{
+    const ProgScan &sc = scans[blockIdx.y];
+    const u32 g = blockIdx.x * 256 + threadIdx.x;
+    if (g == 0 && sc.nbits < sc.total) *sc.status |= PROG_DOWN_DC_REFINE;
+    if (g >= sc.total || (u64)g >= sc.nbits) return;
+    if (((__ldg(sc.bits + (g >> 5)) >> ((g & 24) + (7 - (g & 7)))) & 1u) == 0) return;   // (bytes in file order, MSB first)
+    int16_t *blk = prog_block(sc, g);
+    if (!blk) { *sc.status |= PROG_DOWN_ADDRESS; return; }
+    blk[0] = (int16_t)((uint16_t)blk[0] + (uint16_t)(1u << sc.al));
+}
+
+// Per block of an AC refinement chain's component: bit k set when the coefficient at zig-zag position k is non-zero
+__global__ void __launch_bounds__(256) prog_mask_kernel(const ProgScan *__restrict__ scans, const ProgChain *__restrict__ chains)
+{
+    __shared__ uint8_t sZ[64];
+    const ProgScan &sc = scans[chains[blockIdx.y].first];
+    const u32 z = sc.slot_z[0], n = sc.plane_len[z] / 64;
+    if (threadIdx.x < 64) sZ[threadIdx.x] = c_unzigzag[threadIdx.x];
+    __syncthreads();
+    const u32 b = blockIdx.x * 256 + threadIdx.x;
+    if (b >= n) return;
+    const int16_t *blk = sc.plane[z] + (u64)b * 64;
+    u64 m = 0;
+    for (u32 k = 0; k < 64; k++) m |= (u64)(blk[sZ[k]] != 0) << k;
+    sc.mask[b] = m;
+}
+
+// the correction bits of the non-zero coefficients in `nz` (zig-zag bit mask), one bit each in zig-zag order: the mask of those
+// whose bit is 1
+__device__ __forceinline__ u64 prog_corrections(SyncBits &b, u64 nz)
+{
+    u64 out = 0;
+    while (nz) {
+        const u32 c = min((u32)__popcll(nz), 32u);
+        b.refill();
+        const u32 v = (u32)b.get(c);
+        for (u32 q = 0; q < c; q++) {
+            const u32 k = (u32)__ffsll((long long)nz) - 1;
+            nz &= nz - 1;
+            if ((v >> (c - 1 - q)) & 1u) out |= 1ull << k;
+        }
+    }
+    return out;
+}
+
+__device__ __forceinline__ u64 prog_from(u32 k) { return k >= 64 ? 0ull : ~0ull << k; }
+
+// One AC refinement scan: decode_mcu_ac_refine with the host's eob_run bookkeeping.  Its symbols and bit counts depend only on
+// the bits and on which coefficients are non-zero, so the walk reads the masks and records per block what the host stage would
+// change; prog_apply_kernel changes it.  (A coefficient the scan places is never visited again by the same scan, so corrections
+// only touch coefficients that were non-zero before it.)  All 32 lanes run the walk in step; blocks that start inside an EOB
+// run read one correction bit per non-zero coefficient of the band and nothing else, so the warp takes 32 of them at a time:
+// a prefix sum of their bit counts gives each lane where its bits start.  Lane 0 stores what the serial part records.
+// False when the image must be turned down: a code no table holds, a symbol with s != 1, a zero run past the band end, a read
+// beyond the data or a failed addressing check.  (A lane reads at most 12 bytes past the data: inside the image's buffer.)
+__device__ bool prog_refine_scan(const ProgScan &scan, const EntTable &T)
+{
+    const u32 lane = threadIdx.x & 31;
+    const u32 z = scan.slot_z[0], ss = scan.ss, se = scan.se, mw = scan.mw, total = scan.total, bw = scan.bw[z];
+    const u64 plane_len = scan.plane_len[z], nbits = scan.nbits;
+    uint64_t *const mask = scan.mask, *const rec = scan.rec;
+    const uint32_t *const words = scan.bits;
+    const u64 band = prog_from(ss) & (~0ull >> (63 - se));
+    SyncBits b;
+    b.init(words, 0);
+    u32 eob = 0;
+    for (u32 g = 0; g < total;) {
+        if (eob > 0) {   // ---- up to 32 blocks inside the run, one per lane
+            const u32 n = min(min(eob, 32u), total - g), gl = g + lane;
+            const u32 i = gl / mw, j = gl - (gl / mw) * mw;
+            const u64 at = 64ull * ((u64)i * bw + j);
+            const bool mine = lane < n;
+            if (__any_sync(~0u, mine && at + 64 > plane_len)) return false;
+            const u64 m = mine ? mask[at >> 6] : 0ull;
+            const u64 nz = (m >> 1) ? m & band : 0ull;
+            const u32 c = (u32)__popcll(nz);
+            u32 incl = c;
+            for (u32 d = 1; d < 32; d <<= 1) { const u32 v = __shfl_up_sync(~0u, incl, d); if (lane >= d) incl += v; }
+            const u32 sum = __shfl_sync(~0u, incl, 31);
+            const u64 p0 = b.pos + incl - c;
+            if (b.pos + sum > nbits) return false;
+            if (mine) {
+                u64 corr = 0;
+                if (c) {
+                    const u32 w = (u32)(p0 >> 5), off = (u32)(p0 & 31);
+                    const u64 hi = ((u64)b.word(w) << 32) | b.word(w + 1);
+                    const u64 win = off ? (hi << off) | (b.word(w + 2) >> (32 - off)) : hi;   // the 64 bits from p0
+                    u64 left = nz;
+                    for (u32 q = 0; left; q++, left &= left - 1)
+                        if ((win >> (63 - q)) & 1) corr |= left & (~left + 1);
+                }
+                uint64_t *r = rec + 3 * (at >> 6);
+                r[0] = corr; r[1] = 0; r[2] = 0;
+            }
+            b.init(words, b.pos + sum);
+            eob -= n;
+            g += n;
+            continue;
+        }
+        // ---- a block that starts with a symbol (the same on every lane)
+        const u32 i = g / mw, j = g - i * mw;
+        const u64 at = 64ull * ((u64)i * bw + j);
+        if (at + 64 > plane_len) return false;
+        u64 m = mask[at >> 6];
+        const u64 m0 = m;
+        u64 corr = 0, placed = 0, neg = 0;
+        u32 k = ss;
+        for (;;) {
+            b.refill();
+            int s = sync_huff(b, T, T.lookup[b.peek(9)]);
+            if (s < 0) return false;
+            const u32 rr = (u32)s >> 4;
+            s &= 15;
+            if (s == 0 && rr != 15) {
+                eob = (1u << rr) + (rr ? (u32)b.get(rr) : 0u);
+                break;
+            }
+            bool minus = false;
+            if (s != 0) {
+                if (s != 1) return false;
+                minus = b.get(1) == 0;
+            }
+            // the (rr + 1)-th zero coefficient at or after k: the corrections of the non-zero ones before it come first
+            u64 zeros = ~m & band & prog_from(k);
+            if ((u32)__popcll(zeros) <= rr) return false;
+            for (u32 q = 0; q < rr; q++) zeros &= zeros - 1;
+            const u32 pz = (u32)__ffsll((long long)zeros) - 1;
+            corr |= prog_corrections(b, m & prog_from(k) & ((1ull << pz) - 1));
+            if (b.pos > nbits) return false;
+            if (s != 0) { placed |= 1ull << pz; neg |= (u64)minus << pz; m |= 1ull << pz; }
+            k = pz + 1;
+            if (k > se) break;
+        }
+        if (b.pos > nbits) return false;
+        if (eob > 0) {
+            if (m >> 1) corr |= prog_corrections(b, m & band & prog_from(k));
+            if (b.pos > nbits) return false;
+            eob--;
+        }
+        if (lane == 0) {
+            uint64_t *r = rec + 3 * (at >> 6);
+            r[0] = corr; r[1] = placed; r[2] = neg;
+            if (m != m0) mask[at >> 6] = m;
+        }
+        __syncwarp();
+        g++;
+    }
+    return true;
+}
+
+// One warp per (image, component): its AC refinement scans in file order
+__global__ void __launch_bounds__(32) prog_refine_kernel(const ProgScan *__restrict__ scans, const ProgChain *__restrict__ chains)
+{
+    __shared__ EntTable sT;
+    __shared__ uint8_t sZ[80];
+    const ProgChain ch = chains[blockIdx.x];
+    for (u32 q = 0; q < ch.count; q++) {
+        const ProgScan &sc = scans[ch.first + q];
+        __syncthreads();
+        prog_tables(sc, &sT, sZ, 32);
+        if (!prog_refine_scan(sc, sT)) {
+            if (threadIdx.x == 0) *sc.status |= PROG_DOWN_AC_REFINE;
+            return;
+        }
+    }
+}
+
+// The records of a chain's scans applied to its planes in scan order, one thread per block: a correction adds 2^al away from
+// zero when that bit is clear (decode_mcu_ac_refine), a placed coefficient becomes +-2^al
+__global__ void __launch_bounds__(256) prog_apply_kernel(const ProgScan *__restrict__ scans, const ProgChain *__restrict__ chains)
+{
+    __shared__ uint8_t sZ[64];
+    const ProgChain ch = chains[blockIdx.y];
+    const ProgScan &s0 = scans[ch.first];
+    const u32 z = s0.slot_z[0], n = s0.plane_len[z] / 64;
+    if (threadIdx.x < 64) sZ[threadIdx.x] = c_unzigzag[threadIdx.x];
+    __syncthreads();
+    const u32 bl = blockIdx.x * 256 + threadIdx.x;
+    if (bl >= n || *s0.status != 0) return;
+    const u32 y = bl / s0.bw[z], x = bl - y * s0.bw[z];
+    int16_t *blk = s0.plane[z] + (u64)bl * 64;
+    for (u32 q = 0; q < ch.count; q++) {
+        const ProgScan &sc = scans[ch.first + q];
+        if (x >= sc.mw || (u64)y * sc.mw + x >= sc.total) continue;   // not a block of the scan
+        const uint64_t *r = sc.rec + 3 * (u64)bl;
+        const int p1 = 1 << sc.al;
+        for (u64 c = r[0]; c; c &= c - 1) {
+            int16_t &v = blk[sZ[__ffsll((long long)c) - 1] & 63];
+            if ((v & p1) == 0) v = (int16_t)(v >= 0 ? v + p1 : v - p1);
+        }
+        const u64 neg = r[2];
+        for (u64 c = r[1]; c; c &= c - 1) {
+            const u32 k = (u32)__ffsll((long long)c) - 1;
+            blk[sZ[k] & 63] = (int16_t)((neg >> k) & 1 ? -p1 : p1);
+        }
+    }
+}
+
+int launch_prog_phase(const ProgScan *d_scans, uint32_t n_first, uint32_t max_sub, const uint32_t *dc_ref, uint32_t n_dc_ord,
+                      uint32_t max_dc_blocks, const ProgChain *d_chains, uint32_t n_chain, uint32_t max_blocks, void *stream, int phase)
+{
+    cudaStream_t s = (cudaStream_t)stream;
+    const dim3 grid((max_sub + SYNC_THREADS - 1) / SYNC_THREADS, n_first);
+    if (phase <= PROG_PHASE_DC && (n_first == 0 || max_sub == 0)) return 0;
+    if (phase == PROG_PHASE_ROUNDS)
+        for (u32 r = 0; r < PROG_ROUNDS; r++) prog_round_kernel<<<grid, SYNC_THREADS, 0, s>>>(d_scans, r);
+    else if (phase == PROG_PHASE_ACCEPT) prog_accept_kernel<<<n_first, 1024, 0, s>>>(d_scans);
+    else if (phase == PROG_PHASE_WRITE) prog_write_kernel<<<grid, SYNC_THREADS, 0, s>>>(d_scans);
+    else if (phase == PROG_PHASE_DC) prog_dc_kernel<<<n_first, 1024, 0, s>>>(d_scans);
+    else if (phase == PROG_PHASE_DC_REFINE) {
+        for (u32 r = 0; r < n_dc_ord && max_dc_blocks; r++)
+            prog_dc_refine_kernel<<<dim3((max_dc_blocks + 255) / 256, dc_ref[r + 1] - dc_ref[r]), 256, 0, s>>>(d_scans + dc_ref[r]);
+    } else if (phase == PROG_PHASE_MASK) {
+        if (n_chain && max_blocks) prog_mask_kernel<<<dim3((max_blocks + 255) / 256, n_chain), 256, 0, s>>>(d_scans, d_chains);
+    } else if (phase == PROG_PHASE_AC_REFINE) {
+        if (n_chain) prog_refine_kernel<<<n_chain, 32, 0, s>>>(d_scans, d_chains);
+    } else if (n_chain && max_blocks) prog_apply_kernel<<<dim3((max_blocks + 255) / 256, n_chain), 256, 0, s>>>(d_scans, d_chains);
+    return (int)cudaGetLastError();
+}
+
 }  // namespace zj

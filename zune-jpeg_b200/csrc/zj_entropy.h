@@ -77,4 +77,50 @@ struct SyncImage {
 enum { SYNC_PHASE_ROUNDS = 0, SYNC_PHASE_ACCEPT = 1, SYNC_PHASE_WRITE = 2, SYNC_PHASE_DC = 3 };
 int launch_sync_phase(const SyncImage *d_images, uint32_t n_images, uint32_t max_sub, void *stream, int phase);
 
+// ---- progressive scans, spec and libjpeg output only (zj_entropy.cu, DESIGN.md section 5.6)
+// Every scan of the image is decoded from its own de-stuffed bits into the zeroed whole-image planes of the host stage's
+// progressive loops (mcu_prog.rs).  Phases, each over all scans of its kind in the sub-batch: (1) first scans (DC first, AC
+// first), self-synchronising like the baseline decode; (2) DC refinements, one bit per block; (3) AC refinements, one thread per
+// (image, component) walking that component's refinement scans in file order over non-zero masks, recording per block what
+// changes, then applied to the planes one thread per block.  The host stage only hands over files whose scan
+// script allows this order (every first scan of a component before its refinements of the same kind, first scans of a
+// component on disjoint coefficients).
+// sync rounds launched for first scans (a round after the fixpoint returns at once): their EOB runs let a wrong guess stay
+// consistent for longer than a baseline scan does, and files needing more than SYNC_ROUNDS were found
+constexpr uint32_t PROG_ROUNDS = 64;
+enum { PROG_DC_FIRST = 0, PROG_DC_REFINE = 1, PROG_AC_FIRST = 2, PROG_AC_REFINE = 3 };
+enum { PROG_DOWN_FIRST = 1, PROG_DOWN_ADDRESS = 2, PROG_DOWN_MARKER = 4, PROG_DOWN_DC_REFINE = 8, PROG_DOWN_AC_REFINE = 16 };
+struct ProgScan {
+    const uint32_t *bits;         // de-stuffed scan, big-endian bytes, followed by >= 8 zero bytes
+    uint64_t nbits;
+    const EntTable *tables;       // DC first: the DC table of each scan component; AC scans: the AC table
+    int16_t *plane[3];            // the image's zeroed whole-image planes (raster block order)
+    uint64_t *mask;               // AC refinement: per block of its component, the non-zero coefficients (zig-zag bit order)
+    uint64_t *rec;                // AC refinement: per block of its component, 3 masks (zig-zag bit order) -- coefficients whose
+                                  // correction bit is 1, coefficients the scan places, those of them that are negative
+    uint64_t *exit[2];            // first scans: n_sub states (pos << 16 | slot << 8 | coef) by round parity
+    uint64_t *used;               // first scans: n_sub entries
+    uint32_t *count;              // first scans: n_sub
+    uint32_t *changed;            // first scans: PROG_ROUNDS counters, zeroed
+    int16_t *dc;                  // DC first: total DC differences in block order
+    uint8_t *ok;                  // first scans: written by the accept kernel, 1 = its states are verified
+    uint8_t *status;              // the image's status byte (shared by its scans): non-zero = turned down, PROG_DOWN_* bits say
+                                  // by which phase (racing phases may keep only one of several)
+    uint32_t plane_len[3], bw[3];  // i16 per plane; blocks per plane row
+    uint32_t hs[3], vs[3];        // sampling factors per component
+    uint32_t n_sub, total;        // subsequences (first scans); blocks of the scan (MCUs x blocks per MCU when interleaved)
+    uint32_t kind, ss, se, al;
+    uint32_t nslot, mw, mcu_x;    // blocks per MCU (1: non-interleaved, raster over mw blocks per row); MCUs per row
+    uint32_t marker_check;        // the file's first scan: the host stage needs its bit reader to have met the marker behind it
+    uint8_t slot_z[8], slot_t[8], slot_h[8], slot_v[8];   // block slot -> component, table, h / v offset in the MCU
+};
+struct ProgChain { uint32_t first, count; };   // AC refinement scans [first, first + count) of one (image, component)
+// Queues the phases on `stream`: scans [0, n_first) are first scans (max_sub: the most subsequences of one), dc_ref[r] ..
+// dc_ref[r + 1] the DC refinements of ordinal r (r < n_dc_ord), chains the AC refinement chains (max_blocks: the most blocks of
+// a chain's plane).  phase: PROG_PHASE_*; returns a cudaError_t.
+enum { PROG_PHASE_ROUNDS = 0, PROG_PHASE_ACCEPT = 1, PROG_PHASE_WRITE = 2, PROG_PHASE_DC = 3, PROG_PHASE_DC_REFINE = 4,
+       PROG_PHASE_MASK = 5, PROG_PHASE_AC_REFINE = 6, PROG_PHASE_AC_APPLY = 7, PROG_PHASES = 8 };
+int launch_prog_phase(const ProgScan *d_scans, uint32_t n_first, uint32_t max_sub, const uint32_t *dc_ref, uint32_t n_dc_ord,
+                      uint32_t max_dc_blocks, const ProgChain *d_chains, uint32_t n_chain, uint32_t max_blocks, void *stream, int phase);
+
 }  // namespace zj

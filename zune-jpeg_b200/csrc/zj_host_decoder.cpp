@@ -159,6 +159,7 @@ struct HuffmanTable {  // src/huffman.rs:14-41
     uint8_t bits[17];
     uint8_t values[256];
     bool present;
+    bool progressive;   // built after SOF2: the fast-AC table holds only entries with a value (huffman.rs:224)
 };
 
 // HuffmanTable::new + make_derived_table, src/huffman.rs:45-276
@@ -172,6 +173,7 @@ static void build_huffman(HuffmanTable &p, const uint8_t codes[17], const uint8_
     memcpy(p.values, values, 256);
     p.has_ac_lookup = false;
     p.present = true;
+    p.progressive = is_progressive;
 
     uint8_t huff_size[257] = {0};
     uint32_t huff_code[257] = {0};
@@ -744,16 +746,21 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     // ZJ_USE_EXIF_ORIENTATION and ZJ_USE_GPU_ENTROPY ORed into a spec, libjpeg or scaled value: that value, oriented / with the
     // GPU entropy route of zj_decode_batch_gpu*; every other value keeps its meaning
     static bool spec_value(uint32_t u) { return u == ZJ_USE_SPEC_OUTPUT || u == ZJ_USE_LIBJPEG_OUTPUT || scale_of(u) != 0; }
+    // (ZJ_USE_GPU_PROGRESSIVE counts only next to ZJ_USE_GPU_ENTROPY)
+    static constexpr uint32_t SPEC_BITS = ZJ_USE_EXIF_ORIENTATION | ZJ_USE_GPU_ENTROPY | ZJ_USE_GPU_PROGRESSIVE;
     bool spec_bit(uint32_t bit) const
     {
-        return (options.use_unsafe & bit) && spec_value(options.use_unsafe & ~(uint32_t)(ZJ_USE_EXIF_ORIENTATION | ZJ_USE_GPU_ENTROPY));
+        const uint32_t u = options.use_unsafe;
+        if (bit == ZJ_USE_GPU_PROGRESSIVE && !(u & ZJ_USE_GPU_ENTROPY)) return false;
+        return (u & bit) && spec_value(u & ~SPEC_BITS) && ((u & ZJ_USE_GPU_ENTROPY) || !(u & ZJ_USE_GPU_PROGRESSIVE));
     }
     bool exif_orientation() const { return spec_bit(ZJ_USE_EXIF_ORIENTATION); }
     bool gpu_entropy() const { return spec_bit(ZJ_USE_GPU_ENTROPY); }
+    bool gpu_progressive() const { return spec_bit(ZJ_USE_GPU_PROGRESSIVE); }
     uint32_t use() const
     {
-        const uint32_t u = options.use_unsafe & ~(uint32_t)(ZJ_USE_EXIF_ORIENTATION | ZJ_USE_GPU_ENTROPY);
-        return spec_value(u) ? u : options.use_unsafe;
+        const uint32_t u = options.use_unsafe & ~SPEC_BITS;
+        return spec_value(u) && ((options.use_unsafe & ZJ_USE_GPU_ENTROPY) || !(options.use_unsafe & ZJ_USE_GPU_PROGRESSIVE)) ? u : options.use_unsafe;
     }
     // a one-component image: GRAYSCALE output (headers.rs:278-285, mcu.rs:171-196), except that spec output keeps RGB / RGBA / RGBX
     void gray_input_out_cs()
@@ -1400,12 +1407,25 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         std::vector<uint8_t> bits;
         uint64_t nbits = 0;
         size_t n_sub = 0, bpm = 0;
+        // a progressive frame (zj_entropy.h, ProgScan): every scan's de-stuffed bytes in `bits` (each at a multiple of 4, followed
+        // by >= 8 zero bytes) and the Huffman tables each scan reads, as the walk met them; n_seg is 1 (the image's status)
+        struct Scan {
+            uint32_t kind = 0, ns = 0, ss = 0, se = 0, al = 0, mw = 0, total = 0, nslot = 0;
+            uint8_t slot_z[8] = {}, slot_t[8] = {}, slot_h[8] = {}, slot_v[8] = {};
+            size_t bit_off = 0, tab = 0, ntab = 0;
+            uint64_t nbits = 0;
+            size_t n_sub() const { return (size_t)((nbits + zj::SYNC_BITS - 1) / zj::SYNC_BITS); }
+        };
+        bool prog = false;
+        std::vector<Scan> scans;
+        std::vector<zj::EntTable> ptab;
     };
     // Headers are parsed (reader stands at the first entropy-coded byte).  True when the scan can be handed to the GPU: a
     // baseline scan with restart markers in the state the interval-parallel forms start from.  Everything else -- and every
     // error -- is left to the host stage, which then reports exactly what the reference reports.
     bool gpu_entropy_prepare(const Cursor &reader, GpuPrep &pp)
     {
+        if (spec() && is_progressive) return gpu_progressive() && gpu_entropy_prepare_prog(reader, pp);
         if (spec()) return gpu_entropy() && gpu_entropy_prepare_spec(reader, pp);
         if (is_progressive || restart_interval == 0 || todo != restart_interval) return false;
         if (quirks != ZJ_QUIRK_ALL) return false;   // the GPU form carries the quirks as written; test switches and spec output -> host stage
@@ -1449,13 +1469,13 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
     // The scan's entropy-coded data as the bit reader sees it (bitstream.rs:200-215): FF [FF..] 00 -> FF, and the FF [FF..] of
     // the marker that ends it dropped.  True when that marker is EOI; RSTn (without DRI), DNL, a later scan, any other marker
     // and data without an end marker are left to the host stage.
-    static bool destuff_scan(const Cursor &reader, std::vector<uint8_t> &out)
+    // *end = the position behind the marker, *code = its code; false when the data ends first.  `out` is appended to.
+    static bool destuff_scan(const Cursor &reader, std::vector<uint8_t> &out, size_t *end, uint8_t *code)
     {
         const uint8_t *d = reader.data;
         const size_t n = reader.len;
         size_t p = reader.pos;
-        out.clear();
-        out.reserve(n - std::min(n, p) + 16);
+        out.reserve(out.size() + n - std::min(n, p) + 16);
         while (p < n) {
             const uint8_t *f = (const uint8_t *)memchr(d + p, 0xFF, n - p);
             if (!f) return false;
@@ -1467,9 +1487,18 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
             const uint8_t b = d[p++];
             if (b == 0x00) continue;
             out.pop_back();
-            return b == 0xD9;
+            *end = p;
+            *code = b;
+            return true;
         }
         return false;
+    }
+    static bool destuff_scan(const Cursor &reader, std::vector<uint8_t> &out)
+    {
+        size_t end;
+        uint8_t code;
+        out.clear();
+        return destuff_scan(reader, out, &end, &code) && code == 0xD9;
     }
     // The spec branch (ZJ_USE_GPU_ENTROPY with spec or libjpeg output, quirks off): a baseline frame whose first scan covers
     // every frame component, with factors the fused and spec kernels take, in its scan-start state, whose entropy-coded data
@@ -1510,6 +1539,133 @@ struct zj_decoder {  // Decoder, reference src/decoder.rs:60-121
         pp.n_seg = 1;
         pp.seg_start.assign(2, 0);
         pp.sync = true;
+        return true;
+    }
+    static void ent_table(zj::EntTable &d, const HuffmanTable &src)
+    {
+        memcpy(d.lookup, src.lookup, sizeof(d.lookup));
+        memcpy(d.ac_lookup, src.ac_lookup, sizeof(d.ac_lookup));
+        memcpy(d.maxcode, src.maxcode, sizeof(d.maxcode));
+        memcpy(d.offset, src.offset, sizeof(d.offset));
+        memcpy(d.values, src.values, sizeof(d.values));
+    }
+    // The progressive branch (ZJ_USE_GPU_PROGRESSIVE next to ZJ_USE_GPU_ENTROPY, spec or libjpeg output): walks the file from the
+    // first scan to EOI as decode_progressive would, without decoding, and records every scan (zj_entropy.h, ProgScan).  False --
+    // the host route, with its pixels and errors -- unless every condition of DESIGN.md section 5.6 holds.
+    bool gpu_entropy_prepare_prog(const Cursor &reader0, GpuPrep &pp)
+    {
+        const size_t nc = in_components();
+        if (raster() || four() || restart_interval != 0 || components.size() != nc || (nc != 1 && nc != 3)) return false;
+        if (input_colorspace == ZJ_CS_GRAYSCALE && interleaved) return false;   // finish_progressive_decoding fails there
+        if (reader0.len >= ((size_t)1 << 28)) return false;                        // (bit positions stay below 2^31)
+        try {
+            // decode_progressive's planes, and the checks its loops and finish_progressive_decoding make
+            check_component_dimensions();
+            set_upsampling();
+            size_t mw, mh;
+            if (interleaved) { mw = mcu_x; mh = mcu_y; } else { mw = ((size_t)info.width + 7) / 8; mh = ((size_t)info.height + 7) / 8; }
+            if (interleaved && h_max == 2) mh += mh & 1;
+            for (size_t i = 0; i < 4; i++) plane_len[i] = i < nc ? mw * 64 * components[i].vertical_sample * components[i].horizontal_sample * mh : 0;
+            for (size_t i = 0; i < nc; i++) if (plane_len[i] > 0x7FFFFFFFull) return false;
+            Cursor reader = reader0;
+            uint64_t first_cov[3] = {0, 0, 0}, blocks_all = 0;
+            bool dc_ref[3] = {false, false, false}, ac_ref[3] = {false, false, false};
+            pp.bits.clear();
+            pp.scans.clear();
+            pp.ptab.clear();
+            for (;;) {
+                // ---- the checks of parse_entropy_coded_data (mcu_prog.rs:249-430) for the scan just parsed
+                GpuPrep::Scan sc;
+                if (num_scans == 0 || (size_t)num_scans > nc) return false;
+                sc.ns = num_scans;
+                sc.ss = spec_start; sc.se = spec_end; sc.al = succ_low;
+                const bool dc = num_scans > 1 || spec_start == 0, first = succ_high == 0;   // (scans of several components are DC scans)
+                sc.kind = dc ? (first ? zj::PROG_DC_FIRST : zj::PROG_DC_REFINE) : (first ? zj::PROG_AC_FIRST : zj::PROG_AC_REFINE);
+                if (pp.scans.empty() && !first) return false;
+                if (num_scans == 1) {
+                    if (spec_end != 0 && spec_start == 0) return false;
+                    const size_t k = z_order[0];
+                    if (k >= components.size()) return false;
+                    const Component &c = components[k];
+                    size_t bw, bh;
+                    if (c.component_id == ID_Y || !interleaved) { bw = ((size_t)info.width + 7) / 8; bh = ((size_t)info.height + 7) / 8; }
+                    else { bw = mcu_x; bh = mcu_y; }
+                    sc.mw = (uint32_t)bw;
+                    sc.total = (uint32_t)(bw * bh);
+                    sc.nslot = 1;
+                    sc.slot_z[0] = (uint8_t)k;
+                    const HuffmanTable *t = nullptr;
+                    if (dc) { t = &dc_tables[c.dc_huff_table & 3]; if (!t->present) return false; }
+                    else {
+                        if (c.ac_huff_table >= 4 || !ac_tables[c.ac_huff_table].present || spec_start > spec_end) return false;
+                        t = &ac_tables[c.ac_huff_table];
+                        if (!t->progressive) return false;
+                    }
+                    if (sc.kind != zj::PROG_DC_REFINE) { sc.ntab = 1; pp.ptab.emplace_back(); ent_table(pp.ptab.back(), *t); }
+                } else {
+                    if (spec_end != 0) return false;
+                    for (size_t k = 0; k < num_scans; k++) {
+                        const size_t z = z_order[k];
+                        if (z >= components.size()) return false;
+                        const Component &c = components[z];
+                        if (c.dc_huff_table >= 4 || !dc_tables[c.dc_huff_table].present) return false;
+                        for (size_t v = 0; v < c.vertical_sample; v++)
+                            for (size_t h = 0; h < c.horizontal_sample; h++) {
+                                if (sc.nslot >= 8) return false;
+                                sc.slot_z[sc.nslot] = (uint8_t)z; sc.slot_t[sc.nslot] = (uint8_t)k;
+                                sc.slot_h[sc.nslot] = (uint8_t)h; sc.slot_v[sc.nslot] = (uint8_t)v;
+                                sc.nslot++;
+                            }
+                        if (first) { pp.ptab.emplace_back(); ent_table(pp.ptab.back(), dc_tables[c.dc_huff_table]); sc.ntab++; }
+                    }
+                    sc.mw = (uint32_t)mcu_x;
+                    if ((uint64_t)mcu_x * mcu_y * sc.nslot > 0x7FFFFFFFull) return false;
+                    sc.total = (uint32_t)(mcu_x * mcu_y * sc.nslot);
+                }
+                sc.tab = pp.ptab.size() - sc.ntab;
+                // ---- the phase order: first scans of a component before its refinements, on disjoint coefficients
+                for (size_t k = 0; k < num_scans; k++) {
+                    const size_t z = z_order[k];
+                    const uint64_t band = dc ? 1ull : (~0ull >> (63 - spec_end)) & (~0ull << spec_start);
+                    if (sc.kind == zj::PROG_DC_FIRST || sc.kind == zj::PROG_AC_FIRST) {
+                        if ((dc ? dc_ref[z] : ac_ref[z]) || (first_cov[z] & band)) return false;
+                        first_cov[z] |= band;
+                    } else if (dc) dc_ref[z] = true;
+                    else ac_ref[z] = true;
+                }
+                blocks_all += sc.total;
+                if (blocks_all >= 0x7FFF0000ull) return false;   // (the no-DRI countdown of the host loop never reaches 0)
+                // ---- the scan's bytes up to the marker behind it
+                size_t end;
+                uint8_t code;
+                pp.bits.resize((pp.bits.size() + 3) & ~(size_t)3, 0);
+                sc.bit_off = pp.bits.size();
+                if (!destuff_scan(reader, pp.bits, &end, &code)) return false;
+                sc.nbits = (uint64_t)(pp.bits.size() - sc.bit_off) * 8;
+                pp.bits.resize(pp.bits.size() + 8, 0);
+                if (sc.nbits == 0) return false;
+                pp.scans.push_back(sc);
+                if (pp.scans.size() > options.max_scans) return false;
+                reader.pos = end;
+                // ---- the markers decode_progressive takes behind it: DHT (then the next marker), SOS or EOI
+                Marker m;
+                if (!marker_from_u8(code, &m)) return false;
+                while (m.kind == M_DHT) {
+                    parse_huffman(reader);
+                    BitStream none;
+                    if (!get_marker(reader, none, &m)) return false;
+                }
+                if (m.kind == M_EOI) break;
+                if (m.kind != M_SOS) return false;
+                parse_sos(reader);
+            }
+        } catch (DecodeError &) {
+            return false;
+        }
+        pp.bits.resize(((pp.bits.size() + 3) & ~(size_t)3) + 16, 0);
+        pp.n_seg = 1;
+        pp.seg_start.assign(2, 0);
+        pp.prog = true;
         return true;
     }
     void gpu_entropy_tables(zj::EntTable *t) const   // [dc, ac] per component
@@ -2270,6 +2426,8 @@ struct GpuSlot {
     std::vector<size_t> take, idx;            // images of the sub-batch in stage 1 / images whose pixels are on their way
     std::vector<zj::EntImage> eimg;
     std::vector<zj::SyncImage> simg;
+    std::vector<zj::ProgScan> pscan;          // progressive images' scans in phase order
+    std::vector<zj::ProgChain> pchain;
     std::vector<int16_t *> planes;            // 3 per image of the sub-batch: its device planes
     std::vector<uint8_t *> pix;
     std::vector<size_t> st_off;
@@ -2422,7 +2580,19 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
     auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
     auto footprint = [&](const Item &it, size_t len) {
         size_t b = al(sizeof(zj::EntImage)) + al(6 * sizeof(zj::EntTable)) + al((it.pp.n_seg + 1) * 4) + al(it.pp.n_seg) + 1024 + (dev_out ? 0 : al(it.need));
-        if (!it.pp.sync) b += al(len + 8);
+        if (it.pp.prog) {   // de-stuffed scans and their tables; per first scan its states, counters, DC differences and ok byte;
+                            // per AC refinement scan its block records, per chain the non-zero masks of its component
+            b += al(it.pp.bits.size()) + al(it.pp.ptab.size() * sizeof(zj::EntTable));
+            bool refined[3] = {false, false, false};
+            for (const auto &sc : it.pp.scans) {
+                b += sizeof(zj::ProgScan);
+                if (sc.kind == zj::PROG_AC_REFINE) { refined[sc.slot_z[0]] = true; b += al(it.d->plane_len[sc.slot_z[0]] / 64 * 24); }
+                if (sc.kind != zj::PROG_DC_FIRST && sc.kind != zj::PROG_AC_FIRST) continue;
+                b += 3 * al(sc.n_sub() * 8) + al(sc.n_sub() * 4) + al(zj::PROG_ROUNDS * 4) + al(1);
+                if (sc.kind == zj::PROG_DC_FIRST) b += al((size_t)sc.total * 2);
+            }
+            for (int z = 0; z < 3; z++) if (refined[z]) b += al(it.d->plane_len[z] / 64 * 8) + sizeof(zj::ProgChain);
+        } else if (!it.pp.sync) b += al(len + 8);
         else   // de-stuffed bits, subsequence states (2 exits, entry, count) and DC differences
             b += al(sizeof(zj::SyncImage)) + al(it.pp.bits.size()) + 3 * al(it.pp.n_sub * 8) + al(it.pp.n_sub * 4) +
                  al(it.pp.total * it.pp.bpm * 2) + al(zj::SYNC_ROUNDS * 4);
@@ -2501,7 +2671,7 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
         // interval form get an EntImage, those of the self-synchronising form a SyncImage (slot[t] indexes its array)
         size_t n_int = 0, n_sync = 0;
         std::vector<size_t> slot_of(take.size());
-        for (size_t t = 0; t < take.size(); t++) slot_of[t] = items[take[t]].pp.sync ? n_sync++ : n_int++;
+        for (size_t t = 0; t < take.size(); t++) slot_of[t] = items[take[t]].pp.prog ? 0 : (items[take[t]].pp.sync ? n_sync++ : n_int++);
         sl.eimg.assign(n_int, zj::EntImage{});
         sl.simg.assign(n_sync, zj::SyncImage{});
         std::vector<int16_t *> &planes = sl.planes;
@@ -2512,6 +2682,42 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
         }
         for (size_t t = 0; t < take.size(); t++)
             if (items[take[t]].pp.sync) sl.simg[slot_of[t]].changed = (uint32_t *)carve(zj::SYNC_ROUNDS * 4);
+        // progressive images: their scans in phase order -- first scans, DC refinements by ordinal, AC refinements by (image,
+        // component) chain in file order -- with the first scans' round counters in the cleared block
+        std::vector<std::pair<size_t, size_t>> porder;   // (t, scan)
+        std::vector<uint32_t> dc_ref;
+        std::vector<zj::ProgChain> &chains = sl.pchain;
+        chains.clear();
+        auto kind_of = [&](size_t t, size_t q) { return items[take[t]].pp.scans[q].kind; };
+        for (size_t t = 0; t < take.size(); t++)
+            if (items[take[t]].pp.prog)
+                for (size_t q = 0; q < items[take[t]].pp.scans.size(); q++)
+                    if (kind_of(t, q) == zj::PROG_DC_FIRST || kind_of(t, q) == zj::PROG_AC_FIRST) porder.emplace_back(t, q);
+        const size_t n_first = porder.size();
+        dc_ref.push_back((uint32_t)n_first);
+        for (size_t r = 0;; r++) {
+            const size_t before = porder.size();
+            for (size_t t = 0; t < take.size(); t++) {
+                if (!items[take[t]].pp.prog) continue;
+                size_t seen = 0;
+                for (size_t q = 0; q < items[take[t]].pp.scans.size(); q++)
+                    if (kind_of(t, q) == zj::PROG_DC_REFINE && seen++ == r) { porder.emplace_back(t, q); break; }
+            }
+            if (porder.size() == before) break;
+            dc_ref.push_back((uint32_t)porder.size());
+        }
+        std::vector<std::pair<size_t, int>> chain_of;   // (t, component)
+        for (size_t t = 0; t < take.size(); t++) {
+            if (!items[take[t]].pp.prog) continue;
+            for (int z = 0; z < 3; z++) {
+                const size_t first = porder.size();
+                for (size_t q = 0; q < items[take[t]].pp.scans.size(); q++)
+                    if (kind_of(t, q) == zj::PROG_AC_REFINE && items[take[t]].pp.scans[q].slot_z[0] == z) porder.emplace_back(t, q);
+                if (porder.size() > first) { chains.push_back({(uint32_t)first, (uint32_t)(porder.size() - first)}); chain_of.emplace_back(t, z); }
+            }
+        }
+        sl.pscan.assign(porder.size(), zj::ProgScan{});
+        for (size_t f = 0; f < n_first; f++) sl.pscan[f].changed = (uint32_t *)carve(zj::PROG_ROUNDS * 4);
         bool ok = cudaMemsetAsync(sl.mem, 0, off, sl.s) == cudaSuccess;
         lap("memset planes", sl.s);
         // descriptors, Huffman tables and interval starts of the sub-batch travel as ONE pinned block, the statuses come back as one
@@ -2521,11 +2727,18 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
         for (size_t t = 0; t < take.size(); t++) { sl.st_off[t] = st_total; st_total += items[take[t]].pp.n_seg; seg_words += items[take[t]].pp.n_seg + 1; }
         const size_t off_sync = al(n_int * sizeof(zj::EntImage)), off_tab = off_sync + al(n_sync * sizeof(zj::SyncImage));
         const size_t off_seg = off_tab + al(6 * take.size() * sizeof(zj::EntTable));
-        const size_t meta_bytes = off_seg + al(seg_words * 4);
+        size_t n_ptab = 0;
+        for (size_t t = 0; t < take.size(); t++) n_ptab += items[take[t]].pp.ptab.size();
+        const size_t off_pscan = off_seg + al(seg_words * 4), off_ptab = off_pscan + al(porder.size() * sizeof(zj::ProgScan));
+        const size_t off_chain = off_ptab + al(n_ptab * sizeof(zj::EntTable));
+        const size_t meta_bytes = off_chain + al(chains.size() * sizeof(zj::ProgChain));
         ok = ok && pinned_grow(sl.meta_host, sl.meta_cap, meta_bytes) && pinned_grow(sl.st_host, sl.st_cap, st_total);
         uint8_t *d_meta = carve(meta_bytes), *d_status = carve(st_total);
+        ok = ok && cudaMemsetAsync(d_status, 0, st_total, sl.s) == cudaSuccess;   // (progressive images' kernels only set theirs)
         uint32_t max_seg = 0, max_sub = 0;
-        size_t seg_at = 0;
+        size_t seg_at = 0, ptab_at = 0;
+        std::vector<uint8_t *> d_pbits(take.size(), nullptr);
+        std::vector<size_t> ptab_of(take.size(), 0);
         std::vector<std::pair<uint8_t *, size_t>> uploads;   // (device destination, image): the file, or its de-stuffed scan
         for (size_t t = 0; t < take.size() && ok; t++) {
             const size_t i = take[t];
@@ -2534,6 +2747,15 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
             it.d->gpu_entropy_tables(reinterpret_cast<zj::EntTable *>(sl.meta_host + off_tab) + 6 * t);
             memcpy(sl.meta_host + off_seg + seg_at * 4, it.pp.seg_start.data(), (it.pp.n_seg + 1) * 4);
             sl.pix[t] = dev_out ? out[i] : carve(it.need);
+            if (it.pp.prog) {
+                d_pbits[t] = carve(it.pp.bits.size());
+                uploads.emplace_back(d_pbits[t], i);
+                ptab_of[t] = ptab_at;
+                if (ok) memcpy(sl.meta_host + off_ptab + ptab_at * sizeof(zj::EntTable), it.pp.ptab.data(), it.pp.ptab.size() * sizeof(zj::EntTable));
+                ptab_at += it.pp.ptab.size();
+                seg_at += it.pp.n_seg + 1;
+                continue;
+            }
             if (it.pp.sync) {
                 zj::SyncImage &e = sl.simg[slot_of[t]];
                 const size_t n_sub = it.pp.n_sub, blocks = it.pp.total * it.pp.bpm;
@@ -2587,16 +2809,58 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
             }
             max_seg = std::max(max_seg, e.n_seg);
         }
+        uint32_t max_psub = 0, max_dc = 0, max_blocks = 0;
+        for (size_t x = 0; x < porder.size() && ok; x++) {
+            const size_t t = porder[x].first;
+            const Item &it = items[take[t]];
+            const zj_decoder::GpuPrep::Scan &q = it.pp.scans[porder[x].second];
+            zj::ProgScan &e = sl.pscan[x];
+            e.bits = reinterpret_cast<const uint32_t *>(d_pbits[t] + q.bit_off);
+            e.nbits = q.nbits;
+            e.tables = reinterpret_cast<const zj::EntTable *>(d_meta + off_ptab) + ptab_of[t] + q.tab;
+            e.status = d_status + sl.st_off[t];
+            for (int z = 0; z < 3; z++) {
+                e.plane[z] = planes[3 * t + z];
+                e.plane_len[z] = (uint32_t)it.d->plane_len[z];
+                const bool have = (size_t)z < it.d->components.size();
+                e.hs[z] = have ? (uint32_t)it.d->components[z].horizontal_sample : 0u;
+                e.vs[z] = have ? (uint32_t)it.d->components[z].vertical_sample : 0u;
+                e.bw[z] = have ? (uint32_t)(it.d->components[z].width_stride / 8) : 0u;
+            }
+            e.total = q.total; e.kind = q.kind; e.ss = q.ss; e.se = q.se; e.al = q.al;
+            e.nslot = q.nslot; e.mw = q.mw; e.mcu_x = (uint32_t)it.d->mcu_x;
+            e.marker_check = porder[x].second == 0 ? 1u : 0u;
+            memcpy(e.slot_z, q.slot_z, 8); memcpy(e.slot_t, q.slot_t, 8); memcpy(e.slot_h, q.slot_h, 8); memcpy(e.slot_v, q.slot_v, 8);
+            if (x < n_first) {
+                const size_t n_sub = q.n_sub();
+                e.n_sub = (uint32_t)n_sub;
+                e.exit[0] = (uint64_t *)carve(n_sub * 8); e.exit[1] = (uint64_t *)carve(n_sub * 8);
+                e.used = (uint64_t *)carve(n_sub * 8);
+                e.count = (uint32_t *)carve(n_sub * 4);
+                e.ok = carve(1);
+                if (q.kind == zj::PROG_DC_FIRST) e.dc = (int16_t *)carve((size_t)q.total * 2);
+                max_psub = std::max(max_psub, e.n_sub);
+            } else if (q.kind == zj::PROG_DC_REFINE) max_dc = std::max(max_dc, q.total);
+            else e.rec = (uint64_t *)carve(it.d->plane_len[q.slot_z[0]] / 64 * 24);
+        }
+        for (size_t c = 0; c < chains.size() && ok; c++) {
+            const size_t t = chain_of[c].first, z = (size_t)chain_of[c].second, nb = items[take[t]].d->plane_len[z] / 64;
+            uint64_t *mask = (uint64_t *)carve(nb * 8);
+            for (uint32_t x = chains[c].first; x < chains[c].first + chains[c].count; x++) sl.pscan[x].mask = mask;
+            max_blocks = std::max(max_blocks, (uint32_t)nb);
+        }
         if (ok) {
             memcpy(sl.meta_host, sl.eimg.data(), n_int * sizeof(zj::EntImage));
             memcpy(sl.meta_host + off_sync, sl.simg.data(), n_sync * sizeof(zj::SyncImage));
+            memcpy(sl.meta_host + off_pscan, sl.pscan.data(), sl.pscan.size() * sizeof(zj::ProgScan));
+            memcpy(sl.meta_host + off_chain, chains.data(), chains.size() * sizeof(zj::ProgChain));
         }
         ok = ok && off <= sl.cap && cudaMemcpyAsync(d_meta, sl.meta_host, meta_bytes, cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
         // files (de-stuffed scans) + entropy kernels (behind the cleared planes and the descriptors), then the statuses come back
         for (size_t u = 0; u < uploads.size() && ok; u++) {
             const size_t i = uploads[u].second;
-            const bool sync = items[i].pp.sync;
-            ok = cudaMemcpyAsync(uploads[u].first, sync ? items[i].pp.bits.data() : bufs[i], sync ? items[i].pp.bits.size() : lens[i], cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
+            const bool bits = items[i].pp.sync || items[i].pp.prog;
+            ok = cudaMemcpyAsync(uploads[u].first, bits ? items[i].pp.bits.data() : bufs[i], bits ? items[i].pp.bits.size() : lens[i], cudaMemcpyHostToDevice, sl.s) == cudaSuccess;
         }
         const bool spec = items[take[0]].d->spec();
         ok = ok && zj::launch_entropy(reinterpret_cast<const zj::EntImage *>(d_meta), (uint32_t)n_int, max_seg, sl.s, spec) == 0;
@@ -2623,6 +2887,39 @@ static int decode_batch_gpu_impl(const zj_options *o, const uint8_t *const *bufs
                 down += st != 0;
             }
             fprintf(stderr, "[zj_decode_batch_gpu] sync rounds: images %zu, max %u, mean %.2f, turned down %u\n", n_sync, rmax, rsum / n_sync, down);
+        }
+        static const char *const prog_name[zj::PROG_PHASES] = {"prog rounds", "prog accept", "prog write", "prog DC", "prog DC refine",
+                                                               "prog masks", "prog AC refine", "prog AC apply"};
+        const zj::ProgScan *d_pscan = reinterpret_cast<const zj::ProgScan *>(d_meta + off_pscan);
+        const zj::ProgChain *d_chain = reinterpret_cast<const zj::ProgChain *>(d_meta + off_chain);
+        for (int ph = 0; ph < zj::PROG_PHASES && !porder.empty(); ph++) {
+            ok = ok && zj::launch_prog_phase(d_pscan, (uint32_t)n_first, max_psub, dc_ref.data(), (uint32_t)dc_ref.size() - 1, max_dc,
+                                             d_chain, (uint32_t)chains.size(), max_blocks, sl.s, ph) == 0;
+            lap(prog_name[ph], sl.s);
+        }
+        if (trace && ok && !porder.empty()) {   // rounds of the first scans (PROG_ROUNDS: not settled) and turned-down images
+                                                // (index in the call, PROG_DOWN_* bits)
+            uint32_t rmax = 0;
+            double rsum = 0;
+            for (size_t f = 0; f < n_first; f++) {
+                uint32_t ch[zj::PROG_ROUNDS];
+                cudaMemcpy(ch, sl.pscan[f].changed, sizeof(ch), cudaMemcpyDeviceToHost);
+                uint32_t r = 1;
+                while (r < zj::PROG_ROUNDS && ch[r] != 0) r++;
+                rmax = std::max(rmax, r);
+                rsum += r;
+            }
+            size_t n_prog = 0;
+            std::string down;
+            for (size_t t = 0; t < take.size(); t++) {
+                if (!items[take[t]].pp.prog) continue;
+                n_prog++;
+                uint8_t st = 1;
+                cudaMemcpy(&st, d_status + sl.st_off[t], 1, cudaMemcpyDeviceToHost);
+                if (st) down += " " + std::to_string(take[t]) + "(" + std::to_string(st) + ")";
+            }
+            fprintf(stderr, "[zj_decode_batch_gpu] prog: images %zu, scans %zu, first-scan rounds max %u, mean %.2f, turned down:%s\n",
+                    n_prog, porder.size(), rmax, n_first ? rsum / n_first : 0.0, down.empty() ? " none" : down.c_str());
         }
         ok = ok && (st_total == 0 || cudaMemcpyAsync(sl.st_host, d_status, st_total, cudaMemcpyDeviceToHost, sl.s) == cudaSuccess);
         if (!ok) cudaGetLastError();

@@ -90,6 +90,7 @@ class ZuneJpegOptions:
         self._scale_denom = 1
         self._exif_orientation = False
         self._gpu_entropy = False
+        self._gpu_progressive = False
 
     @staticmethod
     def new() -> "ZuneJpegOptions":
@@ -148,6 +149,11 @@ class ZuneJpegOptions:
     # libjpeg output on the GPU, with or without restart markers (ZJ_USE_GPU_ENTROPY); same results.  Needs spec or libjpeg output.
     def get_gpu_entropy(self): return self._gpu_entropy
     def set_gpu_entropy(self, choice: bool): return self._with(_gpu_entropy=bool(choice))
+    # not in the reference: lets those routes entropy-decode progressive spec and libjpeg output on the GPU as well
+    # (ZJ_USE_GPU_PROGRESSIVE); same results.  Needs set_gpu_entropy(True).  Pays off for large batches only: the AC refinement
+    # scans of each image component are decoded by one warp, ~0.7 s for a 4K q90 file (DESIGN.md section 5.6).
+    def get_gpu_progressive(self): return self._gpu_progressive
+    def set_gpu_progressive(self, choice: bool): return self._with(_gpu_progressive=bool(choice))
 
     def _raw(self) -> ZjOptions:
         o = ZjOptions()
@@ -157,6 +163,8 @@ class ZuneJpegOptions:
             raise ValueError("EXIF orientation needs spec or libjpeg output (set_spec_output(True) or set_libjpeg_output(True))")
         if self._gpu_entropy and not (self._libjpeg_output or self._spec_output):
             raise ValueError("GPU entropy decoding of spec output needs spec or libjpeg output (set_spec_output(True) or set_libjpeg_output(True))")
+        if self._gpu_progressive and not self._gpu_entropy:
+            raise ValueError("GPU entropy decoding of progressive images needs GPU entropy decoding (set_gpu_entropy(True))")
         if self._libjpeg_output:
             o.use_unsafe = _ffi.USE_LIBJPEG_OUTPUT | (self._scale_denom.bit_length() - 1) << _ffi.USE_SCALE_SHIFT
         else:
@@ -165,6 +173,8 @@ class ZuneJpegOptions:
             o.use_unsafe |= _ffi.USE_EXIF_ORIENTATION
         if self._gpu_entropy:
             o.use_unsafe |= _ffi.USE_GPU_ENTROPY
+        if self._gpu_progressive:
+            o.use_unsafe |= _ffi.USE_GPU_PROGRESSIVE
         o.out_colorspace = int(self._out_colorspace)
         o.num_threads = self._num_threads
         o.max_width, o.max_height = self._max_width, self._max_height
@@ -394,7 +404,9 @@ def decode_batch(buffers, options: ZuneJpegOptions | None = None, threads: int =
     `gpu_entropy=True` (zj_decode_batch_gpu): baseline JPEGs with restart markers are entropy-decoded on the GPU as well, one
     restart interval per thread; same results, `stats["gpu_entropy"]` = how many images took that route.  With spec or libjpeg
     output, `options.set_gpu_entropy(True)` lets this route (and `device_out`) take those images too, with or without restart
-    markers (self-synchronising decode); without it they take the host route.
+    markers (self-synchronising decode); without it they take the host route.  `options.set_gpu_progressive(True)` as well lets
+    it take progressive images of these modes too (every scan entropy-decoded on the GPU; same results), and `stats["gpu_entropy"]`
+    counts them.
     `device_out=[(device_ptr, nbytes), ...]` (zj_decode_batch_gpu_device): the pixels stay in device memory; with
     `desc=gpu.OutputDesc(...)` (zj_decode_batch_gpu_device_ex) in the layout / type / scale a GPU consumer wants.
     `devices=[0, 1, ...]` (zj_decode_batch_multi): the batch is cut into contiguous image ranges, one per device of the box
@@ -465,7 +477,8 @@ def decode_batch_resized(buffers, resize, desc=None, rois=None, options: ZuneJpe
     ones decode_batch reports for the same inputs; a crop that does not fit its image, or an image whose channel count is not
     the one the options' colourspace gives, fails with status ZJ_ERR_INVALID_ARG.  The slot of a failed image is not written.
     With spec or libjpeg output and `options.set_gpu_entropy(True)` the entropy stage of baseline images runs on the GPU too
-    (same results); `stats["gpu_entropy"]` = how many images took that route."""
+    (same results), and with `options.set_gpu_progressive(True)` as well that of progressive images; `stats["gpu_entropy"]` =
+    how many images took that route."""
     from . import gpu
     lib = _ffi.load()
     options = options if options is not None else ZuneJpegOptions()
